@@ -2,7 +2,7 @@
 """bench.py -- FHE-RAM hot-path benchmark (BASELINE.json metric: batched reads/s at 2^18 x 4 B,
 plus single read / read_prepare_write / write latency).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one batch of B independent encrypted-address reads (BASELINE.json config 3, B = 1024)
 against a RAM of max_addr = 2^18 words x 4 bytes (README.md:17-34 parameters).  `value` is measured
@@ -14,6 +14,9 @@ libfheram_cuda.so on its own NCCL communicator; the global batch stays B ("stron
 --impl reference times the CPU restatement of the reference's FFT64 path (oracle/, kind "port": the reference
 itself cannot be built here -- no Rust toolchain, Poulpy un-vendored) on inputs made by the oracle's own client side;
 that arm imports nothing of fhe_ram_b200.
+The GPU arm runs from the tree as __graft_entry__.build() left it and writes nothing there.  --dump-outputs DIR writes
+what the last timed step computed (see dump_outputs) so that two builds can be compared output for output: every input
+comes from fixed seeds, so the same arguments give the same inputs on every run.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ F_EXT = 2_363_392   # flop per external product (6 fwd + 8 inv FFT of 2048 pts, 
 F_KS = 1_632_256    # flop per key-switch automorphism (3 + 8 FFT, 3x8 contraction)
 B_EXT = 1.5 * 2**20 + 2 * 96 * 2**10   # bytes per ext product: prepared GGSW + ct in + ct out (int32)
 B_KS = 0.75 * 2**20                    # bytes per key-switch: prepared key (ct stays in shared memory)
+DUMP_BYTES = 48 << 20                  # --dump-outputs budget: a whole batch at 2^18 x 4 B is 805 MB of float64
 
 
 def op_model(max_addr, word_size, base2d, n=4096):
@@ -84,6 +88,7 @@ class ClockSampler:
     def stop(self):
         if self.proc:
             self.proc.terminate()
+            self.proc.wait()
         # samples taken inside the timed window; a window shorter than the sampling period falls back to
         # the samples of the warm-up + timed span (same kernels, same load) and says so
         window = "timed region"
@@ -116,6 +121,17 @@ def make_addresses(fr, params, sk, idxs, threads, first=0):
     with ThreadPoolExecutor(max_workers=threads) as ex:
         list(ex.map(one, range(len(idxs))))
     return out
+
+
+def dump_outputs(out_dir, res, first):
+    """Writes the results of the last timed step: `read_limbs.npy` [n][word_size][glwe_len], the ciphertexts a caller of
+    the batched read receives (float64 holds every limb exactly), for a fixed, seeded sample of n reads that fits
+    DUMP_BYTES, and `read_positions.npy` [n], their positions in the batch."""
+    n = min(len(res), DUMP_BYTES // (res[0].size * 8))
+    pick = np.sort(np.random.default_rng(0).choice(len(res), size=n, replace=False))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "read_limbs.npy", res[pick].astype(np.float64))
+    np.save(out_dir / "read_positions.npy", (first + pick).astype(np.float64))
 
 
 def bench_config(args, world):
@@ -165,7 +181,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--host-format", default="p17", choices=["p17", "i32", "i64"],
                     help="host limb format of the e2e call: packed 17-bit fields, int32, or int64 (Poulpy's containers)")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write a seeded sample of the last timed step's read results to DIR as .npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -239,9 +259,6 @@ def main():
 
     import torch
     import hashlib
-    import __graft_entry__ as g
-    if rank == 0:
-        g.build()
     if world > 1:
         import torch.distributed as dist
         torch.cuda.set_device(local_rank)
@@ -302,8 +319,11 @@ def main():
         ram = fr.Ram.new(params)
         ram.load(cts)
 
+    last_out = [None]   # device pointer of the result arena the latest resident step wrote
+
     def run_resident():
-        return ram.read_batch_device(addr_res, keys)
+        last_out[0] = ram.read_batch_device(addr_res, keys)
+        return last_out[0]
 
     def run_e2e():
         # this rank's host address limbs -> device, prepare, read (all exchange steps), results back on the host
@@ -344,26 +364,29 @@ def main():
     # ---- warm-up, then the device-resident timed region --------------------------------
     sampler = ClockSampler(device)
     sampler.start()
-    for _ in range(args.warmup):
-        run_resident()
-    params.profile(True)
-    l0 = params.launch_count()
-    sampler.mark_start()
-    ms_total = timed(run_resident, args.steps)
-    sampler.mark_end()
-    launches = params.launch_count() - l0
-    prof = params.profile_get()
-    params.profile(False)
-    clocks = sampler.stop()
+    try:  # the sampler's nvidia-smi must not outlive a failed run
+        for _ in range(args.warmup):
+            run_resident()
+        params.profile(True)
+        l0 = params.launch_count()
+        sampler.mark_start()
+        ms_total = timed(run_resident, args.steps)
+        sampler.mark_end()
+        launches = params.launch_count() - l0
+        prof = params.profile_get()
+        params.profile(False)
+    finally:
+        clocks = sampler.stop()
     ms_step = ms_total / args.steps
     value = B / (ms_step * 1e-3)
 
-    # correctness of what was timed: this rank's slice, decrypted, and -- N > 1 -- compared LIMB FOR LIMB with what
-    # ONE GPU computes for the same reads (an unsharded RAM on this rank's GPU, outside every timed region)
-    d_out = run_resident()
+    # correctness of what was timed: this rank's slice of the last timed step, decrypted, and -- N > 1 -- compared LIMB
+    # FOR LIMB with what ONE GPU computes for the same reads (an unsharded RAM on this rank's GPU, outside every timed region)
     res = np.zeros((mine, ws, L), dtype=np.int64)
-    api._check(api.lib().fheram_download_glwe(params.module(), d_out, mine * ws, api._p(res)))
+    api._check(api.lib().fheram_download_glwe(params.module(), last_out[0], mine * ws, api._p(res)))
     check(res)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, first)
     digest = hashlib.sha256(res.tobytes()).hexdigest()
     parity = None
     if world > 1:
