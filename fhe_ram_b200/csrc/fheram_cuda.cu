@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <nccl.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -203,6 +204,7 @@ struct fheram_ctx {
   int device = 0, sm_count = 148;
   int ext9_clusters[2] = {0, 0}; // the same for k_ext9
   int ks8_clusters[2] = {0, 0};  // clusters of k_ks8 that can be resident together: [0] eight SMs each, [1] four
+  int force_ext = 0, force_ks = 0;  // kernels forced by FHERAM_KERNEL (enum Force), FORCE_NONE: the launch-width rule
   cudaStream_t stream = nullptr;
   bool own_stream = true;
   cudaStream_t copy_stream = nullptr;  // uploads of the asynchronous address path
@@ -227,7 +229,6 @@ struct fheram_ctx {
   DevBuf enc_buf[15];  // operands of the encryption kernels, kept between calls (cudaFree synchronizes the device)
   uint64_t enc_stats[3] = {0, 0, 0};  // noise draws sampled on the device / patched by the host / streams resampled on the host
   DevBuf opbuf[3];  // op-level entry points
-  DevBuf split_tmp[2];  // ping-pong ciphertexts of the column-split (latency) schedules
   long long* d_phase = nullptr;  // per-CTA phase cycle counters (fheram_debug_phase_cycles)
   // per-kernel-class CUDA-event timing (fheram_ctx_profile)
   bool profile = false;
@@ -242,36 +243,18 @@ struct fheram_ctx {
   long evk_inv_prep_len() const { return (long)d.dnum_ggsw * 2 * d.size_evk_inv * kM; }
 };
 
-static size_t smem_bytes(int R, int CIN, bool xsmem) {
-  return (size_t)R * CIN * kM * sizeof(double2) + kM * sizeof(double2) +
-         (xsmem ? (size_t)2 * R * kN * sizeof(int) : 0);
-}
+static size_t smem_bytes(int R) { return (size_t)R * kM * sizeof(double2) + kM * sizeof(double2); }
 
 // kernel instantiations used by the schedules
-#define K_EXT      k_vmp<3, 2, 4, 3, MODE_EXT, false>
-#define K_TRACE    k_vmp<3, 1, 4, 3, MODE_TRACE, true>
-#define K_COMBINE2 k_vmp<3, 1, 4, 3, MODE_COMBINE2, true>
-#define K_AUTO3    k_vmp<3, 1, 4, 3, MODE_AUTO, false>
-#define K_AUTO_INV k_vmp<4, 1, 5, 4, MODE_AUTO, false>
-#define K_EXPAND   k_vmp<4, 1, 5, 4, MODE_EXPAND, false>
-// column-split variants (two CTAs per operation, narrow launches)
-#define K_EXT_S      k_vmp<3, 2, 4, 3, MODE_EXT, false, true>
-#define K_TRACE_S    k_vmp<3, 1, 4, 3, MODE_TRACE, true, true>
-#define K_COMBINE2_S k_vmp<3, 1, 4, 3, MODE_COMBINE2, true, true>
+#define K_AUTO3    k_vmp<3, 4, 3, MODE_AUTO>
+#define K_AUTO_INV k_vmp<4, 5, 4, MODE_AUTO>
+#define K_EXPAND   k_vmp<4, 5, 4, MODE_EXPAND>
 
 static int set_attrs() {
-  CU(cudaFuncSetAttribute(K_EXT, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 2, false)));
-  CU(cudaFuncSetAttribute(K_TRACE, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 1, true)));
-  CU(cudaFuncSetAttribute(K_COMBINE2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 1, true)));
-  CU(cudaFuncSetAttribute(K_AUTO3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 1, false)));
-  CU(cudaFuncSetAttribute(K_AUTO_INV, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(4, 1, false)));
-  CU(cudaFuncSetAttribute(K_EXPAND, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(4, 1, false)));
-  CU(cudaFuncSetAttribute(K_EXT_S, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 2, false)));
-  CU(cudaFuncSetAttribute(K_TRACE_S, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 1, true)));
-  CU(cudaFuncSetAttribute(K_COMBINE2_S, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3, 1, true)));
-  CU(cudaFuncSetAttribute(k_ext3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kExt3Smem));
-  CU(cudaFuncSetAttribute(k_ks7<MODE_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs7Smem));
-  CU(cudaFuncSetAttribute(k_ks7<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs7Smem));
+  CU(cudaFuncSetAttribute(K_AUTO3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(3)));
+  CU(cudaFuncSetAttribute(K_AUTO_INV, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(4)));
+  CU(cudaFuncSetAttribute(K_EXPAND, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(4)));
+  CU(cudaFuncSetAttribute(k_ks7, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs7Smem));
   CU(cudaFuncSetAttribute(k_prepare7, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPrep7Smem));
   CU(cudaFuncSetAttribute(k_ext8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kExt8Smem));
   CU(cudaFuncSetAttribute(k_ext9<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ext9_smem(8)));
@@ -284,8 +267,35 @@ static int set_attrs() {
   CU(cudaFuncSetAttribute(k_ks6<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks5<MODE_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks5<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
-  CU(cudaFuncSetAttribute(k_ks4<MODE_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
-  CU(cudaFuncSetAttribute(k_ks4<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
+  CU(cudaFuncSetAttribute(k_ks4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
+  return 0;
+}
+
+// FHERAM_KERNEL: a test / A-B timing hook that forces kernels instead of the launch-width rule (DESIGN.md 3.4), a
+// comma-separated list of at most one external-product name (ext*) and one key-switch name (ks*)
+enum Force { FORCE_NONE, FORCE_EXT8, FORCE_EXT9, FORCE_EXT9C4, FORCE_KS8, FORCE_KS8C4, FORCE_KS7, FORCE_KS6, FORCE_KS5,
+             FORCE_KS4, FORCE_COUNT };
+static const char* const kForceNames[FORCE_COUNT] = {"", "ext8", "ext9", "ext9c4", "ks8", "ks8c4", "ks7", "ks6", "ks5",
+                                                     "ks4"};
+static int parse_force(const char* spec, int* force_ext, int* force_ks) {
+  *force_ext = *force_ks = FORCE_NONE;
+  if (!spec || !*spec) return 0;
+  const std::string list(spec);
+  for (size_t pos = 0; pos <= list.size();) {
+    size_t end = list.find(',', pos);
+    if (end == std::string::npos) end = list.size();
+    const std::string name = list.substr(pos, end - pos);
+    int f = FORCE_NONE;
+    for (int i = 1; i < FORCE_COUNT; i++)
+      if (name == kForceNames[i]) f = i;
+    int* slot = f >= FORCE_KS8 ? force_ks : force_ext;
+    if (f == FORCE_NONE || *slot != FORCE_NONE)
+      return fail(FHERAM_ERR_INVALID,
+                  "FHERAM_KERNEL=%s: expected at most one of ext8 ext9 ext9c4 and one of ks8 ks8c4 ks7 ks6 ks5 ks4, "
+                  "comma-separated", spec);
+    *slot = f;
+    pos = end + 1;
+  }
   return 0;
 }
 
@@ -309,6 +319,8 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
     return fail(FHERAM_ERR_INVALID, "max_addr > N^2: the reference's read loop only supports two coordinates");
   if (d.n_glwe & (d.n_glwe - 1))
     return fail(FHERAM_ERR_INVALID, "max_addr / N must be a power of two");
+  int force_ext = FORCE_NONE, force_ks = FORCE_NONE;
+  TRY(parse_force(getenv("FHERAM_KERNEL"), &force_ext, &force_ks));
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -319,6 +331,8 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
   c->params = *p;
   c->d = d;
   c->device = device;
+  c->force_ext = force_ext;
+  c->force_ks = force_ks;
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   c->sm_count = prop.multiProcessorCount;
@@ -339,11 +353,11 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
   for (int b = 0; b < 64; b++) zeta(7, 2 * b, q++);
   for (int b = 0; b < 128; b++) zeta(8, 2 * b, q++);
   for (int b = 0; b < 512; b++) zeta(9, b, q++);
-  // zeta(9, 2k+1) = i zeta(9, 2k): make the table satisfy it bit for bit, so kernels that derive the
-  // odd entry (k_ext3) agree exactly with those that load it
+  // zeta(9, 2k+1) = i zeta(9, 2k): the odd entries (load_tw34 loads them) are set from the even ones, so the
+  // identity holds bit for bit
   for (int b = 1; b < 512; b += 2) q[b - 512] = make_double2(-q[b - 513].y, q[b - 513].x);
   for (int b = 0; b < 512; b++) zeta(10, 2 * b, q++);
-  // zeta(10, 4k+2) = e^(i pi/4) zeta(10, 4k): same treatment, with the roundings of mul_e8 (kernels_ks3.cuh)
+  // zeta(10, 4k+2) = e^(i pi/4) zeta(10, 4k): same treatment, rounded as ((x - y) r, (x + y) r), r = fl(1/sqrt 2)
   for (int b = 1; b < 512; b += 2) {
     const double2 w = q[b - 513];
     const volatile double dx = w.x - w.y, sx = w.x + w.y;
@@ -414,7 +428,7 @@ extern "C" int fheram_ctx_destroy(fheram_ctx* c) {
   cudaStreamSynchronize(c->stream);
   if (c->comm_prep) { ncclCommDestroy(c->comm_prep); c->comm_prep = nullptr; }
   if (c->comm) { ncclCommDestroy(c->comm); c->comm = nullptr; }
-  c->stage64.release(); c->scratch.release(); c->split_tmp[0].release(); c->split_tmp[1].release();
+  c->stage64.release(); c->scratch.release();
   for (auto& b : c->opbuf) b.release();
   for (auto& b : c->enc_buf) b.release();
   cudaFree(c->d_tw); cudaFree(c->d_tw16); cudaFree(c->d_err);
@@ -687,13 +701,13 @@ static size_t prof_event(fheram_ctx* c) {
   return c->ev_used++;
 }
 enum KClass { KC_EXT = 0, KC_TRACE = 1, KC_COMBINE2 = 2, KC_OTHER = 3, KC_COUNT = 4 };
-template <typename K>
-static int launch(fheram_ctx* c, K kernel, const VmpArgs& a, size_t smem, int cls = KC_OTHER) {
+// one kernel launch on c->stream over a.n_items operations, timed per class `cls` when profiling
+template <typename K, typename... X>
+static int launch(fheram_ctx* c, int cls, K kernel, int grid, int block, size_t smem, const VmpArgs& a, X... extra) {
   if (a.n_items <= 0) return 0;
-  int grid = a.n_items < c->sm_count ? a.n_items : c->sm_count;
   size_t e0 = 0;
   if (c->profile) e0 = prof_event(c);
-  kernel<<<grid, kThreads, smem, c->stream>>>(a);
+  kernel<<<grid, block, smem, c->stream>>>(a, extra...);
   if (c->profile) {
     size_t e1 = prof_event(c);
     c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
@@ -703,143 +717,49 @@ static int launch(fheram_ctx* c, K kernel, const VmpArgs& a, size_t smem, int cl
   return 0;
 }
 
-// column-split launch (latency mode): two CTAs per item, single step
-static bool use_split(const fheram_ctx* c, int n_items) {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_SPLIT"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1 && 2 * n_items <= c->sm_count;
+// ---- the launch-width rule (DESIGN.md 3.4): the kernel of a launch of n operations -----------------
+enum Kernel { KN_EXT9_8, KN_EXT9_4, KN_EXT8, KN_KS8_8, KN_KS8_4, KN_KS7, KN_KS6, KN_KS5, KN_KS4, KN_NONE };
+// external-product chains: one chain per cluster of eight (four) SMs while one wave of clusters holds the launch
+// (kernels_ext9.cuh), else one ciphertext per SM (kernels_ext8.cuh)
+static Kernel select_ext(const fheram_ctx* c, int n) {
+  const int e8 = c->ext9_clusters[0], e4 = c->ext9_clusters[1];
+  if (c->force_ext == FORCE_EXT8) return KN_EXT8;
+  if (c->force_ext == FORCE_EXT9C4 && e4 > 0) return KN_EXT9_4;
+  if (c->force_ext == FORCE_EXT9 && n > e8 && e4 > 0) return KN_EXT9_4;
+  if (n <= e8) return KN_EXT9_8;
+  if (n <= e4) return KN_EXT9_4;
+  return KN_EXT8;
 }
-template <typename K>
-static int launch_split(fheram_ctx* c, K kernel, const VmpArgs& a, size_t smem, int cls) {
-  if (a.n_items <= 0) return 0;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  kernel<<<2 * a.n_items, kThreads, smem, c->stream>>>(a);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+// the k_ks8 rows, shared by trace and combine launches (one chain per cluster of eight or four SMs, kernels_ks8.cuh)
+static Kernel select_ks8(const fheram_ctx* c, int n) {
+  const int cap8 = c->ks8_clusters[0], cap4 = c->ks8_clusters[1];
+  if (c->force_ks == FORCE_KS8C4 && cap4 > 0) return KN_KS8_4;
+  if (n <= cap8) return KN_KS8_8;
+  if (n <= cap4) return KN_KS8_4;
+  if (c->force_ks == FORCE_KS8 && cap4 > 0) return KN_KS8_4;
+  if (c->force_ks == FORCE_KS8 && cap8 > 0) return KN_KS8_8;
+  return KN_NONE;
 }
-// word-domain key-switch kernels with two CTAs per SM (k_ks4; k_ext3 when FHERAM_EXT8=0): FHERAM_KS3=0 falls back to
-// k_vmp, FHERAM_KS3=2 uses them for narrow launches as well
-static int ks3_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_KS3"); v = e ? atoi(e) : 1; }
-  return v;
+// trace chains and one-sided packer levels: wide launches on k_ks7 (two CTAs per SM), narrow ones on the two-SM
+// cluster kernel k_ks6 or the one-SM kernel k_ks5
+static Kernel select_trace(const fheram_ctx* c, int n) {
+  const int S = c->sm_count;
+  if (c->force_ks == FORCE_KS7) return KN_KS7;
+  if (c->force_ks == FORCE_KS5) return KN_KS5;
+  if (c->force_ks == FORCE_KS6 && 2 * n <= S) return KN_KS6;  // k_ks6's per-CTA scratch holds 2 S ciphertexts
+  if (const Kernel k = select_ks8(c, n); k != KN_NONE) return k;
+  if (n > S) return KN_KS7;
+  return 2 * n <= S ? KN_KS6 : KN_KS5;
 }
-// one-operation-per-SM key-switch kernels (kernels_ks5.cuh): FHERAM_KS5 = 0 off, 1 narrow launches
-// (at most one item per SM) only, 2 every launch
-static int ks5_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_KS5"); v = e ? atoi(e) : 1; }
-  return v;
-}
-template <typename K>
-static int launch_ks5(fheram_ctx* c, K kernel, const VmpArgs& a, int cls) {
-  if (a.n_items <= 0) return 0;
-  int grid = a.n_items < c->sm_count ? a.n_items : c->sm_count;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  kernel<<<grid, kThreads5, kKs5Smem, c->stream>>>(a);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
-}
-// two-CTA-cluster trace kernel (kernels_ks6.cuh) for launches of at most sm_count / 2 chains; FHERAM_KS6=0 disables
-static bool use_ks6(const fheram_ctx* c, int n_items) {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_KS6"); v = (e && e[0] == '0') ? 0 : 1; }
-  return v == 1 && 2 * n_items <= c->sm_count;
-}
-template <typename K>
-static int launch_ks6(fheram_ctx* c, K kernel, const VmpArgs& a, int cls) {
-  if (a.n_items <= 0) return 0;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  kernel<<<2 * a.n_items, kThreads5, kKs5Smem, c->stream>>>(a);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
-}
-// cluster key-switch kernels (kernels_ks8.cuh, eight or four SMs per chain): FHERAM_KS8 = 0 off, 1 launches of at
-// most one wave of clusters, 2 every trace / combine launch, 3 the same with four-SM clusters only
-static int ks8_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_KS8"); v = e ? atoi(e) : 1; }
-  return v;
-}
-// cluster variant for n_items key switches: 0 = eight SMs per chain, 1 = four, -1 = not a k_ks8 launch
-static int ks8_variant(const fheram_ctx* c, int n_items) {
-  if (ks8_mode() == 0) return -1;
-  if (ks8_mode() == 3) return c->ks8_clusters[1] > 0 ? 1 : -1;  // four-SM clusters for every launch (tests)
-  if (c->ks8_clusters[0] > 0 && n_items <= c->ks8_clusters[0]) return 0;
-  if (c->ks8_clusters[1] > 0 && n_items <= c->ks8_clusters[1]) return 1;
-  if (ks8_mode() == 2) return c->ks8_clusters[1] > 0 ? 1 : (c->ks8_clusters[0] > 0 ? 0 : -1);
-  return -1;
-}
-template <int MODE>
-static int launch_ks8(fheram_ctx* c, int variant, const VmpArgs& a, int cls) {
-  if (a.n_items <= 0) return 0;
-  const int cl = variant == 0 ? 8 : 4, cap = c->ks8_clusters[variant];
-  const int clusters = a.n_items < cap ? a.n_items : cap;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  if (variant == 0) k_ks8<8, MODE><<<cl * clusters, 512, ks8_smem(8), c->stream>>>(a, c->d_tw16);
-  else k_ks8<4, MODE><<<cl * clusters, 512, ks8_smem(4), c->stream>>>(a, c->d_tw16);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
-}
-// 16-point-per-thread trace kernel (kernels_ks7.cuh): FHERAM_KS7 = 0 off, 1 wide launches, 2 every launch
-static int ks7_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_KS7"); v = e ? atoi(e) : 1; }
-  return v;
-}
-template <typename K>
-static int launch_ks7(fheram_ctx* c, K kernel, const VmpArgs& a, int cls) {
-  if (a.n_items <= 0) return 0;
-  int grid = a.n_items < 2 * c->sm_count ? a.n_items : 2 * c->sm_count;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  kernel<<<grid, 256, kKs7Smem, c->stream>>>(a, c->d_tw16);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
-}
-template <typename K>
-static int launch_ks2(fheram_ctx* c, K kernel, const VmpArgs& a, int cls, size_t smem) {
-  if (a.n_items <= 0) return 0;
-  int grid = a.n_items < 2 * c->sm_count ? a.n_items : 2 * c->sm_count;
-  size_t e0 = 0;
-  if (c->profile) e0 = prof_event(c);
-  kernel<<<grid, kThreads, smem, c->stream>>>(a);
-  if (c->profile) {
-    size_t e1 = prof_event(c);
-    c->ev_recs.push_back({cls, e0, e1, (uint64_t)a.n_items, (uint64_t)a.n_steps});
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+// two-sided combines: as the trace, with k_ks4 (two CTAs per SM) for the wide launches
+static Kernel select_combine(const fheram_ctx* c, int n) {
+  const int S = c->sm_count;
+  if (c->force_ks == FORCE_KS4) return KN_KS4;
+  if (c->force_ks == FORCE_KS5) return KN_KS5;
+  if (c->force_ks == FORCE_KS6 && 2 * n <= S) return KN_KS6;
+  if (const Kernel k = select_ks8(c, n); k != KN_NONE) return k;
+  if (2 * n <= S) return KN_KS6;
+  return n <= S ? KN_KS5 : KN_KS4;
 }
 // vmp_prepare of n_mat matrices
 static int inv_mod_2n(int g) {  // g odd, modulus 2N = 8192: g^(N-1) since the unit group has exponent N
@@ -847,16 +767,8 @@ static int inv_mod_2n(int g) {  // g odd, modulus 2N = 8192: g^(N-1) since the u
   for (int e = kN - 1; e; e >>= 1) { if (e & 1) r = r * b % (2 * kN); b = b * b % (2 * kN); }
   return (int)r;
 }
-// external-product chains on k_ext8 (kernels_ext8.cuh, one ciphertext per SM on the two-exchange transform):
-// FHERAM_EXT8 = 0 off (k_ext3 / k_vmp and GGSWs prepared in their frequency order), 1 (default) every launch.
-// The knob also selects the frequency order in which GGSWs are prepared, so it must not change within a process.
-static int ext8_mode() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("FHERAM_EXT8"); v = e ? atoi(e) : 1; }
-  return v;
-}
 // vmp_prepare of n_mat matrices; gal != 1 prepares phi_gal(matrix) (key-switch keys, see k_vmp);
-// order7: frequency order of the 16-point transform (k_prepare7: consumers k_ks7 / k_ext8)
+// order7: frequency order of the 16-point transform (k_prepare7: consumers k_ks7 / k_ks8 / k_ext8 / k_ext9)
 static int prepare(fheram_ctx* c, const int* raw, long raw_stride, double2* out, long out_stride,
                    int n_mat, int rows, int cin, int lout, int gal = 1, bool order7 = false,
                    cudaStream_t stream = nullptr) {
@@ -878,10 +790,10 @@ static int prepare(fheram_ctx* c, const int* raw, long raw_stride, double2* out,
   CU(cudaGetLastError());
   return 0;
 }
-// CoordinatePrepared::prepare (src/coordinate_prepared.rs:104-116) of n_mat GGSWs, in the order the external-product kernel in use reads
+// CoordinatePrepared::prepare (src/coordinate_prepared.rs:104-116) of n_mat GGSWs, in the frequency order of the
+// external-product kernels (k_prepare7)
 static int prepare_ggsw(fheram_ctx* c, const int* raw, double2* out, int n_mat) {
-  return prepare(c, raw, c->ggsw_raw_len(), out, c->ggsw_prep_len(), n_mat, c->d.dnum_ct, 2, c->d.size_addr, 1,
-                 ext8_mode() != 0);
+  return prepare(c, raw, c->ggsw_raw_len(), out, c->ggsw_prep_len(), n_mat, c->d.dnum_ct, 2, c->d.size_addr, 1, true);
 }
 
 // --------------------------------------------------------------------------------------
@@ -890,7 +802,7 @@ static int prepare_ggsw(fheram_ctx* c, const int* raw, double2* out, int n_mat) 
 struct fheram_keys {
   fheram_ctx* c;
   double2* atk = nullptr;      // [log_n] prepared trace keys
-  double2* atk7 = nullptr;     // trace keys prepared in the frequency order of k_ks7
+  double2* atk7 = nullptr;     // trace keys prepared in the frequency order of k_ks7 / k_ks8 (k_prepare7)
   double2* atk_inv = nullptr;  // prepared atk_ggsw_inv
   double2* tsk = nullptr;      // prepared tsk_ggsw_inv
   int* raw = nullptr;          // fheram_keys_encrypt_sk: the raw keys [atk x log_n | tsk | atk_inv] (fheram_keys_download_raw)
@@ -1088,65 +1000,33 @@ static int run_ext_chain(fheram_ctx* c, int n_items, const int* src, const int* 
   a.n_steps = n_dig;
   for (int s = 0; s < n_dig; s++) a.mat[s] = mats + (size_t)s * c->ggsw_prep_len();
   a.mat_div = mat_div; a.mat_stride = mat_stride;
-  if (ext8_mode() != 0) {
-    if (n_items <= 0) return 0;
-    // launches of at most one wave of clusters: one chain per cluster of eight (four) SMs (kernels_ext9.cuh);
-    // FHERAM_EXT9 = 0 off, 1 default, 2 every launch, 3 every launch on four-SM clusters
-    static int ext9 = -1;
-    if (ext9 < 0) { const char* e = getenv("FHERAM_EXT9"); ext9 = e ? atoi(e) : 1; }
-    int v9 = -1;
-    if (ext9 == 3) v9 = c->ext9_clusters[1] > 0 ? 1 : -1;
-    else if (ext9 >= 1) {
-      if (c->ext9_clusters[0] > 0 && n_items <= c->ext9_clusters[0]) v9 = 0;
-      else if (c->ext9_clusters[1] > 0 && (n_items <= c->ext9_clusters[1] || ext9 == 2)) v9 = 1;
-    }
-    if (v9 >= 0) {
-      const int cl = v9 == 0 ? 8 : 4, cap = c->ext9_clusters[v9];
-      const int clusters = n_items < cap ? n_items : cap;
-      size_t e0 = 0;
-      if (c->profile) e0 = prof_event(c);
-      if (v9 == 0) k_ext9<8><<<cl * clusters, 512, ext9_smem(8), c->stream>>>(a, c->d_tw16);
-      else k_ext9<4><<<cl * clusters, 512, ext9_smem(4), c->stream>>>(a, c->d_tw16);
-      if (c->profile) {
-        size_t e1 = prof_event(c);
-        c->ev_recs.push_back({KC_EXT, e0, e1, (uint64_t)n_items, (uint64_t)n_dig});
-      }
-      c->launches++;
-      CU(cudaGetLastError());
-      return 0;
-    }
-    const int grid = n_items < c->sm_count ? n_items : c->sm_count;
-    size_t e0 = 0;
-    if (c->profile) e0 = prof_event(c);
-    k_ext8<<<grid, kExt8Threads, kExt8Smem, c->stream>>>(a, c->d_tw16);
-    if (c->profile) {
-      size_t e1 = prof_event(c);
-      c->ev_recs.push_back({KC_EXT, e0, e1, (uint64_t)n_items, (uint64_t)n_dig});
-    }
-    c->launches++;
-    CU(cudaGetLastError());
-    return 0;
+  switch (select_ext(c, n_items)) {
+    case KN_EXT9_8:
+      return launch(c, KC_EXT, k_ext9<8>, 8 * std::min(n_items, c->ext9_clusters[0]), 512, ext9_smem(8), a, c->d_tw16);
+    case KN_EXT9_4:
+      return launch(c, KC_EXT, k_ext9<4>, 4 * std::min(n_items, c->ext9_clusters[1]), 512, ext9_smem(4), a, c->d_tw16);
+    default:
+      return launch(c, KC_EXT, k_ext8, std::min(n_items, c->sm_count), kExt8Threads, kExt8Smem, a, c->d_tw16);
   }
-  if (ks3_mode() >= 2) return launch_ks2(c, k_ext3, a, KC_EXT, kExt3Smem);  // forced (kernel-variant tests)
-  if (use_split(c, n_items)) {
-    // narrow launch: one step per launch, two CTAs per ciphertext (one output column each),
-    // ping-pong between two temporaries because both CTAs read both input columns
-    const size_t bytes = sizeof(int) * (size_t)n_items * c->ct_stride();
-    TRY(c->split_tmp[0].ensure(bytes));
-    TRY(c->split_tmp[1].ensure(bytes));
-    for (int s = 0; s < n_dig; s++) {
-      VmpArgs b = a;
-      b.n_steps = 1;
-      b.mat[0] = a.mat[s];
-      if (s > 0) { b.src = (const int*)c->split_tmp[(s - 1) & 1].p; b.src_map = nullptr; b.src_mod = 0; b.src_div = 0; }
-      b.dst = (int*)c->split_tmp[s & 1].p;
-      TRY(launch_split(c, K_EXT_S, b, smem_bytes(3, 2, false), KC_EXT));
-    }
-    CU(cudaMemcpyAsync(dst, c->split_tmp[(n_dig - 1) & 1].p, bytes, cudaMemcpyDeviceToDevice, c->stream));
-    return 0;
+}
+// a key-switch launch of MODE_TRACE or MODE_COMBINE2: step s uses trace key key0 + s, in the frequency order of the
+// selected kernel (k_ks7 and k_ks8 read the keys prepared by k_prepare7, the others those of k_prepare)
+template <int MODE>
+static int launch_ks(fheram_ctx* c, const fheram_keys* k, int key0, VmpArgs a) {
+  const int n = a.n_items, S = c->sm_count, cls = MODE == MODE_TRACE ? KC_TRACE : KC_COMBINE2;
+  const Kernel kn = MODE == MODE_TRACE ? select_trace(c, n) : select_combine(c, n);
+  const double2* keys = (kn == KN_KS7 || kn == KN_KS8_8 || kn == KN_KS8_4) ? k->atk7 : k->atk;
+  for (int s = 0; s < a.n_steps; s++) a.mat[s] = keys + (size_t)(key0 + s) * c->atk_prep_len();
+  switch (kn) {
+    case KN_KS8_8:
+      return launch(c, cls, k_ks8<8, MODE>, 8 * std::min(n, c->ks8_clusters[0]), 512, ks8_smem(8), a, c->d_tw16);
+    case KN_KS8_4:
+      return launch(c, cls, k_ks8<4, MODE>, 4 * std::min(n, c->ks8_clusters[1]), 512, ks8_smem(4), a, c->d_tw16);
+    case KN_KS7: return launch(c, cls, k_ks7, std::min(n, 2 * S), 256, kKs7Smem, a, c->d_tw16);
+    case KN_KS6: return launch(c, cls, k_ks6<MODE>, 2 * n, kThreads5, kKs5Smem, a);
+    case KN_KS5: return launch(c, cls, k_ks5<MODE>, std::min(n, S), kThreads5, kKs5Smem, a);
+    default: return launch(c, cls, k_ks4, std::min(n, 2 * S), kThreads, kKs4Smem, a);
   }
-  if (ks3_mode() >= 1 && n_items > c->sm_count) return launch_ks2(c, k_ext3, a, KC_EXT, kExt3Smem);
-  return launch(c, K_EXT, a, smem_bytes(3, 2, false), KC_EXT);
 }
 // chain of { glwe_rsh(1); automorphism_add with trace key i } for i in [g0, g1)
 // (glwe_trace_inplace, and the one-sided levels of GLWEPacker::combine)
@@ -1157,7 +1037,6 @@ static int run_trace_chain(fheram_ctx* c, const fheram_keys* k, int n_items, con
   a.src_map = src_map; a.src_mod = src_mod; a.src_div = src_div;
   a.n_steps = g1 - g0;
   for (int s = 0; s < a.n_steps; s++) {
-    a.mat[s] = k->atk + (size_t)(g0 + s) * c->atk_prep_len();
     a.gal[s] = (int)((galois(c->d.log_n, g0 + s) + 2 * kN) % (2 * kN));
     a.gal_inv[s] = inv_mod_2n(a.gal[s]);
   }
@@ -1174,73 +1053,17 @@ static int run_trace_chain(fheram_ctx* c, const fheram_keys* k, int n_items, con
     CU(cudaGetLastError());
     return 0;
   }
-  if (const int v8 = ks8_variant(c, n_items); v8 >= 0) {
-    VmpArgs b = a;
-    for (int s = 0; s < b.n_steps; s++) b.mat[s] = k->atk7 + (size_t)(g0 + s) * c->atk_prep_len();
-    return launch_ks8<MODE_TRACE>(c, v8, b, KC_TRACE);
-  }
-  if (ks7_mode() == 2 || (ks7_mode() == 1 && n_items > c->sm_count)) {
-    VmpArgs b = a;
-    for (int s = 0; s < b.n_steps; s++) b.mat[s] = k->atk7 + (size_t)(g0 + s) * c->atk_prep_len();
-    return launch_ks7(c, k_ks7<MODE_TRACE>, b, KC_TRACE);
-  }
-  if (ks5_mode() >= 1 && use_ks6(c, n_items)) return launch_ks6(c, k_ks6<MODE_TRACE>, a, KC_TRACE);
-  if (ks5_mode() == 2 || (ks5_mode() == 1 && n_items <= c->sm_count)) return launch_ks5(c, k_ks5<MODE_TRACE>, a, KC_TRACE);
-  if (ks3_mode() >= 2) return launch_ks2(c, k_ks4<MODE_TRACE>, a, KC_TRACE, kKs4Smem);
-  if (use_split(c, n_items)) {
-    const size_t bytes = sizeof(int) * (size_t)n_items * c->ct_stride();
-    TRY(c->split_tmp[0].ensure(bytes));
-    TRY(c->split_tmp[1].ensure(bytes));
-    for (int s = 0; s < a.n_steps; s++) {
-      VmpArgs b = a;
-      b.n_steps = 1;
-      b.mat[0] = a.mat[s]; b.gal[0] = a.gal[s]; b.gal_inv[0] = a.gal_inv[s];
-      if (s > 0) {
-        b.src = (const int*)c->split_tmp[(s - 1) & 1].p;
-        b.src_map = nullptr; b.src_mod = 0; b.src_div = 0; b.rot_mod = 0; b.rot_mul = 0; b.rot_const = 0;
-      }
-      b.dst = (int*)c->split_tmp[s & 1].p;
-      TRY(launch_split(c, K_TRACE_S, b, smem_bytes(3, 1, true), KC_TRACE));
-    }
-    CU(cudaMemcpyAsync(dst, c->split_tmp[(a.n_steps - 1) & 1].p, bytes, cudaMemcpyDeviceToDevice, c->stream));
-    return 0;
-  }
-  // wide launches: two lean CTAs per SM overlap each other's phases; narrow ones (at most one
-  // item per SM) finish sooner with the single-CTA kernel
-  if (ks3_mode() == 1 && n_items > c->sm_count) return launch_ks2(c, k_ks4<MODE_TRACE>, a, KC_TRACE, kKs4Smem);
-  return launch(c, K_TRACE, a, smem_bytes(3, 1, true), KC_TRACE);
+  return launch_ks<MODE_TRACE>(c, k, g0, a);
 }
 // GLWEPacker::combine, both operands present, at tree level `level` (0-based absolute):
 // in[2i], in[2i+1] -> out[i]
 static int run_combine2(fheram_ctx* c, const fheram_keys* k, int n_items, const int* in, int* out, int level) {
   VmpArgs a = base_args(c, n_items, in, out, c->ct_stride());
   a.n_steps = 1;
-  a.mat[0] = k->atk + (size_t)level * c->atk_prep_len();
   a.gal[0] = (int)((galois(c->d.log_n, level) + 2 * kN) % (2 * kN));
   a.gal_inv[0] = inv_mod_2n(a.gal[0]);
   a.rot_const = 1 << (c->d.log_n - level - 1);  // t
-  if (const int v8 = ks8_variant(c, n_items); v8 >= 0) {
-    VmpArgs b = a;
-    b.mat[0] = k->atk7 + (size_t)level * c->atk_prep_len();
-    return launch_ks8<MODE_COMBINE2>(c, v8, b, KC_COMBINE2);
-  }
-  {
-    static int ks7c = -1;  // two-sided combine on k_ks7: FHERAM_KS7C = 0 off, 1 wide launches, 2 every launch
-    if (ks7c < 0) { const char* e = getenv("FHERAM_KS7C"); ks7c = e ? atoi(e) : 0; }
-    if (ks7c == 2 || (ks7c == 1 && n_items > c->sm_count)) {
-      VmpArgs b = a;
-      b.mat[0] = k->atk7 + (size_t)level * c->atk_prep_len();
-      return launch_ks7(c, k_ks7<MODE_COMBINE2>, b, KC_COMBINE2);
-    }
-  }
-  if (ks5_mode() >= 1 && use_ks6(c, n_items)) return launch_ks6(c, k_ks6<MODE_COMBINE2>, a, KC_COMBINE2);
-  // one item per SM where two CTAs per item no longer fit (75 .. sm_count items): 37-39 us against 45 us of k_vmp
-  if (ks5_mode() == 2 || (ks5_mode() == 1 && n_items <= c->sm_count && 2 * n_items > c->sm_count))
-    return launch_ks5(c, k_ks5<MODE_COMBINE2>, a, KC_COMBINE2);
-  if (ks3_mode() >= 2) return launch_ks2(c, k_ks4<MODE_COMBINE2>, a, KC_COMBINE2, kKs4Smem);
-  if (use_split(c, n_items)) return launch_split(c, K_COMBINE2_S, a, smem_bytes(3, 1, true), KC_COMBINE2);
-  if (ks3_mode() == 1 && n_items > c->sm_count) return launch_ks2(c, k_ks4<MODE_COMBINE2>, a, KC_COMBINE2, kKs4Smem);
-  return launch(c, K_COMBINE2, a, smem_bytes(3, 1, true), KC_COMBINE2);
+  return launch_ks<MODE_COMBINE2>(c, k, level, a);
 }
 
 // GLWEPacker over `width` inputs per group (width a power of two), feed order = index order
@@ -2099,11 +1922,11 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
     // one "matrix" of the prepare kernel = the coord_len[.] consecutive GGSWs of one coordinate of one address
     const int n0 = d.coord_len[0], n1 = d.n_coord > 1 ? d.coord_len[1] : 0;
     double2* own = s.a.prep + (size_t)r->shard * nb * n0 * glen;
-    TRY(prepare(c, s.a.raw, (long)per_addr, own, (long)(n0 * glen), nb, n0 * d.dnum_ct, 2, d.size_addr, 1,
-                ext8_mode() != 0, copy_stream));
+    TRY(prepare(c, s.a.raw, (long)per_addr, own, (long)(n0 * glen), nb, n0 * d.dnum_ct, 2, d.size_addr, 1, true,
+                copy_stream));
     if (n1)
       TRY(prepare(c, s.a.raw + (size_t)n0 * c->ggsw_raw_len(), (long)per_addr, s.a.prep1, (long)(n1 * glen), nb,
-                  n1 * d.dnum_ct, 2, d.size_addr, 1, ext8_mode() != 0, copy_stream));
+                  n1 * d.dnum_ct, 2, d.size_addr, 1, true, copy_stream));
     if (G > 1) NC(ncclAllGather(own, s.a.prep, (size_t)nb * n0 * glen * sizeof(double2), ncclChar, c->comm_prep, copy_stream));
     CU(cudaEventRecord(s.copied, copy_stream));
     return 0;
@@ -2285,7 +2108,7 @@ static int ggsw_invert_device(fheram_ctx* c, const fheram_keys* k, const int* ra
     a.mat[0] = k->atk_inv;
     a.gal[0] = 2 * kN - 1;
     a.gal_inv[0] = 2 * kN - 1;
-    TRY(launch(c, K_AUTO_INV, a, smem_bytes(4, 1, false)));
+    TRY(launch(c, KC_OTHER, K_AUTO_INV, std::min(items, c->sm_count), kThreads, smem_bytes(4), a));
   }
   {
     VmpArgs a = base_args(c, items, inv_raw, inv_raw + glwe4, 2 * glwe4);
@@ -2293,7 +2116,7 @@ static int ggsw_invert_device(fheram_ctx* c, const fheram_keys* k, const int* ra
     a.mat[0] = k->tsk;
     a.gal[0] = 1;
     a.gal_inv[0] = 1;
-    TRY(launch(c, K_EXPAND, a, smem_bytes(4, 1, false)));
+    TRY(launch(c, KC_OTHER, K_EXPAND, std::min(items, c->sm_count), kThreads, smem_bytes(4), a));
   }
   return 0;
 }
@@ -2465,7 +2288,7 @@ extern "C" int fheram_glwe_automorphism(fheram_ctx* c, const fheram_keys* k, int
     a.mat[0] = k->atk + (size_t)gal_idx * c->atk_prep_len();
     a.gal[0] = (int)((galois(c->d.log_n, gal_idx) + 2 * kN) % (2 * kN));
     a.gal_inv[0] = inv_mod_2n(a.gal[0]);
-    TRY(launch(c, K_AUTO3, a, smem_bytes(3, 1, false)));
+    TRY(launch(c, KC_OTHER, K_AUTO3, std::min(n, c->sm_count), kThreads, smem_bytes(3), a));
     res = (int*)c->opbuf[1].p;
   } else {
     TRY(run_trace_chain(c, k, n, res, nullptr, 0, 0, res, gal_idx, gal_idx + 1, 0, 0, 0, mode == 1 ? 1 : -1));

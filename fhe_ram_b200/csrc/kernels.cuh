@@ -243,7 +243,6 @@ __device__ __forceinline__ int rot_index(int i, int k, bool& neg) {
 constexpr int kMaxSteps = 12;
 
 enum Mode : int {
-  MODE_EXT = 0,      // chain of external products (coordinate_prepared.rs:147-177)
   MODE_TRACE = 1,    // chain of { rsh 1; x <- x +/- phi_g(KS(x)) }  (trace / one-sided combine)
   MODE_COMBINE2 = 2, // GLWEPacker two-sided combine
   MODE_AUTO = 3,     // x <- phi_g(normalize(KS(x)))  (glwe_automorphism)
@@ -289,25 +288,22 @@ struct VmpArgs {
   } while (0)
 
 // ======================================================================================
-// The fused kernel.
+// The fused kernel: glwe_automorphism and the GGSW expand rows of the inverse address.
 // Key-switch modes use keys prepared as phi_g(K) (k_prepare with gal_inv): since
 // phi_g(sum_r a_r * K_r) = sum_r phi_g(a_r) * phi_g(K_r), transforming phi_g(x) instead of x makes
 // the inverse transform deliver phi_g(KS(x)) directly in natural coefficient order, so every
 // epilogue works on the thread's own positions (no scatter) and only reads of the small input
 // are gathered.
-//   R     limbs of the input ciphertext that are transformed (rows per input column)
-//   CIN   2: both columns enter the product (GGSW), 1: mask column only (key switch)
+//   R     limbs of the input ciphertext that are transformed (mask column only)
 //   LOUT  limbs of the matrix / big result;   LRES  limbs kept after normalisation
-// Shared memory: R*CIN spectra (32 KiB each) + 32 KiB work + (XSMEM ? 2*R*N ints : 0).
+// Shared memory: R spectra (32 KiB each) + 32 KiB work.
 // ======================================================================================
-// SPLIT (latency mode for narrow launches): two CTAs share one operation, CTA (2*item + c) produces
-// output column c only (both transform the inputs redundantly); single-step launches, src != dst.
-template <int R, int CIN, int LOUT, int LRES, int MODE, bool XSMEM, bool SPLIT = false>
+template <int R, int LOUT, int LRES, int MODE>
 __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
+  static_assert(MODE == MODE_AUTO || MODE == MODE_EXPAND, "automorphism / expand only");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* spectra = reinterpret_cast<double2*>(smem_raw);
-  double2* work = spectra + (size_t)R * CIN * kM;
-  int* xs = reinterpret_cast<int*>(work + kM);  // only if XSMEM
+  double2* work = spectra + (size_t)R * kM;
 
   const int T = threadIdx.x, w = T >> 5, lane = T & 31;
   const Tw34 tw = load_tw34(A.tw, w, lane);
@@ -316,19 +312,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
   long long phase_t0 = A.phase_cycles ? clock64() : 0;
-  const int my_co = SPLIT ? (blockIdx.x & 1) : 0;
-  for (int item = SPLIT ? (blockIdx.x >> 1) : blockIdx.x; item < A.n_items; item += SPLIT ? (gridDim.x >> 1) : gridDim.x) {
+  for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
-    int* scr0 = A.scratch ? A.scratch + (size_t)blockIdx.x * 2 * A.ct_stride : nullptr;
-    int* scr1 = scr0 ? scr0 + A.ct_stride : nullptr;
-    // x buffer: the key-switch input ciphertext (and in-place result for MODE_TRACE)
-    int* xb = XSMEM ? xs : scr0;
 
     const int* src;
     {
       long idx = item;
-      if (MODE == MODE_COMBINE2) idx = 2L * item;
-      else if (A.src_div > 0) idx = item / A.src_div;
+      if (A.src_div > 0) idx = item / A.src_div;
       else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
       src = A.src + idx * A.ct_stride;
     }
@@ -336,86 +326,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
 
     for (int step = 0; step < A.n_steps; step++) {
       const double2* G = A.mat[step] + mat_off;
-
-      // ------------------------------ prologue ------------------------------------
-      if (MODE == MODE_TRACE) {
-        // x = rsh1( step 0 ? rot(src) : x )   (Poulpy glwe_rsh(1) before automorphism_add)
-        int rk = A.rot_const;
-        if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
-        rk &= (2 * kN - 1);
-#pragma unroll 4
-        for (int m = 0; m < 16; m++) {
-          const int i = T + 256 * m;  // 16 positions per thread: i and i + 2048 for m < 8
-#pragma unroll
-          for (int col = 0; col < 2; col++) {
-            int a0, a1, a2;
-            if (step == 0) {
-              // value at i of src * X^rk = +/- src[(i - rk) mod 2N]
-              bool neg;
-              int j = rot_index(i, 2 * kN - rk, neg);
-              a0 = src[CT(col, 0) + j]; a1 = src[CT(col, 1) + j]; a2 = src[CT(col, 2) + j];
-              if (neg) { a0 = -a0; a1 = -a1; a2 = -a2; }
-            } else {
-              a0 = xb[CT(col, 0) + i]; a1 = xb[CT(col, 1) + i]; a2 = xb[CT(col, 2) + i];
-            }
-            int d0, d1, d2;
-            rsh1_3(a0, a1, a2, d0, d1, d2);
-            xb[CT(col, 0) + i] = d0; xb[CT(col, 1) + i] = d1; xb[CT(col, 2) + i] = d2;
-          }
-        }
-      } else if (MODE == MODE_COMBINE2) {
-        // a1 = a X^-t ; D = rsh1(a1 - b) -> xb ; S = rsh1(a1 + b) -> scr1
-        const int* a = src;
-        const int* b = src + A.ct_stride;
-        const int tt = A.rot_const;  // t
-        // loads are staged four positions at a time ahead of the stores: the scratch stores may
-        // alias the source for the compiler, which would otherwise serialise one L2 round trip
-        // per coefficient
-#pragma unroll 1
-        for (int mc = 0; mc < 16; mc += 4) {
-          int av[4][2][3], bv[4][2][3];
-          bool ng[4];
-#pragma unroll
-          for (int mm = 0; mm < 4; mm++) {
-            const int i = T + 256 * (mc + mm);
-            const int j = rot_index(i, tt, ng[mm]);  // (a X^-t)[i] = +/- a[(i + t) mod 2N]
-#pragma unroll
-            for (int col = 0; col < 2; col++)
-#pragma unroll
-              for (int l = 0; l < 3; l++) { av[mm][col][l] = a[CT(col, l) + j]; bv[mm][col][l] = b[CT(col, l) + i]; }
-          }
-#pragma unroll
-          for (int mm = 0; mm < 4; mm++) {
-            const int i = T + 256 * (mc + mm);
-#pragma unroll
-            for (int col = 0; col < 2; col++) {
-              int a0 = av[mm][col][0], a1 = av[mm][col][1], a2 = av[mm][col][2];
-              if (ng[mm]) { a0 = -a0; a1 = -a1; a2 = -a2; }
-              const int b0 = bv[mm][col][0], b1 = bv[mm][col][1], b2 = bv[mm][col][2];
-              int d0, d1, d2;
-              rsh1_3(a0 - b0, a1 - b1, a2 - b2, d0, d1, d2);
-              xb[CT(col, 0) + i] = d0; xb[CT(col, 1) + i] = d1; xb[CT(col, 2) + i] = d2;
-              rsh1_3(a0 + b0, a1 + b1, a2 + b2, d0, d1, d2);
-              scr1[CT(col, 0) + i] = d0; scr1[CT(col, 1) + i] = d1; scr1[CT(col, 2) + i] = d2;
-            }
-          }
-        }
-      }
       PHASE_TICK(0);
       // input of the transforms
-      const int* xin = (MODE == MODE_TRACE || MODE == MODE_COMBINE2) ? xb
-                       : (MODE == MODE_EXT && step > 0) ? dst : src;
-      constexpr bool PERM = (MODE == MODE_TRACE || MODE == MODE_COMBINE2 || MODE == MODE_AUTO);
+      const int* xin = src;
+      constexpr bool PERM = MODE == MODE_AUTO;
       const int ginv = A.gal_inv[step];
-      // the permuted loads below read positions other threads wrote in the prologue
-      if (MODE == MODE_TRACE || MODE == MODE_COMBINE2 || (MODE == MODE_EXT && step > 0)) __syncthreads();
 
       // --------------------------- forward transforms ------------------------------
       // integer limbs of row rho+1 are requested while row rho is converted and transformed
       auto load_row = [&](int rho, int (&v)[16]) {
-        const int limb = rho / CIN;
-        const int col = CIN == 2 ? (rho % CIN) : 1;
-        const int* p = xin + CT(col, limb);
+        const int* p = xin + CT(1, rho);
 #pragma unroll
         for (int m = 0; m < 8; m++) {
           const int i = T + 256 * m;
@@ -435,17 +355,17 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
       int nx[16];
       load_row(0, nx);
 #pragma unroll 1
-      for (int rho = 0; rho < R * CIN; rho++) {
+      for (int rho = 0; rho < R; rho++) {
         double2 x[8];
 #pragma unroll
         for (int m = 0; m < 8; m++) x[m] = make_double2((double)nx[m], (double)nx[m + 8]);
-        if (rho + 1 < R * CIN) load_row(rho + 1, nx);
+        if (rho + 1 < R) load_row(rho + 1, nx);
         fwd_pass1_store(x, spectra + (size_t)rho * kM, T);
       }
       __syncthreads();
       PHASE_TICK(1);
 #pragma unroll 1
-      for (int rho = 0; rho < R * CIN; rho++) fwd_warp_passes(spectra + (size_t)rho * kM, w, lane, tw);
+      for (int rho = 0; rho < R; rho++) fwd_warp_passes(spectra + (size_t)rho * kM, w, lane, tw);
       PHASE_TICK(2);
       // no barrier needed: the contraction reads only what this thread wrote
 
@@ -454,68 +374,39 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
       // from shared memory once for two outputs); carries fit 32 bits (|big| < 2^47).
       // (A register prefetch of the next output's matrix rows across the inverse transform was
       // measured and does not overlap: the L2 port runs at ~55 B/clk/SM either way.)
-      constexpr int NR = R * CIN;
       const int P0 = 256 * w + lane;
       int carryA[16], carryB[16];    // running carry of column 0 / column 1
-      int carry2A[16], carry2B[16];  // COMBINE2: carry of the second normalisation
 #pragma unroll
-      for (int q = 0; q < 16; q++) { carryA[q] = 0; carryB[q] = 0; carry2A[q] = 0; carry2B[q] = 0; }
+      for (int q = 0; q < 16; q++) { carryA[q] = 0; carryB[q] = 0; }
 #pragma unroll 1
       for (int l = LOUT - 1; l >= 0; l--) {
         double2 cur[8], nxt[8];
 #pragma unroll
         for (int j = 0; j < 8; j++) { cur[j] = make_double2(0.0, 0.0); nxt[j] = make_double2(0.0, 0.0); }
-#pragma unroll(NR <= 4 ? NR : 2)
-        for (int rho = 0; rho < NR; rho++) {
+#pragma unroll(R <= 4 ? R : 2)
+        for (int rho = 0; rho < R; rho++) {
           const double2* gp = G + ((size_t)rho * NOUT + l) * kM + P0;
           const double2* ap = spectra + (size_t)rho * kM + P0;
           double2 g0[8], g1[8];
-          if (SPLIT) {
 #pragma unroll
-            for (int j = 0; j < 8; j++) g0[j] = __ldg(gp + (size_t)my_co * LOUT * kM + 32 * j);
+          for (int j = 0; j < 8; j++) { g0[j] = __ldg(gp + 32 * j); g1[j] = __ldg(gp + (size_t)LOUT * kM + 32 * j); }
 #pragma unroll
-            for (int j = 0; j < 8; j++) {
-              const double2 a = ap[32 * j];
-              cur[j].x = fma(a.x, g0[j].x, fma(-a.y, g0[j].y, cur[j].x));
-              cur[j].y = fma(a.x, g0[j].y, fma(a.y, g0[j].x, cur[j].y));
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < 8; j++) { g0[j] = __ldg(gp + 32 * j); g1[j] = __ldg(gp + (size_t)LOUT * kM + 32 * j); }
-#pragma unroll
-            for (int j = 0; j < 8; j++) {
-              const double2 a = ap[32 * j];
-              cur[j].x = fma(a.x, g0[j].x, fma(-a.y, g0[j].y, cur[j].x));
-              cur[j].y = fma(a.x, g0[j].y, fma(a.y, g0[j].x, cur[j].y));
-              nxt[j].x = fma(a.x, g1[j].x, fma(-a.y, g1[j].y, nxt[j].x));
-              nxt[j].y = fma(a.x, g1[j].y, fma(a.y, g1[j].x, nxt[j].y));
-            }
+          for (int j = 0; j < 8; j++) {
+            const double2 a = ap[32 * j];
+            cur[j].x = fma(a.x, g0[j].x, fma(-a.y, g0[j].y, cur[j].x));
+            cur[j].y = fma(a.x, g0[j].y, fma(a.y, g0[j].x, cur[j].y));
+            nxt[j].x = fma(a.x, g1[j].x, fma(-a.y, g1[j].y, nxt[j].x));
+            nxt[j].y = fma(a.x, g1[j].y, fma(a.y, g1[j].x, nxt[j].y));
           }
         }
         PHASE_TICK(3);
 #pragma unroll 1
-        for (int co = SPLIT ? my_co : 0; co < (SPLIT ? my_co + 1 : 2); co++) {
+        for (int co = 0; co < 2; co++) {
           const bool has_small = l < R;  // the small operand has R limbs
-          int xnat[16];  // MODE_TRACE: phi_g(x) body limb; read before any thread overwrites the
-                         // buffer in place, i.e. between the two barriers of the inverse transform
-          inv_transform(cur, work, T, w, lane, tw, [&]() {
-            if (MODE == MODE_TRACE) {
-#pragma unroll
-              for (int q = 0; q < 16; q++) {
-                const int i = T + 256 * (q & 7) + (q >> 3) * kM;
-                bool neg;
-                const int u = auto_index(i, ginv, neg);
-                const int v = (co == 0 && has_small) ? xb[CT(0, l) + u] : 0;
-                xnat[q] = neg ? -v : v;
-              }
-            }
-          });
+          inv_transform(cur, work, T, w, lane, tw, [&]() {});
           PHASE_TICK(4);
-          int sv[16];  // small global operands of this output, requested together (see prologue note)
-          if (MODE == MODE_COMBINE2 && l < LRES) {
-#pragma unroll
-            for (int q = 0; q < 16; q++) sv[q] = scr1[CT(co, l) + T + 256 * (q & 7) + (q >> 3) * kM];
-          } else if (MODE == MODE_EXPAND && co == 1 && has_small) {
+          int sv[16];  // small global operands of this output, requested together
+          if (MODE == MODE_EXPAND && co == 1 && has_small) {
 #pragma unroll
             for (int q = 0; q < 16; q++) sv[q] = xin[CT(0, l) + T + 256 * (q & 7) + (q >> 3) * kM];
           } else if (MODE == MODE_AUTO && co == 0 && has_small) {
@@ -525,72 +416,38 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
               sv[q] = xin[CT(0, l) + auto_index(T + 256 * (q & 7) + (q >> 3) * kM, ginv, ng)];
             }
           }
-          // cur[m] = M * phi_g(vmp)[T + 256 m] (natural order; plain vmp for EXT / EXPAND)
+          // cur[m] = M * phi_g(vmp)[T + 256 m] (natural order; plain vmp for EXPAND)
 #pragma unroll
           for (int q = 0; q < 16; q++) {
             const int i = T + 256 * (q & 7) + (q >> 3) * kM;
             const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
             long long big = __double2ll_rn(v);
             bool neg = false;
-            if (MODE == MODE_TRACE) {
-              // x +/- phi(KS(x)), KS(x) = vmp + body:  phi(body) gathered above
-              big += (long long)xnat[q];
-              if (A.sign < 0) big = -big;
-              if (has_small) big += (long long)xb[CT(co, l) + i];
-            } else if (MODE == MODE_EXPAND) {
+            if (MODE == MODE_EXPAND) {
               if (co == 1 && has_small) big += (long long)sv[q];
-            } else if (MODE == MODE_AUTO || MODE == MODE_COMBINE2) {
+            } else {
               // phi(normalize(KS(x))): run the carry chain in the pre-automorphism sign frame
-              const int u = auto_index(i, ginv, neg);
+              auto_index(i, ginv, neg);
               if (neg) big = -big;
-              if (co == 0 && has_small) big += (long long)(MODE == MODE_AUTO ? sv[q] : xin[CT(0, l) + u]);
+              if (co == 0 && has_small) big += (long long)sv[q];
             }
             const long long t = big + (long long)carryA[q];
             const int c = (int)((t + 65536) >> kK);
             const int dg = (int)t - (c << kK);
             carryA[q] = c;
-            if (l < LRES) {
-              if (MODE == MODE_EXT || MODE == MODE_EXPAND) {
-                dst[CT(co, l) + i] = dg;
-              } else if (MODE == MODE_AUTO) {
-                dst[CT(co, l) + i] = neg ? -dg : dg;
-              } else if (MODE == MODE_TRACE) {
-                xb[CT(co, l) + i] = dg;
-              } else if (MODE == MODE_COMBINE2) {
-                // y = phi(normalize(KS(D))); a' = normalize(S - y); out = a' X^t
-                const int y = neg ? -dg : dg;
-                const int t2 = sv[q] - y + carry2A[q];
-                const int dg2 = sext17i(t2);
-                carry2A[q] = (t2 - dg2) >> kK;
-                bool rneg;
-                const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
-                dst[CT(co, l) + dd] = rneg ? -dg2 : dg2;
-              }
-            }
+            if (l < LRES) dst[CT(co, l) + i] = neg ? -dg : dg;
           }
           PHASE_TICK(5);
-          // rotate the per-column state so the loop body always works on (cur, carryA, carry2A)
-          // (split mode handles one column only: nothing to rotate)
-          if (!SPLIT) {
+          // rotate the per-column state so the loop body always works on (cur, carryA)
 #pragma unroll
-            for (int j = 0; j < 8; j++) { const double2 t = cur[j]; cur[j] = nxt[j]; nxt[j] = t; }
+          for (int j = 0; j < 8; j++) { const double2 t = cur[j]; cur[j] = nxt[j]; nxt[j] = t; }
 #pragma unroll
-            for (int q = 0; q < 16; q++) {
-              int t = carryA[q]; carryA[q] = carryB[q]; carryB[q] = t;
-              if (MODE == MODE_COMBINE2) { t = carry2A[q]; carry2A[q] = carry2B[q]; carry2B[q] = t; }
-            }
-          }
+          for (int q = 0; q < 16; q++) { int t = carryA[q]; carryA[q] = carryB[q]; carryB[q] = t; }
         }
       }
-      if (MODE == MODE_TRACE) __syncthreads();  // xb complete before next step / copy-out
     }  // steps
 
-    if (MODE == MODE_TRACE) {
-      // copy the in-place result to dst (coalesced); split mode: this CTA's column only
-      for (int i = T; i < 2 * R * kN; i += kThreads)
-        if (!SPLIT || ((i / kN) & 1) == my_co) dst[i] = xb[i];
-    }
-    __syncthreads();  // xb / spectra reuse by the next item
+    __syncthreads();  // spectra reuse by the next item
     PHASE_TICK(6);
   }
 }

@@ -1,9 +1,9 @@
 // kernels_ext8.cuh -- external-product chains (CoordinatePrepared::product / product_inplace,
 // src/coordinate_prepared.rs:147-177) on the TWO-EXCHANGE transform of kernels_ks7.cuh, ONE ciphertext per SM.
 //
-// k_ext3 (kernels_ks3.cuh) runs its 14 transforms one after the other on 256 threads x 8 points (three
-// shared-memory exchanges each), keeps two of the six input spectra in shared memory (read back 8 times)
-// and waits one L2 round trip per 32 KiB matrix tile.  Here one CTA of 512 threads = FOUR groups of 128
+// The round-1 kernel (k_ext3, since retired) ran its 14 transforms one after the other on 256 threads x 8 points
+// (three shared-memory exchanges each), kept two of the six input spectra in shared memory (read back 8 times)
+// and waited one L2 round trip per 32 KiB matrix tile.  Here one CTA of 512 threads = FOUR groups of 128
 // threads owns the SM and one ciphertext:
 //   forward     rows rho = 2 limb + col of the input: group g transforms rows g and g + 4 (16 points per thread,
 //               passes of 4 + 4 + 3 stages, private 34 KiB exchange buffer per group, no lock);
@@ -17,7 +17,7 @@
 //               W = lo + hi 2^26 (mod 2^51): the limb-3 group STORES its contribution (+ bias), the three other
 //               contributions of the column are added with native 32-bit shared atomics (no return value, no
 //               64-bit CAS loop, order free); every sum stays below 2^28.  The digits are bit fields of (lo, hi).
-// Same integers as k_ext3 / k_vmp<MODE_EXT>; the prepared GGSWs are in the frequency order of k_prepare7.
+// Same integers as k_ext9 and the oracle's external product; the prepared GGSWs are in the frequency order of k_prepare7.
 // Shared memory 4 (pass-2 twiddles) + 4 x 34 (exchange) + 64 (words) = 204 KiB, 512 tensor-memory columns.
 #pragma once
 #include "kernels_ks7.cuh"
@@ -137,7 +137,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
         const int col = rho & 1, limb = rho >> 1;
         double2 x[16];
         if (step == 0) {
-          // the caller's limbs as they are (any int32), like k_ext3
+          // the caller's limbs as they are (any int32), like k_ext9
           const int* p = src + CT(col, limb) + t;
           asm volatile("" : "+l"(p));
 #pragma unroll

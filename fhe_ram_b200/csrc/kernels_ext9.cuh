@@ -10,7 +10,7 @@
 //             (24 chunks of 8 KiB through a cp.async ring of 7 (3) slots filled since the previous step; the rows of
 //             round one are contracted while round two is transformed), runs ONE inverse transform and stores the
 //             rounded, shifted result as the CTA's contribution slab in L2.
-// One cluster barrier per step, no distributed shared memory, no atomics.  Same integers as k_ext8 / k_ext3; the
+// One cluster barrier per step, no distributed shared memory, no atomics.  Same integers as k_ext8; the
 // prepared GGSWs are in the frequency order of k_prepare7.
 #pragma once
 #include "kernels_ks8.cuh"

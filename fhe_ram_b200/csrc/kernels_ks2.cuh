@@ -1,7 +1,7 @@
 // kernels_ks2.cuh -- tensor memory as LANE-PRIVATE scratch (tcgen05.st / tcgen05.ld, no MMA involved): what every
 // later kernel generation uses to park spectra, twiddles and (k_ks5) matrix tiles.  The digit-domain kernels this file
 // introduced in round 1 (k_ks2 / k_ext2: first two-CTAs-per-SM generation, 96 KiB + 256 tensor-memory columns per CTA)
-// were retired in round 2 (superseded by k_ks4 / k_ks7 and k_ext3 / k_ext8; same integers, DESIGN.md 3).
+// were retired in round 2 (superseded by k_ks4 / k_ks7 and k_ext8; same integers, DESIGN.md 3).
 #pragma once
 #include "kernels.cuh"
 

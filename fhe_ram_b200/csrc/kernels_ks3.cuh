@@ -1,6 +1,5 @@
 // kernels_ks3.cuh -- the integer side of a key switch / external product on 51-bit WORDS instead of per-limb digits
-// (helpers used by every later kernel), and k_ext3, the round-1 external-product kernel (kept behind FHERAM_EXT8=0 for
-// A/B timing and as a parity cross-check of k_ext8).
+// (helpers used by every later kernel).
 //
 // A normalised 3-limb coefficient (balanced base-2^17 digits a0,a1,a2 in [-2^16, 2^16)) is kept
 // on chip as the biased word
@@ -62,182 +61,13 @@ __device__ __forceinline__ unsigned long long magic_bits(double t) {
   return ((unsigned long long)(uint32_t)__double2hiint(t) << 32) | (uint32_t)__double2loint(t);
 }
 
-// ======================================================================================
-// k_ext3: k_ext2 with the padded exchange buffer of transform_pad.cuh (addresses are base + immediate
-// instead of XOR swizzles), three instead of four pass-4 twiddle columns, and digits converted with
-// one DADD instead of I2F.  Same arithmetic and results.
-// ======================================================================================
 // int32 -> double as (2^52 + 2^31 + v) - (2^52 + 2^31)
 __device__ __forceinline__ double int_f64(int v) {
   return __hiloint2double(0x43300000, (int)((uint32_t)v ^ 0x80000000u)) - 4503601774854144.0;
 }
 
-// 36 (padded exchange buffer) + 64 (two spectra) + 8 (pass-4 twiddles b4a, c4a; b4b = i b4a, c4b = e^(i pi/4) c4a)
-// + 4 (pass-3 twiddle table) = 112 KiB
-constexpr size_t kExt3Smem = (size_t)kWorkPad * sizeof(double2) + (size_t)2 * kM * sizeof(double2) +
-                             (size_t)3 * kThreads * sizeof(double2) + 16;
-// w * e^(i pi/4), with exactly the roundings the host uses to build the odd entries of tw10c
-__device__ __forceinline__ double2 mul_e8(double2 w) {
-  const double r = 0.70710678118654757;
-  return make_double2(__dmul_rn(__dadd_rn(w.x, -w.y), r), __dmul_rn(__dadd_rn(w.x, w.y), r));
-}
-
-__global__ void __launch_bounds__(kThreads, 2) k_ext3(const VmpArgs A) {
-  constexpr int NR = 6, LOUT = 4, LRES = 3, NOUT = 2 * LOUT;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  double2* work = reinterpret_cast<double2*>(smem_raw);
-  double2* rows_s = work + kWorkPad;           // spectra of rows 4 and 5
-  double2* tw4s = rows_s + 2 * kM;             // [2][256] pass-4 twiddles b4a, c4a (thread-private columns)
-  double2* tw3s = tw4s + 2 * kThreads;         // [256] pass-3 twiddle table zeta(6,B) | zeta(7,2B) | zeta(8,2k)
-  uint32_t* tmem_base_s = reinterpret_cast<uint32_t*>(tw3s + kThreads);
-
-  const int T = threadIdx.x, w = T >> 5, lane = T & 31;
-  auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
-
-  if (w == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(tmem_base_s)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  BufSync bs{smem_u32(tmem_base_s + 2), 0u};  // exchange-buffer mbarrier in the same 16-byte slot
-  if (T == 0) buf_init(bs.mbar);
-  {
-    const int B4 = 32 * w + lane;
-    tw4s[0 * kThreads + T] = __ldg(A.tw.tw9 + 2 * B4);    // zeta(9, 2 B4 + 1) = i * this one
-    tw4s[1 * kThreads + T] = __ldg(A.tw.tw10c + 2 * B4);  // zeta(10, 4 B4 + 2) = e^(i pi/4) * this one
-    tw3s[T] = __ldg(A.tw.tw6 + T);                        // tw6 | tw7c | tw8c are contiguous
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_base_s;
-  buf_release(bs);  // the buffer starts out free
-  const uint32_t tsp = tmem_base + ((uint32_t)((w & 3) * 32) << 16) + 128 * (w >> 2);  // rows 0..3
-  const int P0 = 256 * w + lane;
-  const PadAddr pa = pad_addr(work, T, w, lane);
-  // pass-3 twiddles from a 4 KiB shared table (8 distinct entries per warp, broadcast within quads):
-  // k_ext2 read them from the constant bank, where 8 distinct addresses per warp serialise in the
-  // address-divergence unit (ncu: ADU pipe 37 %)
-  auto tw3 = [&]() {
-    const int B = 8 * w + (lane >> 2);
-    return Tw4x{tw3s[B], tw3s[64 + B], tw3s[128 + 2 * B], tw3s[128 + 2 * B + 1]};
-  };
-  auto tw4 = [&]() {
-    const double2 b4a = tw4s[T], c4a = tw4s[kThreads + T];
-    return Tw4x{b4a, mul_i(b4a), c4a, mul_e8(c4a)};
-  };
-  long long phase_t0 = A.phase_cycles ? clock64() : 0;
-
-  for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
-    int* dst = A.dst + (size_t)item * A.ct_stride;
-    const int* src;
-    {
-      long idx = item;
-      if (A.src_div > 0) idx = item / A.src_div;
-      else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
-      src = A.src + idx * A.ct_stride;
-    }
-    const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
-
-    for (int step = 0; step < A.n_steps; step++) {
-      const double2* G = A.mat[step] + mat_off;
-      const int* xin = step > 0 ? dst : src;
-      PHASE_TICK(0);
-      // --------------------------- forward transforms ------------------------------
-      {
-        int nx[16];
-        auto load_row = [&](int rho, int (&v)[16]) {
-          // per-thread pointer made opaque: with a (uniform base + thread offset) split the compiler
-          // re-materialises the base in uniform registers for every access (two R2UR per load)
-          const int* p = xin + CT(rho & 1, rho >> 1) + T;
-          asm volatile("" : "+l"(p));
-#pragma unroll
-          for (int m = 0; m < 8; m++) { v[m] = p[256 * m]; v[m + 8] = p[256 * m + kM]; }
-        };
-        load_row(0, nx);
-#pragma unroll 1
-        for (int rho = 0; rho < NR; rho++) {
-          double2 x[8];
-#pragma unroll
-          for (int m = 0; m < 8; m++) x[m] = make_double2(int_f64(nx[m]), int_f64(nx[m + 8]));
-          if (rho + 1 < NR) load_row(rho + 1, nx);
-          fwd_pass1_store_p(x, pa, bs);
-          __syncthreads();
-          fwd_warp_passes_p(pa, w, tw3, tw4, x, bs);
-          if (rho < 4) {
-            const double2 lo[4] = {x[0], x[1], x[2], x[3]};
-            const double2 hi[4] = {x[4], x[5], x[6], x[7]};
-            tm_st4(tsp + 32 * rho, lo);
-            tm_st4(tsp + 32 * rho + 16, hi);
-          } else {
-#pragma unroll
-            for (int j = 0; j < 8; j++) rows_s[(size_t)(rho - 4) * kM + P0 + 32 * j] = x[j];
-          }
-        }
-        tm_wait_st();
-      }
-      PHASE_TICK(2);
-
-      // --------------- contraction + inverse transform + epilogue ------------------
-#pragma unroll 1
-      for (int co = 0; co < 2; co++) {
-        int carry[16];
-#pragma unroll
-        for (int q = 0; q < 16; q++) carry[q] = 0;
-#pragma unroll 1
-        for (int l = LOUT - 1; l >= 0; l--) {
-          const int o = co * LOUT + l;
-          double2 cur[8];
-#pragma unroll
-          for (int j = 0; j < 8; j++) cur[j] = make_double2(0.0, 0.0);
-#pragma unroll 1
-          for (int rho = 0; rho < NR; rho++) {
-            const double2* gp = G + ((size_t)rho * NOUT + o) * kM + P0;
-            double2 g[8];
-#pragma unroll
-            for (int j = 0; j < 8; j++) g[j] = ldg_pinned(gp + 32 * j);
-#pragma unroll
-            for (int h = 0; h < 2; h++) {
-              double2 a[4];
-              if (rho < 4) {
-                tm_ld4(tsp + 32 * rho + 16 * h, a);
-              } else {
-#pragma unroll
-                for (int j = 0; j < 4; j++) a[j] = rows_s[(size_t)(rho - 4) * kM + P0 + 32 * (4 * h + j)];
-              }
-#pragma unroll
-              for (int j = 0; j < 4; j++) {
-                cur[4 * h + j].x = fma(a[j].x, g[4 * h + j].x, fma(-a[j].y, g[4 * h + j].y, cur[4 * h + j].x));
-                cur[4 * h + j].y = fma(a[j].x, g[4 * h + j].y, fma(a[j].y, g[4 * h + j].x, cur[4 * h + j].y));
-              }
-            }
-          }
-          PHASE_TICK(3);
-          inv_transform_p(cur, pa, w, tw3, tw4, bs);
-          PHASE_TICK(4);
-          int* dp = dst + CT(co, l < LRES ? l : 0) + T;
-          asm volatile("" : "+l"(dp));
-#pragma unroll
-          for (int q = 0; q < 16; q++) {
-            const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-            const long long t = __double2ll_rn(v) + (long long)carry[q];
-            const int c = (int)((t + 65536) >> kK);
-            const int dg = (int)t - (c << kK);
-            carry[q] = c;
-            if (l < LRES) dp[256 * (q & 7) + (q >> 3) * kM] = dg;
-          }
-          PHASE_TICK(5);
-        }
-      }
-    }  // steps
-    __syncthreads();
-    PHASE_TICK(6);
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (w == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem_base) : "memory");
-}
-
 // (k_ks3, the first word-domain key-switch kernel -- register accumulators, one tile in flight -- was retired in round 2:
-// k_ks4 does the same with in-place word accumulation and two tiles in flight, k_ks7 with the two-exchange transform.)
+// k_ks4 does the same with in-place word accumulation and two tiles in flight, k_ks7 with the two-exchange transform.
+// k_ext3, the round-1 external product on the padded transform, was retired after k_ext8 / k_ext9 took every launch.)
 
 }  // namespace fheram

@@ -4,6 +4,7 @@
 // and the first tile of every output is fetched during the previous inverse transform.
 // (tools/ablate: without matrix loads k_ks3 runs 76.8 K -> 58.1 K cycles per operation; the loads
 // were three exposed L2 round trips per output.)  Same integers as k_ks3 / k_ks2 / k_vmp.
+// Two-sided combine of GLWEPacker only: the wide launches of the packer tree (the trace kernels took its traces).
 #pragma once
 #include "kernels_ks3.cuh"
 
@@ -11,9 +12,7 @@ namespace fheram {
 
 constexpr size_t kKs4Smem = (size_t)kWorkPad * sizeof(double2) + (size_t)2 * kN * sizeof(long long) + 16;
 
-template <int MODE>
 __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
-  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2, "key-switch modes only");
   constexpr int R = 3, LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* work = reinterpret_cast<double2*>(smem_raw);  // padded exchange buffer (transform_pad.cuh)
@@ -49,44 +48,18 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
   const PadAddr pa = pad_addr(work, T, w, lane);
   auto tw3 = [&]() { double2 t[4]; tm_ld4(ttw, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
   auto tw4 = [&]() { double2 t[4]; tm_ld4(ttw + 16, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
-  const double sgn_d = (MODE == MODE_TRACE && A.sign < 0) ? -1.0 : 1.0;
-  const uint32_t sgn_bit = (MODE == MODE_TRACE && A.sign < 0) ? 1u : 0u;
   long long phase_t0 = A.phase_cycles ? clock64() : 0;
 
   for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
-    // COMBINE2: words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
+    // words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
-    const int* src;
-    {
-      long idx = item;
-      if (MODE == MODE_COMBINE2) idx = 2L * item;
-      else if (A.src_div > 0) idx = item / A.src_div;
-      else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
-      src = A.src + idx * A.ct_stride;
-    }
+    const int* src = A.src + 2L * item * A.ct_stride;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     // ------------------------------ prologue (once per item) ---------------------------
-    if (MODE == MODE_TRACE) {
-      // x = rsh1(src * X^rk)
-      int rk = A.rot_const;
-      if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
-      rk &= (2 * kN - 1);
-#pragma unroll 4
-      for (int m = 0; m < 16; m++) {
-        const int i = T + 256 * m;
-        bool neg;
-        const int j = rot_index(i, 2 * kN - rk, neg);
-#pragma unroll
-        for (int col = 0; col < 2; col++) {
-          long long X = limbs_value(src[CT(col, 0) + j], src[CT(col, 1) + j], src[CT(col, 2) + j]);
-          if (neg) X = -X;
-          xp[col * kN + i] = rsh1_word(X);
-        }
-      }
-    } else {
+    {
       // a1 = a X^-t;  D = rsh1(a1 - b) -> xp;  S = rsh1(a1 + b) -> sw
       const int* a = src;
       const int* b = src + A.ct_stride;
@@ -193,15 +166,14 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
         const int co = 1 - cc;
         unsigned long long* xc = xp + co * kN;
         if (co == 0) {
-          // accumulator init: x_body + s phi_g(x_body)   (COMBINE2: sigma (D_body[u] - bias))
+          // accumulator init: sigma (D_body[u] - bias)
           unsigned long long v0[16];
 #pragma unroll
           for (int q = 0; q < 16; q++) {
-            const int i = T + 256 * (q & 7) + (q >> 3) * kM;
             const int e = (e0 + (q & 7) * d1 + (q >> 3) * d2) & (2 * kN - 1);
             const unsigned long long b = xp[e & (kN - 1)] - kBias51;
-            const bool ng = (((sgn >> q) & 1u) ^ sgn_bit) != 0;
-            v0[q] = (ng ? 0ull - b : b) + (MODE == MODE_TRACE ? xp[i] : 0ull);
+            const bool ng = ((sgn >> q) & 1u) != 0;
+            v0[q] = ng ? 0ull - b : b;
           }
           __syncthreads();  // every gather of the old body column precedes its stores
 #pragma unroll
@@ -257,18 +229,15 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
           PHASE_TICK(4);
           // cur[m] = phi_g(vmp)[T + 256 m] (+ i * [.. + 2048]); round and add into the word
           if (l == 3) {
-            // floor((s r + 2^16) / 2^17) with s the sign frame of the carry chain: the uniform
-            // sign of the trace step, or (COMBINE2) the per-position automorphism sign, for which
-            // floor((-r + 2^16) / 2^17) = -floor((r + 2^16 - 1) / 2^17)
+            // floor((s r + 2^16) / 2^17) with s the sign frame of the carry chain, the per-position
+            // automorphism sign, for which floor((-r + 2^16) / 2^17) = -floor((r + 2^16 - 1) / 2^17)
 #pragma unroll
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
               const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-              double t;
-              if (MODE == MODE_TRACE) t = fma(v, sgn_d, kMagic52 + 65536.0);
-              else t = v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
+              const double t = v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
               const int c3 = (int)__funnelshift_r((uint32_t)__double2loint(t), (uint32_t)__double2hiint(t), 17);
-              if (MODE == MODE_COMBINE2 && co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
+              if (co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
               else xc[i] += (unsigned long long)(long long)c3;
             }
           } else if (l == 2) {
@@ -276,14 +245,14 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
               const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-              xc[i] += magic_bits(fma(v, sgn_d, kMagic52));
+              xc[i] += magic_bits(v + kMagic52);
             }
           } else if (l == 1) {
 #pragma unroll
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
               const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-              xc[i] += magic_bits(fma(v, sgn_d, kMagic52)) << 17;
+              xc[i] += magic_bits(v + kMagic52) << 17;
             }
           } else {
             // last limb: finish the word
@@ -291,23 +260,17 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
               const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-              const double t = fma(v, sgn_d, kMagic52);
+              const double t = v + kMagic52;
               const unsigned long long W = xc[i] + ((unsigned long long)((uint32_t)__double2loint(t) << 2) << 32);
-              if (MODE == MODE_TRACE) {
-                // x <- x + s phi_g(KS(x)):  word = x + s (R + phi(x_body)) + c3
-                const unsigned long long U = W & kMask51;
-                xc[i] = last ? U : rsh1_canon(U);
-              } else {
-                // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:
-                //   word = S - (R + k3) - sigma (D_body[u] - bias)
-                const unsigned long long U = (sw[co * kN + i] - W) & kMask51;
-                bool rneg;
-                const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
+              // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:
+              //   word = S - (R + k3) - sigma (D_body[u] - bias)
+              const unsigned long long U = (sw[co * kN + i] - W) & kMask51;
+              bool rneg;
+              const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
 #pragma unroll
-                for (int ll = 0; ll < 3; ll++) {
-                  const int dg = word_digit(U, ll);
-                  dst[CT(co, ll) + dd] = rneg ? -dg : dg;
-                }
+              for (int ll = 0; ll < 3; ll++) {
+                const int dg = word_digit(U, ll);
+                dst[CT(co, ll) + dd] = rneg ? -dg : dg;
               }
             }
           }
@@ -316,20 +279,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
       }
     }  // steps
 
-    if (MODE == MODE_TRACE) {
-      // own positions only: no barrier needed before reading the words back
-#pragma unroll 4
-      for (int m = 0; m < 16; m++) {
-        const int i = T + 256 * m;
-#pragma unroll
-        for (int col = 0; col < 2; col++) {
-          const unsigned long long U = xp[col * kN + i];
-          dst[CT(col, 0) + i] = word_digit(U, 0);
-          dst[CT(col, 1) + i] = word_digit(U, 1);
-          dst[CT(col, 2) + i] = word_digit(U, 2);
-        }
-      }
-    }
     __syncthreads();  // xp reuse by the next item
     PHASE_TICK(6);
   }

@@ -189,12 +189,9 @@ __global__ void __launch_bounds__(256, 2) k_prepare7(const Prep7Args P) {
 }
 
 // ======================================================================================
-// k_ks7<MODE_TRACE>: chain of { rsh 1; x <- x +/- phi_g(KS(x)) }  (trace / one-sided packer levels)
-// k_ks7<MODE_COMBINE2>: GLWEPacker two-sided combine
+// k_ks7: chain of { rsh 1; x <- x +/- phi_g(KS(x)) }  (trace / one-sided packer levels)
 // ======================================================================================
-template <int MODE>
 __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* __restrict__ tw16) {
-  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2, "key-switch modes only");
   constexpr int LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* tw2 = reinterpret_cast<double2*>(smem_raw);
@@ -239,59 +236,23 @@ __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* 
     return w;
   };
   const T16 tc{buf, tw2, slot + 1, t, g};
-  const double sgn_d = (MODE == MODE_TRACE && A.sign < 0) ? -1.0 : 1.0;
-  const uint32_t sgn_bit = (MODE == MODE_TRACE && A.sign < 0) ? 1u : 0u;
+  const double sgn_d = A.sign < 0 ? -1.0 : 1.0;
+  const uint32_t sgn_bit = A.sign < 0 ? 1u : 0u;
   const int co = g;                         // output column of this group
   unsigned long long* xc = xp + co * kN;    // its words
   long long phase_t0 = A.phase_cycles ? clock64() : 0;
 
   for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
-    // COMBINE2: words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
-    unsigned long long* sw = A.scratch
-        ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
     const int* src;
     {
       long idx = item;
-      if (MODE == MODE_COMBINE2) idx = 2L * item;
-      else if (A.src_div > 0) idx = item / A.src_div;
+      if (A.src_div > 0) idx = item / A.src_div;
       else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
       src = A.src + idx * A.ct_stride;
     }
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
-    if (MODE == MODE_COMBINE2) {
-      // ------------- prologue: a1 = a X^-t;  D = rsh1(a1 - b) -> xp;  S = rsh1(a1 + b) -> sw -------------
-      const int* a = src;
-      const int* b = src + A.ct_stride;
-      const int tt = A.rot_const;
-#pragma unroll 1
-      for (int mc = 0; mc < 16; mc += 4) {
-        int av[4][2][3], bv[4][2][3];
-        bool ng[4];
-#pragma unroll
-        for (int mm = 0; mm < 4; mm++) {
-          const int i = tid + 256 * (mc + mm);
-          const int j = rot_index(i, tt, ng[mm]);  // (a X^-t)[i] = +/- a[(i + t) mod 2N]
-#pragma unroll
-          for (int col = 0; col < 2; col++)
-#pragma unroll
-            for (int l = 0; l < 3; l++) { av[mm][col][l] = a[CT(col, l) + j]; bv[mm][col][l] = b[CT(col, l) + i]; }
-        }
-#pragma unroll
-        for (int mm = 0; mm < 4; mm++) {
-          const int i = tid + 256 * (mc + mm);
-#pragma unroll
-          for (int col = 0; col < 2; col++) {
-            long long Xa = limbs_value(av[mm][col][0], av[mm][col][1], av[mm][col][2]);
-            if (ng[mm]) Xa = -Xa;
-            const long long Xb = limbs_value(bv[mm][col][0], bv[mm][col][1], bv[mm][col][2]);
-            xp[col * kN + i] = rsh1_word(Xa - Xb);
-            sw[col * kN + i] = rsh1_word(Xa + Xb);
-          }
-        }
-      }
-    } else
     // ------------------------------ prologue: x = rsh1(src * X^rk) ------------------------------
     {
       int rk = A.rot_const;
@@ -360,14 +321,14 @@ __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* 
           const int ea = (e0 + m * d1) & (2 * kN - 1);
           const unsigned long long ba = xp[ea & (kN - 1)] - kBias51;
           const bool na = ((ea >= kN ? 1u : 0u) ^ sgn_bit) != 0;
-          v0[m] = (na ? 0ull - ba : ba) + (MODE == MODE_TRACE ? xp[t + 128 * m] : 0ull);
+          v0[m] = (na ? 0ull - ba : ba) + xp[t + 128 * m];
         }
 #pragma unroll
         for (int m = 0; m < 16; m++) {
           const int eb = (e0 + m * d1 + d2) & (2 * kN - 1);
           const unsigned long long bb = xp[eb & (kN - 1)] - kBias51;
           const bool nb = ((eb >= kN ? 1u : 0u) ^ sgn_bit) != 0;
-          v1[m] = (nb ? 0ull - bb : bb) + (MODE == MODE_TRACE ? xp[t + 128 * m + kM] : 0ull);
+          v1[m] = (nb ? 0ull - bb : bb) + xp[t + 128 * m + kM];
         }
         gsync128(1);  // every gather of the old body column precedes its stores
 #pragma unroll
@@ -412,26 +373,13 @@ __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* 
         PHASE_TICK(4);
         // cur[m] = phi_g(vmp)[t + 128 m] + i phi_g(vmp)[t + 128 m + 2048]: round and add into the words
         if (l == 3) {
-          // COMBINE2: the carry chain runs in the pre-automorphism sign frame of each position (see k_ks3)
-          unsigned sgn = 0;
-          if (MODE == MODE_COMBINE2) {
-#pragma unroll
-            for (int m = 0; m < 16; m++) {
-              const int ea = (e0 + m * d1) & (2 * kN - 1);
-              const int eb = (ea + d2) & (2 * kN - 1);
-              sgn |= (ea >= kN ? 1u : 0u) << m;
-              sgn |= (eb >= kN ? 1u : 0u) << (16 + m);
-            }
-          }
 #pragma unroll
           for (int q = 0; q < 32; q++) {
             const int i = t + 128 * (q & 15) + (q >> 4) * kM;
             const double v = (q < 16) ? cur[q & 15].x : cur[q & 15].y;
-            const double tt = MODE == MODE_TRACE ? fma(v, sgn_d, kMagic52 + 65536.0)
-                                                 : v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
+            const double tt = fma(v, sgn_d, kMagic52 + 65536.0);
             const int c3 = (int)__funnelshift_r((uint32_t)__double2loint(tt), (uint32_t)__double2hiint(tt), 17);
-            if (MODE == MODE_COMBINE2 && co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
-            else xc[i] += (unsigned long long)(long long)c3;
+            xc[i] += (unsigned long long)(long long)c3;
           }
         } else if (l == 2) {
 #pragma unroll
@@ -454,20 +402,8 @@ __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* 
             const double v = (q < 16) ? cur[q & 15].x : cur[q & 15].y;
             const double tt = fma(v, sgn_d, kMagic52);
             const unsigned long long W = xc[i] + ((unsigned long long)((uint32_t)__double2loint(tt) << 2) << 32);
-            if (MODE == MODE_TRACE) {
-              const unsigned long long U = W & kMask51;
-              xc[i] = last ? U : rsh1_canon(U);
-            } else {
-              // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:  word = S - (R + k3) [- sigma (D_body[u] - bias)]
-              const unsigned long long U = (sw[co * kN + i] - W) & kMask51;
-              bool rneg;
-              const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
-#pragma unroll
-              for (int ll = 0; ll < 3; ll++) {
-                const int dg = word_digit(U, ll);
-                dst[CT(co, ll) + dd] = rneg ? -dg : dg;
-              }
-            }
+            const unsigned long long U = W & kMask51;
+            xc[i] = last ? U : rsh1_canon(U);
           }
         }
         PHASE_TICK(5);
@@ -478,17 +414,15 @@ __global__ void __launch_bounds__(256, 2) k_ks7(const VmpArgs A, const double2* 
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     }  // steps
 
-    if (MODE == MODE_TRACE) {
 #pragma unroll 4
-      for (int m = 0; m < 16; m++) {
-        const int i = tid + 256 * m;
+    for (int m = 0; m < 16; m++) {
+      const int i = tid + 256 * m;
 #pragma unroll
-        for (int col = 0; col < 2; col++) {
-          const unsigned long long U = xp[col * kN + i];
-          dst[CT(col, 0) + i] = word_digit(U, 0);
-          dst[CT(col, 1) + i] = word_digit(U, 1);
-          dst[CT(col, 2) + i] = word_digit(U, 2);
-        }
+      for (int col = 0; col < 2; col++) {
+        const unsigned long long U = xp[col * kN + i];
+        dst[CT(col, 0) + i] = word_digit(U, 0);
+        dst[CT(col, 1) + i] = word_digit(U, 1);
+        dst[CT(col, 2) + i] = word_digit(U, 2);
       }
     }
     __syncthreads();  // xp reuse by the next item

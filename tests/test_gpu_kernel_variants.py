@@ -1,12 +1,10 @@
 """Every kernel generation behind the same C ABI must give the same limbs as the oracle.
 
-The library picks a kernel per launch from the launch width (external products: k_ext8 always; key switches: narrow
-k_ks6 / k_ks5, wide k_ks7 / k_ks4; the default selection is what test_gpu_parity.py itself runs, and the wide kernels
-are checked at BASELINE sizes in test_gpu_baseline_sizes.py).  The small parity cases of test_gpu_parity.py only
-produce narrow launches, so
-each variant is forced through the whole limb-level parity set (external product, chains, trace,
-packer, read / read_prepare_write / write at four parameter sets, batched, sharded) in a
-subprocess: the selection knobs are read once per process.
+The library picks a kernel per launch from the launch width (DESIGN.md 3.4; the default selection is what
+test_gpu_parity.py itself runs, test_gpu_launch_widths.py pins the rule, and the wide kernels are checked at BASELINE
+sizes in test_gpu_baseline_sizes.py).  The small parity cases of test_gpu_parity.py only produce narrow launches, so
+each kernel is forced with FHERAM_KERNEL through the whole limb-level parity set (external product, chains, trace,
+packer, read / read_prepare_write / write at four parameter sets, batched, sharded) in a subprocess.
 """
 import os
 import subprocess
@@ -23,43 +21,47 @@ SELECT = ("test_external_product_matches_oracle or test_external_product_adversa
           "test_read_rpw_write_bit_exact or test_batched_reads_equal_single_reads or "
           "test_sharded_stages_on_one_gpu")
 
-VARIANTS = {
-    # word-domain key switch with in-place accumulation and two tiles in flight (k_ks4) for every key-switch launch
-    "ks4": {"FHERAM_KS3": "2", "FHERAM_KS5": "0", "FHERAM_KS7": "0", "FHERAM_KS8": "0"},
+# FHERAM_KERNEL values
+VARIANTS = (
+    # word-domain key switch with in-place accumulation and two tiles in flight (k_ks4) for every two-sided combine
+    "ks4",
     # 16-point-per-thread transform with two exchanges, two polynomials per CTA (k_ks7) for every trace chain
-    "ks7": {"FHERAM_KS7": "2", "FHERAM_KS8": "0"},
-    # the same kernel for the packer's two-sided combine as well (k_ks7<MODE_COMBINE2>)
-    "ks7c": {"FHERAM_KS7": "2", "FHERAM_KS7C": "2", "FHERAM_KS8": "0"},
+    "ks7",
     # one operation per SM, 512 threads, tiles parked in tensor memory (k_ks5), trace and combine
-    "ks5": {"FHERAM_KS5": "2", "FHERAM_KS6": "0", "FHERAM_KS7": "0", "FHERAM_KS8": "0"},
-    # the two-SM cluster kernel (k_ks6) for every narrow trace chain (the default hands the narrowest ones to k_ks8)
-    "ks6": {"FHERAM_KS8": "0"},
+    "ks5",
+    # the two-SM cluster kernel (k_ks6) for every narrow trace / combine (the default hands the narrowest ones to k_ks8)
+    "ks6",
     # one key-switch chain per cluster of eight (or, beyond one wave of those, four) SMs, contributions exchanged
     # through L2 (k_ks8), for every trace / combine launch
-    "ks8": {"FHERAM_KS8": "2"},
+    "ks8",
     # the four-SM cluster variant of k_ks8 (two output polynomials per CTA) for every trace / combine launch
-    "ks8c4": {"FHERAM_KS8": "3"},
-    # column-split k_vmp for every narrow key switch (two CTAs per operation, one launch per chain step)
-    "vmp_split": {"FHERAM_KS3": "0", "FHERAM_KS5": "0", "FHERAM_KS7": "0", "FHERAM_KS8": "0"},
+    "ks8c4",
     # one-SM-per-ciphertext external product (k_ext8) for the narrow launches too (the default hands them to k_ext9)
-    "ext8": {"FHERAM_EXT9": "0"},
+    "ext8",
     # one external-product chain per cluster of eight / four SMs (k_ext9) for every launch
-    "ext9": {"FHERAM_EXT9": "2"},
-    "ext9c4": {"FHERAM_EXT9": "3"},
-    # round-1 external-product kernels (k_ext3 forced for every launch, GGSWs prepared in its frequency order)
-    "ext3": {"FHERAM_EXT8": "0", "FHERAM_KS3": "2", "FHERAM_KS8": "0"},
-    # round-1 narrow external product (column-split k_vmp<EXT>) and the single-CTA k_vmp without column split
-    "ext_vmp": {"FHERAM_EXT8": "0", "FHERAM_KS3": "0", "FHERAM_KS5": "0", "FHERAM_KS7": "0", "FHERAM_SPLIT": "0",
-                "FHERAM_KS8": "0"},
-}
+    "ext9",
+    "ext9c4",
+)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", sorted(VARIANTS))
 def test_kernel_variant_is_bit_exact(built, name):
     env = dict(os.environ)
-    env.update(VARIANTS[name])
+    env["FHERAM_KERNEL"] = name
     r = subprocess.run([sys.executable, "-m", "pytest", str(ROOT / "tests" / "test_gpu_parity.py"), "-m", "gpu",
                         "-x", "-q", "-k", SELECT], cwd=ROOT, env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, f"variant {name} {VARIANTS[name]}:\n{r.stdout[-3000:]}\n{r.stderr[-1000:]}"
+    assert r.returncode == 0, f"FHERAM_KERNEL={name}:\n{r.stdout[-3000:]}\n{r.stderr[-1000:]}"
     assert " passed" in r.stdout
+
+
+@pytest.mark.parametrize("spec", ["bogus", "ks5,ks6", "ext8,ext9", "ks6,"])
+def test_unknown_kernel_name_fails_context_creation(built, monkeypatch, spec):
+    """FHERAM_KERNEL is read by every context creation: an unknown name, or two of one class, is an error that lists
+    the valid names (checked before the device, so this runs anywhere)."""
+    import fhe_ram_b200 as fr
+    monkeypatch.setenv("FHERAM_KERNEL", spec)
+    with pytest.raises(fr.FheRamError) as e:
+        fr.Parameters.new().module()
+    assert e.value.code == -1, str(e.value)
+    assert f"FHERAM_KERNEL={spec}" in str(e.value) and "ext9c4" in str(e.value) and "ks8c4" in str(e.value)

@@ -298,8 +298,8 @@ def test_full_size_2pow18_properties(scenario, gpu_keys):
 
 
 def test_wide_kernels_repeatable_and_equal_to_narrow(scenario, gpu_keys):
-    """2^18 x 4 B: a batch (wide launches: k_ext3 / k_ks4, two CTAs per SM, split barriers, in-place word
-    accumulation) must give, limb for limb, what single reads (narrow launches: k_vmp split / k_ks5) give, and the
+    """2^18 x 4 B: a batch (wide launches: k_ext8 / k_ks7 / k_ks4, in-place word accumulation) must give, limb
+    for limb, what single reads (narrow launches: k_ext9 / k_ks8 / k_ks6 / k_ks5) give, and the
     same limbs on every repetition (compute-sanitizer is not available on the GPU pool: races would show up here)."""
     s = scenario(1 << 18, 4, 9)
     fr, p = s.fr, s.params

@@ -17,7 +17,7 @@ ram.encrypt_sk_gpu(data, sk, fr.Source(1), fr.Source(2))            # k_noise_sa
 B = 64
 idxs = np.arange(B, dtype=np.uint32) * 4001 + 7
 addrs = fr.Address.encrypt_sk_gpu(p, idxs, sk, [fr.Source(100 + i) for i in range(B)], [fr.Source(300 + i) for i in range(B)])
-ram.read_batch_device(addrs, keys)                                  # wide: k_ext8, k_ks7, k_ks4<COMBINE2>; narrow tails
+ram.read_batch_device(addrs, keys)                                  # wide: k_ext8, k_ks7, k_ks4; narrow tails
 limbs = addrs.download_raw().reshape(B, -1)
 ram.read_batch_host_p17(api.pack17(limbs[:16]), 16, keys)           # k_unpack17 (+ the pipeline)
 ram.read_batch_host(limbs[:16], 16, keys)                           # k_i64_to_i32, k_i32_to_i64

@@ -1,7 +1,7 @@
 """Development loop of the external-product kernel (run on the B200 box):
   parity of a 4-step coordinate chain against the CPU oracle on random + extreme inputs,
   then device time of BASELINE config 2 (4096 x 1) and of a 4-step chain over 4096 ciphertexts.
-  FHERAM_EXT8=0 selects the round-1 kernels (k_ext3 / split k_vmp) for the same run."""
+  FHERAM_KERNEL=ext8 / ext9 / ext9c4 forces one external-product kernel for the same run."""
 import json
 import os
 import sys
@@ -22,7 +22,7 @@ def main():
     params = fr.Parameters.readme()
     rng = np.random.default_rng(7)
     L, GL = params.glwe_len(), params.ggsw_len()
-    out = {"ext8": os.environ.get("FHERAM_EXT8", "1")}
+    out = {"kernel": os.environ.get("FHERAM_KERNEL", "")}
     if "--no-parity" not in sys.argv:
         orc = Oracle(backend="fft64", max_addr=1 << 18, word_size=4, k_pt=9)
         cts = rng.integers(-(1 << 16), 1 << 16, size=(5, L), dtype=np.int64)

@@ -1,5 +1,5 @@
 """Device time of the narrow launch shapes of a RAM sharded over 8 GPUs (32 ciphertexts per rank) and of the tail of a read
-(4 ciphertexts), under the current kernel selection (FHERAM_KS8 / FHERAM_EXT9 = 0 give the one- and two-SM kernels)."""
+(4 ciphertexts), under the current kernel selection (FHERAM_KERNEL=ks6,ext8 gives the one- and two-SM kernels)."""
 import json, os, sys
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
@@ -14,7 +14,7 @@ keys = fr.EvaluationKeysPrepared.alloc(p).prepare(evk)
 rng = np.random.default_rng(0)
 L, GL = p.glwe_len(), p.ggsw_len()
 ggsws = rng.integers(-(1 << 16), 1 << 16, size=4 * GL, dtype=np.int64)
-out = {"ks8": os.environ.get("FHERAM_KS8", "1"), "ext9": os.environ.get("FHERAM_EXT9", "1")}
+out = {"kernel": os.environ.get("FHERAM_KERNEL", "")}
 for n in (4, 16, 32, 64):
     cts = rng.integers(-(1 << 16), 1 << 16, size=(n, L), dtype=np.int64)
     api.glwe_trace(p, keys, cts); api.coordinate_product(p, cts, ggsws, 4)
