@@ -6,5 +6,5 @@ include/fheram.h), cpp/ (the compiled-language mirror of the reference's Rust AP
 """
 from .api import (  # noqa: F401
     Address, EvaluationKeys, EvaluationKeysPrepared, FheRamError, GLWESecret, Parameters, Ram,
-    Source, cast_u8_to_signed, decrypt_glwe, encrypt_glwe, gen_keys,
+    Source, cast_u8_to_signed, decrypt_glwe, decrypt_ram, decrypt_words_device, encrypt_glwe, gen_keys,
 )

@@ -142,6 +142,9 @@ SIGNATURES = {
     "fheram_debug_encrypt_stats": (C.c_int, [_V, C.POINTER(C.c_uint64)]),
     "fheram_address_encrypt_sk": (C.c_int, [_V, C.c_int, C.c_int, C.POINTER(C.c_uint32), _P64,
                                             C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int]),
+    "fheram_decrypt_ram": (C.c_int, [_PP, _P64, _P64, C.POINTER(C.c_int16), _P64]),
+    "fheram_ram_decrypt_sk": (C.c_int, [_V, _P64, C.POINTER(C.c_int16), _P64]),
+    "fheram_decrypt_words_device": (C.c_int, [_V, _V, C.c_int, _P64, C.POINTER(C.c_int16), _P64]),
 }
 
 _lib = None
@@ -607,6 +610,15 @@ class Ram:
             raise FheRamError(-1, f"invalid data: data.len()/ram_chunks={data.size // ws} != max_addr={p.max_addr()}")
         _check(lib().fheram_ram_encrypt_sk(self.h, data.ctypes.data_as(_PU8), _p(sk.data), source_xa.h, source_xe.h))
 
+    def decrypt_sk(self, sk: GLWESecret, values=None, err=None):
+        """Every byte of the resident RAM, decrypted on the device: (values, err), both [max_addr][word_size]
+        (int16 / int64; `decrypt_ram` on `store()`, bit for bit).  A sharded RAM fills the entries of its own
+        polynomials and leaves the rest of `values` / `err` (zeros when not passed) as they are."""
+        values, err = _dec_out(self.params, values, err)
+        _check(lib().fheram_ram_decrypt_sk(self.h, _p(_sk_limbs(sk)), values.ctypes.data_as(C.POINTER(C.c_int16)),
+                                           _p(err)))
+        return values, err
+
     def load(self, cts: np.ndarray):
         _check(lib().fheram_ram_load(self.h, _p(np.ascontiguousarray(cts, dtype=np.int64))))
 
@@ -718,6 +730,42 @@ def decrypt_glwe(params: Parameters, ct: np.ndarray, want: int, sk: GLWESecret):
     ct = np.ascontiguousarray(ct, dtype=np.int64)
     _check(lib().fheram_decrypt_word(C.byref(params.c), _p(ct), _p(sk.data), int(want), C.byref(v), C.byref(noise)))
     return int(v.value), float(noise.value)
+
+
+def _sk_limbs(sk) -> np.ndarray:
+    return np.ascontiguousarray(sk.data if isinstance(sk, GLWESecret) else sk, dtype=np.int64)
+
+
+def _dec_out(params: Parameters, values, err):
+    shape = (params.max_addr(), params.word_size())
+    values = np.zeros(shape, dtype=np.int16) if values is None else values
+    err = np.zeros(shape, dtype=np.int64) if err is None else err
+    assert values.dtype == np.int16 and values.shape == shape and values.flags.c_contiguous
+    assert err.dtype == np.int64 and err.shape == shape and err.flags.c_contiguous
+    return values, err
+
+
+def decrypt_ram(params: Parameters, cts: np.ndarray, sk):
+    """Every byte of a RAM in `Ram.encrypt_sk` / `Ram.store` layout, decrypted on the CPU (all host threads):
+    (values, err), both [max_addr][word_size].  value = the byte as cast_u8_to_signed(b, min(8, k_pt)) reads it;
+    err = the exact phase error at precision k_ct (log2|err| - k_ct is decrypt_glwe's noise)."""
+    cts = np.ascontiguousarray(cts, dtype=np.int64).reshape(-1)
+    if cts.size != params.word_size() * params.n_glwe() * params.glwe_len():
+        raise FheRamError(-1, "cts is not a whole RAM ([word_size][n_glwe] GLWE)")
+    values, err = _dec_out(params, None, None)
+    _check(lib().fheram_decrypt_ram(C.byref(params.c), _p(cts), _p(_sk_limbs(sk)),
+                                    values.ctypes.data_as(C.POINTER(C.c_int16)), _p(err)))
+    return values, err
+
+
+def decrypt_words_device(params: Parameters, d_ptr: int, n: int, sk):
+    """Coefficient 0 of n device-resident GLWE(k_ct) (int32 [n][limb][col][N], e.g. `Ram.read_batch_device`'s arena
+    with n = reads x word_size), decrypted on the device: (values int16 [n], err int64 [n])."""
+    values = np.zeros(n, dtype=np.int16)
+    err = np.zeros(n, dtype=np.int64)
+    _check(lib().fheram_decrypt_words_device(params.module(), C.c_void_p(int(d_ptr)), int(n), _p(_sk_limbs(sk)),
+                                             values.ctypes.data_as(C.POINTER(C.c_int16)), _p(err)))
+    return values, err
 
 
 # ---- op-level entry points (kernel parity tests, BASELINE.json config 2) ----------------

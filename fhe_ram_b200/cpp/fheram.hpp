@@ -170,6 +170,13 @@ class Ram {  // src/ram.rs:25-29
     for (auto& g : w) flat.insert(flat.end(), g.begin(), g.end());
     check(fheram_ram_write(h_, flat.data(), a.device(), k.raw()));
   }
+  // every byte of the resident RAM decrypted on the device: values / err are [max_addr][word_size] row-major (byte i of
+  // word j at j * word_size + i), the numbers of fheram_decrypt_ram on the stored RAM, bit for bit
+  void decrypt_sk(const GLWESecret& sk, std::vector<int16_t>& values, std::vector<int64_t>& err) {
+    values.assign(p_.max_addr() * p_.word_size(), 0);
+    err.assign(values.size(), 0);
+    check(fheram_ram_decrypt_sk(h_, sk.data.data(), values.data(), err.data()));
+  }
 
  private:
   std::vector<GLWE> split(const std::vector<int64_t>& o) {
@@ -180,5 +187,14 @@ class Ram {  // src/ram.rs:25-29
   Parameters& p_;
   fheram_ram* h_ = nullptr;
 };
+
+// coefficient 0 of n device-resident GLWE(k_ct) (int32 [n][limb][col][N], e.g. a batched read's result arena),
+// decrypted on the device
+inline void decrypt_words_device(Parameters& p, const int32_t* d_glwe, int n, const GLWESecret& sk,
+                                 std::vector<int16_t>& values, std::vector<int64_t>& err) {
+  values.assign((size_t)n, 0);
+  err.assign((size_t)n, 0);
+  check(fheram_decrypt_words_device(p.module(), d_glwe, n, sk.data.data(), values.data(), err.data()));
+}
 
 }  // namespace fheram

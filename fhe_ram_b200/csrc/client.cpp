@@ -1,5 +1,5 @@
 // client.cpp -- client side of the drop-in API (CPU): secret / evaluation-key generation,
-// RAM / address / word encryption and word decryption.  These are the calls of
+// RAM / address / word encryption, and RAM and word decryption.  These are the calls of
 // examples/fhe-ram.rs:34-95,179-237 that run once per key / RAM / address, outside the
 // homomorphic hot path (SURVEY.md 8f ranks moving them to the GPU as the next step).
 //
@@ -16,6 +16,7 @@
 #include <cstdint>
 #include <cstdlib>
 #include <cstring>
+#include <thread>
 #include <vector>
 
 #include "../../include/fheram.h"
@@ -436,15 +437,14 @@ extern "C" int fheram_encrypt_word(const fheram_params* p, uint8_t value, const 
   return 0;
 }
 
-extern "C" int fheram_decrypt_word(const fheram_params* p, const int64_t* glwe, const int64_t* sk,
-                                   int64_t want, int64_t* value, double* noise) {
-  if (check(p) || !glwe || !sk || !value || !noise) return FHERAM_ERR_INVALID;
-  const Dims d = dims(p);
-  Ring R(d.log_n);
-  std::vector<cd> s_spec, spec, prod;
-  R.forward(sk, s_spec);
-  const int n = d.n, S = d.size_ct;
-  std::vector<i64> big((size_t)S * n), tmp(n), pt((size_t)S * n);
+namespace {
+// pt = normalize(body + mask * s) of one GLWE(S limbs): [S][n] balanced digits; big and tmp are scratch
+void decrypt_phase(const Ring& R, int K, int S, const i64* glwe, const std::vector<cd>& s_spec, std::vector<i64>& big,
+                   std::vector<i64>& tmp, i64* pt) {
+  const int n = R.n();
+  std::vector<cd> spec, prod;
+  big.resize((size_t)S * n);
+  tmp.resize(n);
   for (int l = 0; l < S; l++) {
     R.forward(glwe + ((size_t)l * 2 + 1) * n, spec);
     R.mul(spec, s_spec, prod);
@@ -452,7 +452,20 @@ extern "C" int fheram_decrypt_word(const fheram_params* p, const int64_t* glwe, 
     const i64* b = glwe + ((size_t)l * 2) * n;
     for (int i = 0; i < n; i++) big[(size_t)l * n + i] = tmp[i] + b[i];
   }
-  normalize(n, d.K, S, big, pt.data(), 1, 0);
+  normalize(n, K, S, big, pt, 1, 0);
+}
+}  // namespace
+
+extern "C" int fheram_decrypt_word(const fheram_params* p, const int64_t* glwe, const int64_t* sk,
+                                   int64_t want, int64_t* value, double* noise) {
+  if (check(p) || !glwe || !sk || !value || !noise) return FHERAM_ERR_INVALID;
+  const Dims d = dims(p);
+  Ring R(d.log_n);
+  std::vector<cd> s_spec;
+  R.forward(sk, s_spec);
+  const int n = d.n, S = d.size_ct;
+  std::vector<i64> big, tmp, pt((size_t)S * n);
+  decrypt_phase(R, d.K, S, glwe, s_spec, big, tmp, pt.data());
   // examples/fhe-ram.rs:229-235
   const int k = p->k_ct, log_scale = k - p->k_pt;
   i64 v = 0;
@@ -461,6 +474,60 @@ extern "C" int fheram_decrypt_word(const fheram_params* p, const int64_t* glwe, 
   const i64 diff = v - want * ((i64)1 << log_scale);
   *noise = std::log2((double)(diff < 0 ? -diff : diff)) - (double)k;
   *value = (i64)std::llround((double)v / std::exp2((double)log_scale));
+  return 0;
+}
+
+int fheram_decode_shifts(const fheram_params* p, int* vsh, int* ls) {
+  const int S = cdiv(p->k_ct, p->base2k);
+  if (p->k_ct < 1 || p->k_pt >= p->k_ct || S * p->base2k > 62) {
+    fheram_set_error("decryption needs k_pt < k_ct and ceil(k_ct / base2k) * base2k <= 62");
+    return FHERAM_ERR_INVALID;
+  }
+  *vsh = S * p->base2k - p->k_ct;
+  *ls = p->k_ct - p->k_pt;
+  return 0;
+}
+
+// Every byte of a RAM in fheram_encrypt_ram's layout ([word_size][n_glwe] GLWE), each GLWE decrypted as
+// fheram_decrypt_word decrypts coefficient 0, on all host threads.  values / err: [max_addr][word_size].
+extern "C" int fheram_decrypt_ram(const fheram_params* p, const int64_t* cts, const int64_t* sk, int16_t* values,
+                                  int64_t* err) {
+  if (check(p)) return FHERAM_ERR_INVALID;
+  if (!cts || !sk || !values) { fheram_set_error("fheram_decrypt_ram: null argument"); return FHERAM_ERR_INVALID; }
+  int vsh, ls;
+  if (int rc = fheram_decode_shifts(p, &vsh, &ls)) return rc;
+  const Dims d = dims(p);
+  for (int i = 0; i < d.n; i++)
+    if (sk[i] < -1 || sk[i] > 1) { fheram_set_error("secret key is not ternary"); return FHERAM_ERR_INVALID; }
+  Ring R(d.log_n);
+  std::vector<cd> s_spec;
+  R.forward(sk, s_spec);
+  const int n = d.n, S = d.size_ct, ws = p->word_size, G = d.n_glwe;
+  const size_t glwe = fheram_glwe_len(p);
+  const int total = ws * G;
+  unsigned nt = std::thread::hardware_concurrency();
+  nt = nt < 1 ? 1 : nt;
+  if ((int)nt > total) nt = total;
+  auto work = [&](unsigned t) {
+    std::vector<i64> big, tmp, pt((size_t)S * n);
+    for (int g = (int)t; g < total; g += (int)nt) {
+      const int i = g / G, h = g % G;
+      decrypt_phase(R, d.K, S, cts + (size_t)g * glwe, s_spec, big, tmp, pt.data());
+      for (int j = 0; j < n; j++) {
+        const u64 addr = (u64)h * n + j;
+        if (addr >= p->max_addr) break;
+        i64 v = 0;
+        for (int l = 0; l < S; l++) v += pt[(size_t)l * n + j] * ((i64)1 << (d.K * (S - 1 - l)));
+        int64_t e;
+        fheram_decode(v >> vsh, ls, p->k_pt, values + addr * ws + i, &e);
+        if (err) err[addr * ws + i] = e;
+      }
+    }
+  };
+  std::vector<std::thread> th;
+  for (unsigned t = 1; t < nt; t++) th.emplace_back(work, t);
+  work(0);
+  for (auto& t : th) t.join();
   return 0;
 }
 

@@ -27,6 +27,7 @@
 #include "kernels_ks8.cuh"
 #include "kernels_ext9.cuh"
 #include "kernels_enc.cuh"
+#include "kernels_dec.cuh"
 #include "client_internal.h"
 
 using namespace fheram;
@@ -228,6 +229,7 @@ struct fheram_ctx {
   int* pin32 = nullptr;  // pinned host buffer of small downloads (download_i64)
   DevBuf enc_buf[15];  // operands of the encryption kernels, kept between calls (cudaFree synchronizes the device)
   uint64_t enc_stats[3] = {0, 0, 0};  // noise draws sampled on the device / patched by the host / streams resampled on the host
+  DevBuf dec_buf[2];   // decrypted values / errors on their way to the host (zeroed after every download)
   DevBuf opbuf[3];  // op-level entry points
   long long* d_phase = nullptr;  // per-CTA phase cycle counters (fheram_debug_phase_cycles)
   // per-kernel-class CUDA-event timing (fheram_ctx_profile)
@@ -268,6 +270,7 @@ static int set_attrs() {
   CU(cudaFuncSetAttribute(k_ks5<MODE_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks5<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
+  CU(cudaFuncSetAttribute(k_glwe_decrypt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDecSmem));
   return 0;
 }
 
@@ -420,17 +423,20 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
 }
 
 static void wipe_secrets(fheram_ctx* c);
+static void wipe_plaintext(fheram_ctx* c);
 extern "C" int fheram_ctx_destroy(fheram_ctx* c) {
   if (!c) return 0;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
   wipe_secrets(c);
+  wipe_plaintext(c);
   cudaStreamSynchronize(c->stream);
   if (c->comm_prep) { ncclCommDestroy(c->comm_prep); c->comm_prep = nullptr; }
   if (c->comm) { ncclCommDestroy(c->comm); c->comm = nullptr; }
   c->stage64.release(); c->scratch.release();
   for (auto& b : c->opbuf) b.release();
   for (auto& b : c->enc_buf) b.release();
+  for (auto& b : c->dec_buf) b.release();
   cudaFree(c->d_tw); cudaFree(c->d_tw16); cudaFree(c->d_err);
   if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
   if (c->side) {
@@ -1341,15 +1347,35 @@ static void wipe_secrets(fheram_ctx* c) {
   for (int i : idx)
     if (c->enc_buf[i].p) cudaMemsetAsync(c->enc_buf[i].p, 0, c->enc_buf[i].bytes, c->stream);
 }
+// on any failure the secret material already on the device is wiped before returning
+#define ENC_TRY(x) do { int rc_ = (x); if (rc_) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return rc_; } } while (0)
+#define ENC_CU(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
+// s32 = n_sk secrets of 2 N ints each (secret, then N zeros) -> their prepared spectra in enc_buf[5] (2 M double2 each,
+// the secret's first).  The host staging copy s32 is zeroed on every path; the device copies are wiped on failure.
+static int upload_secret(fheram_ctx* c, std::vector<int>& s32) {
+  DevBuf &skraw = c->enc_buf[4], &skspec = c->enc_buf[5];
+  const int n = c->d.n;
+  const int n_sk = (int)(s32.size() / (2 * (size_t)n));
+  auto up = [&]() -> int {
+    TRY(skraw.ensure(sizeof(int) * s32.size()));
+    TRY(skspec.ensure(sizeof(double2) * 2 * kM * n_sk));
+    CU(cudaMemcpyAsync(skraw.p, s32.data(), sizeof(int) * s32.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+  };
+  const int rc = up();
+  volatile int* vs = s32.data();
+  for (size_t i = 0; i < s32.size(); i++) vs[i] = 0;
+  ENC_TRY(rc);
+  ENC_TRY(prepare(c, (const int*)skraw.p, 2 * n, (double2*)skspec.p, 2 * kM, n_sk, 1, 1, 1));
+  return 0;
+}
 static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, const DevBuf& d_noise, bool noise_by_seq,
                        int* d_out, long stride) {
   const int n = c->d.n;
-  DevBuf &skraw = c->enc_buf[4], &skspec = c->enc_buf[5], &pt = c->enc_buf[6], &mono = c->enc_buf[7],
+  DevBuf &skspec = c->enc_buf[5], &pt = c->enc_buf[6], &mono = c->enc_buf[7],
          &seq = c->enc_buf[8], &keys = c->enc_buf[9], &word0 = c->enc_buf[10], &poly = c->enc_buf[12],
          &poly_sel = c->enc_buf[13], &sk_sel = c->enc_buf[14];
-  // on any failure the secret material already on the device is wiped before returning
-#define ENC_TRY(x) do { int rc_ = (x); if (rc_) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return rc_; } } while (0)
-#define ENC_CU(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
   {
     // the secrets the masks are multiplied by: the caller's sk, or (key generation) the n_sk output secrets of the batch
     std::vector<int> s32;
@@ -1359,14 +1385,7 @@ static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, cons
     } else {
       s32 = b.sk_all;
     }
-    const int n_sk = (int)(s32.size() / (2 * (size_t)n));
-    ENC_TRY(skraw.ensure(sizeof(int) * s32.size()));
-    ENC_TRY(skspec.ensure(sizeof(double2) * 2 * kM * n_sk));
-    ENC_CU(cudaMemcpyAsync(skraw.p, s32.data(), sizeof(int) * s32.size(), cudaMemcpyHostToDevice, c->stream));
-    ENC_CU(cudaStreamSynchronize(c->stream));
-    volatile int* vs = s32.data();  // host staging copy of the secret
-    for (size_t i = 0; i < s32.size(); i++) vs[i] = 0;
-    ENC_TRY(prepare(c, (const int*)skraw.p, 2 * n, (double2*)skspec.p, 2 * kM, n_sk, 1, 1, 1));
+    TRY(upload_secret(c, s32));
   }
   auto up = [&](DevBuf& d, const void* h, size_t bytes) -> int {
     if (!bytes) return 0;
@@ -1406,10 +1425,104 @@ static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, cons
   // context belongs to the evaluator (INTEGRATION.md, colocated client / server mode)
   wipe_secrets(c);
   ENC_CU(cudaStreamSynchronize(c->stream));
-#undef ENC_TRY
-#undef ENC_CU
   return 0;
 }
+
+// ---- decryption on the device (DESIGN.md 3.7): k_glwe_decrypt with the secret spectrum of the encryption path ----
+// zero the decrypted values / errors left on the device by a download
+static void wipe_plaintext(fheram_ctx* c) {
+  for (auto& b : c->dec_buf)
+    if (b.p) cudaMemsetAsync(b.p, 0, b.bytes, c->stream);
+}
+// a.in / n_glwe / placement fields set by the caller; n_out entries of values (and of errors when want_err) are left in
+// c->dec_buf.  The secret and its spectrum are wiped before this returns, on every path.
+static int run_decrypt(fheram_ctx* c, const int64_t* sk, DecArgs a, size_t n_out, bool want_err) {
+  const int n = c->d.n;
+  {
+    std::vector<int> s32((size_t)2 * n, 0);
+    for (int i = 0; i < n; i++) s32[i] = (int)sk[i];
+    TRY(upload_secret(c, s32));
+  }
+  ENC_TRY(c->dec_buf[0].ensure(n_out * sizeof(int16_t)));
+  if (want_err) ENC_TRY(c->dec_buf[1].ensure(n_out * sizeof(int64_t)));
+  ENC_TRY(fheram_decode_shifts(&c->params, &a.vsh, &a.ls));
+  a.ct_stride = c->ct_stride(); a.size = c->d.size_ct; a.k_pt = c->params.k_pt;
+  a.sk_spec = (const double2*)c->enc_buf[5].p;
+  a.values = (short*)c->dec_buf[0].p;
+  a.err = want_err ? (long long*)c->dec_buf[1].p : nullptr;
+  a.tw = c->tw;
+  const int grid = a.n_glwe < 2 * c->sm_count ? a.n_glwe : 2 * c->sm_count;
+  k_glwe_decrypt<<<grid, kThreads, kDecSmem, c->stream>>>(a);
+  c->launches++;
+  ENC_CU(cudaGetLastError());
+  wipe_secrets(c);
+  return 0;
+}
+#undef ENC_TRY
+#undef ENC_CU
+// on a failure after run_decrypt: the secret is already wiped, the decrypted values are not
+#define DEC_CU(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { wipe_plaintext(c); cudaStreamSynchronize(c->stream); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
+
+// Every byte of the resident RAM: what fheram_decrypt_ram gives on fheram_ram_store's output.  A sharded RAM fills the
+// entries of its own polynomials (h == shard mod n_shards) and leaves the others as they are.
+extern "C" int fheram_ram_decrypt_sk(fheram_ram* r, const int64_t* sk, int16_t* values, int64_t* err) {
+  if (!r || !sk || !values) return fail(FHERAM_ERR_INVALID, "null argument");
+  fheram_ctx* c = r->c;
+  TRY(check_secret(sk, c->d.n));
+  if (!r->loaded) return fail(FHERAM_ERR_UNINIT, "the RAM was never loaded or encrypted");
+  if (r->state || r->rotated)
+    return fail(FHERAM_ERR_STATE, "the RAM is prepared for write (its data is rotated): call fheram_ram_write first");
+  CU(cudaSetDevice(c->device));
+  const int ws = c->params.word_size, n = c->d.n;
+  const uint64_t max_addr = c->params.max_addr;
+  DecArgs a;
+  memset(&a, 0, sizeof(a));
+  a.in = r->data; a.n_glwe = ws * r->n_local;
+  a.coef0 = 0; a.n_poly = r->n_local; a.word_size = ws; a.shard = r->shard; a.n_shards = r->n_shards;
+  a.max_addr = max_addr;
+  TRY(run_decrypt(c, sk, a, (size_t)r->n_local * n * ws, err != nullptr));
+  // device layout [n_local][N][word_size]: local polynomial hp is the row of entries [h N ws, (h + 1) N ws) of the
+  // caller's arrays, h = shard + n_shards hp; only the last polynomial of the RAM can end before max_addr
+  const size_t row = (size_t)n * ws;
+  int n_full = 0;
+  while (n_full < r->n_local && (r->shard + (uint64_t)r->n_shards * n_full + 1) * n <= max_addr) n_full++;
+  for (int k = 0; k < 2; k++) {
+    if (k == 1 && !err) break;
+    const size_t el = k == 0 ? sizeof(int16_t) : sizeof(int64_t);
+    char* dst = k == 0 ? (char*)values : (char*)err;
+    const char* src = (const char*)c->dec_buf[k].p;
+    if (n_full)
+      DEC_CU(cudaMemcpy2DAsync(dst + (size_t)r->shard * row * el, (size_t)r->n_shards * row * el, src, row * el, row * el,
+                               n_full, cudaMemcpyDeviceToHost, c->stream));
+    if (n_full < r->n_local) {
+      const uint64_t h = r->shard + (uint64_t)r->n_shards * n_full;
+      DEC_CU(cudaMemcpyAsync(dst + h * row * el, src + n_full * row * el, (max_addr - h * n) * ws * el,
+                             cudaMemcpyDeviceToHost, c->stream));
+    }
+  }
+  wipe_plaintext(c);
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+
+// coefficient 0 of n device-resident GLWE(k_ct), [n][limb][col][N] int32 (a read result arena)
+extern "C" int fheram_decrypt_words_device(fheram_ctx* c, const int32_t* d_glwe, int n, const int64_t* sk,
+                                           int16_t* values, int64_t* err) {
+  if (!c || !d_glwe || n < 1 || !sk || !values) return fail(FHERAM_ERR_INVALID, "null argument or n < 1");
+  TRY(check_secret(sk, c->d.n));
+  CU(cudaSetDevice(c->device));
+  DecArgs a;
+  memset(&a, 0, sizeof(a));
+  a.in = d_glwe; a.n_glwe = n; a.coef0 = 1;
+  TRY(run_decrypt(c, sk, a, (size_t)n, err != nullptr));
+  DEC_CU(cudaMemcpyAsync(values, c->dec_buf[0].p, (size_t)n * sizeof(int16_t), cudaMemcpyDeviceToHost, c->stream));
+  if (err)
+    DEC_CU(cudaMemcpyAsync(err, c->dec_buf[1].p, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  wipe_plaintext(c);
+  CU(cudaStreamSynchronize(c->stream));
+  return 0;
+}
+#undef DEC_CU
 
 // Ram::encrypt_sk (src/ram.rs:129-167; SubRam::encrypt_sk :334-380) into the device-resident RAM
 extern "C" int fheram_ram_encrypt_sk(fheram_ram* r, const uint8_t* data, const int64_t* sk,

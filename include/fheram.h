@@ -307,6 +307,25 @@ int fheram_keys_download_raw(fheram_keys *k, int64_t *atk_glwe, int64_t *tsk, in
 /* out = {noise draws sampled on the device, draws re-drawn by the host, streams sampled by the host} so far */
 int fheram_debug_encrypt_stats(fheram_ctx *ctx, uint64_t out[3]);
 
+/* ---- bulk decryption (DESIGN.md 3.7).  One definition for every entry point, per GLWE(k_ct) of S limbs:
+ *   pt = normalize(body + mask * s)  (balanced base-2^K digits, top carry dropped, as fheram_decrypt_word)
+ *   v = (sum_j pt_j 2^(K(S-1-j))) >> (S K - k_ct),  ls = k_ct - k_pt
+ *   value_raw = round_half_away(v / 2^ls)   (fheram_decrypt_word's value)
+ *   value = value_raw reduced into [-2^(k_pt-1), 2^(k_pt-1)),  err = v - value_raw 2^ls  (exact)
+ * fheram_decrypt_word's noise against want = value_raw is log2|err| - k_ct.  For a stored byte b,
+ * value == cast_u8_to_signed(b, min(8, k_pt)).  err may be NULL; sk must be ternary. ---- */
+/* CPU, all host threads: every byte of a RAM in fheram_encrypt_ram / fheram_ram_store's layout.  values / err =
+ * [max_addr][word_size] (byte i of word j at j * word_size + i, the inverse of Ram::encrypt_sk's data) */
+int fheram_decrypt_ram(const fheram_params *p, const int64_t *cts, const int64_t *sk, int16_t *values, int64_t *err);
+/* the same numbers from the resident RAM on the device, bit for bit.  A sharded RAM fills the entries of its own
+ * polynomials (h == shard mod n_shards) and leaves the others as passed.  FHERAM_ERR_UNINIT: never loaded or
+ * encrypted; FHERAM_ERR_STATE: prepared for write (read_prepare_write without its write) */
+int fheram_ram_decrypt_sk(fheram_ram *r, const int64_t *sk, int16_t *values, int64_t *err);
+/* coefficient 0 of n device-resident GLWE(k_ct) in the int32 layout [n][limb][col][N] (e.g. the arena of
+ * fheram_ram_read_batch_device, n = reads x word_size); values / err = [n] */
+int fheram_decrypt_words_device(fheram_ctx *ctx, const int32_t *d_glwe, int n, const int64_t *sk, int16_t *values,
+                                int64_t *err);
+
 #ifdef __cplusplus
 }
 #endif

@@ -97,4 +97,10 @@ extern "C" {
                                xe: *mut fheram_source, glwe: *mut i64) -> c_int;
     pub fn fheram_decrypt_word(p: *const fheram_params, glwe: *const i64, sk: *const i64, want: i64,
                                value: *mut i64, noise: *mut c_double) -> c_int;
+    // bulk decryption (DESIGN.md 3.7): a whole RAM on the CPU / on the device, coefficient 0 of device-resident GLWEs
+    pub fn fheram_decrypt_ram(p: *const fheram_params, cts: *const i64, sk: *const i64, values: *mut i16,
+                              err: *mut i64) -> c_int;
+    pub fn fheram_ram_decrypt_sk(r: *mut fheram_ram, sk: *const i64, values: *mut i16, err: *mut i64) -> c_int;
+    pub fn fheram_decrypt_words_device(c: *mut fheram_ctx, d_glwe: *const i32, n: c_int, sk: *const i64,
+                                       values: *mut i16, err: *mut i64) -> c_int;
 }

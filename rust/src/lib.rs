@@ -193,5 +193,31 @@ impl Ram {
         let a = address.device(&mut self.params);
         check(unsafe { fheram_ram_write(self.h, flat.as_ptr(), a, keys.0) });
     }
+    /// every byte of the resident RAM decrypted on the device: (values, err), [max_addr][word_size] row-major (byte i of
+    /// word j at j * word_size + i); the numbers of `decrypt_ram` on the stored RAM, bit for bit
+    pub fn decrypt_sk(&mut self, sk: &GLWESecret) -> (Vec<i16>, Vec<i64>) {
+        let len = self.params.max_addr() * self.params.word_size();
+        let (mut values, mut err) = (vec![0i16; len], vec![0i64; len]);
+        check(unsafe { fheram_ram_decrypt_sk(self.h, sk.0.as_ptr(), values.as_mut_ptr(), err.as_mut_ptr()) });
+        (values, err)
+    }
+}
+
+/// every byte of a RAM in `fheram_encrypt_ram`'s layout ([word_size][n_glwe] GLWE), decrypted on the CPU: (values, err)
+/// as `Ram::decrypt_sk` returns them
+pub fn decrypt_ram(params: &Parameters, cts: &[i64], sk: &GLWESecret) -> (Vec<i16>, Vec<i64>) {
+    let len = params.max_addr() * params.word_size();
+    let (mut values, mut err) = (vec![0i16; len], vec![0i64; len]);
+    check(unsafe { fheram_decrypt_ram(&params.c, cts.as_ptr(), sk.0.as_ptr(), values.as_mut_ptr(), err.as_mut_ptr()) });
+    (values, err)
+}
+
+/// coefficient 0 of `n` device-resident GLWE(k_ct) (int32 `[n][limb][col][N]`, e.g. a batched read's result arena),
+/// decrypted on the device: (values, err), `n` each
+pub fn decrypt_words_device(params: &mut Parameters, d_glwe: *const i32, n: usize, sk: &GLWESecret) -> (Vec<i16>, Vec<i64>) {
+    let (mut values, mut err) = (vec![0i16; n], vec![0i64; n]);
+    check(unsafe { fheram_decrypt_words_device(params.module(), d_glwe, n as i32, sk.0.as_ptr(), values.as_mut_ptr(),
+                                               err.as_mut_ptr()) });
+    (values, err)
 }
 impl Drop for Ram { fn drop(&mut self) { unsafe { fheram_ram_destroy(self.h); } } }
