@@ -269,7 +269,13 @@ static int set_attrs() {
   CU(cudaFuncSetAttribute(k_ks6<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks5<MODE_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
   CU(cudaFuncSetAttribute(k_ks5<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
-  CU(cudaFuncSetAttribute(k_ks4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
+  CU(cudaFuncSetAttribute(k_ks4<MODE_COMBINE2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
+  // mixed packer level of a tree whose width is not a power of two
+  CU(cudaFuncSetAttribute(k_ks8<8, MODE_MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ks8_smem(8)));
+  CU(cudaFuncSetAttribute(k_ks8<4, MODE_MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ks8_smem(4)));
+  CU(cudaFuncSetAttribute(k_ks6<MODE_MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
+  CU(cudaFuncSetAttribute(k_ks5<MODE_MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs5Smem));
+  CU(cudaFuncSetAttribute(k_ks4<MODE_MIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kKs4Smem));
   CU(cudaFuncSetAttribute(k_glwe_decrypt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDecSmem));
   return 0;
 }
@@ -320,8 +326,6 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
   Derived d = derive(p);
   if (d.n_coord > 2)
     return fail(FHERAM_ERR_INVALID, "max_addr > N^2: the reference's read loop only supports two coordinates");
-  if (d.n_glwe & (d.n_glwe - 1))
-    return fail(FHERAM_ERR_INVALID, "max_addr / N must be a power of two");
   int force_ext = FORCE_NONE, force_ks = FORCE_NONE;
   TRY(parse_force(getenv("FHERAM_KERNEL"), &force_ext, &force_ks));
   int ndev = 0;
@@ -1015,8 +1019,9 @@ static int run_ext_chain(fheram_ctx* c, int n_items, const int* src, const int* 
       return launch(c, KC_EXT, k_ext8, std::min(n_items, c->sm_count), kExt8Threads, kExt8Smem, a, c->d_tw16);
   }
 }
-// a key-switch launch of MODE_TRACE or MODE_COMBINE2: step s uses trace key key0 + s, in the frequency order of the
-// selected kernel (k_ks7 and k_ks8 read the keys prepared by k_prepare7, the others those of k_prepare)
+// a key-switch launch of MODE_TRACE, MODE_COMBINE2 or MODE_MIXED (selected and profiled as a combine): step s uses trace
+// key key0 + s, in the frequency order of the selected kernel (k_ks7 and k_ks8 read the keys prepared by k_prepare7,
+// the others those of k_prepare)
 template <int MODE>
 static int launch_ks(fheram_ctx* c, const fheram_keys* k, int key0, VmpArgs a) {
   const int n = a.n_items, S = c->sm_count, cls = MODE == MODE_TRACE ? KC_TRACE : KC_COMBINE2;
@@ -1031,7 +1036,8 @@ static int launch_ks(fheram_ctx* c, const fheram_keys* k, int key0, VmpArgs a) {
     case KN_KS7: return launch(c, cls, k_ks7, std::min(n, 2 * S), 256, kKs7Smem, a, c->d_tw16);
     case KN_KS6: return launch(c, cls, k_ks6<MODE>, 2 * n, kThreads5, kKs5Smem, a);
     case KN_KS5: return launch(c, cls, k_ks5<MODE>, std::min(n, S), kThreads5, kKs5Smem, a);
-    default: return launch(c, cls, k_ks4, std::min(n, 2 * S), kThreads, kKs4Smem, a);
+    default:
+      return launch(c, cls, k_ks4<MODE == MODE_MIXED ? MODE_MIXED : MODE_COMBINE2>, std::min(n, 2 * S), kThreads, kKs4Smem, a);
   }
 }
 // chain of { glwe_rsh(1); automorphism_add with trace key i } for i in [g0, g1)
@@ -1072,6 +1078,21 @@ static int run_combine2(fheram_ctx* c, const fheram_keys* k, int n_items, const 
   return launch_ks<MODE_COMBINE2>(c, k, level, a);
 }
 
+// GLWEPacker::combine at tree level `level` of a tree whose width m is not a power of two (2^(L-1) < m < 2^L,
+// level = log_n - L, the first level whose a operands are all present): in = groups of m inputs in packer_order,
+// n_items = groups * H (H = 2^(L-1)) pairs; pair i of a group takes the two-sided combine when its b exists and the
+// one-sided one (rsh 1, a + phi_g(a)) otherwise (ops, packer_order).  out[group * H + i], feed order of width H.
+static int run_combine_mixed(fheram_ctx* c, const fheram_keys* k, int n_items, int m, int H, const int* ops,
+                             const int* in, int* out, int level) {
+  VmpArgs a = base_args(c, n_items, in, out, c->ct_stride());
+  a.src_map = ops; a.src_mod = m; a.src_div = H;
+  a.n_steps = 1;
+  a.gal[0] = (int)((galois(c->d.log_n, level) + 2 * kN) % (2 * kN));
+  a.gal_inv[0] = inv_mod_2n(a.gal[0]);
+  a.rot_const = 1 << (c->d.log_n - level - 1);  // t of the two-sided combines
+  return launch_ks<MODE_MIXED>(c, k, level, a);
+}
+
 // GLWEPacker over `width` inputs per group (width a power of two), feed order = index order
 // of `buf` (caller wrote inputs at m = bitrev(h)).  One-sided levels [0, log_n - log2(width_total))
 // must already be applied.  Runs two-sided levels first_level .. first_level + log2(width) - 1,
@@ -1089,6 +1110,42 @@ static int run_pack_levels(fheram_ctx* c, const fheram_keys* k, int groups, int 
   return 0;
 }
 
+// Packer input order of a tree of m inputs (src/ram.rs:424-443: inputs h < m, None beyond).  m a power of two: position p
+// holds input bitrev(p), the feed order.  Otherwise (2^(L-1) < m < 2^L) only the m present inputs, compact: for each pair
+// i < H = 2^(L-1) of level log_n - L, a_i (input h = bitrev_{L-1}(i)) followed by b_i (input h + H) when h + H < m;
+// ops[i] = position of a_i << 1 | (b_i present), the operand table of run_combine_mixed.  The levels below it are
+// one-sided for every input (their b operands are all beyond m).
+static void packer_order(int m, std::vector<int>& order, std::vector<int>& ops) {
+  const int L = ilog2(m);
+  order.clear();
+  ops.clear();
+  if (!(m & (m - 1))) {
+    for (int p = 0; p < m; p++) order.push_back((int)revbits(p, L));
+    return;
+  }
+  const int H = 1 << (L - 1);
+  for (int i = 0; i < H; i++) {
+    const int h = (int)revbits(i, L - 1);
+    const bool two = h + H < m;
+    ops.push_back((int)order.size() << 1 | (two ? 1 : 0));
+    order.push_back(h);
+    if (two) order.push_back(h + H);
+  }
+}
+// the two-sided part of `groups` packer (sub)trees of m inputs each, after their one-sided levels, from tree level
+// first_level on: buf holds the inputs in packer_order (ops on the device); returns the buffer holding the [groups]
+// results.  m a power of two: the levels [first_level, first_level + L) of run_pack_levels (a shard's local tree stops
+// below the top levels, which ram_finish_stage runs); otherwise (a whole tree, first_level = log_n - L) the mixed level,
+// then the levels above it over width H.
+static int run_pack_tree(fheram_ctx* c, const fheram_keys* k, int groups, int m, int first_level, const int* ops,
+                         int* buf, int* tmp, int** result) {
+  const int L = ilog2(m);
+  if (!(m & (m - 1))) return run_pack_levels(c, k, groups, m, first_level, buf, tmp, result);
+  const int H = 1 << (L - 1);
+  TRY(run_combine_mixed(c, k, groups * H, m, H, ops, buf, tmp, first_level));
+  return run_pack_levels(c, k, groups, H, first_level + 1, tmp, buf, result);
+}
+
 // --------------------------------------------------------------------------------------
 // RAM
 // --------------------------------------------------------------------------------------
@@ -1102,7 +1159,8 @@ struct fheram_ram {
   bool rotated = false;      // rpw_local_device rotated SubRam::data in place and rpw_finish_device has not completed:
                              // the reference does both inside one call (src/ram.rs:502-533), so no read may see this state
   bool loaded = false;
-  int* feed_map = nullptr;   // device: [word_size*n_local] feed position -> data index
+  int* feed_map = nullptr;   // device: [word_size*n_local] packer input position -> data index (packer_order)
+  int* mixed_ops = nullptr;  // device: operand table of the mixed packer level (n_local not a power of two)
   DevBuf bufA, bufB;         // work arenas [B][word_size][n_local] GLWE
   DevBuf partial;            // [B][word_size] packed partials
   DevBuf result;             // [B][word_size] results
@@ -1128,6 +1186,9 @@ static int ram_create(fheram_ctx* c, int shard, int n_shards, fheram_ram** out) 
   const Derived& d = c->d;
   if (n_shards < 1 || (n_shards & (n_shards - 1)) || n_shards > d.n_glwe || shard < 0 || shard >= n_shards)
     return fail(FHERAM_ERR_INVALID, "n_shards must be a power of two <= max_addr/N and 0 <= shard < n_shards");
+  if (n_shards > 1 && (d.n_glwe & (d.n_glwe - 1)))
+    return fail(FHERAM_ERR_INVALID, "a sharded RAM needs max_addr/N (rounded up) to be a power of two, here %d",
+                d.n_glwe);
   CU(cudaSetDevice(c->device));
   fheram_ram* r = new fheram_ram();
   r->c = c; r->shard = shard; r->n_shards = n_shards;
@@ -1136,14 +1197,19 @@ static int ram_create(fheram_ctx* c, int shard, int n_shards, fheram_ram** out) 
   CU(cudaMalloc(&r->data, sizeof(int) * (size_t)ws * r->n_local * c->ct_stride()));
   CU(cudaMalloc(&r->tree, sizeof(int) * (size_t)ws * c->ct_stride()));
   CU(cudaMemset(r->tree, 0, sizeof(int) * (size_t)ws * c->ct_stride()));
-  // feed order of the packer (src/ram.rs:425-435): position m of the local tree reads local
-  // polynomial h' = bitrev(m)
+  // input order of the packer (src/ram.rs:425-435, packer_order): position m of the local tree reads local
+  // polynomial h' = order[m]
+  std::vector<int> order, ops;
+  packer_order(r->n_local, order, ops);
   std::vector<int> map((size_t)ws * r->n_local);
-  const int lg = ilog2(r->n_local);
   for (int s = 0; s < ws; s++)
-    for (int m = 0; m < r->n_local; m++) map[(size_t)s * r->n_local + m] = s * r->n_local + (int)revbits(m, lg);
+    for (int m = 0; m < r->n_local; m++) map[(size_t)s * r->n_local + m] = s * r->n_local + order[m];
   CU(cudaMalloc(&r->feed_map, sizeof(int) * map.size()));
   CU(cudaMemcpy(r->feed_map, map.data(), sizeof(int) * map.size(), cudaMemcpyHostToDevice));
+  if (!ops.empty()) {
+    CU(cudaMalloc(&r->mixed_ops, sizeof(int) * ops.size()));
+    CU(cudaMemcpy(r->mixed_ops, ops.data(), sizeof(int) * ops.size(), cudaMemcpyHostToDevice));
+  }
   *out = r;
   return 0;
 }
@@ -1154,7 +1220,7 @@ extern "C" int fheram_ram_create_sharded(fheram_ctx* c, int shard, int n_shards,
 extern "C" int fheram_ram_destroy(fheram_ram* r) {
   if (!r) return 0;
   cudaSetDevice(r->c->device);
-  cudaFree(r->data); cudaFree(r->tree); cudaFree(r->feed_map);
+  cudaFree(r->data); cudaFree(r->tree); cudaFree(r->feed_map); cudaFree(r->mixed_ops);
   if (r->wpin) { cudaStreamSynchronize(r->c->stream); cudaFreeHost(r->wpin); cudaEventDestroy(r->wcopied); }
   r->bufA.release(); r->bufB.release(); r->partial.release(); r->result.release(); r->wbuf.release(); r->wstage.release(); r->all.release(); r->xchg.release(); r->part_all.release();
   for (auto& s : r->pipe.sets) {
@@ -1732,8 +1798,8 @@ static int ram_local_stage(fheram_ram* r, const fheram_address* addr, int first_
   // matrices of the first coordinate of address first_addr, and the distance to the next address
   const long mat_stride = (long)(addr->prep1 ? d.coord_len[0] : d.n_ggsw) * c->ggsw_prep_len();
   const double2* mats = addr->prep + (size_t)first_addr * mat_stride;
-  const int lg_total = ilog2(d.n_glwe);          // two-sided levels of the full tree
-  const int one_sided = d.log_n - lg_total;      // levels with a single non-empty child
+  const int lg_total = ilog2(d.n_glwe);          // levels of the full tree that have a second non-empty child
+  const int one_sided = d.log_n - lg_total;      // levels with a single non-empty child for every input
   if (d.n_coord == 1) {
     // max_addr <= N: product on data[0] only (src/ram.rs:450-452); "partial" = rotated poly
     if (inplace) {
@@ -1754,7 +1820,7 @@ static int ram_local_stage(fheram_ram* r, const fheram_address* addr, int first_
     TRY(run_trace_chain(c, k, items, A, nullptr, 0, 0, A, 0, one_sided));
   }
   int* res = nullptr;
-  TRY(run_pack_levels(c, k, B * ws, nl, one_sided, A, Bb, &res));
+  TRY(run_pack_tree(c, k, B * ws, nl, one_sided, r->mixed_ops, A, Bb, &res));
   CU(cudaMemcpyAsync(r->partial.p, res, sizeof(int) * (size_t)B * ws * L, cudaMemcpyDeviceToDevice, c->stream));
   return 0;
 }
@@ -2364,23 +2430,25 @@ extern "C" int fheram_glwe_trace(fheram_ctx* c, const fheram_keys* k, const int6
 }
 
 extern "C" int fheram_glwe_pack(fheram_ctx* c, const fheram_keys* k, const int64_t* in, int n, int64_t* out) {
-  if (!c || !k || !in || !out || n < 1 || n > kN || (n & (n - 1))) return fail(FHERAM_ERR_INVALID, "n must be a power of two <= N");
+  if (!c || !k || !in || !out || n < 1 || n > kN) return fail(FHERAM_ERR_INVALID, "n must be in 1..N");
   CU(cudaSetDevice(c->device));
   const long L = c->ct_stride();
   TRY(c->opbuf[0].ensure(sizeof(int) * (size_t)n * L));
   TRY(c->opbuf[1].ensure(sizeof(int) * (size_t)n * L));
-  TRY(c->opbuf[2].ensure(sizeof(int) * (size_t)n));
+  TRY(c->opbuf[2].ensure(sizeof(int) * (size_t)2 * n));  // input order | operand table of the mixed level
   TRY(upload_i64(c, in, (size_t)n * L, (int*)c->opbuf[1].p));
-  const int lg = ilog2(n);
-  std::vector<int> map(n);
-  for (int m = 0; m < n; m++) map[m] = (int)revbits(m, lg);
-  CU(cudaMemcpyAsync(c->opbuf[2].p, map.data(), sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+  std::vector<int> map, ops;
+  packer_order(n, map, ops);
+  int* d_map = (int*)c->opbuf[2].p;
+  CU(cudaMemcpyAsync(d_map, map.data(), sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
+  if (!ops.empty())
+    CU(cudaMemcpyAsync(d_map + n, ops.data(), sizeof(int) * ops.size(), cudaMemcpyHostToDevice, c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  const int one_sided = c->d.log_n - lg;
+  const int one_sided = c->d.log_n - ilog2(n);
   int* A = (int*)c->opbuf[0].p;
-  TRY(run_trace_chain(c, k, n, (int*)c->opbuf[1].p, (int*)c->opbuf[2].p, n, 0, A, 0, one_sided));
+  TRY(run_trace_chain(c, k, n, (int*)c->opbuf[1].p, d_map, n, 0, A, 0, one_sided));
   int* res = nullptr;
-  TRY(run_pack_levels(c, k, 1, n, one_sided, A, (int*)c->opbuf[1].p, &res));
+  TRY(run_pack_tree(c, k, 1, n, one_sided, d_map + n, A, (int*)c->opbuf[1].p, &res));
   return download_i64(c, res, (size_t)L, out);
 }
 

@@ -247,6 +247,8 @@ enum Mode : int {
   MODE_COMBINE2 = 2, // GLWEPacker two-sided combine
   MODE_AUTO = 3,     // x <- phi_g(normalize(KS(x)))  (glwe_automorphism)
   MODE_EXPAND = 4,   // GGSW expand row: (KS_tsk(mask), + body on the mask column)
+  MODE_MIXED = 5,    // GLWEPacker level whose pairs may lack their second operand: per item the two-sided
+                     // combine (COMBINE2) or the one-sided one (one TRACE step, no rotation)
 };
 
 struct VmpArgs {
@@ -258,6 +260,8 @@ struct VmpArgs {
   int src_mod;
   int src_div;       // if > 0: index = item / src_div (takes precedence over src_mod)
   // second operand of COMBINE2: a = src[2*item], b = src[2*item+1]
+  // MODE_MIXED: pair p = item % src_div of group item / src_div; op = src_map[p] (offset << 1 | has_b):
+  //   a = src[group * src_mod + (op >> 1)], b = the ciphertext after a when op & 1 (else the one-sided combine)
   int* dst;          // item -> dst + item * ct_stride
   int* scratch;      // per-CTA scratch: gridDim.x * 2 * ct_stride ints
   long ct_stride;    // ints per ciphertext
@@ -278,6 +282,12 @@ struct VmpArgs {
   long long* phase_cycles;
   int stagger;  // k_ks5: cycles by which group 1 trails group 0 after a CTA barrier (tuning knob)
 };
+// MODE_MIXED operands of `item`: returns a; two = whether b (the ciphertext after a) is present
+__device__ __forceinline__ const int* mixed_src(const VmpArgs& A, int item, bool& two) {
+  const int op = A.src_map[item % A.src_div];
+  two = (op & 1) != 0;
+  return A.src + ((long)(item / A.src_div) * A.src_mod + (op >> 1)) * A.ct_stride;
+}
 #define PHASE_TICK(ph)                                                      \
   do {                                                                      \
     if (A.phase_cycles && threadIdx.x == 0) {                               \

@@ -4,7 +4,10 @@
 // and the first tile of every output is fetched during the previous inverse transform.
 // (tools/ablate: without matrix loads k_ks3 runs 76.8 K -> 58.1 K cycles per operation; the loads
 // were three exposed L2 round trips per output.)  Same integers as k_ks3 / k_ks2 / k_vmp.
-// Two-sided combine of GLWEPacker only: the wide launches of the packer tree (the trace kernels took its traces).
+// GLWEPacker combines only: the wide launches of the packer tree (the trace kernels took its traces).
+// MODE_MIXED (the packer level of a tree whose width is not a power of two): items without a second operand take the
+// one-sided combine rsh1(a) + phi_g(KS(rsh1(a))) -- b = 0 and t = 0 below, S + y instead of S - y, and the top-limb
+// rounding of the trace kernels (no pre-automorphism sign frame, the sum is not negated).
 #pragma once
 #include "kernels_ks3.cuh"
 
@@ -12,7 +15,9 @@ namespace fheram {
 
 constexpr size_t kKs4Smem = (size_t)kWorkPad * sizeof(double2) + (size_t)2 * kN * sizeof(long long) + 16;
 
+template <int MODE>
 __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
+  static_assert(MODE == MODE_COMBINE2 || MODE == MODE_MIXED, "combine modes only");
   constexpr int R = 3, LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* work = reinterpret_cast<double2*>(smem_raw);  // padded exchange buffer (transform_pad.cuh)
@@ -55,7 +60,14 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
     // words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
-    const int* src = A.src + 2L * item * A.ct_stride;
+    const int* src;
+    bool two = true;  // MODE_MIXED: the item has its second operand
+    if constexpr (MODE == MODE_MIXED) {
+      src = mixed_src(A, item, two);
+    } else {
+      src = A.src + 2L * item * A.ct_stride;
+    }
+    const bool one = MODE == MODE_MIXED ? !two : false;  // the one-sided combine (a constant unless MODE_MIXED)
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     // ------------------------------ prologue (once per item) ---------------------------
@@ -63,7 +75,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
       // a1 = a X^-t;  D = rsh1(a1 - b) -> xp;  S = rsh1(a1 + b) -> sw
       const int* a = src;
       const int* b = src + A.ct_stride;
-      const int tt = A.rot_const;
+      const int tt = one ? 0 : A.rot_const;
 #pragma unroll 1
       for (int mc = 0; mc < 16; mc += 4) {
         int av[4][2][3], bv[4][2][3];
@@ -75,7 +87,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
 #pragma unroll
           for (int col = 0; col < 2; col++)
 #pragma unroll
-            for (int l = 0; l < 3; l++) { av[mm][col][l] = a[CT(col, l) + j]; bv[mm][col][l] = b[CT(col, l) + i]; }
+            for (int l = 0; l < 3; l++) { av[mm][col][l] = a[CT(col, l) + j]; bv[mm][col][l] = one ? 0 : b[CT(col, l) + i]; }
         }
 #pragma unroll
         for (int mm = 0; mm < 4; mm++) {
@@ -235,7 +247,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
               const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
-              const double t = v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
+              const double t = v + __hiloint2double(0x43380000, (int)(65536u - (one ? 0u : (sgn >> q) & 1u)));
               const int c3 = (int)__funnelshift_r((uint32_t)__double2loint(t), (uint32_t)__double2hiint(t), 17);
               if (co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
               else xc[i] += (unsigned long long)(long long)c3;
@@ -264,9 +276,9 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
               const unsigned long long W = xc[i] + ((unsigned long long)((uint32_t)__double2loint(t) << 2) << 32);
               // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:
               //   word = S - (R + k3) - sigma (D_body[u] - bias)
-              const unsigned long long U = (sw[co * kN + i] - W) & kMask51;
+              const unsigned long long U = (one ? sw[co * kN + i] + W : sw[co * kN + i] - W) & kMask51;
               bool rneg;
-              const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
+              const int dd = rot_index(i, one ? 0 : A.rot_const, rneg);  // a' * X^t
 #pragma unroll
               for (int ll = 0; ll < 3; ll++) {
                 const int dg = word_digit(U, ll);

@@ -69,7 +69,7 @@ __device__ __forceinline__ void inv_transform_g(double2 (&x)[8], const PadAddr& 
 
 template <int MODE>
 __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
-  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2, "key-switch modes only");
+  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2 || MODE == MODE_MIXED, "key-switch modes only");
   constexpr int LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* work_all = reinterpret_cast<double2*>(smem_raw);                         // [2 groups] exchange buffers
@@ -123,19 +123,24 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
     const int* src;
-    {
+    bool two = true;  // MODE_MIXED: the item has its second operand
+    if constexpr (MODE == MODE_MIXED) {
+      src = mixed_src(A, item, two);
+    } else {
       long idx = item;
       if (MODE == MODE_COMBINE2) idx = 2L * item;
       else if (A.src_div > 0) idx = item / A.src_div;
       else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
       src = A.src + idx * A.ct_stride;
     }
+    // this item's path: TRACE steps, or the two-sided combine (a constant unless MODE_MIXED)
+    const bool trace = MODE == MODE_MIXED ? !two : MODE == MODE_TRACE;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     // ---------------- prologue (once per item): group g converts column g -----------------
-    if (MODE == MODE_TRACE) {
-      // x = rsh1(src * X^rk)
-      int rk = A.rot_const;
+    if (trace) {
+      // x = rsh1(src * X^rk)  (MODE_MIXED: the one-sided combine, no rotation)
+      int rk = MODE == MODE_MIXED ? 0 : A.rot_const;
       if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
       rk &= (2 * kN - 1);
 #pragma unroll 4
@@ -253,7 +258,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
           const int e = (e0 + (q & 7) * d1 + (q >> 3) * d2) & (2 * kN - 1);
           const unsigned long long b = xp[e & (kN - 1)] - kBias51;
           const bool ng = (((sgn >> q) & 1u) ^ sgn_bit) != 0;
-          v0[q] = (ng ? 0ull - b : b) + (MODE == MODE_TRACE ? xp[i] : 0ull);
+          v0[q] = (ng ? 0ull - b : b) + (trace ? xp[i] : 0ull);
         }
         group_sync(1);  // every gather of the old body column precedes its stores
 #pragma unroll
@@ -319,10 +324,10 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
             const int i = T + 256 * (q & 7) + (q >> 3) * kM;
             const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
             double t;
-            if (MODE == MODE_TRACE) t = fma(v, sgn_d, kMagic52 + 65536.0);
+            if (trace) t = fma(v, sgn_d, kMagic52 + 65536.0);
             else t = v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
             const int c3 = (int)__funnelshift_r((uint32_t)__double2loint(t), (uint32_t)__double2hiint(t), 17);
-            if (MODE == MODE_COMBINE2 && co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
+            if (!trace && co == 1) xc[i] = (unsigned long long)(long long)c3;  // D mask words are dead
             else xc[i] += (unsigned long long)(long long)c3;
           }
         } else if (l == 2) {
@@ -346,7 +351,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
             const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
             const double t = fma(v, sgn_d, kMagic52);
             const unsigned long long W = xc[i] + ((unsigned long long)((uint32_t)__double2loint(t) << 2) << 32);
-            if (MODE == MODE_TRACE) {
+            if (trace) {
               const unsigned long long U = W & kMask51;
               xc[i] = last ? U : rsh1_canon(U);
             } else {
@@ -370,7 +375,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     }  // steps
 
-    if (MODE == MODE_TRACE) {
+    if (trace) {
 #pragma unroll 4
       for (int m = 0; m < 16; m++) {
         const int i = T + 256 * m;

@@ -37,7 +37,7 @@ __device__ __forceinline__ void st_cluster_u64(uint32_t addr, unsigned long long
 
 template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(const VmpArgs A) {
-  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2, "key-switch modes only");
+  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2 || MODE == MODE_MIXED, "key-switch modes only");
   constexpr int LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* work_all = reinterpret_cast<double2*>(smem_raw);                         // [2 groups] exchange buffers
@@ -92,13 +92,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
     const int* src;
-    {
+    bool two = true;  // MODE_MIXED: the item has its second operand
+    if constexpr (MODE == MODE_MIXED) {
+      src = mixed_src(A, item, two);
+    } else {
       long idx = item;
       if (MODE == MODE_COMBINE2) idx = 2L * item;
       else if (A.src_div > 0) idx = item / A.src_div;
       else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
       src = A.src + idx * A.ct_stride;
     }
+    // this item's path: TRACE steps, or the two-sided combine (a constant unless MODE_MIXED)
+    const bool trace = MODE == MODE_MIXED ? !two : MODE == MODE_TRACE;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     // -------- prologue: both CTAs need the mask column of x (TRACE) / D (COMBINE2), CTA 0 also the body --------
@@ -106,9 +111,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
     {
       const int col = co == 0 ? grp : 1;
       const int m0 = co == 0 ? 0 : 8 * grp, m1 = co == 0 ? 16 : 8 * grp + 8;
-      if (MODE == MODE_TRACE) {
-        // x = rsh1(src * X^rk)
-        int rk = A.rot_const;
+      if (trace) {
+        // x = rsh1(src * X^rk)  (MODE_MIXED: the one-sided combine, no rotation)
+        int rk = MODE == MODE_MIXED ? 0 : A.rot_const;
         if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
         rk &= (2 * kN - 1);
 #pragma unroll 4
@@ -220,7 +225,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
           const int e = (e0 + (q & 7) * d1 + (q >> 3) * d2) & (2 * kN - 1);
           const unsigned long long b = xp[e & (kN - 1)] - kBias51;
           const bool ng = (((sgn >> q) & 1u) ^ sgn_bit) != 0;
-          v0[q] = (ng ? 0ull - b : b) + (MODE == MODE_TRACE ? xp[i] : 0ull);
+          v0[q] = (ng ? 0ull - b : b) + (trace ? xp[i] : 0ull);
         }
         group_sync(1);
 #pragma unroll
@@ -231,7 +236,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncthreads();  // spectra and the body init visible to both groups; every gather of the old mask words done
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      if (MODE == MODE_TRACE) {
+      if (trace) {
         cluster_arrive();  // phase A: this CTA no longer reads the old mask words
       } else if (co == 1) {
         // COMBINE2, mask column: the accumulator starts from zero (the D words were only needed by the gathers)
@@ -286,7 +291,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
           const double v = (q < 8) ? cur[q & 7].x : cur[q & 7].y;
           unsigned long long add;
           if (l == 3) {
-            const double t = MODE == MODE_TRACE ? fma(v, sgn_d, kMagic52 + 65536.0)
+            const double t = trace ? fma(v, sgn_d, kMagic52 + 65536.0)
                                                 : v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
             add = (unsigned long long)(long long)(int)__funnelshift_r((uint32_t)__double2loint(t), (uint32_t)__double2hiint(t), 17);
           } else {
@@ -297,7 +302,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
         }
       }
       __syncthreads();   // all four limbs are in the words of this CTA's column
-      if (MODE == MODE_TRACE) {
+      if (trace) {
         cluster_wait();    // phase A complete: CTA 0 has gathered the old mask words, CTA 1 may overwrite them
         // ------- finish the words (mask to 51 bits, rsh for the next step); CTA 1 mirrors them into CTA 0 -------
 #pragma unroll
@@ -333,7 +338,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
       }
     }  // steps
 
-    if (MODE == MODE_TRACE) {
+    if (trace) {
       // copy-out: every CTA its own column, all 512 threads
 #pragma unroll 4
       for (int q = 0; q < 8; q++) {

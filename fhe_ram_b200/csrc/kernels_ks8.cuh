@@ -20,6 +20,8 @@
 // MODE_COMBINE2 (GLWEPacker two-sided combine, one step): the words are D = rsh1(a X^-t - b), the base term of the
 // body column is s phi_g(D_body) only, and the output is normalize(S - y) X^t with S = rsh1(a X^-t + b) rebuilt from the
 // operands at the end.
+// MODE_MIXED (the packer level of a tree whose width is not a power of two): per item either MODE_COMBINE2 or one
+// MODE_TRACE step without rotation (the one-sided combine), chosen by the operand table (mixed_src, kernels.cuh).
 // Same integers as every other generation (tests/test_gpu_kernel_variants.py: "ks8"); keys in the order of k_prepare7.
 #pragma once
 #include "kernels_ext8.cuh"
@@ -64,7 +66,7 @@ __device__ __forceinline__ void cp_async_wait_n(int n) {
 template <int CL, int MODE>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const VmpArgs A, const double2* __restrict__ tw16) {
   static_assert(CL == 8 || CL == 4, "cluster of eight or four CTAs");
-  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2, "key-switch modes only");
+  static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2 || MODE == MODE_MIXED, "key-switch modes only");
   constexpr int LOUT = 4, NOUT = 2 * LOUT;
   constexpr int OPC = NOUT / CL;      // output polynomials per CTA
   constexpr int R = ks8_ring(CL);     // ring slots per output group
@@ -142,17 +144,22 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
   for (int item = cluster_id; item < A.n_items; item += n_clusters) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
     const int* src;
-    {
+    bool two = true;  // MODE_MIXED: the item has its second operand
+    if constexpr (MODE == MODE_MIXED) {
+      src = mixed_src(A, item, two);
+    } else {
       long idx = item;
       if (MODE == MODE_COMBINE2) idx = 2L * item;
       else if (A.src_div > 0) idx = item / A.src_div;
       else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
       src = A.src + idx * A.ct_stride;
     }
+    // this item's path: TRACE steps, or the two-sided combine (a constant unless MODE_MIXED)
+    const bool trace = MODE == MODE_MIXED ? !two : MODE == MODE_TRACE;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
     if (out_group) ring_fill(A.mat[0] + mat_off);
 
-    int rk = A.rot_const;
+    int rk = MODE == MODE_MIXED && trace ? 0 : A.rot_const;  // MODE_MIXED: the one-sided combine has no rotation
     if (MODE == MODE_TRACE) {
       if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
       rk &= (2 * kN - 1);
@@ -160,7 +167,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
     // the words before step 0 of column col at position i:
     // TRACE x = rsh1(src X^rk);  COMBINE2 D = rsh1(a X^-t - b) (plus = false) or S = rsh1(a X^-t + b) (plus = true)
     auto x_src = [&](int col, int i, bool plus) {
-      if (MODE == MODE_TRACE) {
+      if (trace) {
         bool neg;
         const int j = rot_index(i, 2 * kN - rk, neg);
         long long X = limbs_value(src[CT(col, 0) + j], src[CT(col, 1) + j], src[CT(col, 2) + j]);
@@ -258,7 +265,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
             const int e = (i * ginv) & (2 * kN - 1);
             const unsigned long long b = x_body(e & (kN - 1)) - kBias51;
             const bool ng = ((e >= kN ? 1u : 0u) ^ sgn_bit) != 0;
-            __stcg(Bout + i, (ng ? 0ull - b : b) + (MODE == MODE_TRACE ? x_body(i) : 0ull));
+            __stcg(Bout + i, (ng ? 0ull - b : b) + (trace ? x_body(i) : 0ull));
           }
         }
       }
@@ -295,7 +302,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
         // cur[m] = phi_g(vmp)[t + 128 m] + i phi_g(vmp)[t + 128 m + 2048] of limb l: round, shift to the limb's place
         unsigned long long* go = Cout + (size_t)o * kN + t;
         unsigned sgn = 0;
-        if (MODE == MODE_COMBINE2 && l == 3) {
+        if (!trace && l == 3) {
           // the carry chain runs in the pre-automorphism sign frame of each position (see k_ks3)
 #pragma unroll
           for (int m = 0; m < 16; m++) {
@@ -311,7 +318,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
           const double v = (q < 16) ? cur[q & 15].x : cur[q & 15].y;
           unsigned long long add;
           if (l == 3) {
-            const double tt = MODE == MODE_TRACE ? fma(v, sgn_d, kMagic52 + 65536.0)
+            const double tt = trace ? fma(v, sgn_d, kMagic52 + 65536.0)
                                                  : v + __hiloint2double(0x43380000, (int)(65536u - ((sgn >> q) & 1u)));
             add = (unsigned long long)(long long)(int)__funnelshift_r((uint32_t)__double2loint(tt),
                                                                       (uint32_t)__double2hiint(tt), 17);
@@ -339,10 +346,10 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
       for (int m = 0; m < 2 * kN / CL / 512; m++) {
         const int wi = rank * (2 * kN / CL) + tid + 512 * m;
         const int col = wi >> 12, i = wi & (kN - 1);
-        unsigned long long w = col == 1 ? (MODE == MODE_TRACE ? xm[i] : 0ull) : __ldcg(Bin + i);
+        unsigned long long w = col == 1 ? (trace ? xm[i] : 0ull) : __ldcg(Bin + i);
 #pragma unroll
         for (int ll = 0; ll < LOUT; ll++) w += __ldcg(Cin + (size_t)(col * LOUT + ll) * kN + i);
-        if (MODE == MODE_TRACE) {
+        if (trace) {
           const unsigned long long U = w & kMask51;
           dst[CT(col, 0) + i] = word_digit(U, 0);
           dst[CT(col, 1) + i] = word_digit(U, 1);

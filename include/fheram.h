@@ -240,7 +240,8 @@ int fheram_coordinate_product(fheram_ctx *ctx, const int64_t *glwe_in, int n, co
 int fheram_glwe_trace(fheram_ctx *ctx, const fheram_keys *k, const int64_t *in, int n, int start,
                       int end, int64_t *out);
 /* GLWEPacker: add(Some(in[rev(j)])) for rev(j) < n else add(None), then flush
- * (src/ram.rs:424-449); n a power of two <= N.  Coefficient h of out = coefficient 0 of in[h] */
+ * (src/ram.rs:424-449); any 1 <= n <= N (the read schedule of a RAM with n polynomials per sub-RAM, including its
+ * mixed level when n is not a power of two).  Coefficient h of out = coefficient 0 of in[h] */
 int fheram_glwe_pack(fheram_ctx *ctx, const fheram_keys *k, const int64_t *in, int n, int64_t *out);
 /* glwe_automorphism (mode 0) / _add (1) / _sub_negate (2) with trace key gal_idx, after an
  * optional glwe_rsh(1) (rsh != 0): n ciphertexts */
