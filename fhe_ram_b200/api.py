@@ -44,11 +44,21 @@ class CParams(C.Structure):
     ]
 
 
+class CSeed(C.Structure):
+    """fheram_seed: the state of a mask Source (ChaCha20 key, stream position in 32-bit words)"""
+    _fields_ = [("key", C.c_uint32 * 8), ("word0", C.c_uint64)]
+
+
+# seeds as numpy records (one per address of a batch), laid out as fheram_seed
+SEED_DTYPE = np.dtype([("key", "<u4", (8,)), ("word0", "<u8")], align=True)
+assert SEED_DTYPE.itemsize == C.sizeof(CSeed)
+
 _P64 = C.POINTER(C.c_int64)
 _PU8 = C.POINTER(C.c_uint8)
 _V = C.c_void_p
 _PV = C.POINTER(C.c_void_p)
 _PP = C.POINTER(CParams)
+_PS = C.POINTER(CSeed)
 
 # every symbol include/fheram.h declares: name -> (restype, argtypes)
 SIGNATURES = {
@@ -145,6 +155,15 @@ SIGNATURES = {
     "fheram_decrypt_ram": (C.c_int, [_PP, _P64, _P64, C.POINTER(C.c_int16), _P64]),
     "fheram_ram_decrypt_sk": (C.c_int, [_V, _P64, C.POINTER(C.c_int16), _P64]),
     "fheram_decrypt_words_device": (C.c_int, [_V, _V, C.c_int, _P64, C.POINTER(C.c_int16), _P64]),
+    "fheram_source_seed": (C.c_int, [_V, _PS]),
+    "fheram_encrypt_ram_seeded": (C.c_int, [_PP, _PU8, _P64, _V, _V, _P64, _PS]),
+    "fheram_encrypt_address_seeded": (C.c_int, [_PP, C.c_uint32, _P64, _V, _V, _P64, _PS]),
+    "fheram_ram_expand": (C.c_int, [_PP, _P64, _PS, _P64]),
+    "fheram_address_expand": (C.c_int, [_PP, _P64, _PS, _P64]),
+    "fheram_address_load_seeded": (C.c_int, [_V, _P64, _PS, C.c_int, _PV]),
+    "fheram_ram_read_batch_host_seeded": (C.c_int, [_V, C.POINTER(C.c_uint32), _PS, C.c_int, _V,
+                                                    C.POINTER(C.c_int32)]),
+    "fheram_ram_load_seeded": (C.c_int, [_V, _P64, _PS]),
 }
 
 _lib = None
@@ -327,6 +346,19 @@ def unpack17(packed: np.ndarray, n: int) -> np.ndarray:
     return out
 
 
+def _ps(seeds: np.ndarray, n: int):
+    assert seeds.dtype == SEED_DTYPE and seeds.flags["C_CONTIGUOUS"] and seeds.size == n, \
+        f"{n} seed(s) of SEED_DTYPE expected"
+    return seeds.ctypes.data_as(_PS)
+
+
+def _seeds(seeds) -> np.ndarray:
+    """one SEED_DTYPE array from an array of seeds or a list of them"""
+    if isinstance(seeds, (list, tuple)):
+        seeds = np.concatenate([np.asarray(x, dtype=SEED_DTYPE).reshape(-1) for x in seeds])
+    return np.ascontiguousarray(np.asarray(seeds, dtype=SEED_DTYPE).reshape(-1))
+
+
 def host_register(a: np.ndarray):
     _check(lib().fheram_host_register(a.ctypes.data_as(C.c_void_p), a.nbytes))
 
@@ -356,6 +388,12 @@ class Source:
     def fill_bytes(self, n: int) -> np.ndarray:
         out = np.zeros(n, dtype=np.uint8)
         lib().fheram_source_fill_bytes(self.h, out.ctypes.data_as(_PU8), n)
+        return out
+
+    def seed(self) -> np.ndarray:
+        """the seed of the current position (one SEED_DTYPE record, shape (1,))"""
+        out = np.zeros(1, dtype=SEED_DTYPE)
+        _check(lib().fheram_source_seed(self.h, _ps(out, 1)))
         return out
 
     def __del__(self):
@@ -469,6 +507,44 @@ class Address:
                                             source_xe.h, _p(self.data)))
         self._drop()
         return self
+
+    @staticmethod
+    def encrypt_sk_seeded(params: Parameters, value: int, sk: GLWESecret, source_xa: Source, source_xe: Source):
+        """Address::encrypt_sk in the seeded form (include/fheram.h): (bodies int64 [n_ggsw][dnum][2][size][N]
+        flattened, seed).  The rows with ci = 1 carry their plaintext in the body, so the limbs differ from
+        `encrypt_sk`'s (same phase, same noise); both Sources end where `encrypt_sk` leaves them."""
+        bodies = np.zeros(params.n_ggsw() * params.ggsw_len() // 2, dtype=np.int64)
+        seed = np.zeros(1, dtype=SEED_DTYPE)
+        _check(lib().fheram_encrypt_address_seeded(C.byref(params.c), int(value), _p(sk.data), source_xa.h,
+                                                   source_xe.h, _p(bodies), _ps(seed, 1)))
+        return bodies, seed
+
+    @classmethod
+    def expand(cls, params: Parameters, bodies: np.ndarray, seeds, count: int = 1) -> "Address":
+        """full limbs of `count` seeded addresses (CPU): what the device expansion builds"""
+        seeds = _seeds(seeds)
+        bodies = np.ascontiguousarray(bodies, dtype=np.int64).reshape(count, -1)
+        per = params.n_ggsw() * params.ggsw_len()
+        if bodies.shape[1] != per // 2 or seeds.size != count:
+            raise FheRamError(-1, "bodies / seeds do not hold `count` addresses")
+        out = np.zeros((count, per), dtype=np.int64)
+        for i in range(count):
+            _check(lib().fheram_address_expand(C.byref(params.c), _p(bodies[i]), _ps(seeds[i:i + 1], 1), _p(out[i])))
+        return cls.from_limbs(params, out, count)
+
+    @classmethod
+    def load_seeded(cls, params: Parameters, bodies: np.ndarray, seeds, count: int = 1) -> "Address":
+        """`count` seeded addresses made resident and prepared; the masks are regenerated on the device"""
+        seeds = _seeds(seeds)
+        bodies = np.ascontiguousarray(bodies, dtype=np.int64).reshape(-1)
+        if bodies.size != count * params.n_ggsw() * params.ggsw_len() // 2:
+            raise FheRamError(-1, "bodies do not hold `count` addresses")
+        a = cls.__new__(cls)
+        a.params, a.data, a.count = params, None, count
+        h = C.c_void_p()
+        _check(lib().fheram_address_load_seeded(params.module(), _p(bodies), _ps(seeds, count), count, C.byref(h)))
+        a.h = h
+        return a
 
     @classmethod
     def from_limbs(cls, params: Parameters, limbs: np.ndarray, count: int = 1) -> "Address":
@@ -598,6 +674,37 @@ class Ram:
         self.load(cts)
         return cts
 
+    def encrypt_sk_seeded(self, data, sk: GLWESecret, source_xa: Source, source_xe: Source):
+        """Ram::encrypt_sk in the seeded form (CPU), then `load_seeded`: returns (bodies, seed).  Expanded, they are
+        exactly the limbs `encrypt_sk` returns from the same Sources."""
+        p = self.params
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        if data.size != p.max_addr() * p.word_size():
+            raise FheRamError(-1, f"invalid data: {data.size} bytes != max_addr * word_size")
+        bodies = np.zeros(self.glwe_count() * p.glwe_len() // 2, dtype=np.int64)
+        seed = np.zeros(1, dtype=SEED_DTYPE)
+        _check(lib().fheram_encrypt_ram_seeded(C.byref(p.c), data.ctypes.data_as(_PU8), _p(sk.data), source_xa.h,
+                                               source_xe.h, _p(bodies), _ps(seed, 1)))
+        self.load_seeded(bodies, seed)
+        return bodies, seed
+
+    @staticmethod
+    def expand(params: Parameters, bodies: np.ndarray, seed) -> np.ndarray:
+        """full limbs of a seeded RAM (CPU), in `encrypt_sk` / `store` layout"""
+        bodies = np.ascontiguousarray(bodies, dtype=np.int64).reshape(-1)
+        cts = np.zeros(2 * bodies.size, dtype=np.int64)
+        if cts.size != params.word_size() * params.n_glwe() * params.glwe_len():
+            raise FheRamError(-1, "bodies are not a whole RAM")
+        _check(lib().fheram_ram_expand(C.byref(params.c), _p(bodies), _ps(_seeds(seed), 1), _p(cts)))
+        return cts
+
+    def load_seeded(self, bodies: np.ndarray, seed):
+        """`load` of a seeded RAM (bodies of the whole RAM; a sharded RAM expands its own polynomials)"""
+        bodies = np.ascontiguousarray(bodies, dtype=np.int64).reshape(-1)
+        if 2 * bodies.size != self.glwe_count() * self.params.glwe_len():
+            raise FheRamError(-1, "bodies are not a whole RAM")
+        _check(lib().fheram_ram_load_seeded(self.h, _p(bodies), _ps(_seeds(seed), 1)))
+
     def encrypt_sk_gpu(self, data, sk: GLWESecret, source_xa: Source, source_xe: Source) -> None:
         """src/ram.rs:129-167 on the device (k_glwe_encrypt), straight into the resident RAM: the same
         limbs as `encrypt_sk` from the same Sources, without the host round trip."""
@@ -691,6 +798,19 @@ class Ram:
             out = np.zeros((n, self.params.word_size(), self.params.glwe_len()), dtype=np.int32)
         _check(lib().fheram_ram_read_batch_host_p17(self.h, a.ctypes.data_as(C.POINTER(C.c_uint32)), n, keys.h,
                                                     out.reshape(-1).ctypes.data_as(C.POINTER(C.c_int32))))
+        return out
+
+    def read_batch_host_seeded(self, bodies_p17: np.ndarray, seeds, n: int, keys: EvaluationKeysPrepared,
+                               out=None) -> np.ndarray:
+        """n seeded addresses: their bodies packed by `pack17` and one seed each; int32 limbs out"""
+        a = np.ascontiguousarray(bodies_p17, dtype=np.uint32).reshape(-1)
+        if a.size != n * self.params.n_ggsw() * self.params.ggsw_len() // 2 * 17 // 32:
+            raise FheRamError(-1, "bodies_p17 does not hold n packed addresses")
+        if out is None:
+            out = np.zeros((n, self.params.word_size(), self.params.glwe_len()), dtype=np.int32)
+        _check(lib().fheram_ram_read_batch_host_seeded(self.h, a.ctypes.data_as(C.POINTER(C.c_uint32)),
+                                                       _ps(_seeds(seeds), n), n, keys.h,
+                                                       out.reshape(-1).ctypes.data_as(C.POINTER(C.c_int32))))
         return out
 
     def read_batch_device(self, addresses: Address, keys: EvaluationKeysPrepared) -> int:

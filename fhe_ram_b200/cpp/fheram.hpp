@@ -36,6 +36,11 @@ class Source {  // poulpy_hal::source::Source
   uint32_t next_u32() { return fheram_source_next_u32(h_); }
   void fill_bytes(std::vector<uint8_t>& v) { fheram_source_fill_bytes(h_, v.data(), v.size()); }
   fheram_source* raw() { return h_; }
+  fheram_seed seed() const {  // the state of the stream here (seeded ciphertexts, fheram.h)
+    fheram_seed s;
+    check(fheram_source_seed(h_, &s));
+    return s;
+  }
 
  private:
   fheram_source* h_;
@@ -121,18 +126,33 @@ class Address {  // src/address.rs:21-24
   void encrypt_sk(const Parameters& p, uint32_t value, const GLWESecret& sk, Source& xa, Source& xe) {  // :86-109
     check(fheram_encrypt_address(&p.c, value, sk.data.data(), xa.raw(), xe.raw(), data.data()));
     if (h_) { fheram_address_destroy(h_); h_ = nullptr; }
+    seeded_ = false;
+    bodies.clear();
+  }
+  // the seeded form (fheram.h): bodies + the mask Source's seed, half the bytes; data = its expanded limbs (another
+  // valid encryption than encrypt_sk's), device() uploads the bodies and regenerates the masks on the GPU
+  void encrypt_sk_seeded(const Parameters& p, uint32_t value, const GLWESecret& sk, Source& xa, Source& xe) {
+    bodies.resize(data.size() / 2);
+    check(fheram_encrypt_address_seeded(&p.c, value, sk.data.data(), xa.raw(), xe.raw(), bodies.data(), &seed));
+    check(fheram_address_expand(&p.c, bodies.data(), &seed, data.data()));
+    if (h_) { fheram_address_destroy(h_); h_ = nullptr; }
+    seeded_ = true;
   }
   fheram_address* device() {  // resident + CoordinatePrepared::prepare
-    if (!h_) check(fheram_address_load(p_.module(), data.data(), &h_));
+    if (!h_) check(seeded_ ? fheram_address_load_seeded(p_.module(), bodies.data(), &seed, 1, &h_)
+                           : fheram_address_load(p_.module(), data.data(), &h_));
     return h_;
   }
   ~Address() { if (h_) fheram_address_destroy(h_); }
   std::vector<int64_t> data;
+  std::vector<int64_t> bodies;  // seeded form only
+  fheram_seed seed{};
 
  private:
   explicit Address(Parameters& p) : data(p.n_ggsw() * p.ggsw_len()), p_(p) {}
   Parameters& p_;
   fheram_address* h_ = nullptr;
+  bool seeded_ = false;
 };
 
 using GLWE = std::vector<int64_t>;
@@ -153,6 +173,29 @@ class Ram {  // src/ram.rs:25-29
     if (data.size() / p_.word_size() != p_.max_addr()) throw Panic(-1, "invalid data: data.len()/ram_chunks != max_addr");
     // on the device, straight into the resident RAM: the limbs fheram_encrypt_ram + fheram_ram_load would install
     check(fheram_ram_encrypt_sk(h_, data.data(), sk.data.data(), xa.raw(), xe.raw()));
+  }
+  // Ram::encrypt_sk on the client (CPU) in the seeded form, then load_seeded: bodies + seed are what a separated
+  // client ships (half the bytes of the limbs), and they expand to exactly the limbs of fheram_encrypt_ram
+  void encrypt_sk_seeded(const std::vector<uint8_t>& data, const GLWESecret& sk, Source& xa, Source& xe,
+                         std::vector<int64_t>& bodies, fheram_seed& seed) {
+    if (data.size() != p_.max_addr() * p_.word_size()) throw Panic(-1, "invalid data: data.len() != max_addr * ram_chunks");
+    bodies.resize(p_.word_size() * p_.n_glwe() * p_.glwe_len() / 2);
+    check(fheram_encrypt_ram_seeded(&p_.c, data.data(), sk.data.data(), xa.raw(), xe.raw(), bodies.data(), &seed));
+    load_seeded(bodies, seed);
+  }
+  void load_seeded(const std::vector<int64_t>& bodies, const fheram_seed& seed) {
+    if (bodies.size() != p_.word_size() * p_.n_glwe() * p_.glwe_len() / 2) throw Panic(-1, "bodies are not a whole RAM");
+    check(fheram_ram_load_seeded(h_, bodies.data(), &seed));
+  }
+  // n seeded addresses from host buffers: bodies packed by fheram_pack17, one seed each; int32 limbs out
+  std::vector<int32_t> read_batch_host_seeded(const std::vector<uint32_t>& bodies_p17, const std::vector<fheram_seed>& seeds,
+                                              const EvaluationKeysPrepared& k) {
+    const int n = (int)seeds.size();
+    if (bodies_p17.size() != (size_t)n * p_.n_ggsw() * p_.ggsw_len() / 2 * 17 / 32)
+      throw Panic(-1, "bodies_p17 does not hold one packed address per seed");
+    std::vector<int32_t> out((size_t)n * p_.word_size() * p_.glwe_len());
+    check(fheram_ram_read_batch_host_seeded(h_, bodies_p17.data(), seeds.data(), n, k.raw(), out.data()));
+    return out;
   }
   std::vector<GLWE> read(Address& a, const EvaluationKeysPrepared& k) {  // :172-191
     std::vector<int64_t> out(p_.word_size() * p_.glwe_len());

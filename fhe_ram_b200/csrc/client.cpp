@@ -283,17 +283,38 @@ void atk_encrypt(const Ring& R, int K, i64* key, int rows, int size, int k_noise
   gglwe_encrypt(R, K, key, rows, size, k_noise, sk, so, xa, xe);
 }
 
+// seeded: the rows with ci = 1 carry scalar * s in the body instead of scalar in the mask (same phase, raw mask)
 void ggsw_encrypt(const Ring& R, const Dims& d, int k_addr, i64* ggsw, const i64* scalar,
-                  const std::vector<cd>& sk_spec, fheram_source* xa, fheram_source* xe) {
+                  const std::vector<cd>& sk_spec, fheram_source* xa, fheram_source* xe, bool seeded = false) {
   const int n = d.n, S = d.size_addr;
   const size_t glwe = (size_t)2 * S * n;
-  std::vector<i64> pt((size_t)S * n);
+  std::vector<i64> pt((size_t)S * n), pt_s, ms;
+  if (seeded) {  // scalar * s: a signed rotation of the secret, exact through the transform
+    std::vector<cd> spec, prod;
+    R.forward(scalar, spec);
+    R.mul(spec, sk_spec, prod);
+    ms.resize(n);
+    R.inverse(prod, ms.data());
+    pt_s.resize((size_t)S * n);
+  }
   for (int r = 0; r < d.dnum_ct; r++) {
     std::fill(pt.begin(), pt.end(), 0);
     memcpy(pt.data() + (size_t)r * n, scalar, sizeof(i64) * n);
-    for (int ci = 0; ci < 2; ci++)
-      glwe_encrypt(R, d.K, ggsw + ((size_t)r * 2 + ci) * glwe, S, k_addr, pt.data(), r + 1, ci, sk_spec, xa, xe);
+    if (seeded) {
+      std::fill(pt_s.begin(), pt_s.end(), 0);
+      memcpy(pt_s.data() + (size_t)r * n, ms.data(), sizeof(i64) * n);
+    }
+    for (int ci = 0; ci < 2; ci++) {
+      const bool body = seeded && ci == 1;
+      glwe_encrypt(R, d.K, ggsw + ((size_t)r * 2 + ci) * glwe, S, k_addr, body ? pt_s.data() : pt.data(), r + 1,
+                   body ? 0 : ci, sk_spec, xa, xe);
+    }
   }
+}
+
+// body columns of n_glwe GLWEs of `size` limbs: [n_glwe][size][2][N] -> [n_glwe][size][N]
+void take_bodies(int n, int size, size_t n_glwe, const i64* ct, i64* bodies) {
+  for (size_t t = 0; t < n_glwe * size; t++) memcpy(bodies + t * n, ct + t * 2 * n, sizeof(i64) * n);
 }
 
 // value * 2^-k placed in `size` limbs (torus wrap), coefficient idx
@@ -349,16 +370,17 @@ extern "C" int fheram_keygen(const fheram_params* p, const int64_t* sk, fheram_s
   return 0;
 }
 
-extern "C" int fheram_encrypt_ram(const fheram_params* p, const uint8_t* data, const int64_t* sk,
-                                  fheram_source* xa, fheram_source* xe, int64_t* cts) {
-  if (check(p) || !data || !sk || !xa || !xe || !cts) return FHERAM_ERR_INVALID;
+namespace {
+// Ram::encrypt_sk: every GLWE into cts, or (cts null) its body column into bodies
+int encrypt_ram(const fheram_params* p, const uint8_t* data, const int64_t* sk, fheram_source* xa,
+                fheram_source* xe, int64_t* cts, int64_t* bodies) {
   const Dims d = dims(p);
   Ring R(d.log_n);
   std::vector<cd> s_spec;
   R.forward(sk, s_spec);
   const int ws = p->word_size, pt_size = cdiv(p->k_pt, d.K);
   const size_t glwe = fheram_glwe_len(p);
-  std::vector<i64> pt((size_t)pt_size * d.n);
+  std::vector<i64> pt((size_t)pt_size * d.n), one(cts ? 0 : glwe);
   for (int i = 0; i < ws; i++)           // src/ram.rs:161-166
     for (int h = 0; h < d.n_glwe; h++) { // src/ram.rs:358-379
       std::fill(pt.begin(), pt.end(), 0);
@@ -367,10 +389,19 @@ extern "C" int fheram_encrypt_ram(const fheram_params* p, const uint8_t* data, c
         const i64 v = addr < p->max_addr ? (i64)(int8_t)data[addr * ws + i] : 0;  // :364
         encode_coeff(d.n, d.K, pt.data(), pt_size, j, v, p->k_pt);                // :368
       }
-      glwe_encrypt(R, d.K, cts + ((size_t)i * d.n_glwe + h) * glwe, d.size_ct, p->k_ct, pt.data(), pt_size, 0,
-                   s_spec, xa, xe);
+      const size_t g = (size_t)i * d.n_glwe + h;
+      i64* ct = cts ? cts + g * glwe : one.data();
+      glwe_encrypt(R, d.K, ct, d.size_ct, p->k_ct, pt.data(), pt_size, 0, s_spec, xa, xe);
+      if (!cts) take_bodies(d.n, d.size_ct, 1, ct, bodies + g * glwe / 2);
     }
   return 0;
+}
+}  // namespace
+
+extern "C" int fheram_encrypt_ram(const fheram_params* p, const uint8_t* data, const int64_t* sk,
+                                  fheram_source* xa, fheram_source* xe, int64_t* cts) {
+  if (check(p) || !data || !sk || !xa || !xe || !cts) return FHERAM_ERR_INVALID;
+  return encrypt_ram(p, data, sk, xa, xe, cts, nullptr);
 }
 
 int fheram_address_monomials(const fheram_params* p, uint32_t value, int32_t* pos_out, int32_t* sign_out) {
@@ -403,9 +434,10 @@ int fheram_address_monomials(const fheram_params* p, uint32_t value, int32_t* po
   return g;
 }
 
-extern "C" int fheram_encrypt_address(const fheram_params* p, uint32_t value, const int64_t* sk,
-                                      fheram_source* xa, fheram_source* xe, int64_t* ggsw) {
-  if (check(p) || !sk || !xa || !xe || !ggsw) return FHERAM_ERR_INVALID;
+namespace {
+// Address::encrypt_sk: every GGSW into ggsw, or (ggsw null) the seeded form's body columns into bodies
+int encrypt_address(const fheram_params* p, uint32_t value, const int64_t* sk, fheram_source* xa,
+                    fheram_source* xe, int64_t* ggsw, int64_t* bodies) {
   const Dims d = dims(p);
   int32_t pos[64], sign[64];
   const int n_ggsw = fheram_address_monomials(p, value, pos, sign);
@@ -414,13 +446,22 @@ extern "C" int fheram_encrypt_address(const fheram_params* p, uint32_t value, co
   std::vector<cd> s_spec;
   R.forward(sk, s_spec);
   const size_t ggsw_len = fheram_ggsw_len(p);
-  std::vector<i64> scalar(d.n, 0);
+  std::vector<i64> scalar(d.n, 0), one(ggsw ? 0 : ggsw_len);
   for (int g = 0; g < n_ggsw; g++) {
     scalar[pos[g]] = sign[g];
-    ggsw_encrypt(R, d, p->k_addr, ggsw + (size_t)g * ggsw_len, scalar.data(), s_spec, xa, xe);
+    i64* out = ggsw ? ggsw + (size_t)g * ggsw_len : one.data();
+    ggsw_encrypt(R, d, p->k_addr, out, scalar.data(), s_spec, xa, xe, !ggsw);
+    if (!ggsw) take_bodies(d.n, d.size_addr, (size_t)d.dnum_ct * 2, out, bodies + (size_t)g * ggsw_len / 2);
     scalar[pos[g]] = 0;
   }
   return 0;
+}
+}  // namespace
+
+extern "C" int fheram_encrypt_address(const fheram_params* p, uint32_t value, const int64_t* sk,
+                                      fheram_source* xa, fheram_source* xe, int64_t* ggsw) {
+  if (check(p) || !sk || !xa || !xe || !ggsw) return FHERAM_ERR_INVALID;
+  return encrypt_address(p, value, sk, xa, xe, ggsw, nullptr);
 }
 
 extern "C" int fheram_encrypt_word(const fheram_params* p, uint8_t value, const int64_t* sk,
@@ -434,6 +475,70 @@ extern "C" int fheram_encrypt_word(const fheram_params* p, uint8_t value, const 
   std::vector<i64> pt((size_t)pt_size * d.n, 0);
   encode_coeff(d.n, d.K, pt.data(), pt_size, 0, (i64)value, p->k_pt);  // examples/fhe-ram.rs:197
   glwe_encrypt(R, d.K, glwe, d.size_ct, p->k_ct, pt.data(), pt_size, 0, s_spec, xa, xe);
+  return 0;
+}
+
+// ---- seeded ciphertexts (fheram.h): bodies + the mask Source's state ----
+extern "C" int fheram_source_seed(const fheram_source* s, fheram_seed* seed) {
+  if (!s || !seed) { fheram_set_error("fheram_source_seed: null argument"); return FHERAM_ERR_INVALID; }
+  fheram_source_tell(s, seed->key, &seed->word0);
+  return 0;
+}
+
+namespace {
+int check_seeded(const fheram_params* p, const int64_t* sk, const fheram_source* xa, const fheram_source* xe,
+                 const void* bodies, const fheram_seed* seed) {
+  if (check(p)) return FHERAM_ERR_INVALID;
+  if (!sk || !xa || !xe || !bodies || !seed) { fheram_set_error("null argument"); return FHERAM_ERR_INVALID; }
+  if (xa == xe) { fheram_set_error("mask and noise need distinct Sources"); return FHERAM_ERR_INVALID; }
+  return 0;
+}
+
+// n_glwe GLWEs of `size` limbs from their bodies ([n_glwe][size][N]) and the mask stream of seed
+void expand(const Dims& d, int size, size_t n_glwe, const i64* bodies, const fheram_seed* seed, i64* out) {
+  fheram_source s;
+  memcpy(s.key, seed->key, sizeof(s.key));
+  fheram_source_skip_words(&s, seed->word0);
+  const size_t n = (size_t)d.n;
+  for (size_t t = 0; t < n_glwe * size; t++) {  // (GLWE, limb) in stream order, as glwe_encrypt draws them
+    memcpy(out + t * 2 * n, bodies + t * n, sizeof(i64) * n);
+    i64* a = out + (t * 2 + 1) * n;
+    for (size_t i = 0; i < n; i++) a[i] = digit(d.K, (i64)s.next());
+  }
+}
+}  // namespace
+
+extern "C" int fheram_encrypt_ram_seeded(const fheram_params* p, const uint8_t* data, const int64_t* sk,
+                                         fheram_source* xa, fheram_source* xe, int64_t* bodies, fheram_seed* seed) {
+  if (int rc = check_seeded(p, sk, xa, xe, bodies, seed)) return rc;
+  if (!data) { fheram_set_error("null argument"); return FHERAM_ERR_INVALID; }
+  fheram_source_tell(xa, seed->key, &seed->word0);
+  return encrypt_ram(p, data, sk, xa, xe, nullptr, bodies);
+}
+
+extern "C" int fheram_encrypt_address_seeded(const fheram_params* p, uint32_t value, const int64_t* sk,
+                                             fheram_source* xa, fheram_source* xe, int64_t* bodies,
+                                             fheram_seed* seed) {
+  if (int rc = check_seeded(p, sk, xa, xe, bodies, seed)) return rc;
+  fheram_source_tell(xa, seed->key, &seed->word0);
+  return encrypt_address(p, value, sk, xa, xe, nullptr, bodies);
+}
+
+extern "C" int fheram_ram_expand(const fheram_params* p, const int64_t* bodies, const fheram_seed* seed,
+                                 int64_t* cts) {
+  if (check(p)) return FHERAM_ERR_INVALID;
+  if (!bodies || !seed || !cts) { fheram_set_error("fheram_ram_expand: null argument"); return FHERAM_ERR_INVALID; }
+  const Dims d = dims(p);
+  expand(d, d.size_ct, (size_t)p->word_size * d.n_glwe, bodies, seed, cts);
+  return 0;
+}
+
+extern "C" int fheram_address_expand(const fheram_params* p, const int64_t* bodies, const fheram_seed* seed,
+                                     int64_t* ggsw) {
+  if (check(p)) return FHERAM_ERR_INVALID;
+  if (!bodies || !seed || !ggsw) { fheram_set_error("fheram_address_expand: null argument"); return FHERAM_ERR_INVALID; }
+  const Dims d = dims(p);
+  expand(d, d.size_addr, (size_t)d.n_ggsw * d.dnum_ct * 2, bodies, seed, ggsw);
   return 0;
 }
 

@@ -8,6 +8,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -230,6 +231,7 @@ struct fheram_ctx {
   DevBuf enc_buf[15];  // operands of the encryption kernels, kept between calls (cudaFree synchronizes the device)
   uint64_t enc_stats[3] = {0, 0, 0};  // noise draws sampled on the device / patched by the host / streams resampled on the host
   DevBuf dec_buf[2];   // decrypted values / errors on their way to the host (zeroed after every download)
+  DevBuf seed_buf[2];  // seeded loads: the seeds and the stream position of every GLWE
   DevBuf opbuf[3];  // op-level entry points
   long long* d_phase = nullptr;  // per-CTA phase cycle counters (fheram_debug_phase_cycles)
   // per-kernel-class CUDA-event timing (fheram_ctx_profile)
@@ -441,6 +443,7 @@ extern "C" int fheram_ctx_destroy(fheram_ctx* c) {
   for (auto& b : c->opbuf) b.release();
   for (auto& b : c->enc_buf) b.release();
   for (auto& b : c->dec_buf) b.release();
+  for (auto& b : c->seed_buf) b.release();
   cudaFree(c->d_tw); cudaFree(c->d_tw16); cudaFree(c->d_err);
   if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
   if (c->side) {
@@ -635,6 +638,14 @@ __global__ void k_unpack17(const uint32_t* __restrict__ in, int* __restrict__ ou
     out[i] = (int)(f << 15) >> 15;
   }
 }
+// reports (and clears) the range flag k_i64_to_i32 / k_glwe_expand set on a limb outside +-2^30
+static int take_range_error(fheram_ctx* c) {
+  int err = 0;
+  CU(cudaMemcpy(&err, c->d_err, sizeof(int), cudaMemcpyDeviceToHost));
+  if (!err) return 0;
+  CU(cudaMemset(c->d_err, 0, sizeof(int)));
+  return fail(FHERAM_ERR_RANGE, "limb outside +-2^30: ciphertext limbs must be (nearly) normalised");
+}
 static int upload_i64(fheram_ctx* c, const int64_t* h, size_t n, int* d_out) {
   const size_t chunk = (size_t)64 << 20;  // limbs per staging pass (512 MiB of int64)
   for (size_t off = 0; off < n; off += chunk) {
@@ -645,13 +656,7 @@ static int upload_i64(fheram_ctx* c, const int64_t* h, size_t n, int* d_out) {
     c->launches++;
     CU(cudaStreamSynchronize(c->stream));
   }
-  int err = 0;
-  CU(cudaMemcpy(&err, c->d_err, sizeof(int), cudaMemcpyDeviceToHost));
-  if (err) {
-    CU(cudaMemset(c->d_err, 0, sizeof(int)));
-    return fail(FHERAM_ERR_RANGE, "limb outside +-2^30: ciphertext limbs must be (nearly) normalised");
-  }
-  return 0;
+  return take_range_error(c);
 }
 static int download_i64(fheram_ctx* c, const int* d_in, size_t n, int64_t* h) {
   if (n <= kSmallDownload) {
@@ -986,6 +991,69 @@ extern "C" int fheram_address_prepare(fheram_address* a) {  // CoordinatePrepare
 extern "C" int fheram_address_load(fheram_ctx* c, const int64_t* ggsw, fheram_address** out) {
   return fheram_address_load_batch(c, ggsw, 1, out);
 }
+
+// ---- seeded uploads (fheram.h fheram_seed): bodies from the host, masks regenerated by k_glwe_expand ----
+static_assert(sizeof(Seed) == sizeof(fheram_seed) && offsetof(fheram_seed, word0) == offsetof(Seed, word0),
+              "Seed mirrors fheram_seed");
+static int launch_expand(fheram_ctx* c, const ExpandArgs& a, cudaStream_t st) {
+  const long items = (long)a.n_glwe * a.size;
+  const int grid = items < 8L * c->sm_count ? (int)items : 8 * c->sm_count;
+  k_glwe_expand<<<grid, kThreads, 0, st>>>(a);
+  c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
+// one pass of a seeded upload from int64 bodies: a.n_glwe GLWEs' bodies (host) through the staging buffer into
+// k_glwe_expand (a.out, a.ct_stride, a.size, a.seeds, a.glwe_per_stream and a.seq set by the caller)
+static int expand_pass_i64(fheram_ctx* c, const int64_t* bodies, ExpandArgs a) {
+  const size_t limbs = (size_t)a.n_glwe * a.size * c->d.n;
+  TRY(c->stage64.ensure(limbs * sizeof(int64_t)));
+  CU(cudaMemcpyAsync(c->stage64.p, bodies, limbs * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+  a.body64 = (const long long*)c->stage64.p;
+  a.body17 = nullptr;
+  a.err = c->d_err;
+  TRY(launch_expand(c, a, c->stream));
+  CU(cudaStreamSynchronize(c->stream));  // the host buffer and the staging buffer are reused by the next pass
+  return 0;
+}
+extern "C" int fheram_address_load_seeded(fheram_ctx* c, const int64_t* bodies, const fheram_seed* seeds, int n,
+                                          fheram_address** out) {
+  if (!c || !bodies || !seeds || !out || n < 1) return fail(FHERAM_ERR_INVALID, "bad argument");
+  CU(cudaSetDevice(c->device));
+  const Derived& d = c->d;
+  const int per = d.n_ggsw * d.dnum_ct * 2;                     // GLWEs per address, one stream
+  const size_t body_per = (size_t)per * d.size_addr * d.n;      // body limbs per address
+  const size_t nm = (size_t)n * d.n_ggsw;
+  fheram_address* a = new fheram_address();
+  a->c = c; a->count = n;
+  auto run = [&]() -> int {
+    CU(cudaMalloc(&a->raw, sizeof(int) * nm * c->ggsw_raw_len()));
+    CU(cudaMalloc(&a->prep, sizeof(double2) * nm * c->ggsw_prep_len()));
+    DevBuf& d_seed = c->seed_buf[0];
+    TRY(d_seed.ensure(sizeof(Seed) * n));
+    CU(cudaMemcpyAsync(d_seed.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, c->stream));
+    const size_t step_l = ((size_t)64 << 20) / body_per;        // addresses per pass: at most 64 Mi staged limbs
+    const int step = step_l < 1 ? 1 : (step_l > (size_t)n ? n : (int)step_l);
+    for (int i0 = 0; i0 < n; i0 += step) {
+      const int m = n - i0 < step ? n - i0 : step;
+      ExpandArgs e;
+      memset(&e, 0, sizeof(e));
+      e.out = a->raw + (size_t)i0 * d.n_ggsw * c->ggsw_raw_len();
+      e.ct_stride = (long)2 * d.size_addr * d.n;
+      e.n_glwe = m * per; e.size = d.size_addr;
+      e.seeds = (const Seed*)d_seed.p + i0;
+      e.glwe_per_stream = per;
+      TRY(expand_pass_i64(c, bodies + (size_t)i0 * body_per, e));
+    }
+    TRY(take_range_error(c));
+    TRY(prepare_ggsw(c, a->raw, a->prep, (int)nm));  // CoordinatePrepared::prepare, as fheram_address_load_batch
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+  };
+  if (int rc = run()) { fheram_address_destroy(a); return rc; }
+  *out = a;
+  return 0;
+}
 extern "C" int fheram_address_count(const fheram_address* a) { return a ? a->count : 0; }
 extern "C" int fheram_address_destroy(fheram_address* a) {
   if (!a) return 0;
@@ -1178,6 +1246,7 @@ struct fheram_ram {
     cudaEvent_t out_ready[2] = {nullptr, nullptr}, out_done[2] = {nullptr, nullptr};
     cudaStream_t copy_stream = nullptr, down_stream = nullptr;
     int cap = 0;
+    DevBuf seeds;            // the seeds of a seeded batch
   } pipe;
 };
 
@@ -1234,6 +1303,7 @@ extern "C" int fheram_ram_destroy(fheram_ram* r) {
     if (r->pipe.out_ready[i]) cudaEventDestroy(r->pipe.out_ready[i]);
     if (r->pipe.out_done[i]) cudaEventDestroy(r->pipe.out_done[i]);
   }
+  r->pipe.seeds.release();
   if (r->pipe.copy_stream) cudaStreamDestroy(r->pipe.copy_stream);
   if (r->pipe.down_stream) cudaStreamDestroy(r->pipe.down_stream);
   delete r;
@@ -1260,6 +1330,47 @@ extern "C" int fheram_ram_load(fheram_ram* r, const int64_t* cts) {
       TRY(upload_i64(c, gathered.data(), (size_t)r->n_local * L, r->data + (size_t)s * r->n_local * L));
     }
   }
+  r->loaded = true;
+  r->state = false;
+  r->rotated = false;
+  return 0;
+}
+// bodies: the FULL RAM's bodies [word_size][n_glwe][size_ct][N]; a sharded RAM expands h = shard + n_shards*h'
+extern "C" int fheram_ram_load_seeded(fheram_ram* r, const int64_t* bodies, const fheram_seed* seed) {
+  if (!r || !bodies || !seed) return fail(FHERAM_ERR_INVALID, "null argument");
+  fheram_ctx* c = r->c;
+  CU(cudaSetDevice(c->device));
+  const int ws = c->params.word_size, G = c->d.n_glwe, S = c->d.size_ct, nl = r->n_local;
+  const size_t B = (size_t)S * c->d.n;  // body limbs per GLWE
+  const long L = c->ct_stride();
+  // stream position of every local GLWE: polynomial h of sub-RAM s is GLWE s G + h of the RAM (one stream)
+  std::vector<int> seq((size_t)ws * nl);
+  for (int s = 0; s < ws; s++)
+    for (int hp = 0; hp < nl; hp++) seq[(size_t)s * nl + hp] = s * G + r->shard + r->n_shards * hp;
+  DevBuf &d_seed = c->seed_buf[0], &d_seq = c->seed_buf[1];
+  TRY(d_seed.ensure(sizeof(Seed)));
+  TRY(d_seq.ensure(sizeof(int) * seq.size()));
+  CU(cudaMemcpyAsync(d_seed.p, seed, sizeof(Seed), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(d_seq.p, seq.data(), sizeof(int) * seq.size(), cudaMemcpyHostToDevice, c->stream));
+  std::vector<int64_t> gathered(r->n_shards > 1 ? (size_t)nl * B : 0);
+  for (int s = 0; s < ws; s++) {  // one pass per sub-RAM
+    const int64_t* src = bodies + (size_t)s * G * B;
+    if (r->n_shards > 1) {
+      for (int hp = 0; hp < nl; hp++)
+        memcpy(gathered.data() + (size_t)hp * B, src + (size_t)(r->shard + r->n_shards * hp) * B, sizeof(int64_t) * B);
+      src = gathered.data();
+    }
+    ExpandArgs e;
+    memset(&e, 0, sizeof(e));
+    e.out = r->data + (size_t)s * nl * L;
+    e.ct_stride = L;
+    e.n_glwe = nl; e.size = S;
+    e.seeds = (const Seed*)d_seed.p;
+    e.glwe_per_stream = nl;
+    e.seq = (const int*)d_seq.p + (size_t)s * nl;
+    TRY(expand_pass_i64(c, src, e));
+  }
+  TRY(take_range_error(c));
   r->loaded = true;
   r->state = false;
   r->rotated = false;
@@ -2002,10 +2113,13 @@ extern "C" int fheram_ram_read(fheram_ram* r, const fheram_address* addr, const 
 // GGSWs are all-gathered over NVLink (NCCL, in place), every rank rotates + packs its own polynomials for all
 // n_ranks * nb reads of the chunk, the packed partials are exchanged with one all-to-all, and each rank finishes its
 // own nb reads (top log2 n_ranks packer levels, second coordinate, trace).
-// in_fmt: 8 (int64 limbs), 4 (int32 limbs) or 17 (packed 17-bit fields, fheram_pack17)
+// in_fmt: 8 (int64 limbs), 4 (int32 limbs), 17 (packed 17-bit fields, fheram_pack17) or kSeededP17 (the bodies
+// packed as in 17, the masks regenerated from seeds[n] by k_glwe_expand)
+constexpr int kSeededP17 = -17;
 static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt, int n, const fheram_keys* k,
-                                void* out_host, int out_bytes) {
-  if (!r || !ggsw_host || !k || !out_host || n < 1) return fail(FHERAM_ERR_INVALID, "bad argument");
+                                void* out_host, int out_bytes, const fheram_seed* seeds = nullptr) {
+  if (!r || !ggsw_host || !k || !out_host || n < 1 || (in_fmt == kSeededP17 && !seeds))
+    return fail(FHERAM_ERR_INVALID, "bad argument");
   if (k->c != r->c) return fail(FHERAM_ERR_INVALID, "handles belong to different contexts");
   if (!r->loaded) return fail(FHERAM_ERR_UNINIT, "unitialized memory: self.data.len()=0 (src/ram.rs:182-185)");
   if (r->state || r->rotated) return fail(FHERAM_ERR_STATE, "invalid call to Memory.read: internal state is true (src/ram.rs:393-396)");
@@ -2061,6 +2175,11 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
   if (G > 1) TRYC(r->xchg.ensure(sizeof(int) * (size_t)G * chunk * ws * L));
   Set* sets = hp.sets;
   cudaStream_t copy_stream = hp.copy_stream;
+  const int glwe_per_addr = d.n_ggsw * d.dnum_ct * 2;
+  if (in_fmt == kSeededP17) {
+    TRYC(hp.seeds.ensure(sizeof(Seed) * n));
+    CUC(cudaMemcpyAsync(hp.seeds.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, copy_stream));
+  }
   // chunk boundaries: the first chunk is small (its upload overlaps nothing), the sizes then double up to the full
   // chunk, and the schedule is laid out from the END so that no tiny chunk (narrow launches) trails a batch that is
   // not a multiple of the chunk: n = 128 -> 8, 8, 16, 32, 64;  n = 1024 -> 8, 8, 16, 32, 64, 64, ...
@@ -2089,7 +2208,8 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
     const int b0 = start[ci], nb = start[ci + 1] - b0;
     if (ci >= 2) CU(cudaStreamWaitEvent(copy_stream, s.freed, 0));
     void* dst = in_fmt == 4 ? (void*)s.a.raw : (void*)s.stage;  // int32 limbs land where the prepare kernel reads them
-    const size_t addr_bytes = in_fmt == 17 ? per_addr * 17 / 8 : per_addr * in_fmt;  // per_addr is a multiple of 4096
+    const size_t addr_bytes = in_fmt == 17 ? per_addr * 17 / 8 :           // per_addr is a multiple of 4096
+                              in_fmt == kSeededP17 ? per_addr / 2 * 17 / 8 : per_addr * in_fmt;
     CU(cudaMemcpyAsync(dst, in + (size_t)b0 * addr_bytes, (size_t)nb * addr_bytes, cudaMemcpyHostToDevice, copy_stream));
     if (in_fmt == 8) {
       k_i64_to_i32<<<c->sm_count * 8, 256, 0, copy_stream>>>(s.stage, s.a.raw, (size_t)nb * per_addr, c->d_err);
@@ -2097,6 +2217,16 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
     } else if (in_fmt == 17) {
       k_unpack17<<<c->sm_count * 8, 256, 0, copy_stream>>>((const uint32_t*)s.stage, s.a.raw, (size_t)nb * per_addr);
       c->launches++;
+    } else if (in_fmt == kSeededP17) {
+      ExpandArgs e;
+      memset(&e, 0, sizeof(e));
+      e.out = s.a.raw;
+      e.ct_stride = (long)2 * d.size_addr * d.n;
+      e.n_glwe = nb * glwe_per_addr; e.size = d.size_addr;
+      e.body17 = (const uint32_t*)s.stage;
+      e.seeds = (const Seed*)hp.seeds.p + b0;
+      e.glwe_per_stream = glwe_per_addr;
+      TRY(launch_expand(c, e, copy_stream));
     }
     // one "matrix" of the prepare kernel = the coord_len[.] consecutive GGSWs of one coordinate of one address
     const int n0 = d.coord_len[0], n1 = d.n_coord > 1 ? d.coord_len[1] : 0;
@@ -2164,6 +2294,11 @@ extern "C" int fheram_ram_read_batch_host(fheram_ram* r, const int64_t* ggsw_hos
 extern "C" int fheram_ram_read_batch_host_p17(fheram_ram* r, const uint32_t* ggsw_packed, int n, const fheram_keys* k,
                                               int32_t* out_host) {
   return read_batch_host_impl(r, ggsw_packed, 17, n, k, out_host, 4);
+}
+// seeded addresses: bodies packed as in _p17 (half its bytes) and one seed per address, results as int32 limbs
+extern "C" int fheram_ram_read_batch_host_seeded(fheram_ram* r, const uint32_t* bodies_p17, const fheram_seed* seeds,
+                                                 int n, const fheram_keys* k, int32_t* out_host) {
+  return read_batch_host_impl(r, bodies_p17, kSeededP17, n, k, out_host, 4, seeds);
 }
 // compact host format: the same limbs as int32 (normalised digits fit 17 bits), addresses and results
 extern "C" int fheram_ram_read_batch_host_i32(fheram_ram* r, const int32_t* ggsw_host, int n, const fheram_keys* k,

@@ -55,6 +55,74 @@ __device__ __forceinline__ void chacha20_block(const uint32_t* key, unsigned lon
 }
 #undef FHERAM_QR
 
+// Seeded ciphertexts (fheram.h fheram_seed): the mask of every GLWE regenerated from its Source's ChaCha20 stream, the
+// body copied from int64 limbs or unpacked from 17-bit fields (fheram_pack17) in the same pass.
+struct Seed {                 // layout of fheram_seed
+  uint32_t key[8];
+  unsigned long long word0;   // stream position (32-bit words) of the first mask draw
+};
+struct ExpandArgs {
+  int* out;                   // GLWE j at out + j * ct_stride, [limb][col][N] int32 (col 0 = body)
+  long ct_stride;
+  int n_glwe, size;           // limbs per GLWE
+  const long long* body64;    // bodies [n_glwe][size][N] as int64 limbs, or
+  const uint32_t* body17;     //   as packed 17-bit fields (limb i = bits [17 i, 17 i + 17))
+  int* err;                   // set when an int64 body limb lies outside +-2^30 (k_i64_to_i32's rule)
+  const Seed* seeds;          // [n_streams]
+  int glwe_per_stream;        // GLWE j draws from stream j / glwe_per_stream ...
+  const int* seq;             // ... as that stream's seq[j]-th GLWE (null: j % glwe_per_stream)
+};
+// One CTA per (GLWE, limb), grid-stride.  Mask coefficient i of limb l of the stream's GLWE jl is the low 17 bits,
+// sign-extended, of stream word word0 + 2 ((jl size + l) N + i): each thread produces whole ChaCha20 blocks, the
+// coefficients whose low words fall in them go through shared memory so that the stores to the mask column coalesce.
+__global__ void __launch_bounds__(kThreads) k_glwe_expand(const ExpandArgs A) {
+  __shared__ __align__(16) int a_s[kN];
+  const int T = threadIdx.x;
+  for (long item = blockIdx.x; item < (long)A.n_glwe * A.size; item += gridDim.x) {
+    const int j = (int)(item / A.size), l = (int)(item % A.size);
+    const int stream = j / A.glwe_per_stream, jl = A.seq ? A.seq[j] : j % A.glwe_per_stream;
+    const Seed& sd = A.seeds[stream];
+    uint32_t key_s[8];
+#pragma unroll
+    for (int i = 0; i < 8; i++) key_s[i] = __ldg(sd.key + i);
+    int* ob = A.out + (size_t)j * A.ct_stride + (size_t)l * 2 * kN;
+    int* oa = ob + kN;
+    const unsigned long long base = __ldg(&sd.word0) + 2ull * ((unsigned long long)jl * A.size + l) * kN;
+    const unsigned long long b0 = base >> 4;
+    const int r = (int)(base & 15);
+    const int nblk = ((r + 2 * kN - 2) >> 4) + 1;
+    for (int blk = T; blk < nblk; blk += kThreads) {
+      uint32_t o[16];
+      chacha20_block(key_s, b0 + blk, o);
+#pragma unroll
+      for (int k = 0; k < 16; k++) {
+        const int off = blk * 16 + k - r;
+        if (off >= 0 && off < 2 * kN && !(off & 1)) a_s[off >> 1] = sext17i((int)(o[k] & 0x1ffffu));
+      }
+    }
+    __syncthreads();
+    for (int i = T; i < kN / 4; i += kThreads) reinterpret_cast<int4*>(oa)[i] = reinterpret_cast<const int4*>(a_s)[i];
+    const size_t t = (size_t)j * A.size + l;  // body limb t of the input
+    if (A.body64) {
+      const long long* in = A.body64 + t * kN;
+      for (int i = T; i < kN; i += kThreads) {
+        const long long v = in[i];
+        if (v > 0x3fffffffLL || v < -0x40000000LL) *A.err = 1;
+        ob[i] = (int)v;
+      }
+    } else {
+      const uint32_t* in = A.body17 + t * (kN * 17 / 32);  // kN * 17 bits: a whole number of words
+      for (int i = T; i < kN; i += kThreads) {
+        const int bit = 17 * i, w = bit >> 5, sh = bit & 31;
+        unsigned long long two = in[w];
+        if (sh > 15) two |= (unsigned long long)in[w + 1] << 32;
+        ob[i] = sext17i((int)((uint32_t)(two >> sh) & 0x1ffffu));
+      }
+    }
+    __syncthreads();  // a_s is rewritten by the next item
+  }
+}
+
 // Encryption noise on the device: sample k of a stream is client.cpp's fheram_source::gauss(3.2, 19.2) on the
 // stream words 4k .. 4k+3 (two 53-bit uniforms, Box-Muller cosine branch, rounded to the nearest integer), as
 // long as no earlier draw of the stream was rejected.  libm and CUDA agree on log / cos only to a few ulp, so

@@ -191,6 +191,10 @@ class ShardedRamLib:
         fn = {"i64": self.ram.read_batch_host, "i32": self.ram.read_batch_host_i32, "p17": self.ram.read_batch_host_p17}[fmt]
         return fn(my_addr_limbs, n, keys, out)
 
+    def read_batch_host_seeded(self, my_bodies_p17, my_seeds, n, keys, out=None):
+        """THIS rank's n seeded addresses (packed bodies + one seed each); returns this rank's n results"""
+        return self.ram.read_batch_host_seeded(my_bodies_p17, my_seeds, n, keys, out)
+
     def read_prepare_write(self, addr, keys) -> np.ndarray:
         return self.ram.read_prepare_write(addr, keys)
 

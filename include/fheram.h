@@ -327,6 +327,49 @@ int fheram_ram_decrypt_sk(fheram_ram *r, const int64_t *sk, int16_t *values, int
 int fheram_decrypt_words_device(fheram_ctx *ctx, const int32_t *d_glwe, int n, const int64_t *sk, int16_t *values,
                                 int64_t *err);
 
+/* ---- seeded ciphertexts (DESIGN.md 3.6): the body columns plus the state of the mask Source, half the bytes of the
+ * limbs.  A seed is the mask Source before the first mask draw of the object.  Mask coefficient i of limb l of GLWE j
+ * of the object is the low base2k bits, sign-extended, of stream word word0 + 2 ((j S + l) N + i) (S = the GLWE's
+ * limb count): what fheram_encrypt_ram / fheram_encrypt_address draw.  Bodies are the body columns in Poulpy's order
+ * with the column dropped:
+ *   RAM      [word_size][n_glwe][size_ct][N], GLWE j = s n_glwe + h, one seed for the whole RAM;
+ *   address  [n_ggsw][dnum_ct][2 ci][size_addr][N], GLWE j = (g dnum_ct + r) 2 + ci, one seed per address.
+ * A seeded RAM expands to exactly the limbs of fheram_encrypt_ram from the same Sources.  A seeded address is a
+ * different, equally valid encryption: the plaintext +/-X^pos of the rows with ci = 1, which fheram_encrypt_address
+ * adds to the mask, is moved into the body (body = normalize(-a s + e + X^pos s), mask = a), so that the mask is the
+ * raw stream.  Every row has the phase and the noise of fheram_encrypt_address's row, bit for bit, but reads with a
+ * seeded address give other limbs than reads with the full one; they decrypt to the same values.
+ * A seed discloses every draw of its Source: the mask Source of a seeded object must serve mask draws only. ---- */
+typedef struct fheram_seed {
+  uint32_t key[8];
+  uint64_t word0;
+} fheram_seed;
+/* the seed of a Source's current position */
+int fheram_source_seed(const fheram_source *s, fheram_seed *seed);
+/* Ram::encrypt_sk as bodies + seed: bodies = the body columns of fheram_encrypt_ram from the same Sources, which are
+ * left where it leaves them.  xa != xe */
+int fheram_encrypt_ram_seeded(const fheram_params *p, const uint8_t *data, const int64_t *sk, fheram_source *xa,
+                              fheram_source *xe, int64_t *bodies, fheram_seed *seed);
+/* Address::encrypt_sk as bodies + seed (the ci = 1 rows carry their plaintext in the body, see above); both Sources
+ * are left where fheram_encrypt_address leaves them.  xa != xe */
+int fheram_encrypt_address_seeded(const fheram_params *p, uint32_t value, const int64_t *sk, fheram_source *xa,
+                                  fheram_source *xe, int64_t *bodies, fheram_seed *seed);
+/* CPU expansion to full limbs (the reference of the device expansion): cts in fheram_encrypt_ram's layout, ggsw in
+ * fheram_encrypt_address's */
+int fheram_ram_expand(const fheram_params *p, const int64_t *bodies, const fheram_seed *seed, int64_t *cts);
+int fheram_address_expand(const fheram_params *p, const int64_t *bodies, const fheram_seed *seed, int64_t *ggsw);
+/* n seeded addresses made resident and prepared, as fheram_address_load_batch: bodies = n addresses' bodies one
+ * after the other, seeds = [n]; the masks are regenerated on the device (k_glwe_expand) */
+int fheram_address_load_seeded(fheram_ctx *ctx, const int64_t *bodies, const fheram_seed *seeds, int n,
+                               fheram_address **out);
+/* fheram_ram_read_batch_host_p17 with seeded addresses: bodies_p17 = the n addresses' bodies packed as fheram_pack17
+ * packs limbs (half the bytes of the _p17 format), seeds = [n]; results as int32 limbs.  A sharded RAM follows the
+ * contract of the _p17 call: every rank passes its own addresses and receives its own results */
+int fheram_ram_read_batch_host_seeded(fheram_ram *r, const uint32_t *bodies_p17, const fheram_seed *seeds, int n,
+                                      const fheram_keys *k, int32_t *out);
+/* fheram_ram_load of a seeded RAM (bodies in the RAM layout above); a sharded RAM loads its own polynomials */
+int fheram_ram_load_seeded(fheram_ram *r, const int64_t *bodies, const fheram_seed *seed);
+
 #ifdef __cplusplus
 }
 #endif

@@ -17,6 +17,13 @@ pub struct fheram_params {
     pub decomp_n: [i32; 8],
     pub max_addr: u64,
 }
+/// state of a mask Source: the seed of a seeded ciphertext (include/fheram.h)
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct fheram_seed {
+    pub key: [u32; 8],
+    pub word0: u64,
+}
 macro_rules! opaque { ($($n:ident),*) => { $(#[repr(C)] pub struct $n { _p: [u8; 0] })* } }
 opaque!(fheram_ctx, fheram_keys, fheram_address, fheram_ram, fheram_source);
 
@@ -103,4 +110,18 @@ extern "C" {
     pub fn fheram_ram_decrypt_sk(r: *mut fheram_ram, sk: *const i64, values: *mut i16, err: *mut i64) -> c_int;
     pub fn fheram_decrypt_words_device(c: *mut fheram_ctx, d_glwe: *const i32, n: c_int, sk: *const i64,
                                        values: *mut i16, err: *mut i64) -> c_int;
+    // seeded ciphertexts (DESIGN.md 3.6): bodies + the mask Source's seed, masks regenerated on the device
+    pub fn fheram_source_seed(s: *const fheram_source, seed: *mut fheram_seed) -> c_int;
+    pub fn fheram_encrypt_ram_seeded(p: *const fheram_params, data: *const u8, sk: *const i64, xa: *mut fheram_source,
+                                     xe: *mut fheram_source, bodies: *mut i64, seed: *mut fheram_seed) -> c_int;
+    pub fn fheram_encrypt_address_seeded(p: *const fheram_params, value: u32, sk: *const i64, xa: *mut fheram_source,
+                                         xe: *mut fheram_source, bodies: *mut i64, seed: *mut fheram_seed) -> c_int;
+    pub fn fheram_ram_expand(p: *const fheram_params, bodies: *const i64, seed: *const fheram_seed, cts: *mut i64) -> c_int;
+    pub fn fheram_address_expand(p: *const fheram_params, bodies: *const i64, seed: *const fheram_seed,
+                                 ggsw: *mut i64) -> c_int;
+    pub fn fheram_address_load_seeded(c: *mut fheram_ctx, bodies: *const i64, seeds: *const fheram_seed, n: c_int,
+                                      out: *mut *mut fheram_address) -> c_int;
+    pub fn fheram_ram_read_batch_host_seeded(r: *mut fheram_ram, bodies_p17: *const u32, seeds: *const fheram_seed,
+                                             n: c_int, k: *const fheram_keys, out: *mut i32) -> c_int;
+    pub fn fheram_ram_load_seeded(r: *mut fheram_ram, bodies: *const i64, seed: *const fheram_seed) -> c_int;
 }

@@ -109,21 +109,39 @@ impl EvaluationKeysPrepared {
 }
 impl Drop for EvaluationKeysPrepared { fn drop(&mut self) { if !self.0.is_null() { unsafe { fheram_keys_destroy(self.0); } } } }
 
-/// src/address.rs:21-24
-pub struct Address { pub data: Vec<i64>, dev: *mut fheram_address }
+/// src/address.rs:21-24.  `seeded`: the bodies and seed of `encrypt_sk_seeded`, uploaded in place of `data`
+pub struct Address { pub data: Vec<i64>, pub seeded: Option<(Vec<i64>, fheram_seed)>, dev: *mut fheram_address }
 impl Address {
     pub fn alloc_from_params(params: &Parameters) -> Self {
         let n = unsafe { fheram_n_ggsw(&params.c) as usize * fheram_ggsw_len(&params.c) };
-        Address { data: vec![0; n], dev: std::ptr::null_mut() }
+        Address { data: vec![0; n], seeded: None, dev: std::ptr::null_mut() }
     }
     pub fn alloc(params: &Parameters) -> Self { Self::alloc_from_params(params) }
     /// src/address.rs:86-109
     pub fn encrypt_sk(&mut self, params: &Parameters, value: u32, sk: &GLWESecret, xa: &mut Source, xe: &mut Source) {
         check(unsafe { fheram_encrypt_address(&params.c, value, sk.0.as_ptr(), xa.0, xe.0, self.data.as_mut_ptr()) });
+        self.seeded = None;
+        self.drop_device();
+    }
+    /// the seeded form (include/fheram.h): bodies + the mask Source's seed, half the bytes.  `data` becomes its
+    /// expanded limbs, another valid encryption of the same address than `encrypt_sk`'s
+    pub fn encrypt_sk_seeded(&mut self, params: &Parameters, value: u32, sk: &GLWESecret, xa: &mut Source,
+                             xe: &mut Source) {
+        let mut bodies = vec![0i64; self.data.len() / 2];
+        let mut seed = fheram_seed::default();
+        check(unsafe { fheram_encrypt_address_seeded(&params.c, value, sk.0.as_ptr(), xa.0, xe.0, bodies.as_mut_ptr(),
+                                                     &mut seed) });
+        check(unsafe { fheram_address_expand(&params.c, bodies.as_ptr(), &seed, self.data.as_mut_ptr()) });
+        self.seeded = Some((bodies, seed));
         self.drop_device();
     }
     fn device(&mut self, params: &mut Parameters) -> *const fheram_address {
-        if self.dev.is_null() { check(unsafe { fheram_address_load(params.module(), self.data.as_ptr(), &mut self.dev) }); }
+        if self.dev.is_null() {
+            match &self.seeded {
+                Some((b, s)) => check(unsafe { fheram_address_load_seeded(params.module(), b.as_ptr(), s, 1, &mut self.dev) }),
+                None => check(unsafe { fheram_address_load(params.module(), self.data.as_ptr(), &mut self.dev) }),
+            }
+        }
         self.dev
     }
     fn drop_device(&mut self) { if !self.dev.is_null() { unsafe { fheram_address_destroy(self.dev); } self.dev = std::ptr::null_mut(); } }
@@ -170,6 +188,32 @@ impl Ram {
         assert!(data.len() / p.word_size() == p.max_addr(), "invalid data: data.len()/ram_chunks != max_addr");
         // on the device, straight into the resident RAM (the limbs fheram_encrypt_ram + fheram_ram_load would install)
         check(unsafe { fheram_ram_encrypt_sk(self.h, data.as_ptr(), sk.0.as_ptr(), xa.0, xe.0) });
+    }
+    /// `encrypt_sk` on the client (CPU) in the seeded form, then `load_seeded`; returns (bodies, seed), what a
+    /// separated client ships: they expand to exactly the limbs of `fheram_encrypt_ram`
+    pub fn encrypt_sk_seeded(&mut self, data: &[u8], sk: &GLWESecret, xa: &mut Source, xe: &mut Source)
+                             -> (Vec<i64>, fheram_seed) {
+        let p = &self.params;
+        assert!(data.len() == p.max_addr() * p.word_size(), "invalid data: data.len() != max_addr * ram_chunks");
+        let n_glwe = unsafe { fheram_n_glwe_per_subram(&p.c) } as usize;
+        let mut bodies = vec![0i64; p.word_size() * n_glwe * p.glwe_len() / 2];
+        let mut seed = fheram_seed::default();
+        check(unsafe { fheram_encrypt_ram_seeded(&p.c, data.as_ptr(), sk.0.as_ptr(), xa.0, xe.0, bodies.as_mut_ptr(),
+                                                 &mut seed) });
+        self.load_seeded(&bodies, &seed);
+        (bodies, seed)
+    }
+    /// `fheram_ram_load` of a seeded RAM (a sharded RAM expands its own polynomials)
+    pub fn load_seeded(&mut self, bodies: &[i64], seed: &fheram_seed) {
+        check(unsafe { fheram_ram_load_seeded(self.h, bodies.as_ptr(), seed) });
+    }
+    /// n = seeds.len() seeded addresses from host buffers (bodies packed by `fheram_pack17`); int32 limbs out
+    pub fn read_batch_host_seeded(&mut self, bodies_p17: &[u32], seeds: &[fheram_seed], keys: &EvaluationKeysPrepared)
+                                  -> Vec<i32> {
+        let mut out = vec![0i32; seeds.len() * self.params.word_size() * self.params.glwe_len()];
+        check(unsafe { fheram_ram_read_batch_host_seeded(self.h, bodies_p17.as_ptr(), seeds.as_ptr(), seeds.len() as i32,
+                                                         keys.0, out.as_mut_ptr()) });
+        out
     }
     fn split(&self, flat: Vec<i64>) -> Vec<GLWE> { flat.chunks(self.params.glwe_len()).map(|c| c.to_vec()).collect() }
     /// src/ram.rs:172-191
