@@ -86,6 +86,7 @@ SIGNATURES = {
                                              C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "fheram_fp64_peak_probe": (C.c_int, [_V, C.c_int, C.POINTER(C.c_double)]),
     "fheram_debug_phase_cycles": (C.c_int, [_V, C.c_int, C.POINTER(C.c_longlong)]),
+    "fheram_debug_device_bytes": (C.c_uint64, []),
     "fheram_host_register": (C.c_int, [_V, C.c_size_t]),
     "fheram_host_unregister": (C.c_int, [_V]),
     "fheram_keys_prepare": (C.c_int, [_V, _P64, _P64, _P64, _PV]),

@@ -6,12 +6,14 @@
 #include <nccl.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cmath>
 #include <cstdarg>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -182,23 +184,53 @@ static int ilog2(int x) { int l = 0; while ((1 << l) < x) l++; return l; }
 // --------------------------------------------------------------------------------------
 // context
 // --------------------------------------------------------------------------------------
+static std::atomic<uint64_t> g_device_bytes{0};  // live bytes of every DevBuf of the process
+extern "C" uint64_t fheram_debug_device_bytes(void) { return g_device_bytes.load(); }
+
+// the one owner of device memory in this file (move-only): freed when its owner goes away
+template <typename T = void>
 struct DevBuf {
-  void* p = nullptr;
+  T* p = nullptr;
   size_t bytes = 0;
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), bytes(o.bytes) { o.p = nullptr; o.bytes = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept { std::swap(p, o.p); std::swap(bytes, o.bytes); return *this; }
+  ~DevBuf() { release(); }
+  operator T*() const { return p; }
   int ensure(size_t need) {
     if (need <= bytes) return 0;
     // growing while kernels that read the old buffer may still be queued: wait for them explicitly (cudaFree would
     // also synchronise the device, but the guarantee should not hang on an implementation detail of the allocator)
-    if (p) { cudaDeviceSynchronize(); cudaFree(p); }
-    p = nullptr; bytes = 0;
-    cudaError_t e = cudaMalloc(&p, need);
+    if (p) cudaDeviceSynchronize();
+    release();
+    cudaError_t e = cudaMalloc((void**)&p, need);
     if (e != cudaSuccess) return fail(FHERAM_ERR_CUDA, "cudaMalloc(%zu): %s", need, cudaGetErrorString(e));
     bytes = need;
+    g_device_bytes += need;
     return 0;
   }
-  void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
+  void release() { if (p) { cudaFree(p); g_device_bytes -= bytes; } p = nullptr; bytes = 0; }
 };
 
+// runs f when the scope is left, unless dismissed first
+template <typename F>
+struct OnExit {
+  F f;
+  bool armed = true;
+  ~OnExit() { if (armed) f(); }
+  void dismiss() { armed = false; }
+};
+template <typename F>
+static OnExit<F> on_exit(F f) { return OnExit<F>{f}; }
+
+// operands of the encryption and decryption kernels, kept between calls (cudaFree synchronizes the device)
+struct EncBufs {
+  struct Secret {  // secret-key material and PRNG state: wipe_secrets zeroes exactly these
+    DevBuf<> noise_keys, noise_word0, sk, sk_spec;  // noise Source keys / positions, 2 N int secrets, their spectra
+    DevBuf<> mask_keys, mask_word0, noise, poly;    // mask Source keys / positions, sampled noise, s and s * s
+  } secret;
+  DevBuf<> noise_flags, noise_n_flags, pt, mono, seq, poly_sel, sk_sel;
+};
 constexpr size_t kSmallDownload = (size_t)1 << 19;  // limbs (2 MiB of int32): up to 21 GLWEs at N = 4096, k = 51
 struct fheram_ctx {
   fheram_params params;
@@ -215,31 +247,38 @@ struct fheram_ctx {
   cudaStream_t side = nullptr;
   cudaEvent_t side_fork = nullptr, side_join = nullptr;
   bool on_side = false;
-  // multi-GPU (SURVEY.md 8e): one context per rank, NCCL communicator over NVLink (fheram_comm_init)
+  // multi-GPU (SURVEY.md 8e): one context per rank, a communicator over NVLink (fheram_comm_init)
   ncclComm_t comm = nullptr;
   ncclComm_t comm_prep = nullptr;  // second communicator: all-gather of prepared GGSWs on the upload stream, beside the reads
   int n_ranks = 1, rank = 0;
-  double2* d_tw = nullptr;  // tw6 | tw7c | tw8c | tw9 | tw10c
-  double2* d_tw16 = nullptr;  // twiddles of the 16-point transform (kernels_ks7.cuh): [16][16] | [128][7]
+  DevBuf<double2> d_tw;  // tw6 | tw7c | tw8c | tw9 | tw10c
+  DevBuf<double2> d_tw16;  // twiddles of the 16-point transform (kernels_ks7.cuh): [16][16] | [128][7]
   Twiddles tw;
-  int* d_err = nullptr;
+  DevBuf<int> d_err;
   uint64_t launches = 0;
-  DevBuf stage64;   // int64 staging for uploads / downloads
-  DevBuf scratch;   // per-CTA scratch of the vmp kernels
-  DevBuf scratch_side;
+  DevBuf<> stage64;   // int64 staging for uploads / downloads
+  DevBuf<> scratch;   // per-CTA scratch of the vmp kernels
+  DevBuf<> scratch_side;
   int* pin32 = nullptr;  // pinned host buffer of small downloads (download_i64)
-  DevBuf enc_buf[15];  // operands of the encryption kernels, kept between calls (cudaFree synchronizes the device)
+  EncBufs enc;
   uint64_t enc_stats[3] = {0, 0, 0};  // noise draws sampled on the device / patched by the host / streams resampled on the host
-  DevBuf dec_buf[2];   // decrypted values / errors on their way to the host (zeroed after every download)
-  DevBuf seed_buf[2];  // seeded loads: the seeds and the stream position of every GLWE
-  DevBuf opbuf[3];  // op-level entry points
-  long long* d_phase = nullptr;  // per-CTA phase cycle counters (fheram_debug_phase_cycles)
+  DevBuf<> dec_values, dec_err;  // decrypted values / errors on their way to the host (zeroed after every download)
+  DevBuf<> seeds, seed_seq;      // seeded loads: the seeds and the stream position of every GLWE
+  DevBuf<> op_ct, op_ct2, op_aux;  // op-level entry points: ciphertexts, a second operand, GGSWs or index tables
+  DevBuf<long long> d_phase;  // per-CTA phase cycle counters (fheram_debug_phase_cycles)
   // per-kernel-class CUDA-event timing (fheram_ctx_profile)
   bool profile = false;
   std::vector<cudaEvent_t> ev_pool;
   struct EvRec { int cls; size_t e0, e1; uint64_t items, steps; };
   std::vector<EvRec> ev_recs;
   size_t ev_used = 0;
+  ~fheram_ctx() {
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+    if (side) { cudaStreamDestroy(side); cudaEventDestroy(side_fork); cudaEventDestroy(side_join); }
+    for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
+    if (pin32) cudaFreeHost(pin32);
+    if (own_stream && stream) cudaStreamDestroy(stream);
+  }
   long ct_stride() const { return (long)2 * d.size_ct * d.n; }          // ints per GLWE(k_ct)
   long ggsw_raw_len() const { return (long)d.dnum_ct * 4 * d.size_addr * d.n; }
   long ggsw_prep_len() const { return (long)d.dnum_ct * 2 * 2 * d.size_addr * kM; }  // double2
@@ -336,7 +375,7 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
     return fail(FHERAM_ERR_CUDA, "no CUDA device: %s (there is no CPU fallback)", cudaGetErrorString(e));
   if (device < 0 || device >= ndev) return fail(FHERAM_ERR_INVALID, "device %d out of range", device);
   CU(cudaSetDevice(device));
-  fheram_ctx* c = new fheram_ctx();
+  auto c = std::make_unique<fheram_ctx>();
   c->params = *p;
   c->d = d;
   c->device = device;
@@ -345,11 +384,9 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   c->sm_count = prop.multiProcessorCount;
-  if (prop.major < 10) {
-    delete c;
+  if (prop.major < 10)
     return fail(FHERAM_ERR_CUDA, "device %s is sm_%d%d; this library is built for sm_100a only",
                 prop.name, prop.major, prop.minor);
-  }
   CU(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   TRY(set_attrs());
   // twiddles
@@ -374,7 +411,7 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
     q[b - 512] = make_double2(dx * r, sx * r);
   }
   CU(cudaMemcpyToSymbol(c_tw_lo, lo.data(), sizeof(double2) * 64));
-  CU(cudaMalloc(&c->d_tw, sizeof(double2) * hi.size()));
+  TRY(c->d_tw.ensure(sizeof(double2) * hi.size()));
   CU(cudaMemcpy(c->d_tw, hi.data(), sizeof(double2) * hi.size(), cudaMemcpyHostToDevice));
   c->tw.tw6 = c->d_tw;
   c->tw.tw7c = c->d_tw + 64;
@@ -395,10 +432,10 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
       zeta(8, 2 * t, p); zeta(9, 4 * t, p + 1); zeta(9, 4 * t + 2, p + 2);
       for (int k = 0; k < 4; k++) zeta(10, 8 * t + 2 * k, p + 3 + k);
     }
-    CU(cudaMalloc(&c->d_tw16, sizeof(double2) * kTw16Len));
+    TRY(c->d_tw16.ensure(sizeof(double2) * kTw16Len));
     CU(cudaMemcpy(c->d_tw16, t16.data(), sizeof(double2) * kTw16Len, cudaMemcpyHostToDevice));
   }
-  CU(cudaMalloc(&c->d_err, sizeof(int)));
+  TRY(c->d_err.ensure(sizeof(int)));
   CU(cudaMemset(c->d_err, 0, sizeof(int)));
   TRY(c->scratch.ensure((size_t)c->sm_count * 2 * c->ct_stride() * sizeof(int)));
   for (int v = 0; v < 2; v++) {
@@ -424,7 +461,7 @@ extern "C" int fheram_ctx_create(const fheram_params* p, int device, fheram_ctx*
     if (e2 != cudaSuccess) { n = 0; (void)cudaGetLastError(); }
     c->ext9_clusters[v] = n < cap ? n : cap;
   }
-  *out = c;
+  *out = c.release();
   return 0;
 }
 
@@ -437,22 +474,10 @@ extern "C" int fheram_ctx_destroy(fheram_ctx* c) {
   wipe_secrets(c);
   wipe_plaintext(c);
   cudaStreamSynchronize(c->stream);
-  if (c->comm_prep) { ncclCommDestroy(c->comm_prep); c->comm_prep = nullptr; }
-  if (c->comm) { ncclCommDestroy(c->comm); c->comm = nullptr; }
-  c->stage64.release(); c->scratch.release();
-  for (auto& b : c->opbuf) b.release();
-  for (auto& b : c->enc_buf) b.release();
-  for (auto& b : c->dec_buf) b.release();
-  for (auto& b : c->seed_buf) b.release();
-  cudaFree(c->d_tw); cudaFree(c->d_tw16); cudaFree(c->d_err);
-  if (c->copy_stream) { cudaStreamSynchronize(c->copy_stream); cudaStreamDestroy(c->copy_stream); }
-  if (c->side) {
-    cudaStreamSynchronize(c->side); cudaStreamDestroy(c->side);
-    cudaEventDestroy(c->side_fork); cudaEventDestroy(c->side_join);
-  }
-  c->scratch_side.release();
-  if (c->pin32) cudaFreeHost(c->pin32);
-  if (c->own_stream) cudaStreamDestroy(c->stream);
+  if (c->comm_prep) ncclCommDestroy(c->comm_prep);
+  if (c->comm) ncclCommDestroy(c->comm);
+  if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+  if (c->side) cudaStreamSynchronize(c->side);
   delete c;
   return 0;
 }
@@ -572,14 +597,15 @@ __global__ void k_fp64_probe(double* out, int iters) {
 extern "C" int fheram_fp64_peak_probe(fheram_ctx* c, int reps, double* tflops) {
   CU(cudaSetDevice(c->device));
   const int blocks = c->sm_count * 4, threads = 512, iters = 4096;
-  double* d = nullptr;
-  CU(cudaMalloc(&d, sizeof(double) * blocks * threads));
-  cudaEvent_t e0, e1;
+  DevBuf<double> d;
+  TRY(d.ensure(sizeof(double) * blocks * threads));
+  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  auto destroy_events = on_exit([&] { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); });
   CU(cudaEventCreate(&e0)); CU(cudaEventCreate(&e1));
   double best = 0;
   for (int r = 0; r < reps + 1; r++) {
     CU(cudaEventRecord(e0, c->stream));
-    k_fp64_probe<<<blocks, threads, 0, c->stream>>>(d, iters);
+    k_fp64_probe<<<blocks, threads, 0, c->stream>>>(d.p, iters);
     CU(cudaEventRecord(e1, c->stream));
     CU(cudaEventSynchronize(e1));
     float ms = 0;
@@ -587,8 +613,6 @@ extern "C" int fheram_fp64_peak_probe(fheram_ctx* c, int reps, double* tflops) {
     double tf = (double)blocks * threads * iters * 64 * 2 / (ms * 1e-3) / 1e12;
     if (r > 0 && tf > best) best = tf;
   }
-  CU(cudaEventDestroy(e0)); CU(cudaEventDestroy(e1));
-  CU(cudaFree(d));
   *tflops = best;
   return 0;
 }
@@ -600,7 +624,7 @@ extern "C" int fheram_debug_phase_cycles(fheram_ctx* c, int enable, long long ou
   CU(cudaStreamSynchronize(c->stream));
   const size_t n = (size_t)c->sm_count * 2 * 8;
   if (enable) {
-    if (!c->d_phase) CU(cudaMalloc(&c->d_phase, sizeof(long long) * n));
+    TRY(c->d_phase.ensure(sizeof(long long) * n));
     CU(cudaMemset(c->d_phase, 0, sizeof(long long) * n));
     return 0;
   }
@@ -609,8 +633,7 @@ extern "C" int fheram_debug_phase_cycles(fheram_ctx* c, int enable, long long ou
   CU(cudaMemcpy(h.data(), c->d_phase, sizeof(long long) * n, cudaMemcpyDeviceToHost));
   for (int i = 0; i < 8; i++) out[i] = 0;
   for (size_t i = 0; i < n; i++) out[i % 8] += h[i];
-  CU(cudaFree(c->d_phase));
-  c->d_phase = nullptr;
+  c->d_phase.release();
   return 0;
 }
 extern "C" int fheram_host_register(void* p, size_t bytes) {
@@ -815,12 +838,12 @@ static int prepare_ggsw(fheram_ctx* c, const int* raw, double2* out, int n_mat) 
 // keys
 // --------------------------------------------------------------------------------------
 struct fheram_keys {
-  fheram_ctx* c;
-  double2* atk = nullptr;      // [log_n] prepared trace keys
-  double2* atk7 = nullptr;     // trace keys prepared in the frequency order of k_ks7 / k_ks8 (k_prepare7)
-  double2* atk_inv = nullptr;  // prepared atk_ggsw_inv
-  double2* tsk = nullptr;      // prepared tsk_ggsw_inv
-  int* raw = nullptr;          // fheram_keys_encrypt_sk: the raw keys [atk x log_n | tsk | atk_inv] (fheram_keys_download_raw)
+  fheram_ctx* c = nullptr;
+  DevBuf<double2> atk;      // [log_n] prepared trace keys
+  DevBuf<double2> atk7;     // trace keys prepared in the frequency order of k_ks7 / k_ks8 (k_prepare7)
+  DevBuf<double2> atk_inv;  // prepared atk_ggsw_inv
+  DevBuf<double2> tsk;      // prepared tsk_ggsw_inv
+  DevBuf<int> raw;          // fheram_keys_encrypt_sk: the raw keys [atk x log_n | tsk | atk_inv] (fheram_keys_download_raw)
 };
 
 // EvaluationKeysPrepared::prepare (src/keys.rs:57-71) from raw int32 keys already on the device:
@@ -829,10 +852,10 @@ static int keys_prepare_device(fheram_ctx* c, const int* d_atk, const int* d_tsk
   const Derived& d = c->d;
   const size_t atk_raw = (size_t)d.dnum_ct * 2 * d.size_evk_trace * d.n;
   const size_t inv_raw = (size_t)d.dnum_ggsw * 2 * d.size_evk_inv * d.n;
-  CU(cudaMalloc(&k->atk, sizeof(double2) * c->atk_prep_len() * d.log_n));
-  CU(cudaMalloc(&k->atk7, sizeof(double2) * c->atk_prep_len() * d.log_n));
-  CU(cudaMalloc(&k->atk_inv, sizeof(double2) * c->evk_inv_prep_len()));
-  CU(cudaMalloc(&k->tsk, sizeof(double2) * c->evk_inv_prep_len()));
+  TRY(k->atk.ensure(sizeof(double2) * c->atk_prep_len() * d.log_n));
+  TRY(k->atk7.ensure(sizeof(double2) * c->atk_prep_len() * d.log_n));
+  TRY(k->atk_inv.ensure(sizeof(double2) * c->evk_inv_prep_len()));
+  TRY(k->tsk.ensure(sizeof(double2) * c->evk_inv_prep_len()));
   // trace key i is stored as phi_{g_i}(key): the kernels transform phi_g(x) and get phi_g(KS(x)); once per
   // transform family (frequency orders of k_prepare and k_prepare7)
   for (int i = 0; i < d.log_n; i++) {
@@ -853,26 +876,24 @@ extern "C" int fheram_keys_prepare(fheram_ctx* c, const int64_t* atk_glwe, const
   if (!c || !atk_glwe || !tsk || !atk_inv || !out) return fail(FHERAM_ERR_INVALID, "null argument");
   CU(cudaSetDevice(c->device));
   const Derived& d = c->d;
-  fheram_keys* k = new fheram_keys();
+  auto k = std::make_unique<fheram_keys>();
   k->c = c;
   const size_t atk_raw = (size_t)d.dnum_ct * 2 * d.size_evk_trace * d.n;
   const size_t inv_raw = (size_t)d.dnum_ggsw * 2 * d.size_evk_inv * d.n;
-  int* tmp = nullptr;
-  CU(cudaMalloc(&tmp, sizeof(int) * (atk_raw * d.log_n + 2 * inv_raw)));
-  int *d_atk = tmp, *d_tsk = tmp + atk_raw * d.log_n, *d_inv = d_tsk + inv_raw;
+  DevBuf<int> tmp;
+  TRY(tmp.ensure(sizeof(int) * (atk_raw * d.log_n + 2 * inv_raw)));
+  int *d_atk = tmp.p, *d_tsk = tmp.p + atk_raw * d.log_n, *d_inv = d_tsk + inv_raw;
   TRY(upload_i64(c, atk_glwe, atk_raw * d.log_n, d_atk));
   TRY(upload_i64(c, tsk, inv_raw, d_tsk));
   TRY(upload_i64(c, atk_inv, inv_raw, d_inv));
-  TRY(keys_prepare_device(c, d_atk, d_tsk, d_inv, k));
-  CU(cudaFree(tmp));
-  *out = k;
+  TRY(keys_prepare_device(c, d_atk, d_tsk, d_inv, k.get()));
+  *out = k.release();
   return 0;
 }
 
 extern "C" int fheram_keys_destroy(fheram_keys* k) {
   if (!k) return 0;
   cudaSetDevice(k->c->device);
-  cudaFree(k->atk); cudaFree(k->atk7); cudaFree(k->atk_inv); cudaFree(k->tsk); cudaFree(k->raw);
   delete k;
   return 0;
 }
@@ -881,41 +902,45 @@ extern "C" int fheram_keys_destroy(fheram_keys* k) {
 // addresses
 // --------------------------------------------------------------------------------------
 struct fheram_address {
-  fheram_ctx* c;
+  fheram_ctx* c = nullptr;
   int count = 0;
-  int* raw = nullptr;        // [count][n_ggsw] raw GGSW, int32
-  double2* prep = nullptr;   // [count][n_ggsw] prepared GGSW
+  DevBuf<int> raw;         // [count][n_ggsw] raw GGSW, int32
+  DevBuf<double2> prep;    // [count][n_ggsw] prepared GGSW
   // split layout of the sharded host pipeline (prep1 != nullptr): prep = [count][coord_len[0]] prepared GGSWs of the
   // first coordinate (every rank needs them for its local stage: all-gathered), prep1 = [own reads][coord_len[1]] of
   // the second coordinate, which only the finishing rank needs (address `prep1_first` of the set is its entry 0)
-  double2* prep1 = nullptr;
+  DevBuf<double2> prep1;
   int prep1_first = 0;
   // CoordinatePrepared::prepare_inv of every digit (src/ram.rs:260-271,278-289): a cache of the address handle,
   // built by read_prepare_write (off the critical path of the write that follows) or lazily by write
-  mutable int* inv_raw = nullptr;    // [n_ggsw] GGSW(X^+digit)
-  mutable double2* inv_prep = nullptr;
+  mutable DevBuf<int> inv_raw;    // [n_ggsw] GGSW(X^+digit)
+  mutable DevBuf<double2> inv_prep;
   mutable bool inv_ready = false;
   // asynchronous slice upload (multi-GPU host-buffer pipeline): int64 staging, copy-stream events
-  long long* stage = nullptr;
-  size_t stage_cap = 0;
+  DevBuf<long long> stage;
   cudaEvent_t uploaded = nullptr, released = nullptr;
   bool released_valid = false;
+  ~fheram_address() { if (uploaded) cudaEventDestroy(uploaded); if (released) cudaEventDestroy(released); }
+  // n addresses of raw and prepared GGSWs
+  int alloc(fheram_ctx* ctx, int n) {
+    c = ctx; count = n;
+    const size_t nm = (size_t)n * c->d.n_ggsw;
+    TRY(raw.ensure(sizeof(int) * nm * c->ggsw_raw_len()));
+    return prep.ensure(sizeof(double2) * nm * c->ggsw_prep_len());
+  }
 };
 
 extern "C" int fheram_address_load_batch(fheram_ctx* c, const int64_t* ggsw, int n, fheram_address** out) {
   if (!c || !ggsw || !out || n < 1) return fail(FHERAM_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(c->device));
-  const Derived& d = c->d;
-  fheram_address* a = new fheram_address();
-  a->c = c; a->count = n;
-  const size_t nm = (size_t)n * d.n_ggsw;
-  CU(cudaMalloc(&a->raw, sizeof(int) * nm * c->ggsw_raw_len()));
-  CU(cudaMalloc(&a->prep, sizeof(double2) * nm * c->ggsw_prep_len()));
+  auto a = std::make_unique<fheram_address>();
+  TRY(a->alloc(c, n));
+  const size_t nm = (size_t)n * c->d.n_ggsw;
   TRY(upload_i64(c, ggsw, nm * c->ggsw_raw_len(), a->raw));
   // CoordinatePrepared::prepare, src/coordinate_prepared.rs:104-116
   TRY(prepare_ggsw(c, a->raw, a->prep, (int)nm));
   CU(cudaStreamSynchronize(c->stream));
-  *out = a;
+  *out = a.release();
   return 0;
 }
 // Multi-GPU upload path: allocate n addresses, fill slices of the raw limbs (host upload of this
@@ -923,15 +948,12 @@ extern "C" int fheram_address_load_batch(fheram_ctx* c, const int64_t* ggsw, int
 extern "C" int fheram_address_alloc(fheram_ctx* c, int n, fheram_address** out) {
   if (!c || !out || n < 1) return fail(FHERAM_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(c->device));
-  fheram_address* a = new fheram_address();
-  a->c = c; a->count = n;
-  const size_t nm = (size_t)n * c->d.n_ggsw;
-  CU(cudaMalloc(&a->raw, sizeof(int) * nm * c->ggsw_raw_len()));
-  CU(cudaMalloc(&a->prep, sizeof(double2) * nm * c->ggsw_prep_len()));
-  *out = a;
+  auto a = std::make_unique<fheram_address>();
+  TRY(a->alloc(c, n));
+  *out = a.release();
   return 0;
 }
-extern "C" int32_t* fheram_address_raw_ptr(fheram_address* a) { return a ? a->raw : nullptr; }
+extern "C" int32_t* fheram_address_raw_ptr(fheram_address* a) { return a ? a->raw.p : nullptr; }
 extern "C" int fheram_address_upload_slice(fheram_address* a, const int64_t* ggsw, int first, int count) {
   if (!a || !ggsw || first < 0 || count < 1 || first + count > a->count) return fail(FHERAM_ERR_INVALID, "bad slice");
   fheram_ctx* c = a->c;
@@ -951,18 +973,12 @@ extern "C" int fheram_address_upload_slice_async(fheram_address* a, const int64_
   if (!c->copy_stream) CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   const size_t per = (size_t)c->d.n_ggsw * c->ggsw_raw_len();
   const size_t n = (size_t)count * per;
-  if (a->stage_cap < n) {
-    CU(cudaStreamSynchronize(c->copy_stream));
-    cudaFree(a->stage);
-    a->stage = nullptr; a->stage_cap = 0;
-    CU(cudaMalloc(&a->stage, sizeof(long long) * n));
-    a->stage_cap = n;
-  }
+  TRY(a->stage.ensure(sizeof(long long) * n));  // waits for the copy stream before it grows
   a->inv_ready = false;
   if (!a->uploaded) CU(cudaEventCreateWithFlags(&a->uploaded, cudaEventDisableTiming));
   if (a->released_valid) CU(cudaStreamWaitEvent(c->copy_stream, a->released, 0));
-  CU(cudaMemcpyAsync(a->stage, ggsw, sizeof(long long) * n, cudaMemcpyHostToDevice, c->copy_stream));
-  k_i64_to_i32<<<c->sm_count * 8, 256, 0, c->copy_stream>>>(a->stage, a->raw + (size_t)first * per, n, c->d_err);
+  CU(cudaMemcpyAsync(a->stage.p, ggsw, sizeof(long long) * n, cudaMemcpyHostToDevice, c->copy_stream));
+  k_i64_to_i32<<<c->sm_count * 8, 256, 0, c->copy_stream>>>(a->stage.p, a->raw + (size_t)first * per, n, c->d_err);
   c->launches++;
   CU(cudaGetLastError());
   CU(cudaEventRecord(a->uploaded, c->copy_stream));
@@ -1024,34 +1040,27 @@ extern "C" int fheram_address_load_seeded(fheram_ctx* c, const int64_t* bodies, 
   const int per = d.n_ggsw * d.dnum_ct * 2;                     // GLWEs per address, one stream
   const size_t body_per = (size_t)per * d.size_addr * d.n;      // body limbs per address
   const size_t nm = (size_t)n * d.n_ggsw;
-  fheram_address* a = new fheram_address();
-  a->c = c; a->count = n;
-  auto run = [&]() -> int {
-    CU(cudaMalloc(&a->raw, sizeof(int) * nm * c->ggsw_raw_len()));
-    CU(cudaMalloc(&a->prep, sizeof(double2) * nm * c->ggsw_prep_len()));
-    DevBuf& d_seed = c->seed_buf[0];
-    TRY(d_seed.ensure(sizeof(Seed) * n));
-    CU(cudaMemcpyAsync(d_seed.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, c->stream));
-    const size_t step_l = ((size_t)64 << 20) / body_per;        // addresses per pass: at most 64 Mi staged limbs
-    const int step = step_l < 1 ? 1 : (step_l > (size_t)n ? n : (int)step_l);
-    for (int i0 = 0; i0 < n; i0 += step) {
-      const int m = n - i0 < step ? n - i0 : step;
-      ExpandArgs e;
-      memset(&e, 0, sizeof(e));
-      e.out = a->raw + (size_t)i0 * d.n_ggsw * c->ggsw_raw_len();
-      e.ct_stride = (long)2 * d.size_addr * d.n;
-      e.n_glwe = m * per; e.size = d.size_addr;
-      e.seeds = (const Seed*)d_seed.p + i0;
-      e.glwe_per_stream = per;
-      TRY(expand_pass_i64(c, bodies + (size_t)i0 * body_per, e));
-    }
-    TRY(take_range_error(c));
-    TRY(prepare_ggsw(c, a->raw, a->prep, (int)nm));  // CoordinatePrepared::prepare, as fheram_address_load_batch
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
-  };
-  if (int rc = run()) { fheram_address_destroy(a); return rc; }
-  *out = a;
+  auto a = std::make_unique<fheram_address>();
+  TRY(a->alloc(c, n));
+  TRY(c->seeds.ensure(sizeof(Seed) * n));
+  CU(cudaMemcpyAsync(c->seeds.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, c->stream));
+  const size_t step_l = ((size_t)64 << 20) / body_per;        // addresses per pass: at most 64 Mi staged limbs
+  const int step = step_l < 1 ? 1 : (step_l > (size_t)n ? n : (int)step_l);
+  for (int i0 = 0; i0 < n; i0 += step) {
+    const int m = n - i0 < step ? n - i0 : step;
+    ExpandArgs e;
+    memset(&e, 0, sizeof(e));
+    e.out = a->raw + (size_t)i0 * d.n_ggsw * c->ggsw_raw_len();
+    e.ct_stride = (long)2 * d.size_addr * d.n;
+    e.n_glwe = m * per; e.size = d.size_addr;
+    e.seeds = (const Seed*)c->seeds.p + i0;
+    e.glwe_per_stream = per;
+    TRY(expand_pass_i64(c, bodies + (size_t)i0 * body_per, e));
+  }
+  TRY(take_range_error(c));
+  TRY(prepare_ggsw(c, a->raw, a->prep, (int)nm));  // CoordinatePrepared::prepare, as fheram_address_load_batch
+  CU(cudaStreamSynchronize(c->stream));
+  *out = a.release();
   return 0;
 }
 extern "C" int fheram_address_count(const fheram_address* a) { return a ? a->count : 0; }
@@ -1059,9 +1068,6 @@ extern "C" int fheram_address_destroy(fheram_address* a) {
   if (!a) return 0;
   cudaSetDevice(a->c->device);
   if (a->c->copy_stream) cudaStreamSynchronize(a->c->copy_stream);
-  cudaFree(a->raw); cudaFree(a->prep); cudaFree(a->inv_raw); cudaFree(a->inv_prep); cudaFree(a->stage);
-  if (a->uploaded) cudaEventDestroy(a->uploaded);
-  if (a->released) cudaEventDestroy(a->released);
   delete a;
   return 0;
 }
@@ -1080,11 +1086,11 @@ static int run_ext_chain(fheram_ctx* c, int n_items, const int* src, const int* 
   a.mat_div = mat_div; a.mat_stride = mat_stride;
   switch (select_ext(c, n_items)) {
     case KN_EXT9_8:
-      return launch(c, KC_EXT, k_ext9<8>, 8 * std::min(n_items, c->ext9_clusters[0]), 512, ext9_smem(8), a, c->d_tw16);
+      return launch(c, KC_EXT, k_ext9<8>, 8 * std::min(n_items, c->ext9_clusters[0]), 512, ext9_smem(8), a, c->d_tw16.p);
     case KN_EXT9_4:
-      return launch(c, KC_EXT, k_ext9<4>, 4 * std::min(n_items, c->ext9_clusters[1]), 512, ext9_smem(4), a, c->d_tw16);
+      return launch(c, KC_EXT, k_ext9<4>, 4 * std::min(n_items, c->ext9_clusters[1]), 512, ext9_smem(4), a, c->d_tw16.p);
     default:
-      return launch(c, KC_EXT, k_ext8, std::min(n_items, c->sm_count), kExt8Threads, kExt8Smem, a, c->d_tw16);
+      return launch(c, KC_EXT, k_ext8, std::min(n_items, c->sm_count), kExt8Threads, kExt8Smem, a, c->d_tw16.p);
   }
 }
 // a key-switch launch of MODE_TRACE, MODE_COMBINE2 or MODE_MIXED (selected and profiled as a combine): step s uses trace
@@ -1098,10 +1104,10 @@ static int launch_ks(fheram_ctx* c, const fheram_keys* k, int key0, VmpArgs a) {
   for (int s = 0; s < a.n_steps; s++) a.mat[s] = keys + (size_t)(key0 + s) * c->atk_prep_len();
   switch (kn) {
     case KN_KS8_8:
-      return launch(c, cls, k_ks8<8, MODE>, 8 * std::min(n, c->ks8_clusters[0]), 512, ks8_smem(8), a, c->d_tw16);
+      return launch(c, cls, k_ks8<8, MODE>, 8 * std::min(n, c->ks8_clusters[0]), 512, ks8_smem(8), a, c->d_tw16.p);
     case KN_KS8_4:
-      return launch(c, cls, k_ks8<4, MODE>, 4 * std::min(n, c->ks8_clusters[1]), 512, ks8_smem(4), a, c->d_tw16);
-    case KN_KS7: return launch(c, cls, k_ks7, std::min(n, 2 * S), 256, kKs7Smem, a, c->d_tw16);
+      return launch(c, cls, k_ks8<4, MODE>, 4 * std::min(n, c->ks8_clusters[1]), 512, ks8_smem(4), a, c->d_tw16.p);
+    case KN_KS7: return launch(c, cls, k_ks7, std::min(n, 2 * S), 256, kKs7Smem, a, c->d_tw16.p);
     case KN_KS6: return launch(c, cls, k_ks6<MODE>, 2 * n, kThreads5, kKs5Smem, a);
     case KN_KS5: return launch(c, cls, k_ks5<MODE>, std::min(n, S), kThreads5, kKs5Smem, a);
     default:
@@ -1221,33 +1227,44 @@ struct fheram_ram {
   fheram_ctx* c;
   int shard = 0, n_shards = 1;
   int n_local = 0;           // local polynomials per sub-RAM
-  int* data = nullptr;       // [word_size][n_local] GLWE   (SubRam::data, src/ram.rs:299)
-  int* tree = nullptr;       // [word_size] GLWE            (SubRam::tree[0][0], src/ram.rs:300)
+  DevBuf<int> data;          // [word_size][n_local] GLWE   (SubRam::data, src/ram.rs:299)
+  DevBuf<int> tree;          // [word_size] GLWE            (SubRam::tree[0][0], src/ram.rs:300)
   bool state = false;        // src/ram.rs:302
   bool rotated = false;      // rpw_local_device rotated SubRam::data in place and rpw_finish_device has not completed:
                              // the reference does both inside one call (src/ram.rs:502-533), so no read may see this state
   bool loaded = false;
-  int* feed_map = nullptr;   // device: [word_size*n_local] packer input position -> data index (packer_order)
-  int* mixed_ops = nullptr;  // device: operand table of the mixed packer level (n_local not a power of two)
-  DevBuf bufA, bufB;         // work arenas [B][word_size][n_local] GLWE
-  DevBuf partial;            // [B][word_size] packed partials
-  DevBuf result;             // [B][word_size] results
-  DevBuf wbuf;               // uploaded write words
-  DevBuf wstage;             // their int64 staging
+  DevBuf<int> feed_map;      // device: [word_size*n_local] packer input position -> data index (packer_order)
+  DevBuf<int> mixed_ops;     // device: operand table of the mixed packer level (n_local not a power of two)
+  DevBuf<> bufA, bufB;       // work arenas [B][word_size][n_local] GLWE
+  DevBuf<> partial;          // [B][word_size] packed partials
+  DevBuf<> result;           // [B][word_size] results
+  DevBuf<> wbuf;             // uploaded write words
+  DevBuf<> wstage;           // their int64 staging
   void* wpin = nullptr;      // pinned host copy of the words of the write in flight
   cudaEvent_t wcopied = nullptr;
-  DevBuf all;                // results of a chunked batched read
-  DevBuf xchg;               // sharded: partials received from the other ranks, [n_shards][reads][word_size]
-  DevBuf part_all;           // sharded, device-resident batch: partials of every read before the exchange
+  DevBuf<> all;              // results of a chunked batched read
+  DevBuf<> xchg;             // sharded: partials received from the other ranks, [n_shards][reads][word_size]
+  DevBuf<> part_all;         // sharded, device-resident batch: partials of every read before the exchange
   struct HostPipe {          // fheram_ram_read_batch_host: double-buffered upload pipeline
-    struct Set { long long* stage = nullptr; fheram_address a; cudaEvent_t copied = nullptr, freed = nullptr; };
+    struct Set {
+      DevBuf<long long> stage;
+      fheram_address a;
+      cudaEvent_t copied = nullptr, freed = nullptr;
+      ~Set() { if (copied) cudaEventDestroy(copied); if (freed) cudaEventDestroy(freed); }
+    };
     Set sets[2];
-    long long* out_stage[2] = {nullptr, nullptr};
+    DevBuf<long long> out_stage[2];
     cudaEvent_t out_ready[2] = {nullptr, nullptr}, out_done[2] = {nullptr, nullptr};
     cudaStream_t copy_stream = nullptr, down_stream = nullptr;
     int cap = 0;
-    DevBuf seeds;            // the seeds of a seeded batch
+    DevBuf<> seeds;          // the seeds of a seeded batch
+    ~HostPipe() {
+      for (cudaEvent_t e : {out_ready[0], out_ready[1], out_done[0], out_done[1]}) if (e) cudaEventDestroy(e);
+      if (copy_stream) cudaStreamDestroy(copy_stream);
+      if (down_stream) cudaStreamDestroy(down_stream);
+    }
   } pipe;
+  ~fheram_ram() { if (wpin) cudaFreeHost(wpin); if (wcopied) cudaEventDestroy(wcopied); }
 };
 
 static int ram_create(fheram_ctx* c, int shard, int n_shards, fheram_ram** out) {
@@ -1259,12 +1276,12 @@ static int ram_create(fheram_ctx* c, int shard, int n_shards, fheram_ram** out) 
     return fail(FHERAM_ERR_INVALID, "a sharded RAM needs max_addr/N (rounded up) to be a power of two, here %d",
                 d.n_glwe);
   CU(cudaSetDevice(c->device));
-  fheram_ram* r = new fheram_ram();
+  auto r = std::make_unique<fheram_ram>();
   r->c = c; r->shard = shard; r->n_shards = n_shards;
   r->n_local = d.n_glwe / n_shards;
   const int ws = c->params.word_size;
-  CU(cudaMalloc(&r->data, sizeof(int) * (size_t)ws * r->n_local * c->ct_stride()));
-  CU(cudaMalloc(&r->tree, sizeof(int) * (size_t)ws * c->ct_stride()));
+  TRY(r->data.ensure(sizeof(int) * (size_t)ws * r->n_local * c->ct_stride()));
+  TRY(r->tree.ensure(sizeof(int) * (size_t)ws * c->ct_stride()));
   CU(cudaMemset(r->tree, 0, sizeof(int) * (size_t)ws * c->ct_stride()));
   // input order of the packer (src/ram.rs:425-435, packer_order): position m of the local tree reads local
   // polynomial h' = order[m]
@@ -1273,13 +1290,13 @@ static int ram_create(fheram_ctx* c, int shard, int n_shards, fheram_ram** out) 
   std::vector<int> map((size_t)ws * r->n_local);
   for (int s = 0; s < ws; s++)
     for (int m = 0; m < r->n_local; m++) map[(size_t)s * r->n_local + m] = s * r->n_local + order[m];
-  CU(cudaMalloc(&r->feed_map, sizeof(int) * map.size()));
+  TRY(r->feed_map.ensure(sizeof(int) * map.size()));
   CU(cudaMemcpy(r->feed_map, map.data(), sizeof(int) * map.size(), cudaMemcpyHostToDevice));
   if (!ops.empty()) {
-    CU(cudaMalloc(&r->mixed_ops, sizeof(int) * ops.size()));
+    TRY(r->mixed_ops.ensure(sizeof(int) * ops.size()));
     CU(cudaMemcpy(r->mixed_ops, ops.data(), sizeof(int) * ops.size(), cudaMemcpyHostToDevice));
   }
-  *out = r;
+  *out = r.release();
   return 0;
 }
 extern "C" int fheram_ram_create(fheram_ctx* c, fheram_ram** out) { return ram_create(c, 0, 1, out); }
@@ -1289,23 +1306,7 @@ extern "C" int fheram_ram_create_sharded(fheram_ctx* c, int shard, int n_shards,
 extern "C" int fheram_ram_destroy(fheram_ram* r) {
   if (!r) return 0;
   cudaSetDevice(r->c->device);
-  cudaFree(r->data); cudaFree(r->tree); cudaFree(r->feed_map); cudaFree(r->mixed_ops);
-  if (r->wpin) { cudaStreamSynchronize(r->c->stream); cudaFreeHost(r->wpin); cudaEventDestroy(r->wcopied); }
-  r->bufA.release(); r->bufB.release(); r->partial.release(); r->result.release(); r->wbuf.release(); r->wstage.release(); r->all.release(); r->xchg.release(); r->part_all.release();
-  for (auto& s : r->pipe.sets) {
-    cudaFree(s.stage); cudaFree(s.a.raw); cudaFree(s.a.prep); cudaFree(s.a.prep1);
-    s.a.raw = nullptr; s.a.prep = nullptr; s.a.prep1 = nullptr;
-    if (s.copied) cudaEventDestroy(s.copied);
-    if (s.freed) cudaEventDestroy(s.freed);
-  }
-  for (int i = 0; i < 2; i++) {
-    cudaFree(r->pipe.out_stage[i]);
-    if (r->pipe.out_ready[i]) cudaEventDestroy(r->pipe.out_ready[i]);
-    if (r->pipe.out_done[i]) cudaEventDestroy(r->pipe.out_done[i]);
-  }
-  r->pipe.seeds.release();
-  if (r->pipe.copy_stream) cudaStreamDestroy(r->pipe.copy_stream);
-  if (r->pipe.down_stream) cudaStreamDestroy(r->pipe.down_stream);
+  if (r->wpin) cudaStreamSynchronize(r->c->stream);  // the copy out of the pinned words
   delete r;
   return 0;
 }
@@ -1347,7 +1348,7 @@ extern "C" int fheram_ram_load_seeded(fheram_ram* r, const int64_t* bodies, cons
   std::vector<int> seq((size_t)ws * nl);
   for (int s = 0; s < ws; s++)
     for (int hp = 0; hp < nl; hp++) seq[(size_t)s * nl + hp] = s * G + r->shard + r->n_shards * hp;
-  DevBuf &d_seed = c->seed_buf[0], &d_seq = c->seed_buf[1];
+  DevBuf<> &d_seed = c->seeds, &d_seq = c->seed_seq;
   TRY(d_seed.ensure(sizeof(Seed)));
   TRY(d_seq.ensure(sizeof(int) * seq.size()));
   CU(cudaMemcpyAsync(d_seed.p, seed, sizeof(Seed), cudaMemcpyHostToDevice, c->stream));
@@ -1433,9 +1434,12 @@ static double enc_bound_guard() {
   if (g < 0) { const char* e = getenv("FHERAM_ENC_BOUND_GUARD"); g = e ? atof(e) : enc_guard(); if (!(g >= 1e-12)) g = 1e-12; }
   return g;
 }
-// Noise of n_streams Sources (per_stream draws each, stream-major) into d_noise, and every Source advanced as
-// that many fheram_source::gauss draws advance it.
-static int sample_noise(fheram_ctx* c, fheram_source* const* xe, int n_streams, size_t per_stream, DevBuf& d_noise) {
+static void wipe_secrets(fheram_ctx* c);
+// Noise of n_streams Sources (per_stream draws each, stream-major) into c->enc.secret.noise, and every Source advanced
+// as that many fheram_source::gauss draws advance it.  On failure the secret material on the device is wiped.
+static int sample_noise(fheram_ctx* c, fheram_source* const* xe, int n_streams, size_t per_stream) {
+  auto wipe = on_exit([&] { wipe_secrets(c); cudaStreamSynchronize(c->stream); });
+  DevBuf<>& d_noise = c->enc.secret.noise;
   TRY(d_noise.ensure((size_t)n_streams * per_stream));
   std::vector<int8_t> host;
   auto host_stream = [&](int s) -> int {
@@ -1458,36 +1462,36 @@ static int sample_noise(fheram_ctx* c, fheram_source* const* xe, int n_streams, 
     for (auto& t : th) t.join();
     CU(cudaMemcpy(d_noise.p, all.data(), all.size(), cudaMemcpyHostToDevice));
     c->enc_stats[2] += n_streams;
+    wipe.dismiss();
     return 0;
   }
   const unsigned max_flags = 1u << 16;
   std::vector<uint32_t> keys((size_t)8 * n_streams);
   std::vector<unsigned long long> w0(n_streams);
   for (int s = 0; s < n_streams; s++) fheram_source_tell(xe[s], &keys[8 * s], (uint64_t*)&w0[s]);
-  DevBuf &dk = c->enc_buf[0], &dw = c->enc_buf[1], &df = c->enc_buf[2], &dn = c->enc_buf[3];
-#define NZ_TRY(x) TRY(x)
-#define NZ_CU(x) CU(x)
-  NZ_TRY(dk.ensure(keys.size() * sizeof(uint32_t)));
-  NZ_TRY(dw.ensure(w0.size() * sizeof(unsigned long long)));
-  NZ_TRY(df.ensure((size_t)max_flags * sizeof(unsigned long long)));
-  NZ_TRY(dn.ensure(sizeof(unsigned)));
-  NZ_CU(cudaMemcpyAsync(dk.p, keys.data(), keys.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-  NZ_CU(cudaMemcpyAsync(dw.p, w0.data(), w0.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
-  NZ_CU(cudaMemsetAsync(dn.p, 0, sizeof(unsigned), c->stream));
+  DevBuf<> &dk = c->enc.secret.noise_keys, &dw = c->enc.secret.noise_word0, &df = c->enc.noise_flags,
+           &dn = c->enc.noise_n_flags;
+  TRY(dk.ensure(keys.size() * sizeof(uint32_t)));
+  TRY(dw.ensure(w0.size() * sizeof(unsigned long long)));
+  TRY(df.ensure((size_t)max_flags * sizeof(unsigned long long)));
+  TRY(dn.ensure(sizeof(unsigned)));
+  CU(cudaMemcpyAsync(dk.p, keys.data(), keys.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(dw.p, w0.data(), w0.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemsetAsync(dn.p, 0, sizeof(unsigned), c->stream));
   NoiseArgs a;
   a.out = (signed char*)d_noise.p; a.n_streams = n_streams; a.per_stream = (long)per_stream;
   a.keys = (const uint32_t*)dk.p; a.word0 = (const unsigned long long*)dw.p; a.guard = enc_guard(); a.bound_guard = enc_bound_guard();
   a.n_flags = (unsigned*)dn.p; a.flags = (unsigned long long*)df.p; a.max_flags = max_flags;
   k_noise_sample<<<c->sm_count * 8, 256, 0, c->stream>>>(a);
   c->launches++;
-  NZ_CU(cudaGetLastError());
+  CU(cudaGetLastError());
   unsigned n_flags = 0;
-  NZ_CU(cudaMemcpyAsync(&n_flags, dn.p, sizeof(unsigned), cudaMemcpyDeviceToHost, c->stream));
-  NZ_CU(cudaStreamSynchronize(c->stream));
+  CU(cudaMemcpyAsync(&n_flags, dn.p, sizeof(unsigned), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
   std::vector<char> redo(n_streams, n_flags > max_flags ? 1 : 0);  // more reports than slots: host sampling for all
   if (n_flags && n_flags <= max_flags) {
     std::vector<unsigned long long> flags(n_flags);
-    NZ_CU(cudaMemcpy(flags.data(), df.p, (size_t)n_flags * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(flags.data(), df.p, (size_t)n_flags * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
     for (unsigned long long f : flags)
       if ((f >> 39) & 1) redo[(size_t)(f >> 40)] = 1;
     for (unsigned long long f : flags) {
@@ -1495,16 +1499,15 @@ static int sample_noise(fheram_ctx* c, fheram_source* const* xe, int n_streams, 
       if (((f >> 39) & 1) || redo[s]) continue;
       const unsigned long long k = f & ((1ull << 39) - 1);
       const int8_t v = fheram_source_noise_at(xe[s], 4ull * k);
-      NZ_CU(cudaMemcpy((char*)d_noise.p + s * per_stream + k, &v, 1, cudaMemcpyHostToDevice));
+      CU(cudaMemcpy((char*)d_noise.p + s * per_stream + k, &v, 1, cudaMemcpyHostToDevice));
       c->enc_stats[1]++;
     }
   }
   for (int s = 0; s < n_streams; s++) {
-    if (redo[s]) NZ_TRY(host_stream(s));
+    if (redo[s]) TRY(host_stream(s));
     else { fheram_source_skip_words(xe[s], 4ull * per_stream); c->enc_stats[0] += per_stream; }
   }
-#undef NZ_TRY
-#undef NZ_CU
+  wipe.dismiss();
   return 0;
 }
 extern "C" int fheram_debug_encrypt_stats(fheram_ctx* c, uint64_t out[3]) {
@@ -1518,41 +1521,37 @@ static int check_secret(const int64_t* sk, int n) {  // before any Source moves
     if (sk[i] < -1 || sk[i] > 1) return fail(FHERAM_ERR_INVALID, "secret key is not ternary");
   return 0;
 }
-// zero every device buffer that held secret-key material or PRNG state of an encryption call
+// zero every device buffer that held secret-key material or PRNG state of an encryption or decryption call
 static void wipe_secrets(fheram_ctx* c) {
-  const int idx[] = {0, 1, 4, 5, 9, 10, 11, 12};  // noise Source keys / positions, sk, sk spectrum, mask Source keys / positions, noise, s and s*s
-  for (int i : idx)
-    if (c->enc_buf[i].p) cudaMemsetAsync(c->enc_buf[i].p, 0, c->enc_buf[i].bytes, c->stream);
+  EncBufs::Secret& s = c->enc.secret;
+  static_assert(sizeof(EncBufs::Secret) == 8 * sizeof(DevBuf<>), "wipe_secrets lists every member of EncBufs::Secret");
+  for (DevBuf<>* b : {&s.noise_keys, &s.noise_word0, &s.sk, &s.sk_spec, &s.mask_keys, &s.mask_word0, &s.noise, &s.poly})
+    if (b->p) cudaMemsetAsync(b->p, 0, b->bytes, c->stream);
 }
-// on any failure the secret material already on the device is wiped before returning
-#define ENC_TRY(x) do { int rc_ = (x); if (rc_) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return rc_; } } while (0)
-#define ENC_CU(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { wipe_secrets(c); cudaStreamSynchronize(c->stream); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
-// s32 = n_sk secrets of 2 N ints each (secret, then N zeros) -> their prepared spectra in enc_buf[5] (2 M double2 each,
-// the secret's first).  The host staging copy s32 is zeroed on every path; the device copies are wiped on failure.
+// s32 = n_sk secrets of 2 N ints each (secret, then N zeros) -> their prepared spectra in c->enc.secret.sk_spec (2 M
+// double2 each, the secret's first).  The host staging copy s32 is zeroed on every path; the callers wipe the device
+// copies.
 static int upload_secret(fheram_ctx* c, std::vector<int>& s32) {
-  DevBuf &skraw = c->enc_buf[4], &skspec = c->enc_buf[5];
+  DevBuf<> &skraw = c->enc.secret.sk, &skspec = c->enc.secret.sk_spec;
   const int n = c->d.n;
   const int n_sk = (int)(s32.size() / (2 * (size_t)n));
-  auto up = [&]() -> int {
-    TRY(skraw.ensure(sizeof(int) * s32.size()));
-    TRY(skspec.ensure(sizeof(double2) * 2 * kM * n_sk));
-    CU(cudaMemcpyAsync(skraw.p, s32.data(), sizeof(int) * s32.size(), cudaMemcpyHostToDevice, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    return 0;
-  };
-  const int rc = up();
-  volatile int* vs = s32.data();
-  for (size_t i = 0; i < s32.size(); i++) vs[i] = 0;
-  ENC_TRY(rc);
-  ENC_TRY(prepare(c, (const int*)skraw.p, 2 * n, (double2*)skspec.p, 2 * kM, n_sk, 1, 1, 1));
-  return 0;
+  auto zero_host = on_exit([&] {
+    volatile int* vs = s32.data();
+    for (size_t i = 0; i < s32.size(); i++) vs[i] = 0;
+  });
+  TRY(skraw.ensure(sizeof(int) * s32.size()));
+  TRY(skspec.ensure(sizeof(double2) * 2 * kM * n_sk));
+  CU(cudaMemcpyAsync(skraw.p, s32.data(), sizeof(int) * s32.size(), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
+  return prepare(c, (const int*)skraw.p, 2 * n, (double2*)skspec.p, 2 * kM, n_sk, 1, 1, 1);
 }
-static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, const DevBuf& d_noise, bool noise_by_seq,
-                       int* d_out, long stride) {
+// the secret, its spectrum, the ChaCha20 keys of the Sources and the raw noise do not outlive the call, on any path:
+// the context belongs to the evaluator (INTEGRATION.md, colocated client / server mode)
+static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, bool noise_by_seq, int* d_out,
+                       long stride) {
+  auto wipe = on_exit([&] { wipe_secrets(c); cudaStreamSynchronize(c->stream); });
   const int n = c->d.n;
-  DevBuf &skspec = c->enc_buf[5], &pt = c->enc_buf[6], &mono = c->enc_buf[7],
-         &seq = c->enc_buf[8], &keys = c->enc_buf[9], &word0 = c->enc_buf[10], &poly = c->enc_buf[12],
-         &poly_sel = c->enc_buf[13], &sk_sel = c->enc_buf[14];
+  EncBufs& e = c->enc;
   {
     // the secrets the masks are multiplied by: the caller's sk, or (key generation) the n_sk output secrets of the batch
     std::vector<int> s32;
@@ -1564,81 +1563,79 @@ static int run_encrypt(fheram_ctx* c, const int64_t* sk, const EncBatch& b, cons
     }
     TRY(upload_secret(c, s32));
   }
-  auto up = [&](DevBuf& d, const void* h, size_t bytes) -> int {
+  auto up = [&](DevBuf<>& d, const void* h, size_t bytes) -> int {
     if (!bytes) return 0;
     TRY(d.ensure(bytes));
     CU(cudaMemcpyAsync(d.p, h, bytes, cudaMemcpyHostToDevice, c->stream));
     return 0;
   };
-  ENC_TRY(up(pt, b.pt.data(), b.pt.size()));
-  ENC_TRY(up(mono, b.mono.data(), b.mono.size() * sizeof(int)));
-  ENC_TRY(up(seq, b.seq.data(), b.seq.size() * sizeof(int)));
-  ENC_TRY(up(keys, b.keys.data(), b.keys.size() * sizeof(uint32_t)));
-  ENC_TRY(up(word0, b.word0.data(), b.word0.size() * sizeof(unsigned long long)));
-  ENC_TRY(up(poly, b.poly.data(), b.poly.size() * sizeof(short)));
-  ENC_TRY(up(poly_sel, b.poly_sel.data(), b.poly_sel.size() * sizeof(int)));
-  ENC_TRY(up(sk_sel, b.sk_sel.data(), b.sk_sel.size() * sizeof(int)));
+  TRY(up(e.pt, b.pt.data(), b.pt.size()));
+  TRY(up(e.mono, b.mono.data(), b.mono.size() * sizeof(int)));
+  TRY(up(e.seq, b.seq.data(), b.seq.size() * sizeof(int)));
+  TRY(up(e.secret.mask_keys, b.keys.data(), b.keys.size() * sizeof(uint32_t)));
+  TRY(up(e.secret.mask_word0, b.word0.data(), b.word0.size() * sizeof(unsigned long long)));
+  TRY(up(e.secret.poly, b.poly.data(), b.poly.size() * sizeof(short)));
+  TRY(up(e.poly_sel, b.poly_sel.data(), b.poly_sel.size() * sizeof(int)));
+  TRY(up(e.sk_sel, b.sk_sel.data(), b.sk_sel.size() * sizeof(int)));
   EncArgs a;
   a.out = d_out; a.ct_stride = stride; a.n_glwe = b.n_glwe; a.size = b.size;
   a.nl = (b.k_noise + kK - 1) / kK - 1; a.sh = (a.nl + 1) * kK - b.k_noise;
-  a.sk_spec = (const double2*)skspec.p;
-  a.noise = (const signed char*)d_noise.p; a.noise_by_seq = noise_by_seq ? 1 : 0;
-  a.pt = b.pt.empty() ? nullptr : (const signed char*)pt.p;
+  a.sk_spec = (const double2*)e.secret.sk_spec.p;
+  a.noise = (const signed char*)e.secret.noise.p; a.noise_by_seq = noise_by_seq ? 1 : 0;
+  a.pt = b.pt.empty() ? nullptr : (const signed char*)e.pt.p;
   a.pt_l = b.pt_l; a.pt_sh = b.pt_sh;
-  a.mono = b.mono.empty() ? nullptr : (const int*)mono.p;
-  a.poly = b.poly.empty() ? nullptr : (const short*)poly.p;
-  a.poly_sel = b.poly.empty() ? nullptr : (const int*)poly_sel.p;
-  a.sk_sel = b.sk_sel.empty() ? nullptr : (const int*)sk_sel.p;
-  a.seq = b.seq.empty() ? nullptr : (const int*)seq.p;
-  a.keys = (const uint32_t*)keys.p;
-  a.word0 = (const unsigned long long*)word0.p;
+  a.mono = b.mono.empty() ? nullptr : (const int*)e.mono.p;
+  a.poly = b.poly.empty() ? nullptr : (const short*)e.secret.poly.p;
+  a.poly_sel = b.poly.empty() ? nullptr : (const int*)e.poly_sel.p;
+  a.sk_sel = b.sk_sel.empty() ? nullptr : (const int*)e.sk_sel.p;
+  a.seq = b.seq.empty() ? nullptr : (const int*)e.seq.p;
+  a.keys = (const uint32_t*)e.secret.mask_keys.p;
+  a.word0 = (const unsigned long long*)e.secret.mask_word0.p;
   a.glwe_per_stream = b.glwe_per_stream;
   a.tw = c->tw;
   const int grid = b.n_glwe < 2 * c->sm_count ? b.n_glwe : 2 * c->sm_count;
   k_glwe_encrypt<<<grid, kThreads, 0, c->stream>>>(a);
   c->launches++;
-  ENC_CU(cudaGetLastError());
-  // the secret, its spectrum, the ChaCha20 keys of the Sources and the raw noise do not outlive the call: the
-  // context belongs to the evaluator (INTEGRATION.md, colocated client / server mode)
+  CU(cudaGetLastError());
+  wipe.dismiss();
   wipe_secrets(c);
-  ENC_CU(cudaStreamSynchronize(c->stream));
+  CU(cudaStreamSynchronize(c->stream));
   return 0;
 }
 
 // ---- decryption on the device (DESIGN.md 3.7): k_glwe_decrypt with the secret spectrum of the encryption path ----
 // zero the decrypted values / errors left on the device by a download
 static void wipe_plaintext(fheram_ctx* c) {
-  for (auto& b : c->dec_buf)
-    if (b.p) cudaMemsetAsync(b.p, 0, b.bytes, c->stream);
+  for (DevBuf<>* b : {&c->dec_values, &c->dec_err})
+    if (b->p) cudaMemsetAsync(b->p, 0, b->bytes, c->stream);
 }
 // a.in / n_glwe / placement fields set by the caller; n_out entries of values (and of errors when want_err) are left in
-// c->dec_buf.  The secret and its spectrum are wiped before this returns, on every path.
+// c->dec_values / c->dec_err.  The secret and its spectrum are wiped before this returns, on every path; the caller
+// downloads and synchronises.
 static int run_decrypt(fheram_ctx* c, const int64_t* sk, DecArgs a, size_t n_out, bool want_err) {
+  auto wipe = on_exit([&] { wipe_secrets(c); cudaStreamSynchronize(c->stream); });
   const int n = c->d.n;
   {
     std::vector<int> s32((size_t)2 * n, 0);
     for (int i = 0; i < n; i++) s32[i] = (int)sk[i];
     TRY(upload_secret(c, s32));
   }
-  ENC_TRY(c->dec_buf[0].ensure(n_out * sizeof(int16_t)));
-  if (want_err) ENC_TRY(c->dec_buf[1].ensure(n_out * sizeof(int64_t)));
-  ENC_TRY(fheram_decode_shifts(&c->params, &a.vsh, &a.ls));
+  TRY(c->dec_values.ensure(n_out * sizeof(int16_t)));
+  if (want_err) TRY(c->dec_err.ensure(n_out * sizeof(int64_t)));
+  TRY(fheram_decode_shifts(&c->params, &a.vsh, &a.ls));
   a.ct_stride = c->ct_stride(); a.size = c->d.size_ct; a.k_pt = c->params.k_pt;
-  a.sk_spec = (const double2*)c->enc_buf[5].p;
-  a.values = (short*)c->dec_buf[0].p;
-  a.err = want_err ? (long long*)c->dec_buf[1].p : nullptr;
+  a.sk_spec = (const double2*)c->enc.secret.sk_spec.p;
+  a.values = (short*)c->dec_values.p;
+  a.err = want_err ? (long long*)c->dec_err.p : nullptr;
   a.tw = c->tw;
   const int grid = a.n_glwe < 2 * c->sm_count ? a.n_glwe : 2 * c->sm_count;
   k_glwe_decrypt<<<grid, kThreads, kDecSmem, c->stream>>>(a);
   c->launches++;
-  ENC_CU(cudaGetLastError());
+  CU(cudaGetLastError());
+  wipe.dismiss();
   wipe_secrets(c);
   return 0;
 }
-#undef ENC_TRY
-#undef ENC_CU
-// on a failure after run_decrypt: the secret is already wiped, the decrypted values are not
-#define DEC_CU(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { wipe_plaintext(c); cudaStreamSynchronize(c->stream); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
 
 // Every byte of the resident RAM: what fheram_decrypt_ram gives on fheram_ram_store's output.  A sharded RAM fills the
 // entries of its own polynomials (h == shard mod n_shards) and leaves the others as they are.
@@ -1650,6 +1647,7 @@ extern "C" int fheram_ram_decrypt_sk(fheram_ram* r, const int64_t* sk, int16_t* 
   if (r->state || r->rotated)
     return fail(FHERAM_ERR_STATE, "the RAM is prepared for write (its data is rotated): call fheram_ram_write first");
   CU(cudaSetDevice(c->device));
+  auto wipe = on_exit([&] { wipe_plaintext(c); cudaStreamSynchronize(c->stream); });
   const int ws = c->params.word_size, n = c->d.n;
   const uint64_t max_addr = c->params.max_addr;
   DecArgs a;
@@ -1667,16 +1665,17 @@ extern "C" int fheram_ram_decrypt_sk(fheram_ram* r, const int64_t* sk, int16_t* 
     if (k == 1 && !err) break;
     const size_t el = k == 0 ? sizeof(int16_t) : sizeof(int64_t);
     char* dst = k == 0 ? (char*)values : (char*)err;
-    const char* src = (const char*)c->dec_buf[k].p;
+    const char* src = (const char*)(k == 0 ? c->dec_values.p : c->dec_err.p);
     if (n_full)
-      DEC_CU(cudaMemcpy2DAsync(dst + (size_t)r->shard * row * el, (size_t)r->n_shards * row * el, src, row * el, row * el,
+      CU(cudaMemcpy2DAsync(dst + (size_t)r->shard * row * el, (size_t)r->n_shards * row * el, src, row * el, row * el,
                                n_full, cudaMemcpyDeviceToHost, c->stream));
     if (n_full < r->n_local) {
       const uint64_t h = r->shard + (uint64_t)r->n_shards * n_full;
-      DEC_CU(cudaMemcpyAsync(dst + h * row * el, src + n_full * row * el, (max_addr - h * n) * ws * el,
+      CU(cudaMemcpyAsync(dst + h * row * el, src + n_full * row * el, (max_addr - h * n) * ws * el,
                              cudaMemcpyDeviceToHost, c->stream));
     }
   }
+  wipe.dismiss();
   wipe_plaintext(c);
   CU(cudaStreamSynchronize(c->stream));
   return 0;
@@ -1688,18 +1687,18 @@ extern "C" int fheram_decrypt_words_device(fheram_ctx* c, const int32_t* d_glwe,
   if (!c || !d_glwe || n < 1 || !sk || !values) return fail(FHERAM_ERR_INVALID, "null argument or n < 1");
   TRY(check_secret(sk, c->d.n));
   CU(cudaSetDevice(c->device));
+  auto wipe = on_exit([&] { wipe_plaintext(c); cudaStreamSynchronize(c->stream); });
   DecArgs a;
   memset(&a, 0, sizeof(a));
   a.in = d_glwe; a.n_glwe = n; a.coef0 = 1;
   TRY(run_decrypt(c, sk, a, (size_t)n, err != nullptr));
-  DEC_CU(cudaMemcpyAsync(values, c->dec_buf[0].p, (size_t)n * sizeof(int16_t), cudaMemcpyDeviceToHost, c->stream));
-  if (err)
-    DEC_CU(cudaMemcpyAsync(err, c->dec_buf[1].p, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaMemcpyAsync(values, c->dec_values.p, (size_t)n * sizeof(int16_t), cudaMemcpyDeviceToHost, c->stream));
+  if (err) CU(cudaMemcpyAsync(err, c->dec_err.p, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  wipe.dismiss();
   wipe_plaintext(c);
   CU(cudaStreamSynchronize(c->stream));
   return 0;
 }
-#undef DEC_CU
 
 // Ram::encrypt_sk (src/ram.rs:129-167; SubRam::encrypt_sk :334-380) into the device-resident RAM
 extern "C" int fheram_ram_encrypt_sk(fheram_ram* r, const uint8_t* data, const int64_t* sk,
@@ -1721,10 +1720,9 @@ extern "C" int fheram_ram_encrypt_sk(fheram_ram* r, const uint8_t* data, const i
   fheram_source_tell(xa, b.keys.data(), (uint64_t*)&b.word0[0]);
   b.glwe_per_stream = (int)total;
   // noise in the order of src/ram.rs:161-166 (sub-RAM major), every polynomial of every shard: one stream
-  DevBuf& d_noise = c->enc_buf[11];
   {
     fheram_source* xes[1] = {xe};
-    TRY(sample_noise(c, xes, 1, total * n, d_noise));
+    TRY(sample_noise(c, xes, 1, total * n));
   }
   b.pt.resize((size_t)b.n_glwe * n); b.seq.resize(b.n_glwe);
   for (int s = 0; s < ws; s++)
@@ -1737,7 +1735,7 @@ extern "C" int fheram_ram_encrypt_sk(fheram_ram* r, const uint8_t* data, const i
         b.pt[jl * n + j] = addr < p.max_addr ? (int8_t)data[addr * ws + s] : 0;  // src/ram.rs:364
       }
     }
-  TRY(run_encrypt(c, sk, b, d_noise, true, r->data, c->ct_stride()));
+  TRY(run_encrypt(c, sk, b, true, r->data, c->ct_stride()));
   fheram_source_skip_words(xa, 2ull * d.size_ct * n * total);
   r->loaded = true;
   r->state = false;
@@ -1779,10 +1777,9 @@ extern "C" int fheram_address_encrypt_sk(fheram_address* a, int first, int count
   b.keys.resize((size_t)8 * n_sources); b.word0.resize(n_sources);
   for (int i = 0; i < n_sources; i++) fheram_source_tell(xa[i], &b.keys[8 * i], (uint64_t*)&b.word0[i]);
   b.glwe_per_stream = n_sources == 1 ? b.n_glwe : per;
-  DevBuf& d_noise = c->enc_buf[11];
-  TRY(sample_noise(c, xe, n_sources, (size_t)b.n_glwe / n_sources * n, d_noise));
+  TRY(sample_noise(c, xe, n_sources, (size_t)b.n_glwe / n_sources * n));
   const long stride = (long)2 * d.size_addr * n;
-  TRY(run_encrypt(c, sk, b, d_noise, false, a->raw + (size_t)first * d.n_ggsw * c->ggsw_raw_len(), stride));
+  TRY(run_encrypt(c, sk, b, false, a->raw + (size_t)first * d.n_ggsw * c->ggsw_raw_len(), stride));
   for (int i = 0; i < n_sources; i++)
     fheram_source_skip_words(xa[i], 2ull * d.size_addr * n * (n_sources == 1 ? (uint64_t)b.n_glwe : (uint64_t)per));
   a->inv_ready = false;
@@ -1804,9 +1801,9 @@ extern "C" int fheram_keys_encrypt_sk(fheram_ctx* c, const int64_t* sk, fheram_s
   TRY(check_secret(sk, n));
   const size_t atk_raw = (size_t)d.dnum_ct * 2 * d.size_evk_trace * n;
   const size_t inv_raw = (size_t)d.dnum_ggsw * 2 * d.size_evk_inv * n;
-  fheram_keys* k = new fheram_keys();
+  auto k = std::make_unique<fheram_keys>();
   k->c = c;
-  CU(cudaMalloc(&k->raw, sizeof(int) * (atk_raw * log_n + 2 * inv_raw)));
+  TRY(k->raw.ensure(sizeof(int) * (atk_raw * log_n + 2 * inv_raw)));
   int *d_atk = k->raw, *d_tsk = k->raw + atk_raw * log_n, *d_inv = d_tsk + inv_raw;
   // phi_q(s): coefficient i of s goes to i q mod 2N with the sign of the wrap (client.cpp automorphism)
   auto autom = [&](long q, int* o) {
@@ -1854,17 +1851,16 @@ extern "C" int fheram_keys_encrypt_sk(fheram_ctx* c, const int64_t* sk, fheram_s
     b.keys.resize(8); b.word0.resize(1);
     fheram_source_tell(xa, b.keys.data(), (uint64_t*)&b.word0[0]);
     b.glwe_per_stream = b.n_glwe;
-    DevBuf& d_noise = c->enc_buf[11];
     fheram_source* xes[1] = {xe};
-    TRY(sample_noise(c, xes, 1, (size_t)b.n_glwe * n, d_noise));
-    TRY(run_encrypt(c, sk, b, d_noise, false, P.dst, (long)2 * P.size * n));
+    TRY(sample_noise(c, xes, 1, (size_t)b.n_glwe * n));
+    TRY(run_encrypt(c, sk, b, false, P.dst, (long)2 * P.size * n));
     fheram_source_skip_words(xa, 2ull * P.size * n * (uint64_t)b.n_glwe);
     volatile int* vs = b.sk_all.data();
     for (size_t i = 0; i < b.sk_all.size(); i++) vs[i] = 0;
   }
   { volatile short* vp = poly.data(); for (size_t i = 0; i < poly.size(); i++) vp[i] = 0; }
-  TRY(keys_prepare_device(c, d_atk, d_tsk, d_inv, k));
-  *out = k;
+  TRY(keys_prepare_device(c, d_atk, d_tsk, d_inv, k.get()));
+  *out = k.release();
   return 0;
 }
 // raw limbs of keys made by fheram_keys_encrypt_sk, in the layout fheram_keygen writes (tests; a client that wants to
@@ -2071,7 +2067,7 @@ extern "C" int fheram_ram_read_batch_device(fheram_ram* r, const fheram_address*
   const int B = addr->count, ws = c->params.word_size;
   const long L = c->ct_stride();
   const int chunk = batch_chunk(r);
-  DevBuf& all = r->all;  // results of every chunk
+  DevBuf<>& all = r->all;  // results of every chunk
   if (B <= chunk) {
     TRY(ram_local_stage(r, addr, 0, B, k, false));
     TRY(ram_finish_stage(r, (const int*)r->partial.p, B, 0, B, addr, 0, k, false));
@@ -2110,7 +2106,7 @@ extern "C" int fheram_ram_read(fheram_ram* r, const fheram_address* addr, const 
 // third stream.
 // Sharded RAM (fheram_comm_init done): every rank passes ITS n addresses and receives ITS n results; the global batch
 // is the concatenation over ranks.  Per chunk: each rank uploads and prepares only its own addresses, the prepared
-// GGSWs are all-gathered over NVLink (NCCL, in place), every rank rotates + packs its own polynomials for all
+// GGSWs are all-gathered over NVLink (ncclAllGather, in place), every rank rotates + packs its own polynomials for all
 // n_ranks * nb reads of the chunk, the packed partials are exchanged with one all-to-all, and each rank finishes its
 // own nb reads (top log2 n_ranks packer levels, second coordinate, trace).
 // in_fmt: 8 (int64 limbs), 4 (int32 limbs), 17 (packed 17-bit fields, fheram_pack17) or kSeededP17 (the bodies
@@ -2139,46 +2135,41 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
   // (cudaMalloc / cudaFree of gigabytes per call cost more than the copies they serve)
   typedef fheram_ram::HostPipe::Set Set;
   fheram_ram::HostPipe& hp = r->pipe;
-  int rc = 0;
-  auto cleanup = [&]() {
-    cudaStreamSynchronize(hp.copy_stream);
-    cudaStreamSynchronize(c->stream);
-    if (hp.down_stream) cudaStreamSynchronize(hp.down_stream);
-  };
-#define TRYC(x) do { rc = (x); if (rc) { cleanup(); return rc; } } while (0)
-#define CUC(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) { cleanup(); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, cudaGetErrorString(e_)); } } while (0)
-#define NCC(x) do { ncclResult_t e_ = (x); if (e_ != ncclSuccess) { cleanup(); return fail(FHERAM_ERR_CUDA, "%s: %s", #x, ncclGetErrorString(e_)); } } while (0)
   if (!hp.copy_stream) CU(cudaStreamCreateWithFlags(&hp.copy_stream, cudaStreamNonBlocking));
   if (!hp.down_stream) CU(cudaStreamCreateWithFlags(&hp.down_stream, cudaStreamNonBlocking));
   if (hp.cap < chunk) {
     for (auto& s : hp.sets) {
-      cudaFree(s.stage); cudaFree(s.a.raw); cudaFree(s.a.prep); cudaFree(s.a.prep1);
-      s.stage = nullptr; s.a.raw = nullptr; s.a.prep = nullptr; s.a.prep1 = nullptr;
+      s.stage.release(); s.a.raw.release(); s.a.prep.release(); s.a.prep1.release();
       s.a.c = c;
-      CU(cudaMalloc(&s.stage, sizeof(long long) * chunk * per_addr));       // int64 staging of the own slice
-      CU(cudaMalloc(&s.a.raw, sizeof(int) * chunk * per_addr));             // raw limbs of the own slice
+      TRY(s.stage.ensure(sizeof(long long) * chunk * per_addr));       // int64 staging of the own slice
+      TRY(s.a.raw.ensure(sizeof(int) * chunk * per_addr));             // raw limbs of the own slice
       // prepared GGSWs: first coordinate of every rank's slice (all-gathered), second coordinate of the own slice
-      CU(cudaMalloc(&s.a.prep, (size_t)G * chunk * d.coord_len[0] * glen * sizeof(double2)));
-      if (d.n_coord > 1) CU(cudaMalloc(&s.a.prep1, (size_t)chunk * d.coord_len[1] * glen * sizeof(double2)));
+      TRY(s.a.prep.ensure((size_t)G * chunk * d.coord_len[0] * glen * sizeof(double2)));
+      if (d.n_coord > 1) TRY(s.a.prep1.ensure((size_t)chunk * d.coord_len[1] * glen * sizeof(double2)));
       if (!s.copied) CU(cudaEventCreateWithFlags(&s.copied, cudaEventDisableTiming));
       if (!s.freed) CU(cudaEventCreateWithFlags(&s.freed, cudaEventDisableTiming));
     }
     for (int i = 0; i < 2; i++) {
-      cudaFree(hp.out_stage[i]);
-      hp.out_stage[i] = nullptr;
-      CU(cudaMalloc(&hp.out_stage[i], sizeof(long long) * (size_t)chunk * ws * L));
+      hp.out_stage[i].release();
+      TRY(hp.out_stage[i].ensure(sizeof(long long) * (size_t)chunk * ws * L));
       if (!hp.out_ready[i]) CU(cudaEventCreateWithFlags(&hp.out_ready[i], cudaEventDisableTiming));
       if (!hp.out_done[i]) CU(cudaEventCreateWithFlags(&hp.out_done[i], cudaEventDisableTiming));
     }
     hp.cap = chunk;
   }
-  if (G > 1) TRYC(r->xchg.ensure(sizeof(int) * (size_t)G * chunk * ws * L));
+  // every return from here on leaves the three streams of the pipeline idle
+  auto drain = on_exit([&] {
+    cudaStreamSynchronize(hp.copy_stream);
+    cudaStreamSynchronize(c->stream);
+    cudaStreamSynchronize(hp.down_stream);
+  });
+  if (G > 1) TRY(r->xchg.ensure(sizeof(int) * (size_t)G * chunk * ws * L));
   Set* sets = hp.sets;
   cudaStream_t copy_stream = hp.copy_stream;
   const int glwe_per_addr = d.n_ggsw * d.dnum_ct * 2;
   if (in_fmt == kSeededP17) {
-    TRYC(hp.seeds.ensure(sizeof(Seed) * n));
-    CUC(cudaMemcpyAsync(hp.seeds.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, copy_stream));
+    TRY(hp.seeds.ensure(sizeof(Seed) * n));
+    CU(cudaMemcpyAsync(hp.seeds.p, seeds, sizeof(Seed) * n, cudaMemcpyHostToDevice, copy_stream));
   }
   // chunk boundaries: the first chunk is small (its upload overlaps nothing), the sizes then double up to the full
   // chunk, and the schedule is laid out from the END so that no tiny chunk (narrow launches) trails a batch that is
@@ -2207,84 +2198,74 @@ static int read_batch_host_impl(fheram_ram* r, const void* ggsw_host, int in_fmt
     Set& s = sets[ci & 1];
     const int b0 = start[ci], nb = start[ci + 1] - b0;
     if (ci >= 2) CU(cudaStreamWaitEvent(copy_stream, s.freed, 0));
-    void* dst = in_fmt == 4 ? (void*)s.a.raw : (void*)s.stage;  // int32 limbs land where the prepare kernel reads them
+    void* dst = in_fmt == 4 ? (void*)s.a.raw.p : (void*)s.stage.p;  // int32 limbs land where the prepare kernel reads them
     const size_t addr_bytes = in_fmt == 17 ? per_addr * 17 / 8 :           // per_addr is a multiple of 4096
                               in_fmt == kSeededP17 ? per_addr / 2 * 17 / 8 : per_addr * in_fmt;
     CU(cudaMemcpyAsync(dst, in + (size_t)b0 * addr_bytes, (size_t)nb * addr_bytes, cudaMemcpyHostToDevice, copy_stream));
     if (in_fmt == 8) {
-      k_i64_to_i32<<<c->sm_count * 8, 256, 0, copy_stream>>>(s.stage, s.a.raw, (size_t)nb * per_addr, c->d_err);
+      k_i64_to_i32<<<c->sm_count * 8, 256, 0, copy_stream>>>(s.stage.p, s.a.raw.p, (size_t)nb * per_addr, c->d_err);
       c->launches++;
     } else if (in_fmt == 17) {
-      k_unpack17<<<c->sm_count * 8, 256, 0, copy_stream>>>((const uint32_t*)s.stage, s.a.raw, (size_t)nb * per_addr);
+      k_unpack17<<<c->sm_count * 8, 256, 0, copy_stream>>>((const uint32_t*)s.stage.p, s.a.raw.p, (size_t)nb * per_addr);
       c->launches++;
     } else if (in_fmt == kSeededP17) {
       ExpandArgs e;
       memset(&e, 0, sizeof(e));
-      e.out = s.a.raw;
+      e.out = s.a.raw.p;
       e.ct_stride = (long)2 * d.size_addr * d.n;
       e.n_glwe = nb * glwe_per_addr; e.size = d.size_addr;
-      e.body17 = (const uint32_t*)s.stage;
+      e.body17 = (const uint32_t*)s.stage.p;
       e.seeds = (const Seed*)hp.seeds.p + b0;
       e.glwe_per_stream = glwe_per_addr;
       TRY(launch_expand(c, e, copy_stream));
     }
     // one "matrix" of the prepare kernel = the coord_len[.] consecutive GGSWs of one coordinate of one address
     const int n0 = d.coord_len[0], n1 = d.n_coord > 1 ? d.coord_len[1] : 0;
-    double2* own = s.a.prep + (size_t)r->shard * nb * n0 * glen;
-    TRY(prepare(c, s.a.raw, (long)per_addr, own, (long)(n0 * glen), nb, n0 * d.dnum_ct, 2, d.size_addr, 1, true,
+    double2* own = s.a.prep.p + (size_t)r->shard * nb * n0 * glen;
+    TRY(prepare(c, s.a.raw.p, (long)per_addr, own, (long)(n0 * glen), nb, n0 * d.dnum_ct, 2, d.size_addr, 1, true,
                 copy_stream));
     if (n1)
-      TRY(prepare(c, s.a.raw + (size_t)n0 * c->ggsw_raw_len(), (long)per_addr, s.a.prep1, (long)(n1 * glen), nb,
+      TRY(prepare(c, s.a.raw.p + (size_t)n0 * c->ggsw_raw_len(), (long)per_addr, s.a.prep1.p, (long)(n1 * glen), nb,
                   n1 * d.dnum_ct, 2, d.size_addr, 1, true, copy_stream));
-    if (G > 1) NC(ncclAllGather(own, s.a.prep, (size_t)nb * n0 * glen * sizeof(double2), ncclChar, c->comm_prep, copy_stream));
+    if (G > 1) NC(ncclAllGather(own, s.a.prep.p, (size_t)nb * n0 * glen * sizeof(double2), ncclChar, c->comm_prep, copy_stream));
     CU(cudaEventRecord(s.copied, copy_stream));
     return 0;
   };
-  TRYC(issue_copy(0));
+  TRY(issue_copy(0));
   for (int ci = 0; ci < n_chunks; ci++) {
-    if (ci + 1 < n_chunks) TRYC(issue_copy(ci + 1));
+    if (ci + 1 < n_chunks) TRY(issue_copy(ci + 1));
     Set& s = sets[ci & 1];
     const int b0 = start[ci], nb = start[ci + 1] - b0;
     s.a.count = G * nb;
     s.a.prep1_first = r->shard * nb;
-    CUC(cudaStreamWaitEvent(c->stream, s.copied, 0));
-    TRYC(ram_local_stage(r, &s.a, 0, G * nb, k, false));
+    CU(cudaStreamWaitEvent(c->stream, s.copied, 0));
+    TRY(ram_local_stage(r, &s.a, 0, G * nb, k, false));
     const int* gathered = (const int*)r->partial.p;
     if (G > 1) {
-      TRYC(all_to_all_i32(c, (const int*)r->partial.p, (int*)r->xchg.p, (size_t)nb * ws * L));
+      TRY(all_to_all_i32(c, (const int*)r->partial.p, (int*)r->xchg.p, (size_t)nb * ws * L));
       gathered = (const int*)r->xchg.p;
     }
-    TRYC(ram_finish_stage(r, gathered, nb, 0, nb, &s.a, r->shard * nb, k, false));
-    CUC(cudaEventRecord(s.freed, c->stream));
+    TRY(ram_finish_stage(r, gathered, nb, 0, nb, &s.a, r->shard * nb, k, false));
+    CU(cudaEventRecord(s.freed, c->stream));
     // results: widened on the compute stream if the host wants int64, downloaded on a third stream (overlaps the
     // next chunk's reads)
-    long long* os = hp.out_stage[ci & 1];
-    if (ci >= 2) CUC(cudaStreamWaitEvent(c->stream, hp.out_done[ci & 1], 0));
+    long long* os = hp.out_stage[ci & 1].p;
+    if (ci >= 2) CU(cudaStreamWaitEvent(c->stream, hp.out_done[ci & 1], 0));
     const size_t n_res = (size_t)nb * ws * L;
     if (out_bytes == 8) {
       k_i32_to_i64<<<c->sm_count * 4, 256, 0, c->stream>>>((const int*)r->result.p, os, n_res);
       c->launches++;
     } else {
-      CUC(cudaMemcpyAsync(os, r->result.p, sizeof(int) * n_res, cudaMemcpyDeviceToDevice, c->stream));
+      CU(cudaMemcpyAsync(os, r->result.p, sizeof(int) * n_res, cudaMemcpyDeviceToDevice, c->stream));
     }
-    CUC(cudaEventRecord(hp.out_ready[ci & 1], c->stream));
-    CUC(cudaStreamWaitEvent(hp.down_stream, hp.out_ready[ci & 1], 0));
-    CUC(cudaMemcpyAsync(out + (size_t)b0 * ws * L * out_bytes, os, n_res * out_bytes, cudaMemcpyDeviceToHost, hp.down_stream));
-    CUC(cudaEventRecord(hp.out_done[ci & 1], hp.down_stream));
+    CU(cudaEventRecord(hp.out_ready[ci & 1], c->stream));
+    CU(cudaStreamWaitEvent(hp.down_stream, hp.out_ready[ci & 1], 0));
+    CU(cudaMemcpyAsync(out + (size_t)b0 * ws * L * out_bytes, os, n_res * out_bytes, cudaMemcpyDeviceToHost, hp.down_stream));
+    CU(cudaEventRecord(hp.out_done[ci & 1], hp.down_stream));
   }
-  CUC(cudaStreamSynchronize(c->stream));
-  CUC(cudaStreamSynchronize(hp.down_stream));
-  int err = 0;
-  CUC(cudaMemcpy(&err, c->d_err, sizeof(int), cudaMemcpyDeviceToHost));
-  cleanup();
-#undef TRYC
-#undef CUC
-#undef NCC
-  if (err) {
-    cudaMemset(c->d_err, 0, sizeof(int));
-    return fail(FHERAM_ERR_RANGE, "limb outside +-2^30: ciphertext limbs must be (nearly) normalised");
-  }
-  return 0;
+  CU(cudaStreamSynchronize(c->stream));
+  CU(cudaStreamSynchronize(hp.down_stream));
+  return take_range_error(c);
 }
 extern "C" int fheram_ram_read_batch_host(fheram_ram* r, const int64_t* ggsw_host, int n, const fheram_keys* k,
                                           int64_t* out_host) {
@@ -2439,10 +2420,8 @@ static int address_prepare_inv(const fheram_address* a, const fheram_keys* k) {
   const Derived& d = c->d;
   if (a->count != 1) return fail(FHERAM_ERR_INVALID, "write takes a single address");
   if (a->inv_ready) return 0;
-  if (!a->inv_raw) {
-    CU(cudaMalloc(&a->inv_raw, sizeof(int) * (size_t)d.n_ggsw * c->ggsw_raw_len()));
-    CU(cudaMalloc(&a->inv_prep, sizeof(double2) * (size_t)d.n_ggsw * c->ggsw_prep_len()));
-  }
+  TRY(a->inv_raw.ensure(sizeof(int) * (size_t)d.n_ggsw * c->ggsw_raw_len()));
+  TRY(a->inv_prep.ensure(sizeof(double2) * (size_t)d.n_ggsw * c->ggsw_prep_len()));
   TRY(ggsw_invert_device(c, k, a->raw, d.n_ggsw, a->inv_raw));
   TRY(prepare_ggsw(c, a->inv_raw, a->inv_prep, d.n_ggsw));
   a->inv_ready = true;
@@ -2537,15 +2516,15 @@ extern "C" int fheram_coordinate_product(fheram_ctx* c, const int64_t* in, int n
     return fail(FHERAM_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(c->device));
   const long L = c->ct_stride();
-  TRY(c->opbuf[0].ensure(sizeof(int) * (size_t)n * L));
-  TRY(c->opbuf[1].ensure(sizeof(int) * (size_t)n_ggsw * c->ggsw_raw_len()));
-  TRY(c->opbuf[2].ensure(sizeof(double2) * (size_t)n_ggsw * c->ggsw_prep_len()));
-  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->opbuf[0].p));
-  TRY(upload_i64(c, ggsws, (size_t)n_ggsw * c->ggsw_raw_len(), (int*)c->opbuf[1].p));
-  TRY(prepare_ggsw(c, (int*)c->opbuf[1].p, (double2*)c->opbuf[2].p, n_ggsw));
-  TRY(run_ext_chain(c, n, (int*)c->opbuf[0].p, nullptr, 0, (int*)c->opbuf[0].p, (double2*)c->opbuf[2].p,
+  TRY(c->op_ct.ensure(sizeof(int) * (size_t)n * L));
+  TRY(c->op_ct2.ensure(sizeof(int) * (size_t)n_ggsw * c->ggsw_raw_len()));
+  TRY(c->op_aux.ensure(sizeof(double2) * (size_t)n_ggsw * c->ggsw_prep_len()));
+  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->op_ct.p));
+  TRY(upload_i64(c, ggsws, (size_t)n_ggsw * c->ggsw_raw_len(), (int*)c->op_ct2.p));
+  TRY(prepare_ggsw(c, (int*)c->op_ct2.p, (double2*)c->op_aux.p, n_ggsw));
+  TRY(run_ext_chain(c, n, (int*)c->op_ct.p, nullptr, 0, (int*)c->op_ct.p, (double2*)c->op_aux.p,
                     n_ggsw, 0, 0));
-  return download_i64(c, (int*)c->opbuf[0].p, (size_t)n * L, out);
+  return download_i64(c, (int*)c->op_ct.p, (size_t)n * L, out);
 }
 extern "C" int fheram_external_product_batch(fheram_ctx* c, const int64_t* in, int n, const int64_t* ggsw,
                                              int64_t* out) {
@@ -2558,32 +2537,32 @@ extern "C" int fheram_glwe_trace(fheram_ctx* c, const fheram_keys* k, const int6
     return fail(FHERAM_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(c->device));
   const long L = c->ct_stride();
-  TRY(c->opbuf[0].ensure(sizeof(int) * (size_t)n * L));
-  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->opbuf[0].p));
-  if (end > start) TRY(run_trace_chain(c, k, n, (int*)c->opbuf[0].p, nullptr, 0, 0, (int*)c->opbuf[0].p, start, end));
-  return download_i64(c, (int*)c->opbuf[0].p, (size_t)n * L, out);
+  TRY(c->op_ct.ensure(sizeof(int) * (size_t)n * L));
+  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->op_ct.p));
+  if (end > start) TRY(run_trace_chain(c, k, n, (int*)c->op_ct.p, nullptr, 0, 0, (int*)c->op_ct.p, start, end));
+  return download_i64(c, (int*)c->op_ct.p, (size_t)n * L, out);
 }
 
 extern "C" int fheram_glwe_pack(fheram_ctx* c, const fheram_keys* k, const int64_t* in, int n, int64_t* out) {
   if (!c || !k || !in || !out || n < 1 || n > kN) return fail(FHERAM_ERR_INVALID, "n must be in 1..N");
   CU(cudaSetDevice(c->device));
   const long L = c->ct_stride();
-  TRY(c->opbuf[0].ensure(sizeof(int) * (size_t)n * L));
-  TRY(c->opbuf[1].ensure(sizeof(int) * (size_t)n * L));
-  TRY(c->opbuf[2].ensure(sizeof(int) * (size_t)2 * n));  // input order | operand table of the mixed level
-  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->opbuf[1].p));
+  TRY(c->op_ct.ensure(sizeof(int) * (size_t)n * L));
+  TRY(c->op_ct2.ensure(sizeof(int) * (size_t)n * L));
+  TRY(c->op_aux.ensure(sizeof(int) * (size_t)2 * n));  // input order | operand table of the mixed level
+  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->op_ct2.p));
   std::vector<int> map, ops;
   packer_order(n, map, ops);
-  int* d_map = (int*)c->opbuf[2].p;
+  int* d_map = (int*)c->op_aux.p;
   CU(cudaMemcpyAsync(d_map, map.data(), sizeof(int) * n, cudaMemcpyHostToDevice, c->stream));
   if (!ops.empty())
     CU(cudaMemcpyAsync(d_map + n, ops.data(), sizeof(int) * ops.size(), cudaMemcpyHostToDevice, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   const int one_sided = c->d.log_n - ilog2(n);
-  int* A = (int*)c->opbuf[0].p;
-  TRY(run_trace_chain(c, k, n, (int*)c->opbuf[1].p, d_map, n, 0, A, 0, one_sided));
+  int* A = (int*)c->op_ct.p;
+  TRY(run_trace_chain(c, k, n, (int*)c->op_ct2.p, d_map, n, 0, A, 0, one_sided));
   int* res = nullptr;
-  TRY(run_pack_tree(c, k, 1, n, one_sided, d_map + n, A, (int*)c->opbuf[1].p, &res));
+  TRY(run_pack_tree(c, k, 1, n, one_sided, d_map + n, A, (int*)c->op_ct2.p, &res));
   return download_i64(c, res, (size_t)L, out);
 }
 
@@ -2594,18 +2573,18 @@ extern "C" int fheram_glwe_automorphism(fheram_ctx* c, const fheram_keys* k, int
   if ((mode == 0) == (rsh != 0)) return fail(FHERAM_ERR_INVALID, "mode 0 runs without rsh, modes 1/2 with rsh=1 (the fused kernels' shapes)");
   CU(cudaSetDevice(c->device));
   const long L = c->ct_stride();
-  TRY(c->opbuf[0].ensure(sizeof(int) * (size_t)n * L));
-  TRY(c->opbuf[1].ensure(sizeof(int) * (size_t)n * L));
-  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->opbuf[0].p));
-  int* res = (int*)c->opbuf[0].p;
+  TRY(c->op_ct.ensure(sizeof(int) * (size_t)n * L));
+  TRY(c->op_ct2.ensure(sizeof(int) * (size_t)n * L));
+  TRY(upload_i64(c, in, (size_t)n * L, (int*)c->op_ct.p));
+  int* res = (int*)c->op_ct.p;
   if (mode == 0) {
-    VmpArgs a = base_args(c, n, (int*)c->opbuf[0].p, (int*)c->opbuf[1].p, L);
+    VmpArgs a = base_args(c, n, (int*)c->op_ct.p, (int*)c->op_ct2.p, L);
     a.n_steps = 1;
     a.mat[0] = k->atk + (size_t)gal_idx * c->atk_prep_len();
     a.gal[0] = (int)((galois(c->d.log_n, gal_idx) + 2 * kN) % (2 * kN));
     a.gal_inv[0] = inv_mod_2n(a.gal[0]);
     TRY(launch(c, KC_OTHER, K_AUTO3, std::min(n, c->sm_count), kThreads, smem_bytes(3), a));
-    res = (int*)c->opbuf[1].p;
+    res = (int*)c->op_ct2.p;
   } else {
     TRY(run_trace_chain(c, k, n, res, nullptr, 0, 0, res, gal_idx, gal_idx + 1, 0, 0, 0, mode == 1 ? 1 : -1));
   }
@@ -2616,9 +2595,9 @@ extern "C" int fheram_ggsw_invert(fheram_ctx* c, const fheram_keys* k, const int
   if (!c || !k || !ggsw || !out || n < 1) return fail(FHERAM_ERR_INVALID, "bad argument");
   CU(cudaSetDevice(c->device));
   const size_t len = (size_t)n * c->ggsw_raw_len();
-  TRY(c->opbuf[0].ensure(sizeof(int) * len));
-  TRY(c->opbuf[1].ensure(sizeof(int) * len));
-  TRY(upload_i64(c, ggsw, len, (int*)c->opbuf[0].p));
-  TRY(ggsw_invert_device(c, k, (int*)c->opbuf[0].p, n, (int*)c->opbuf[1].p));
-  return download_i64(c, (int*)c->opbuf[1].p, len, out);
+  TRY(c->op_ct.ensure(sizeof(int) * len));
+  TRY(c->op_ct2.ensure(sizeof(int) * len));
+  TRY(upload_i64(c, ggsw, len, (int*)c->op_ct.p));
+  TRY(ggsw_invert_device(c, k, (int*)c->op_ct.p, n, (int*)c->op_ct2.p));
+  return download_i64(c, (int*)c->op_ct2.p, len, out);
 }

@@ -98,6 +98,9 @@ int fheram_fp64_peak_probe(fheram_ctx *ctx, int reps, double *tflops);
  * counting, enable = 0 reads {prologue, forward pass 1, forward warp passes, contraction, inverse
  * transform, epilogue, rest, -} into out and stops. */
 int fheram_debug_phase_cycles(fheram_ctx *ctx, int enable, long long out[8]);
+/* debug: bytes of device memory the library holds right now, over every context, handle and device
+ * of the process (a leak check that does not depend on other users of the GPU) */
+uint64_t fheram_debug_device_bytes(void);
 /* pin / unpin a caller-owned host buffer (cudaHostRegister) so uploads run at PCIe speed */
 int fheram_host_register(void *p, size_t bytes);
 int fheram_host_unregister(void *p);
