@@ -20,8 +20,6 @@
 
 #include "../../include/fheram.h"
 #include "kernels.cuh"
-#include "kernels_ks2.cuh"
-#include "kernels_ks3.cuh"
 #include "kernels_ks4.cuh"
 #include "kernels_ks5.cuh"
 #include "kernels_ks6.cuh"
@@ -252,7 +250,7 @@ struct fheram_ctx {
   ncclComm_t comm_prep = nullptr;  // second communicator: all-gather of prepared GGSWs on the upload stream, beside the reads
   int n_ranks = 1, rank = 0;
   DevBuf<double2> d_tw;  // tw6 | tw7c | tw8c | tw9 | tw10c
-  DevBuf<double2> d_tw16;  // twiddles of the 16-point transform (kernels_ks7.cuh): [16][16] | [128][7]
+  DevBuf<double2> d_tw16;  // twiddles of the 16-point transform (transform16.cuh): [16][16] | [128][7]
   Twiddles tw;
   DevBuf<int> d_err;
   uint64_t launches = 0;

@@ -53,7 +53,13 @@ __device__ __forceinline__ double2 ldg_pinned(const double2* p) {
   asm volatile("ld.global.nc.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
   return v;
 }
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ double2 mul_i(double2 w) { return make_double2(-w.y, w.x); }
+// acc += a g (complex multiply-accumulate of the contraction)
+__device__ __forceinline__ void cmac(double2& acc, const double2 a, const double2 g) {
+  acc.x = fma(a.x, g.x, fma(-a.y, g.y, acc.x));
+  acc.y = fma(a.x, g.y, fma(a.y, g.x, acc.y));
+}
 __device__ __forceinline__ double2 conj_(double2 w) { return make_double2(w.x, -w.y); }
 
 // forward butterfly: (x, y) <- (x + w y, x - w y), 6 FP64 FMA-pipe ops
@@ -288,6 +294,20 @@ __device__ __forceinline__ const int* mixed_src(const VmpArgs& A, int item, bool
   two = (op & 1) != 0;
   return A.src + ((long)(item / A.src_div) * A.src_mod + (op >> 1)) * A.ct_stride;
 }
+// source ciphertext of `item` through src_div / src_mod / src_map
+__device__ __forceinline__ const int* item_src(const VmpArgs& A, int item) {
+  long idx = item;
+  if (A.src_div > 0) idx = item / A.src_div;
+  else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
+  return A.src + idx * A.ct_stride;
+}
+// the same for the key-switch modes: COMBINE2 reads the pair at 2 item, MODE_MIXED the operand table (two = b present)
+template <int MODE>
+__device__ __forceinline__ const int* mode_src(const VmpArgs& A, int item, bool& two) {
+  if constexpr (MODE == MODE_MIXED) return mixed_src(A, item, two);
+  else if constexpr (MODE == MODE_COMBINE2) return A.src + 2L * item * A.ct_stride;
+  else return item_src(A, item);
+}
 #define PHASE_TICK(ph)                                                      \
   do {                                                                      \
     if (A.phase_cycles && threadIdx.x == 0) {                               \
@@ -325,13 +345,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
   for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
 
-    const int* src;
-    {
-      long idx = item;
-      if (A.src_div > 0) idx = item / A.src_div;
-      else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
-      src = A.src + idx * A.ct_stride;
-    }
+    const int* src = item_src(A, item);
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     for (int step = 0; step < A.n_steps; step++) {
@@ -403,10 +417,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_vmp(const VmpArgs A) {
 #pragma unroll
           for (int j = 0; j < 8; j++) {
             const double2 a = ap[32 * j];
-            cur[j].x = fma(a.x, g0[j].x, fma(-a.y, g0[j].y, cur[j].x));
-            cur[j].y = fma(a.x, g0[j].y, fma(a.y, g0[j].x, cur[j].y));
-            nxt[j].x = fma(a.x, g1[j].x, fma(-a.y, g1[j].y, nxt[j].x));
-            nxt[j].y = fma(a.x, g1[j].y, fma(a.y, g1[j].x, nxt[j].y));
+            cmac(cur[j], a, g0[j]);
+            cmac(nxt[j], a, g1[j]);
           }
         }
         PHASE_TICK(3);

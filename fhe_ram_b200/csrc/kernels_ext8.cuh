@@ -1,10 +1,7 @@
 // kernels_ext8.cuh -- external-product chains (CoordinatePrepared::product / product_inplace,
-// src/coordinate_prepared.rs:147-177) on the TWO-EXCHANGE transform of kernels_ks7.cuh, ONE ciphertext per SM.
+// src/coordinate_prepared.rs:147-177) on the TWO-EXCHANGE transform of transform16.cuh, ONE ciphertext per SM.
 //
-// The round-1 kernel (k_ext3, since retired) ran its 14 transforms one after the other on 256 threads x 8 points
-// (three shared-memory exchanges each), kept two of the six input spectra in shared memory (read back 8 times)
-// and waited one L2 round trip per 32 KiB matrix tile.  Here one CTA of 512 threads = FOUR groups of 128
-// threads owns the SM and one ciphertext:
+// One CTA of 512 threads = FOUR groups of 128 threads owns the SM and one ciphertext:
 //   forward     rows rho = 2 limb + col of the input: group g transforms rows g and g + 4 (16 points per thread,
 //               passes of 4 + 4 + 3 stages, private 34 KiB exchange buffer per group, no lock);
 //               ALL six spectra live in tensor memory (6 x 64 columns; thread t of every group is tensor-memory
@@ -12,7 +9,7 @@
 //   contraction group g owns output column g & 1, limbs {3, 2} (g < 2) or {1, 0}: per output 24 chunks of
 //   + inverse   4 frequencies x 6 rows, the matrix chunk of step c + 1 in flight while chunk c is multiplied
 //               (the tile stream never drains: no round trip per tile), then inverse16 and the word update
-//   words       the ciphertext between the steps of a chain stays on chip as 51-bit words (kernels_ks3.cuh),
+//   words       the ciphertext between the steps of a chain stays on chip as 51-bit words (words.cuh),
 //               kept as two 32-bit halves lo = W mod 2^26 (+ carries), hi = W >> 26 (+ carries) with
 //               W = lo + hi 2^26 (mod 2^51): the limb-3 group STORES its contribution (+ bias), the three other
 //               contributions of the column are added with native 32-bit shared atomics (no return value, no
@@ -20,7 +17,10 @@
 // Same integers as k_ext9 and the oracle's external product; the prepared GGSWs are in the frequency order of k_prepare7.
 // Shared memory 4 (pass-2 twiddles) + 4 x 34 (exchange) + 64 (words) = 204 KiB, 512 tensor-memory columns.
 #pragma once
-#include "kernels_ks7.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
+#include "transform16.cuh"
+#include "words.cuh"
 
 // groups 2, 3 start contracting rows 0..3 while groups 0, 1 transform rows 4, 5 (0: all groups wait for the six rows)
 // timing ablations (results are garbage): 1 no matrix stream, 2 no tensor-memory loads in the contraction
@@ -41,17 +41,6 @@ constexpr int kExt8Threads = 512;
 constexpr size_t kExt8Smem = (size_t)256 * sizeof(double2) + (size_t)4 * kPad16 * sizeof(double2) +
                              (size_t)4 * kN * sizeof(uint32_t) + 32;
 
-__device__ __forceinline__ void pair_arrive(int id) { asm volatile("bar.arrive %0, 256;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void pair_sync(int id) { asm volatile("bar.sync %0, 256;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void cp_async16(const void* smem, const void* gmem) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void red_add_u32(uint32_t* p, uint32_t v) {
-  asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(smem_u32(p)), "r"(v) : "memory");
-}
 // digit fields of the word W = lo + hi 2^26 (limb 0 = bits 34..50, limb 1 = 17..33, limb 2 = 0..16)
 __device__ __forceinline__ uint32_t word_field(uint32_t lo, uint32_t hi, int limb) {
   if (limb == 2) return lo & 0x1ffffu;
@@ -60,7 +49,7 @@ __device__ __forceinline__ uint32_t word_field(uint32_t lo, uint32_t hi, int lim
 }
 
 __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const double2* __restrict__ tw16) {
-  constexpr int NR = 6, LOUT = 4, NOUT = 2 * LOUT;
+  constexpr int NR = 6, LOUT = 4;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double2* tw2 = reinterpret_cast<double2*>(smem_raw);
   double2* bufs = tw2 + 256;
@@ -71,46 +60,21 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
   const int tid = threadIdx.x, g = tid >> 7, t = tid & 127;
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc<512>(slot);
   if (tid < 256) tw2[tid] = __ldg(tw16 + tid);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *slot;
   const uint32_t tsp = tmem_base + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);  // spectrum rho at column 64 rho
   const uint32_t ttw = tsp + 384;                                              // 7 pass-3 twiddles (28 columns)
-  if (g == 0) {
-    const Tw3x w = load_tw3x(tw16, t);
-    const double2 p0[4] = {w.w8, w.w9a, w.w9b, w.w10[0]};
-    const double2 p1[4] = {w.w10[1], w.w10[2], w.w10[3], w.w10[3]};
-    tm_st4(ttw, p0);
-    tm_st4(ttw + 16, p1);
-    tm_wait_st();
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  auto t3f = [&]() {
-    double2 p0[4], p1[4];
-    tm_ld4(ttw, p0);
-    tm_ld4(ttw + 16, p1);
-    Tw3x w;
-    w.w8 = p0[0]; w.w9a = p0[1]; w.w9b = p0[2]; w.w10[0] = p0[3];
-    w.w10[1] = p1[0]; w.w10[2] = p1[1]; w.w10[3] = p1[2];
-    return w;
-  };
+  if (g == 0) park_tw3x(ttw, tw16, t);
+  tmem_sync();
+  auto t3f = [&]() { return tm_tw3x(ttw); };
   const T16 tc{bufs + g * kPad16, tw2, nullptr, t, g};
   const int co = g & 1;                    // output column of this group
   uint32_t* clo = xlo + co * kN + t;       // its words, position t (+ 128 m, + 2048)
   uint32_t* chi = xhi + co * kN + t;
   const int pair_bar = 5 + co;             // barriers 1..4: the groups (gsync128)
   long long phase_t0 = A.phase_cycles ? clock64() : 0;
-  // groups of a pair leave every CTA-wide barrier A.stagger cycles apart, so that one is in a register pass (FP64 pipe)
-  // while the other exchanges (shared-memory pipe) instead of both queueing for the same unit
-  auto skew = [&]() {};
   // SMs start a quarter of a step apart: the grid is uniform, so without it every SM streams its matrix tiles in the
   // same thousands of cycles and the L2 (21.8 TB/s in total, tools/tile_stage_probe.cu) is the bound of that phase
   if (A.stagger > 0) {
@@ -120,13 +84,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
 
   for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
-    const int* src;
-    {
-      long idx = item;
-      if (A.src_div > 0) idx = item / A.src_div;
-      else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
-      src = A.src + idx * A.ct_stride;
-    }
+    const int* src = item_src(A, item);
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
     for (int step = 0; step < A.n_steps; step++) {
@@ -164,18 +122,13 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
       };
       fwd_row(g);
       tm_wait_st();
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();  // rows 0..3 visible to every group
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      skew();
+      tmem_sync();  // rows 0..3 visible to every group
       if (!FHERAM_EXT8_STAGGER) {
         if (g < 2) {
           fwd_row(g + 4);
           tm_wait_st();
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();  // six spectra visible to every group; every read of the old words is done
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tmem_sync();  // six spectra visible to every group; every read of the old words is done
       } else if (g < 2) {
         // rows 4 and 5 while groups 2 and 3 already contract rows 0..3 (their matrix stream then runs beside these
         // transforms and, one output later, beside the inverse transforms of groups 0 and 1)
@@ -191,20 +144,12 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
       // ----------------- contraction + inverse transform + word update: two outputs per group -----------------
       constexpr int kDepth = 4;
       double2* stage = tc.buf + t;  // slot (s, j) of this thread: stage[(4 s + j) * 128]
-      auto stage_issue = [&](const double2* gp, int c) {
-        const double2* np = gp + (size_t)(c >> 2) * NOUT * kM + 512 * (c & 3);
-#pragma unroll
-        for (int j = 0; j < 4; j++) cp_async16(stage + (4 * (c % kDepth) + j) * 128, np + 128 * j);
-        cp_async_commit();
-      };
-      auto stage_begin = [&](const double2* gp) {
-#pragma unroll
-        for (int c = 0; c < kDepth - 1; c++) stage_issue(gp, c);
-      };
+      auto stage_issue = [&](const double2* gp, int c) { ring_issue(stage, gp, c, c % kDepth); };
+      auto stage_begin = [&](const double2* gp) { ring_fill<kDepth - 1>(stage, gp); };
 #pragma unroll 1
       for (int k = 0; k < 2; k++) {
         const int l = (g < 2 ? 3 : 1) - k;
-        const double2* gp = G + (size_t)(co * LOUT + l) * kM + t;  // + rho NOUT kM + 128 r
+        const double2* gp = G + (size_t)(co * LOUT + l) * kM + t;  // + rho 2 LOUT kM + 128 r
         // 24 chunks of (row rho = c >> 2, frequencies r = 4 (c & 3) .. + 3).  The matrix stream is staged by cp.async
         // (16 bytes per thread and value, thread-private slots, completion by groups: no registers and no scoreboard
         // held by the values in flight) in the group's exchange buffer, idle during the contraction: kDepth - 1
@@ -220,7 +165,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
 #pragma unroll
         for (int c = 0; c < 4 * NR; c++) {
           if (c + 1 < 4 * NR) {
-            const double2* np = gp + (size_t)((c + 1) >> 2) * NOUT * kM + 512 * ((c + 1) & 3);
+            const double2* np = gp + (size_t)((c + 1) >> 2) * 2 * LOUT * kM + 512 * ((c + 1) & 3);
 #pragma unroll
             for (int j = 0; j < 4; j++) gb[(c + 1) & 1][j] = ldg_pinned(np + 128 * j);
           }
@@ -231,12 +176,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
           double2 a[4];
           tm_ld4(tsp + 64 * (c >> 2) + 16 * (c & 3), a);
 #pragma unroll
-          for (int j = 0; j < 4; j++) {
-            double2& acc = cur[4 * (c & 3) + j];
-            const double2 m = gb[c & 1][j];
-            acc.x = fma(a[j].x, m.x, fma(-a[j].y, m.y, acc.x));
-            acc.y = fma(a[j].x, m.y, fma(a[j].y, m.x, acc.y));
-          }
+          for (int j = 0; j < 4; j++) cmac(cur[4 * (c & 3) + j], a[j], gb[c & 1][j]);
         }
 #else
         if (k == 0) stage_begin(gp);
@@ -267,11 +207,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
             tm_ld4(tsp + 64 * (c >> 2) + 16 * (c & 3), a);
           }
 #pragma unroll
-          for (int j = 0; j < 4; j++) {
-            double2& acc = cur[4 * (c & 3) + j];
-            acc.x = fma(a[j].x, m[j].x, fma(-a[j].y, m[j].y, acc.x));
-            acc.y = fma(a[j].x, m[j].y, fma(a[j].y, m[j].x, acc.y));
-          }
+          for (int j = 0; j < 4; j++) cmac(cur[4 * (c & 3) + j], a[j], m[j]);
         }
 #endif
         gsync128(g);  // every staged value is read before the inverse transform's first store into the buffer
@@ -285,9 +221,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
           for (int q = 0; q < 32; q++) {
             const int off = 128 * (q & 15) + (q >> 4) * kM;
             const double v = (q < 16) ? cur[q & 15].x : cur[q & 15].y;
-            const double tt = v + (kMagic52 + 65536.0);
-            const int c3 = (int)__funnelshift_r((uint32_t)__double2loint(tt), (uint32_t)__double2hiint(tt), 17);
-            const unsigned long long W = ((unsigned long long)(long long)c3 + kBias51) & kMask51;
+            const unsigned long long W = (limb_word(v, 3, 1.0, true, 0u) + kBias51) & kMask51;
             clo[off] = (uint32_t)W & 0x3ffffffu;
             chi[off] = (uint32_t)(W >> 26);
           }
@@ -323,10 +257,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
         PHASE_TICK(5);
       }
       // every contribution landed before the next step's reads; every spectrum read precedes the next stores
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      skew();
+      tmem_sync();
     }  // steps
 
     // digits of the final words -> dst (coalesced)
@@ -344,9 +275,7 @@ __global__ void __launch_bounds__(kExt8Threads, 1) k_ext8(const VmpArgs A, const
     __syncthreads();  // words reuse by the next item
     PHASE_TICK(6);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+  tmem_free<512>(tmem_base, tid < 32);
 }
 
 }  // namespace fheram

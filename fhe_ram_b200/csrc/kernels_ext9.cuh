@@ -13,7 +13,10 @@
 // One cluster barrier per step, no distributed shared memory, no atomics.  Same integers as k_ext8; the
 // prepared GGSWs are in the frequency order of k_prepare7.
 #pragma once
-#include "kernels_ks8.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
+#include "transform16.cuh"
+#include "words.cuh"
 
 namespace fheram {
 
@@ -44,37 +47,15 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ext9(cons
   const int l = o & 3;
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc<512>(slot);
   if (tid < 256) tw2[tid] = __ldg(tw16 + tid);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *slot;
   const uint32_t tsp = tmem_base + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);  // spectrum rho at column 64 rho
   const uint32_t ttw = tsp + 384;                                              // 7 pass-3 twiddles (28 columns)
-  if (g == 0) {
-    const Tw3x w = load_tw3x(tw16, t);
-    const double2 p0[4] = {w.w8, w.w9a, w.w9b, w.w10[0]};
-    const double2 p1[4] = {w.w10[1], w.w10[2], w.w10[3], w.w10[3]};
-    tm_st4(ttw, p0);
-    tm_st4(ttw + 16, p1);
-    tm_wait_st();
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  auto t3f = [&]() {
-    double2 p0[4], p1[4];
-    tm_ld4(ttw, p0);
-    tm_ld4(ttw + 16, p1);
-    Tw3x w;
-    w.w8 = p0[0]; w.w9a = p0[1]; w.w9b = p0[2]; w.w10[0] = p0[3];
-    w.w10[1] = p1[0]; w.w10[2] = p1[1]; w.w10[3] = p1[2];
-    return w;
-  };
+  if (g == 0) park_tw3x(ttw, tw16, t);
+  tmem_sync();
+  auto t3f = [&]() { return tm_tw3x(ttw); };
   // group 3 runs its inverse transform in the exchange buffer of group 1 (idle after the forward transforms)
   const T16 tc{bufs + (g < 3 ? g : 1) * kPad16, tw2, nullptr, t, g};
 
@@ -82,17 +63,6 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ext9(cons
   // per cluster: contribution slabs C[2 parities][8 outputs][N]
   unsigned long long* Cs = reinterpret_cast<unsigned long long*>(A.scratch) + (size_t)cluster_id * kKs8ScratchWords;
   double2* stage = ring + og * (R * 512) + t;  // slot s, value j of this thread: stage[(4 s + j) * 128]
-  auto ring_issue = [&](const double2* gp, int c, int s) {
-    const double2* np = gp + (size_t)(c >> 2) * NOUT * kM + 512 * (c & 3);
-#pragma unroll
-    for (int j = 0; j < 4; j++) cp_async16(stage + (4 * s + j) * 128, np + 128 * j);
-    cp_async_commit();
-  };
-  auto ring_fill = [&](const double2* Gmat) {
-    const double2* gp = Gmat + (size_t)o * kM + t;
-#pragma unroll
-    for (int c = 0; c < R; c++) ring_issue(gp, c, c);
-  };
 
   for (int item = cluster_id; item < A.n_items; item += n_clusters) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
@@ -104,7 +74,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ext9(cons
       src = A.src + idx * A.ct_stride;
     }
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
-    if (out_group) ring_fill(A.mat[0] + mat_off);
+    if (out_group) ring_fill<R>(stage, A.mat[0] + mat_off + (size_t)o * kM + t);
 
     for (int step = 0; step < A.n_steps; step++) {
       const bool last = step + 1 == A.n_steps, first = step == 0;
@@ -188,16 +158,12 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ext9(cons
           const int s = c % R;
 #pragma unroll
           for (int j = 0; j < 4; j++) m[j] = stage[(4 * s + j) * 128];
-          if (c + R < NCH) ring_issue(gp, c + R, s);  // refill the slot just read
+          if (c + R < NCH) ring_issue(stage, gp, c + R, s);  // refill the slot just read
           tm_ld4(tsp + 64 * (c >> 2) + 16 * (c & 3), a);
 #pragma unroll
-          for (int j = 0; j < 4; j++) {
-            double2& acc = cur[4 * (c & 3) + j];
-            acc.x = fma(a[j].x, m[j].x, fma(-a[j].y, m[j].y, acc.x));
-            acc.y = fma(a[j].x, m[j].y, fma(a[j].y, m[j].x, acc.y));
-          }
+          for (int j = 0; j < 4; j++) cmac(cur[4 * (c & 3) + j], a[j], m[j]);
         }
-        if (!last) ring_fill(A.mat[step + 1] + mat_off);  // lands during the inverse transform and the next forward
+        if (!last) ring_fill<R>(stage, A.mat[step + 1] + mat_off + (size_t)o * kM + t);  // lands during the inverse + next forward
         inverse16(cur, tc, t3f);
         // cur[m] = vmp[t + 128 m] + i vmp[t + 128 m + 2048] of limb l: round, shift to the limb's place in the word
         unsigned long long* go = Cout + (size_t)o * kN + t;
@@ -243,9 +209,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ext9(cons
     cluster_arrive();  // the next item rewrites the slabs
     cluster_wait();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+  tmem_free<512>(tmem_base, tid < 32);
 }
 
 }  // namespace fheram

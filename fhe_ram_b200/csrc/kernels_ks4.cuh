@@ -1,15 +1,15 @@
-// kernels_ks4.cuh -- k_ks3 (key switch on 51-bit words, padded transforms) with the matrix stream
-// software-pipelined: words are accumulated in place in shared memory instead of 32 registers, the
-// registers hold a second matrix tile, so the L2 round trip of tile t+1 overlaps the FMAs of tile t
-// and the first tile of every output is fetched during the previous inverse transform.
-// (tools/ablate: without matrix loads k_ks3 runs 76.8 K -> 58.1 K cycles per operation; the loads
-// were three exposed L2 round trips per output.)  Same integers as k_ks3 / k_ks2 / k_vmp.
-// GLWEPacker combines only: the wide launches of the packer tree (the trace kernels took its traces).
+// kernels_ks4.cuh -- GLWEPacker combines on the wide launches of the packer tree: one key switch per CTA of 256 threads,
+// two CTAs per SM, padded 8-point transforms (transform_pad.cuh), 51-bit words (words.cuh).  The matrix stream is
+// software-pipelined: words are accumulated in place in shared memory instead of 32 registers, the registers hold a
+// second matrix tile, so the L2 round trip of tile t+1 overlaps the FMAs of tile t and the first tile of every output
+// is fetched during the previous inverse transform.
 // MODE_MIXED (the packer level of a tree whose width is not a power of two): items without a second operand take the
 // one-sided combine rsh1(a) + phi_g(KS(rsh1(a))) -- b = 0 and t = 0 below, S + y instead of S - y, and the top-limb
 // rounding of the trace kernels (no pre-automorphism sign frame, the sum is not negated).
 #pragma once
-#include "kernels_ks3.cuh"
+#include "tmem.cuh"
+#include "transform_pad.cuh"
+#include "words.cuh"
 
 namespace fheram {
 
@@ -27,32 +27,20 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
   const int T = threadIdx.x, w = T >> 5, lane = T & 31;
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (w == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(tmem_base_s)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (w == 0) tmem_alloc<256>(tmem_base_s);
   BufSync bs{smem_u32(tmem_base_s + 2), 0u};  // exchange-buffer mbarrier in the same 16-byte slot
   if (T == 0) buf_init(bs.mbar);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *tmem_base_s;
   buf_release(bs);  // the buffer starts out free
   // this thread's 128 columns: spectra rows at +0/+32/+64, twiddles at +96 (pass 3) / +112 (pass 4)
   const uint32_t tsp = tmem_base + ((uint32_t)((w & 3) * 32) << 16) + 128 * (w >> 2);
   const uint32_t ttw = tsp + 96;
-  {
-    const Tw34 t = load_tw34(A.tw, w, lane);
-    const double2 p3[4] = {t.a3, t.b3, t.c3, t.d3};
-    const double2 p4[4] = {t.b4a, t.b4b, t.c4a, t.c4b};
-    tm_st4(ttw, p3);
-    tm_st4(ttw + 16, p4);
-    tm_wait_st();
-  }
+  park_tw34(ttw, A.tw, w, lane);
   const int P0 = 256 * w + lane;
   const PadAddr pa = pad_addr(work, T, w, lane);
-  auto tw3 = [&]() { double2 t[4]; tm_ld4(ttw, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
-  auto tw4 = [&]() { double2 t[4]; tm_ld4(ttw + 16, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
+  auto tw3 = [&]() { return tm_tw3(ttw); };
+  auto tw4 = [&]() { return tm_tw4(ttw); };
   long long phase_t0 = A.phase_cycles ? clock64() : 0;
 
   for (int item = blockIdx.x; item < A.n_items; item += gridDim.x) {
@@ -60,13 +48,8 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
     // words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
-    const int* src;
     bool two = true;  // MODE_MIXED: the item has its second operand
-    if constexpr (MODE == MODE_MIXED) {
-      src = mixed_src(A, item, two);
-    } else {
-      src = A.src + 2L * item * A.ct_stride;
-    }
+    const int* src = mode_src<MODE>(A, item, two);
     const bool one = MODE == MODE_MIXED ? !two : false;  // the one-sided combine (a constant unless MODE_MIXED)
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
 
@@ -134,20 +117,14 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
           // digit rho = bits [17 (2 - rho), +17) of the word = (funnel(lo, hi, s1) >> s2) & (2^17 - 1)
           // (shift amounts kept loop-variant on purpose: with per-rho code the compiler hoists all
           // 48 digits out of the loop and spills them)
-          const int s1 = rho == 0 ? 31 : (rho == 1 ? 17 : 0);
-          const int s2 = rho == 0 ? 3 : 0;
           unsigned sg = 0;
 #pragma unroll
           for (int m = 0; m < 8; m++) {
             const int ea = (e0 + m * d1) & (2 * kN - 1);
             const int eb = (ea + d2) & (2 * kN - 1);
-            const unsigned long long wa = xp[kN + (ea & (kN - 1))];
-            const unsigned long long wb = xp[kN + (eb & (kN - 1))];
             const uint32_t na = ea >= kN ? 0x80000000u : 0u, nb = eb >= kN ? 0x80000000u : 0u;
             sg |= (na >> (31 - m)) | (nb >> (23 - m));
-            x[m] = make_double2(
-                field_f64((__funnelshift_r((uint32_t)wa, (uint32_t)(wa >> 32), s1) >> s2) & 0x1ffffu, na),
-                field_f64((__funnelshift_r((uint32_t)wb, (uint32_t)(wb >> 32), s1) >> s2) & 0x1ffffu, nb));
+            x[m] = gather_digits(xp + kN, ea, eb, rho);
           }
           sgn = sg;
           if (!(FHERAM_ABL & 4)) {
@@ -183,9 +160,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
 #pragma unroll
           for (int q = 0; q < 16; q++) {
             const int e = (e0 + (q & 7) * d1 + (q >> 3) * d2) & (2 * kN - 1);
-            const unsigned long long b = xp[e & (kN - 1)] - kBias51;
-            const bool ng = ((sgn >> q) & 1u) != 0;
-            v0[q] = ng ? 0ull - b : b;
+            v0[q] = body_base(xp[e & (kN - 1)], ((sgn >> q) & 1u) != 0, 0ull);
           }
           __syncthreads();  // every gather of the old body column precedes its stores
 #pragma unroll
@@ -204,10 +179,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
               double2 a[4];
               tm_ld4(tsp + 32 * rho + 16 * h, a);
 #pragma unroll
-              for (int j = 0; j < 4; j++) {
-                cur[4 * h + j].x = fma(a[j].x, g[4 * h + j].x, fma(-a[j].y, g[4 * h + j].y, cur[4 * h + j].x));
-                cur[4 * h + j].y = fma(a[j].x, g[4 * h + j].y, fma(a[j].y, g[4 * h + j].x, cur[4 * h + j].y));
-              }
+              for (int j = 0; j < 4; j++) cmac(cur[4 * h + j], a[j], g[4 * h + j]);
             }
           };
           {
@@ -241,8 +213,6 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
           PHASE_TICK(4);
           // cur[m] = phi_g(vmp)[T + 256 m] (+ i * [.. + 2048]); round and add into the word
           if (l == 3) {
-            // floor((s r + 2^16) / 2^17) with s the sign frame of the carry chain, the per-position
-            // automorphism sign, for which floor((-r + 2^16) / 2^17) = -floor((r + 2^16 - 1) / 2^17)
 #pragma unroll
             for (int q = 0; q < 16; q++) {
               const int i = T + 256 * (q & 7) + (q >> 3) * kM;
@@ -277,13 +247,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
               // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:
               //   word = S - (R + k3) - sigma (D_body[u] - bias)
               const unsigned long long U = (one ? sw[co * kN + i] + W : sw[co * kN + i] - W) & kMask51;
-              bool rneg;
-              const int dd = rot_index(i, one ? 0 : A.rot_const, rneg);  // a' * X^t
-#pragma unroll
-              for (int ll = 0; ll < 3; ll++) {
-                const int dg = word_digit(U, ll);
-                dst[CT(co, ll) + dd] = rneg ? -dg : dg;
-              }
+              put_digits_rot(dst, co, i, U, one ? 0 : A.rot_const);
             }
           }
           PHASE_TICK(5);
@@ -294,9 +258,7 @@ __global__ void __launch_bounds__(kThreads, 2) k_ks4(const VmpArgs A) {
     __syncthreads();  // xp reuse by the next item
     PHASE_TICK(6);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (w == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem_base) : "memory");
+  tmem_free<256>(tmem_base, w == 0);
 }
 
 }  // namespace fheram

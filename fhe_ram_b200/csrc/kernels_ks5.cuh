@@ -1,7 +1,7 @@
 // kernels_ks5.cuh -- key switch (trace chains, two-sided packer combine) with ONE operation per SM
 // spread over a CTA of 512 threads = two groups of 8 warps.
 //
-// Why: tools/ablate shows k_ks3/k_ks4 are bound by per-CTA latency, not by a saturated unit: the
+// Why: tools/ablate shows k_ks4 is bound by per-CTA latency, not by a saturated unit: the
 // contraction waits one L2 round trip per matrix tile (the registers of 256 threads hold 32 KiB in
 // flight), and with two CTAs per SM there is no tensor memory or shared memory left to stage tiles.
 // Here both groups work on the SAME ciphertext (group g owns output column g: contraction, inverse
@@ -16,56 +16,17 @@
 // contraction then reads tiles from registers / tensor memory and no longer waits on L2.
 // A single operation per SM also finishes in about half the time, which is what the narrow stages
 // of a single read need (top of the packer tree, the final trace on word_size ciphertexts).
-// Integer side (51-bit words), transforms and results are those of k_ks3 / k_ks4.
+// Integer side (51-bit words), transforms and results are those of k_ks4.
 #pragma once
-#include "kernels_ks4.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
+#include "transform_pad.cuh"
+#include "words.cuh"
 
 namespace fheram {
 
 constexpr int kThreads5 = 512;
 constexpr size_t kKs5Smem = (size_t)2 * kWorkPad * sizeof(double2) + (size_t)2 * kN * sizeof(long long) + 32;
-
-__device__ __forceinline__ void group_sync(int grp) { asm volatile("bar.sync %0, 256;" ::"r"(1 + grp) : "memory"); }
-
-// transform pieces of transform_pad.cuh with the block barrier restricted to the group and three
-// hooks in the inverse (tile prefetch points, several hundred cycles apart)
-template <typename F3, typename F4, typename H>
-__device__ __forceinline__ void inv_transform_g(double2 (&x)[8], const PadAddr& p, int w, int grp, F3&& tw3, F4&& tw4,
-                                                BufSync& bs, H&& hook) {
-  hook(0);
-  {
-    const Tw4x t = tw4();
-    ibf(x[0], x[1], t.c); ibf(x[2], x[3], mul_i(t.c));
-    ibf(x[4], x[5], t.d); ibf(x[6], x[7], mul_i(t.d));
-    ibf(x[0], x[2], t.a); ibf(x[1], x[3], t.a); ibf(x[4], x[6], t.b); ibf(x[5], x[7], t.b);
-  }
-  buf_acquire(bs);
-#pragma unroll
-  for (int j = 0; j < 8; j++) p.C[j] = x[j];
-  __syncwarp();
-#pragma unroll
-  for (int m = 0; m < 8; m++) x[m] = p.B[4 * m + (m >> 1)];
-  {
-    const Tw4x t = tw3();
-    radix8_inv<true>(x, t.a, t.b, t.c, t.d);
-  }
-  hook(1);
-  __syncwarp();
-#pragma unroll
-  for (int m = 0; m < 8; m++) p.B[4 * m] = x[m];
-  __syncwarp();
-#pragma unroll
-  for (int m = 0; m < 8; m++) x[m] = p.A[36 * m];
-  radix8_inv<true>(x, c_tw_lo[8 + w], c_tw_lo[16 + 2 * w], c_tw_lo[32 + 4 * w], c_tw_lo[32 + 4 * w + 2]);
-#pragma unroll
-  for (int m = 0; m < 8; m++) p.A[36 * m] = x[m];
-  group_sync(grp);
-#pragma unroll
-  for (int m = 0; m < 8; m++) x[m] = p.D[kBlk * m];
-  buf_release(bs);
-  hook(2);
-  radix8_inv<true>(x, c_tw_lo[1], c_tw_lo[2], c_tw_lo[4], c_tw_lo[6]);
-}
 
 template <int MODE>
 __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
@@ -79,15 +40,10 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
   const int tid = threadIdx.x, grp = tid >> 8, T = tid & 255, w = T >> 5, lane = T & 31;
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc<512>(slot);
   BufSync bs{smem_u32(slot + 2 + 2 * grp), 0u};
   if (T == 0) buf_init(bs.mbar);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *slot;
   buf_release(bs);  // the group's buffer starts out free
   // columns of thread position (w, lane), the same for both groups: spectra +0/+32/+64, twiddles +96
@@ -95,22 +51,13 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
   const uint32_t tsp = tmem_base + ((uint32_t)((w & 3) * 32) << 16) + 256 * (w >> 2);
   const uint32_t ttw = tsp + 96;
   const uint32_t tpark = tsp + 128 + 64 * grp;
-  if (grp == 0) {
-    const Tw34 t = load_tw34(A.tw, w, lane);
-    const double2 p3[4] = {t.a3, t.b3, t.c3, t.d3};
-    const double2 p4[4] = {t.b4a, t.b4b, t.c4a, t.c4b};
-    tm_st4(ttw, p3);
-    tm_st4(ttw + 16, p4);
-    tm_wait_st();
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  if (grp == 0) park_tw34(ttw, A.tw, w, lane);
+  tmem_sync();
 
   const int P0 = 256 * w + lane;
   const PadAddr pa = pad_addr(work_all + grp * kWorkPad, T, w, lane);
-  auto tw3 = [&]() { double2 t[4]; tm_ld4(ttw, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
-  auto tw4 = [&]() { double2 t[4]; tm_ld4(ttw + 16, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
+  auto tw3 = [&]() { return tm_tw3(ttw); };
+  auto tw4 = [&]() { return tm_tw4(ttw); };
   const double sgn_d = (MODE == MODE_TRACE && A.sign < 0) ? -1.0 : 1.0;
   const uint32_t sgn_bit = (MODE == MODE_TRACE && A.sign < 0) ? 1u : 0u;
   const int co = grp;                       // output column of this group
@@ -122,17 +69,8 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
     // COMBINE2: words of S = rsh1(a X^-t + b), [2 cols][N], in this CTA's global scratch
     unsigned long long* sw = A.scratch
         ? reinterpret_cast<unsigned long long*>(A.scratch + (size_t)blockIdx.x * A.ct_stride) : nullptr;
-    const int* src;
     bool two = true;  // MODE_MIXED: the item has its second operand
-    if constexpr (MODE == MODE_MIXED) {
-      src = mixed_src(A, item, two);
-    } else {
-      long idx = item;
-      if (MODE == MODE_COMBINE2) idx = 2L * item;
-      else if (A.src_div > 0) idx = item / A.src_div;
-      else if (A.src_mod > 0) { int r = item % A.src_mod; idx = A.src_map ? A.src_map[r] : r; }
-      src = A.src + idx * A.ct_stride;
-    }
+    const int* src = mode_src<MODE>(A, item, two);
     // this item's path: TRACE steps, or the two-sided combine (a constant unless MODE_MIXED)
     const bool trace = MODE == MODE_MIXED ? !two : MODE == MODE_TRACE;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
@@ -140,18 +78,9 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
     // ---------------- prologue (once per item): group g converts column g -----------------
     if (trace) {
       // x = rsh1(src * X^rk)  (MODE_MIXED: the one-sided combine, no rotation)
-      int rk = MODE == MODE_MIXED ? 0 : A.rot_const;
-      if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
-      rk &= (2 * kN - 1);
+      const int rk = trace_rot(A, item, MODE == MODE_MIXED ? 0 : A.rot_const);
 #pragma unroll 4
-      for (int m = 0; m < 16; m++) {
-        const int i = T + 256 * m;
-        bool neg;
-        const int j = rot_index(i, 2 * kN - rk, neg);
-        long long X = limbs_value(src[CT(co, 0) + j], src[CT(co, 1) + j], src[CT(co, 2) + j]);
-        if (neg) X = -X;
-        xc[i] = rsh1_word(X);
-      }
+      for (int m = 0; m < 16; m++) xc[T + 256 * m] = trace_word(src, co, T + 256 * m, rk);
     } else {
       // a1 = a X^-t;  D = rsh1(a1 - b) -> xp;  S = rsh1(a1 + b) -> sw
       const int* a = src;
@@ -224,18 +153,10 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
       for (int rho = (grp == 0 ? 0 : 2); rho < (grp == 0 ? 2 : 3); rho++) {
         double2 x[8];
         // digit rho = bits [17 (2 - rho), +17) of the word = (funnel(lo, hi, s1) >> s2) & (2^17 - 1)
-        const int s1 = rho == 0 ? 31 : (rho == 1 ? 17 : 0);
-        const int s2 = rho == 0 ? 3 : 0;
 #pragma unroll
         for (int m = 0; m < 8; m++) {
           const int ea = (e0 + m * d1) & (2 * kN - 1);
-          const int eb = (ea + d2) & (2 * kN - 1);
-          const unsigned long long wa = xp[kN + (ea & (kN - 1))];
-          const unsigned long long wb = xp[kN + (eb & (kN - 1))];
-          const uint32_t na = ea >= kN ? 0x80000000u : 0u, nb = eb >= kN ? 0x80000000u : 0u;
-          x[m] = make_double2(
-              field_f64((__funnelshift_r((uint32_t)wa, (uint32_t)(wa >> 32), s1) >> s2) & 0x1ffffu, na),
-              field_f64((__funnelshift_r((uint32_t)wb, (uint32_t)(wb >> 32), s1) >> s2) & 0x1ffffu, nb));
+          x[m] = gather_digits(xp + kN, ea, (ea + d2) & (2 * kN - 1), rho);
         }
         fwd_pass1_store_p(x, pa, bs);
         group_sync(grp);
@@ -266,9 +187,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
       }
       if (step == 0) prefetch(2);
       tm_wait_st();
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();  // spectra (tensor memory) and the body-column init are visible to both groups
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tmem_sync();  // spectra (tensor memory) and the body-column init are visible to both groups
       if (grp == 1 && A.stagger > 0) {
         // the groups run identical phase sequences: offset them so that one group's butterflies
         // overlap the other's shared-memory exchanges instead of colliding with its butterflies
@@ -289,10 +208,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
             double2 a[4];
             tm_ld4(tsp + 32 * rho + 16 * h, a);
 #pragma unroll
-            for (int j = 0; j < 4; j++) {
-              cur[4 * h + j].x = fma(a[j].x, g[4 * h + j].x, fma(-a[j].y, g[4 * h + j].y, cur[4 * h + j].x));
-              cur[4 * h + j].y = fma(a[j].x, g[4 * h + j].y, fma(a[j].y, g[4 * h + j].x, cur[4 * h + j].y));
-            }
+            for (int j = 0; j < 4; j++) cmac(cur[4 * h + j], a[j], g[4 * h + j]);
           }
         };
         tm_wait_st();  // parked tiles of this output
@@ -318,7 +234,6 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
         PHASE_TICK(4);
         // cur[m] = phi_g(vmp)[T + 256 m] (+ i * [.. + 2048]); round and add into the word
         if (l == 3) {
-          // floor((s r + 2^16) / 2^17) with s the sign frame of the carry chain (see k_ks3)
 #pragma unroll
           for (int q = 0; q < 16; q++) {
             const int i = T + 256 * (q & 7) + (q >> 3) * kM;
@@ -355,14 +270,7 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
               const unsigned long long U = W & kMask51;
               xc[i] = last ? U : rsh1_canon(U);
             } else {
-              const unsigned long long U = (sw[co * kN + i] - W) & kMask51;
-              bool rneg;
-              const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
-#pragma unroll
-              for (int ll = 0; ll < 3; ll++) {
-                const int dg = word_digit(U, ll);
-                dst[CT(co, ll) + dd] = rneg ? -dg : dg;
-              }
+              put_digits_rot(dst, co, i, (sw[co * kN + i] - W) & kMask51, A.rot_const);
             }
           }
         }
@@ -370,27 +278,17 @@ __global__ void __launch_bounds__(kThreads5, 1) k_ks5(const VmpArgs A) {
       }
       // both columns complete (the next forward gathers the mask words, the next body init gathers
       // the body words) and every read of the spectra precedes the next forward's tensor-memory stores
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tmem_sync();
     }  // steps
 
     if (trace) {
 #pragma unroll 4
-      for (int m = 0; m < 16; m++) {
-        const int i = T + 256 * m;
-        const unsigned long long U = xc[i];
-        dst[CT(co, 0) + i] = word_digit(U, 0);
-        dst[CT(co, 1) + i] = word_digit(U, 1);
-        dst[CT(co, 2) + i] = word_digit(U, 2);
-      }
+      for (int m = 0; m < 16; m++) put_digits(dst, co, T + 256 * m, xc[T + 256 * m]);
     }
     __syncthreads();  // xp reuse by the next item
     PHASE_TICK(6);
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+  tmem_free<512>(tmem_base, tid < 32);
 }
 
 }  // namespace fheram

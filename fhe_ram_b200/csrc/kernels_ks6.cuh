@@ -14,29 +14,15 @@
 // Everything else (51-bit words, padded transforms, matrix tiles parked in tensor memory during the inverse
 // transform) is k_ks5.  Same integers as every other generation (tests/test_gpu_kernel_variants.py: "ks6").
 #pragma once
-#include "kernels_ks5.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
+#include "transform_pad.cuh"
+#include "words.cuh"
 
 namespace fheram {
 
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-// address of the same shared-memory location in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t saddr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void st_cluster_u64(uint32_t addr, unsigned long long v) {
-  asm volatile("st.shared::cluster.u64 [%0], %1;" ::"r"(addr), "l"(v) : "memory");
-}
-
 template <int MODE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(const VmpArgs A) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(512, 1) k_ks6(const VmpArgs A) {
   static_assert(MODE == MODE_TRACE || MODE == MODE_COMBINE2 || MODE == MODE_MIXED, "key-switch modes only");
   constexpr int LOUT = 4, NOUT = 2 * LOUT;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -48,36 +34,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
   const int co = (int)cluster_ctarank();  // output column of this CTA
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc<512>(slot);
   BufSync bs{smem_u32(slot + 2 + 2 * grp), 0u};
   if (T == 0) buf_init(bs.mbar);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *slot;
   buf_release(bs);
   const uint32_t tsp = tmem_base + ((uint32_t)((w & 3) * 32) << 16) + 256 * (w >> 2);
   const uint32_t ttw = tsp + 96;
   const uint32_t tpark = tsp + 128 + 64 * grp;
-  if (grp == 0) {
-    const Tw34 t = load_tw34(A.tw, w, lane);
-    const double2 p3[4] = {t.a3, t.b3, t.c3, t.d3};
-    const double2 p4[4] = {t.b4a, t.b4b, t.c4a, t.c4b};
-    tm_st4(ttw, p3);
-    tm_st4(ttw + 16, p4);
-    tm_wait_st();
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  if (grp == 0) park_tw34(ttw, A.tw, w, lane);
+  tmem_sync();
 
   const int P0 = 256 * w + lane;
   const PadAddr pa = pad_addr(work_all + grp * kWorkPad, T, w, lane);
-  auto tw3 = [&]() { double2 t[4]; tm_ld4(ttw, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
-  auto tw4 = [&]() { double2 t[4]; tm_ld4(ttw + 16, t); return Tw4x{t[0], t[1], t[2], t[3]}; };
+  auto tw3 = [&]() { return tm_tw3(ttw); };
+  auto tw4 = [&]() { return tm_tw4(ttw); };
   const double sgn_d = (MODE == MODE_TRACE && A.sign < 0) ? -1.0 : 1.0;
   const uint32_t sgn_bit = (MODE == MODE_TRACE && A.sign < 0) ? 1u : 0u;
   unsigned long long* xc = xp + co * kN;  // the words this CTA produces
@@ -113,9 +85,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
       const int m0 = co == 0 ? 0 : 8 * grp, m1 = co == 0 ? 16 : 8 * grp + 8;
       if (trace) {
         // x = rsh1(src * X^rk)  (MODE_MIXED: the one-sided combine, no rotation)
-        int rk = MODE == MODE_MIXED ? 0 : A.rot_const;
-        if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
-        rk &= (2 * kN - 1);
+        const int rk = trace_rot(A, item, MODE == MODE_MIXED ? 0 : A.rot_const);
 #pragma unroll 4
         for (int m = m0; m < m1; m++) {
           const int i = T + 256 * m;
@@ -233,9 +203,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
       }
       if (step == 0) prefetch(2);
       tm_wait_st();
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncthreads();  // spectra and the body init visible to both groups; every gather of the old mask words done
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tmem_sync();  // spectra and the body init visible to both groups; every gather of the old mask words done
       if (trace) {
         cluster_arrive();  // phase A: this CTA no longer reads the old mask words
       } else if (co == 1) {
@@ -258,10 +226,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
             double2 a[4];
             tm_ld4(tsp + 32 * rho + 16 * h, a);
 #pragma unroll
-            for (int j = 0; j < 4; j++) {
-              cur[4 * h + j].x = fma(a[j].x, g[4 * h + j].x, fma(-a[j].y, g[4 * h + j].y, cur[4 * h + j].x));
-              cur[4 * h + j].y = fma(a[j].x, g[4 * h + j].y, fma(a[j].y, g[4 * h + j].x, cur[4 * h + j].y));
-            }
+            for (int j = 0; j < 4; j++) cmac(cur[4 * h + j], a[j], g[4 * h + j]);
           }
         };
         tm_wait_st();
@@ -314,49 +279,30 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads5, 1) k_ks6(
           if (co == 1) st_cluster_u64(remote_mask + 8u * (uint32_t)i, Un);
         }
         cluster_arrive();  // phase B: new mask words written on both sides
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tmem_sync();
         cluster_wait();    // ... and visible before the next step's gathers
       } else {
         // y = phi_g(normalize(KS(D)));  out = normalize(S - y) X^t:  word = S - (R + k3) [- sigma (D_body[u] - bias)]
 #pragma unroll
         for (int q = 0; q < 8; q++) {
           const int i = tid + 512 * q;
-          const unsigned long long U = (sw[i] - xc[i]) & kMask51;
-          bool rneg;
-          const int dd = rot_index(i, A.rot_const, rneg);  // a' * X^t
-#pragma unroll
-          for (int ll = 0; ll < 3; ll++) {
-            const int dg = word_digit(U, ll);
-            dst[CT(co, ll) + dd] = rneg ? -dg : dg;
-          }
+          put_digits_rot(dst, co, i, (sw[i] - xc[i]) & kMask51, A.rot_const);
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tmem_sync();
       }
     }  // steps
 
     if (trace) {
       // copy-out: every CTA its own column, all 512 threads
 #pragma unroll 4
-      for (int q = 0; q < 8; q++) {
-        const int i = tid + 512 * q;
-        const unsigned long long U = xc[i];
-        dst[CT(co, 0) + i] = word_digit(U, 0);
-        dst[CT(co, 1) + i] = word_digit(U, 1);
-        dst[CT(co, 2) + i] = word_digit(U, 2);
-      }
+      for (int q = 0; q < 8; q++) put_digits(dst, co, tid + 512 * q, xc[tid + 512 * q]);
     }
     // the next item's prologue rewrites the word buffers (CTA 0's mask column is also written by CTA 1)
     cluster_arrive();
     __syncthreads();
     cluster_wait();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+  tmem_free<512>(tmem_base, tid < 32);
 }
 
 }  // namespace fheram

@@ -8,7 +8,7 @@
 // mask column over distributed shared memory (8.8 B/clk, tools/dsmem_probe.cu): 18.3 us per step.  Here a step is
 //   phase A   every CTA rebuilds the mask words in its shared memory: old word + the four limb contributions of the
 //             previous step, read from L2 (4 x 32 KiB, coalesced), reduced mod 2^51 and shifted (rsh 1);
-//   forward   groups 0, 1, 2 (128 threads x 16 points, kernels_ks7.cuh) transform one mask limb each -- the same three
+//   forward   groups 0, 1, 2 (128 threads x 16 points, transform16.cuh) transform one mask limb each -- the same three
 //             transforms in all eight CTAs, the spectra stay in the CTA's tensor memory;
 //   output    group 3 contracts the three spectra with ITS column of the key (the 96 KiB were prefetched by cp.async
 //             into a ring of 11 x 8 KiB since the previous step's contraction ended: no L2 round trip on the critical
@@ -24,7 +24,10 @@
 // MODE_TRACE step without rotation (the one-sided combine), chosen by the operand table (mixed_src, kernels.cuh).
 // Same integers as every other generation (tests/test_gpu_kernel_variants.py: "ks8"); keys in the order of k_prepare7.
 #pragma once
-#include "kernels_ext8.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
+#include "transform16.cuh"
+#include "words.cuh"
 
 namespace fheram {
 
@@ -39,28 +42,11 @@ namespace fheram {
     }                                                                            \
   } while (0)
 
-constexpr size_t kKs8ScratchWords = (size_t)2 * 8 * kN + 2 * kN;  // u64 per cluster (576 KiB)
 // staged 8 KiB chunks (of the 12 of one output column) per output group
 __host__ __device__ constexpr int ks8_ring(int cl) { return cl == 8 ? 11 : 5; }
 constexpr size_t ks8_smem(int cl) {
   return (size_t)256 * sizeof(double2) + (size_t)3 * kPad16 * sizeof(double2) + (size_t)kN * sizeof(unsigned long long) +
          (size_t)(8 / cl) * ks8_ring(cl) * 512 * sizeof(double2) + 32;
-}
-
-__device__ __forceinline__ void cp_async_wait_n(int n) {
-  switch (n) {
-    case 0: cp_async_wait<0>(); break;
-    case 1: cp_async_wait<1>(); break;
-    case 2: cp_async_wait<2>(); break;
-    case 3: cp_async_wait<3>(); break;
-    case 4: cp_async_wait<4>(); break;
-    case 5: cp_async_wait<5>(); break;
-    case 6: cp_async_wait<6>(); break;
-    case 7: cp_async_wait<7>(); break;
-    case 8: cp_async_wait<8>(); break;
-    case 9: cp_async_wait<9>(); break;
-    default: cp_async_wait<10>(); break;
-  }
 }
 
 template <int CL, int MODE>
@@ -86,37 +72,15 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
   const int l = o & 3;                  // (column o >> 2: 0 body, 1 mask)
   auto CT = [](int col, int limb) { return (limb * 2 + col) * kN; };
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(slot)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc<256>(slot);
   if (tid < 256) tw2[tid] = __ldg(tw16 + tid);
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tmem_sync();
   const uint32_t tmem_base = *slot;
   const uint32_t tsp = tmem_base + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);  // spectra rows at +0 / +64 / +128
   const uint32_t ttw = tsp + 192;                                             // 7 pass-3 twiddles (28 columns)
-  if (g == 0) {
-    const Tw3x w = load_tw3x(tw16, t);
-    const double2 p0[4] = {w.w8, w.w9a, w.w9b, w.w10[0]};
-    const double2 p1[4] = {w.w10[1], w.w10[2], w.w10[3], w.w10[3]};
-    tm_st4(ttw, p0);
-    tm_st4(ttw + 16, p1);
-    tm_wait_st();
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  auto t3f = [&]() {
-    double2 p0[4], p1[4];
-    tm_ld4(ttw, p0);
-    tm_ld4(ttw + 16, p1);
-    Tw3x w;
-    w.w8 = p0[0]; w.w9a = p0[1]; w.w9b = p0[2]; w.w10[0] = p0[3];
-    w.w10[1] = p1[0]; w.w10[2] = p1[1]; w.w10[3] = p1[2];
-    return w;
-  };
+  if (g == 0) park_tw3x(ttw, tw16, t);
+  tmem_sync();
+  auto t3f = [&]() { return tm_tw3x(ttw); };
   // group 3 runs its inverse transform in the exchange buffer of group 1 (idle after the forward transforms)
   const T16 tc{bufs + (g < 3 ? g : 1) * kPad16, tw2, nullptr, t, g};
   const double sgn_d = (MODE == MODE_TRACE && A.sign < 0) ? -1.0 : 1.0;
@@ -129,17 +93,6 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
   const bool prof = A.phase_cycles != nullptr && cluster_id == 0 && rank == A.stagger;
   long long pt0 = 0;
   double2* stage = ring + og * (R * 512) + t;  // slot s, value j of this thread: stage[(4 s + j) * 128]
-  auto ring_issue = [&](const double2* gp, int c, int s) {
-    const double2* np = gp + (size_t)(c >> 2) * NOUT * kM + 512 * (c & 3);
-#pragma unroll
-    for (int j = 0; j < 4; j++) cp_async16(stage + (4 * s + j) * 128, np + 128 * j);
-    cp_async_commit();
-  };
-  auto ring_fill = [&](const double2* Gmat) {
-    const double2* gp = Gmat + (size_t)o * kM + t;
-#pragma unroll
-    for (int c = 0; c < R; c++) ring_issue(gp, c, c);
-  };
 
   for (int item = cluster_id; item < A.n_items; item += n_clusters) {
     int* dst = A.dst + (size_t)item * A.ct_stride;
@@ -157,22 +110,15 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
     // this item's path: TRACE steps, or the two-sided combine (a constant unless MODE_MIXED)
     const bool trace = MODE == MODE_MIXED ? !two : MODE == MODE_TRACE;
     const size_t mat_off = A.mat_div > 0 ? (size_t)(item / A.mat_div) * A.mat_stride : 0;
-    if (out_group) ring_fill(A.mat[0] + mat_off);
+    if (out_group) ring_fill<R>(stage, A.mat[0] + mat_off + (size_t)o * kM + t);
 
-    int rk = MODE == MODE_MIXED && trace ? 0 : A.rot_const;  // MODE_MIXED: the one-sided combine has no rotation
-    if (MODE == MODE_TRACE) {
-      if (A.rot_mod > 0) rk += A.rot_mul * (item % A.rot_mod);
-      rk &= (2 * kN - 1);
-    }
+    // MODE_MIXED: the one-sided combine has no rotation
+    const int rk = MODE == MODE_TRACE ? trace_rot(A, item, A.rot_const) : (MODE == MODE_MIXED && trace ? 0 : A.rot_const);
     // the words before step 0 of column col at position i:
     // TRACE x = rsh1(src X^rk);  COMBINE2 D = rsh1(a X^-t - b) (plus = false) or S = rsh1(a X^-t + b) (plus = true)
     auto x_src = [&](int col, int i, bool plus) {
       if (trace) {
-        bool neg;
-        const int j = rot_index(i, 2 * kN - rk, neg);
-        long long X = limbs_value(src[CT(col, 0) + j], src[CT(col, 1) + j], src[CT(col, 2) + j]);
-        if (neg) X = -X;
-        return rsh1_word(X);
+        return trace_word(src, col, i, rk);
       } else {
         const int* pa = src;
         const int* pb = src + A.ct_stride;
@@ -225,18 +171,10 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
         {
           const int rho = g;
           double2 x[16];
-          const int s1 = rho == 0 ? 31 : (rho == 1 ? 17 : 0);
-          const int s2 = rho == 0 ? 3 : 0;
 #pragma unroll
           for (int m = 0; m < 16; m++) {
             const int ea = (e0 + m * d1) & (2 * kN - 1);
-            const int eb = (ea + d2) & (2 * kN - 1);
-            const unsigned long long wa = xm[ea & (kN - 1)];
-            const unsigned long long wb = xm[eb & (kN - 1)];
-            const uint32_t na = ea >= kN ? 0x80000000u : 0u, nb = eb >= kN ? 0x80000000u : 0u;
-            x[m] = make_double2(
-                field_f64((__funnelshift_r((uint32_t)wa, (uint32_t)(wa >> 32), s1) >> s2) & 0x1ffffu, na),
-                field_f64((__funnelshift_r((uint32_t)wb, (uint32_t)(wb >> 32), s1) >> s2) & 0x1ffffu, nb));
+            x[m] = gather_digits(xm, ea, (ea + d2) & (2 * kN - 1), rho);
           }
           forward16(x, tc, t3f);
 #pragma unroll
@@ -286,17 +224,13 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
           const int s = c % R;
 #pragma unroll
           for (int j = 0; j < 4; j++) m[j] = stage[(4 * s + j) * 128];
-          if (c + R < 12) ring_issue(gp, c + R, s);  // refill the slot just read
+          if (c + R < 12) ring_issue(stage, gp, c + R, s);  // refill the slot just read
           tm_ld4(tsp + 64 * (c >> 2) + 16 * (c & 3), a);
 #pragma unroll
-          for (int j = 0; j < 4; j++) {
-            double2& acc = cur[4 * (c & 3) + j];
-            acc.x = fma(a[j].x, m[j].x, fma(-a[j].y, m[j].y, acc.x));
-            acc.y = fma(a[j].x, m[j].y, fma(a[j].y, m[j].x, acc.y));
-          }
+          for (int j = 0; j < 4; j++) cmac(cur[4 * (c & 3) + j], a[j], m[j]);
         }
         KS8_TICK(5);
-        if (!last) ring_fill(A.mat[step + 1] + mat_off);  // lands during the inverse transform and the next forward
+        if (!last) ring_fill<R>(stage, A.mat[step + 1] + mat_off + (size_t)o * kM + t);  // lands during the inverse and the next forward
         inverse16(cur, tc, t3f);
         KS8_TICK(6);
         // cur[m] = phi_g(vmp)[t + 128 m] + i phi_g(vmp)[t + 128 m + 2048] of limb l: round, shift to the limb's place
@@ -370,9 +304,7 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(512, 1) k_ks8(const
     cluster_arrive();  // the next item rewrites the slabs and the mask words
     cluster_wait();
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem_base) : "memory");
+  tmem_free<256>(tmem_base, tid < 32);
 }
 
 }  // namespace fheram

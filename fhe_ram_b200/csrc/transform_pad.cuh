@@ -1,10 +1,9 @@
 // transform_pad.cuh -- the 2048-point transform of kernels.cuh with PADDED exchange buffers.
 //
 // kernels.cuh keeps every 16-byte shared-memory access of the exchanges conflict free with XOR
-// swizzles (S1/S2), which costs one LOP3 + one LEA per access (about 100 integer instructions per
-// warp and transform, a quarter of the non-FP64 instruction stream of k_ks2/k_ext2).  Here the same
-// accesses are made conflict free by padding instead, so that every address is a per-thread base
-// register plus a compile-time immediate:
+// swizzles (S1/S2), which costs one LOP3 + one LEA per access.  Here the same accesses are made
+// conflict free by padding instead, so that every address is a per-thread base register plus a
+// compile-time immediate:
 //   a warp's 256-element block occupies 288 slots;
 //   P1(e) = e + 4 (e >> 5)   (4 slots after every 32 elements)  for the exchanges of passes 1-3,
 //   P2(e) = e + (e >> 3)     (1 slot after every 8 elements)    for the exchange of passes 3-4.
@@ -17,11 +16,14 @@
 // and results are bit-identical and the prepared matrices are shared.
 #pragma once
 #include "kernels.cuh"
+#include "sync.cuh"
+#include "tmem.cuh"
 
+// timing ablations for tools/ablate.sh (results are garbage when non-zero): 1 no matrix loads, 2 no inverse
+// transforms, 4 no forward transforms (k_ks4), 8 no warp-local exchanges, 16 no butterflies
 #ifndef FHERAM_ABL
 #define FHERAM_ABL 0
 #endif
-// timing ablations (results are garbage): 8 = no warp-local exchanges, 16 = no butterflies
 #define ABL_XCH if (!(FHERAM_ABL & 8))
 #define ABL_BFLY if (!(FHERAM_ABL & 16))
 
@@ -47,6 +49,18 @@ __device__ __forceinline__ PadAddr pad_addr(double2* work, int T, int w, int lan
 }
 
 struct Tw4x { double2 a, b, c, d; };  // four twiddles of one pass
+
+// pass-3/4 twiddles of thread (w, lane) parked in tensor memory columns ttw .. ttw + 31, and their loaders
+__device__ __forceinline__ void park_tw34(uint32_t ttw, const Twiddles& tw, int w, int lane) {
+  const Tw34 t = load_tw34(tw, w, lane);
+  const double2 p3[4] = {t.a3, t.b3, t.c3, t.d3};
+  const double2 p4[4] = {t.b4a, t.b4b, t.c4a, t.c4b};
+  tm_st4(ttw, p3);
+  tm_st4(ttw + 16, p4);
+  tm_wait_st();
+}
+__device__ __forceinline__ Tw4x tm_tw3(uint32_t ttw) { double2 t[4]; tm_ld4(ttw, t); return Tw4x{t[0], t[1], t[2], t[3]}; }
+__device__ __forceinline__ Tw4x tm_tw4(uint32_t ttw) { double2 t[4]; tm_ld4(ttw + 16, t); return Tw4x{t[0], t[1], t[2], t[3]}; }
 
 // Split barrier protecting the exchange buffer between transforms (write-after-read): a warp
 // RELEASES the buffer (one mbarrier arrival per warp) once it has read everything it needs, and a
@@ -164,6 +178,46 @@ __device__ __forceinline__ void inv_transform_p(double2 (&x)[8], const PadAddr& 
   for (int m = 0; m < 8; m++) x[m] = p.D[kBlk * m];
   buf_release(bs);
   ABL_BFLY radix8_inv<true>(x, c_tw_lo[1], c_tw_lo[2], c_tw_lo[4], c_tw_lo[6]);
+}
+
+// inv_transform_p with the block barrier restricted to the group and three
+// hooks in the inverse (tile prefetch points, several hundred cycles apart)
+template <typename F3, typename F4, typename H>
+__device__ __forceinline__ void inv_transform_g(double2 (&x)[8], const PadAddr& p, int w, int grp, F3&& tw3, F4&& tw4,
+                                                BufSync& bs, H&& hook) {
+  hook(0);
+  {
+    const Tw4x t = tw4();
+    ibf(x[0], x[1], t.c); ibf(x[2], x[3], mul_i(t.c));
+    ibf(x[4], x[5], t.d); ibf(x[6], x[7], mul_i(t.d));
+    ibf(x[0], x[2], t.a); ibf(x[1], x[3], t.a); ibf(x[4], x[6], t.b); ibf(x[5], x[7], t.b);
+  }
+  buf_acquire(bs);
+#pragma unroll
+  for (int j = 0; j < 8; j++) p.C[j] = x[j];
+  __syncwarp();
+#pragma unroll
+  for (int m = 0; m < 8; m++) x[m] = p.B[4 * m + (m >> 1)];
+  {
+    const Tw4x t = tw3();
+    radix8_inv<true>(x, t.a, t.b, t.c, t.d);
+  }
+  hook(1);
+  __syncwarp();
+#pragma unroll
+  for (int m = 0; m < 8; m++) p.B[4 * m] = x[m];
+  __syncwarp();
+#pragma unroll
+  for (int m = 0; m < 8; m++) x[m] = p.A[36 * m];
+  radix8_inv<true>(x, c_tw_lo[8 + w], c_tw_lo[16 + 2 * w], c_tw_lo[32 + 4 * w], c_tw_lo[32 + 4 * w + 2]);
+#pragma unroll
+  for (int m = 0; m < 8; m++) p.A[36 * m] = x[m];
+  group_sync(grp);
+#pragma unroll
+  for (int m = 0; m < 8; m++) x[m] = p.D[kBlk * m];
+  buf_release(bs);
+  hook(2);
+  radix8_inv<true>(x, c_tw_lo[1], c_tw_lo[2], c_tw_lo[4], c_tw_lo[6]);
 }
 
 }  // namespace fheram

@@ -81,7 +81,7 @@ def test_trace_matches_oracle(scenario, gpu_keys):
 
 def _extreme_glwe(rng, params, n):
     """ciphertexts whose digits sit on the edges of the balanced range: the word-domain kernels
-    (kernels_ks3.cuh) replace digit carry chains by arithmetic mod 2^51 on biased words, so the cases to
+    (words.cuh) replace digit carry chains by arithmetic mod 2^51 on biased words, so the cases to
     pin are -2^16 (whose negation under a rotation / automorphism is the non-canonical +2^16), 2^16 - 1,
     and values whose top digit wraps"""
     L = params.glwe_len()
