@@ -165,6 +165,9 @@ SIGNATURES = {
     "fheram_ram_read_batch_host_seeded": (C.c_int, [_V, C.POINTER(C.c_uint32), _PS, C.c_int, _V,
                                                     C.POINTER(C.c_int32)]),
     "fheram_ram_load_seeded": (C.c_int, [_V, _P64, _PS]),
+    "fheram_ram_read_plain": (C.c_int, [_V, C.POINTER(C.c_uint32), C.c_int, _V, _P64]),
+    "fheram_ram_read_plain_device": (C.c_int, [_V, C.POINTER(C.c_uint32), C.c_int, _V, _PV]),
+    "fheram_ram_write_plain": (C.c_int, [_V, C.c_uint32, _P64, _V]),
 }
 
 _lib = None
@@ -819,6 +822,46 @@ class Ram:
         d = C.c_void_p()
         _check(lib().fheram_ram_read_batch_device(self.h, addresses.device(), keys.h, C.byref(d)))
         return int(d.value)
+
+    # ---- plaintext addresses (include/fheram.h): the address is disclosed to the server, the words stay encrypted ----
+    @staticmethod
+    def _addrs(addrs) -> np.ndarray:
+        a = np.asarray(addrs, dtype=np.int64).reshape(-1)
+        if a.size and (a.min() < 0 or a.max() >= 1 << 32):
+            raise FheRamError(-1, "addresses must be in [0, 2^32)")
+        return np.ascontiguousarray(a, dtype=np.uint32)
+
+    def read_plain(self, addrs, keys: EvaluationKeysPrepared, out=None) -> np.ndarray:
+        """[n][word_size] GLWE: TRACE(data[s][h] X^-j) for each address a = h N + j.  A shard without a communicator
+        fills the entries of the addresses it holds and leaves the rest of `out` (zeros when not passed) as it is."""
+        a = self._addrs(addrs)
+        out = self._out(a.size) if out is None else out
+        assert out.dtype == np.int64 and out.flags.c_contiguous and out.size == a.size * self.params.word_size() * \
+            self.params.glwe_len()
+        _check(lib().fheram_ram_read_plain(self.h, a.ctypes.data_as(C.POINTER(C.c_uint32)), int(a.size), keys.h,
+                                           _p(out.reshape(-1))))
+        return out
+
+    def read_plain_device(self, addrs, keys: EvaluationKeysPrepared) -> int:
+        """read_plain into the RAM's device arena ([n][word_size] GLWE, int32 limbs); returns its device pointer"""
+        a = self._addrs(addrs)
+        d = C.c_void_p()
+        _check(lib().fheram_ram_read_plain_device(self.h, a.ctypes.data_as(C.POINTER(C.c_uint32)), int(a.size),
+                                                  keys.h, C.byref(d)))
+        return int(d.value)
+
+    def write_plain(self, addr: int, w, keys: EvaluationKeysPrepared) -> None:
+        """data[s][h] = normalize(data[s][h] - TRACE(data[s][h] X^-j) X^j + w[s] X^j) for a = h N + j; w = word_size
+        GLWE as `write` takes it (sharded RAM with a communicator: rank 0's, the other ranks may pass None)"""
+        if not 0 <= int(addr) < 1 << 32:
+            raise FheRamError(-1, "addresses must be in [0, 2^32)")
+        if w is None:
+            _check(lib().fheram_ram_write_plain(self.h, int(addr), None, keys.h))
+            return
+        w = np.ascontiguousarray(w, dtype=np.int64).reshape(-1)
+        if w.size != self.params.word_size() * self.params.glwe_len():
+            raise FheRamError(-1, "w must hold word_size GLWE")
+        _check(lib().fheram_ram_write_plain(self.h, int(addr), _p(w), keys.h))
 
     def close(self):
         if self.h is not None:

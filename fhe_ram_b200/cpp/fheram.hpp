@@ -213,6 +213,22 @@ class Ram {  // src/ram.rs:25-29
     for (auto& g : w) flat.insert(flat.end(), g.begin(), g.end());
     check(fheram_ram_write(h_, flat.data(), a.device(), k.raw()));
   }
+  // reads / writes at plaintext addresses (include/fheram.h): the address is disclosed to the server, the words stay
+  // encrypted.  read_plain: one [word_size] GLWE per address
+  std::vector<std::vector<GLWE>> read_plain(const std::vector<uint32_t>& addrs, const EvaluationKeysPrepared& k) {
+    std::vector<int64_t> out(addrs.size() * p_.word_size() * p_.glwe_len());
+    check(fheram_ram_read_plain(h_, addrs.data(), (int)addrs.size(), k.raw(), out.data()));
+    std::vector<std::vector<GLWE>> r;
+    const size_t per = p_.word_size() * p_.glwe_len();
+    for (size_t b = 0; b < addrs.size(); b++) r.push_back(split(std::vector<int64_t>(out.begin() + b * per, out.begin() + (b + 1) * per)));
+    return r;
+  }
+  void write_plain(uint32_t addr, const std::vector<GLWE>& w, const EvaluationKeysPrepared& k) {
+    if (w.size() != p_.word_size()) throw Panic(-1, "assertion failed: w.len() == self.subrams.len()");
+    std::vector<int64_t> flat;
+    for (auto& g : w) flat.insert(flat.end(), g.begin(), g.end());
+    check(fheram_ram_write_plain(h_, addr, flat.data(), k.raw()));
+  }
   // every byte of the resident RAM decrypted on the device: values / err are [max_addr][word_size] row-major (byte i of
   // word j at j * word_size + i), the numbers of fheram_decrypt_ram on the stored RAM, bit for bit
   void decrypt_sk(const GLWESecret& sk, std::vector<int16_t>& values, std::vector<int64_t>& err) {

@@ -1243,6 +1243,7 @@ struct fheram_ram {
   DevBuf<> all;              // results of a chunked batched read
   DevBuf<> xchg;             // sharded: partials received from the other ranks, [n_shards][reads][word_size]
   DevBuf<> part_all;         // sharded, device-resident batch: partials of every read before the exchange
+  DevBuf<> plain_tab;        // plaintext-address calls: (source, rotation) of every item, then its place (sharded)
   struct HostPipe {          // fheram_ram_read_batch_host: double-buffered upload pipeline
     struct Set {
       DevBuf<long long> stage;
@@ -2426,23 +2427,12 @@ static int address_prepare_inv(const fheram_address* a, const fheram_keys* k) {
   return 0;
 }
 
-// Ram::write (src/ram.rs:226-294).  Works on sharded RAMs without communication: the steps that
-// touch tree[0][0] are replicated on every rank, the rest touches only local polynomials.
-extern "C" int fheram_ram_write(fheram_ram* r, const int64_t* w, const fheram_address* addr,
-                                const fheram_keys* k) {
-  if (!r || !addr || !k) return fail(FHERAM_ERR_INVALID, "null argument");
+// The written words ([word_size] GLWE) into r->wbuf as int32 limbs, on the context stream.  bcast: rank 0's words are
+// broadcast over the communicator and the other ranks pass none.
+static int stage_words(fheram_ram* r, const int64_t* w, bool bcast) {
   fheram_ctx* c = r->c;
-  const bool bcast = r->n_shards != 1 && comm_matches(c, r->shard, r->n_shards);
-  // with a communicator the written word is rank 0's, broadcast over NVLink: the other ranks may pass NULL
-  if (!w && !(bcast && r->shard != 0)) return fail(FHERAM_ERR_INVALID, "null argument");
-  if (addr->c != c || k->c != c) return fail(FHERAM_ERR_INVALID, "handles belong to different contexts");
-  if (!r->state)
-    return fail(FHERAM_ERR_NOT_READY, "invalid call to Memory.write: internal state is false -> requires calling Memory.read_prepare_write (src/ram.rs:555-558)");
-  CU(cudaSetDevice(c->device));
-  const Derived& d = c->d;
-  const int ws = c->params.word_size, nl = r->n_local;
+  const int ws = c->params.word_size;
   const long L = c->ct_stride();
-  const int per = ws * nl;
   TRY(r->wbuf.ensure(sizeof(int) * (size_t)ws * L));
   if (!bcast || r->shard == 0) {
     // staged through a buffer of its own and not waited for: the copy out of pageable memory returns once the
@@ -2463,6 +2453,27 @@ extern "C" int fheram_ram_write(fheram_ram* r, const int64_t* w, const fheram_ad
     c->launches++;
   }
   if (bcast) NC(ncclBroadcast(r->wbuf.p, r->wbuf.p, (size_t)ws * L, ncclInt32, 0, c->comm, c->stream));
+  return 0;
+}
+
+// Ram::write (src/ram.rs:226-294).  Works on sharded RAMs without communication: the steps that
+// touch tree[0][0] are replicated on every rank, the rest touches only local polynomials.
+extern "C" int fheram_ram_write(fheram_ram* r, const int64_t* w, const fheram_address* addr,
+                                const fheram_keys* k) {
+  if (!r || !addr || !k) return fail(FHERAM_ERR_INVALID, "null argument");
+  fheram_ctx* c = r->c;
+  const bool bcast = r->n_shards != 1 && comm_matches(c, r->shard, r->n_shards);
+  // with a communicator the written word is rank 0's, broadcast over NVLink: the other ranks may pass NULL
+  if (!w && !(bcast && r->shard != 0)) return fail(FHERAM_ERR_INVALID, "null argument");
+  if (addr->c != c || k->c != c) return fail(FHERAM_ERR_INVALID, "handles belong to different contexts");
+  if (!r->state)
+    return fail(FHERAM_ERR_NOT_READY, "invalid call to Memory.write: internal state is false -> requires calling Memory.read_prepare_write (src/ram.rs:555-558)");
+  CU(cudaSetDevice(c->device));
+  const Derived& d = c->d;
+  const int ws = c->params.word_size, nl = r->n_local;
+  const long L = c->ct_stride();
+  const int per = ws * nl;
+  TRY(stage_words(r, w, bcast));
   TRY(r->bufA.ensure(sizeof(int) * (size_t)per * L));
   TRY(r->bufB.ensure(sizeof(int) * (size_t)per * L));
   int* A = (int*)r->bufA.p;
@@ -2502,6 +2513,151 @@ extern "C" int fheram_ram_write(fheram_ram* r, const int64_t* w, const fheram_ad
   // no host synchronisation: the call returns with the work queued on the context stream, like every *_device entry
   // point; the next call on this RAM is ordered after it, fheram_ctx_synchronize / any download waits for it
   r->state = false;  // src/ram.rs:648
+  return 0;
+}
+
+// --------------------------------------------------------------------------------------
+// reads and writes at plaintext addresses (DESIGN.md 3.8): address a is coefficient j = a mod N of polynomial
+// h = a / N of every sub-RAM, which lives on shard h mod n_shards as local polynomial h / n_shards
+// --------------------------------------------------------------------------------------
+static int check_plain_args(const fheram_ram* r, const fheram_keys* k, const uint32_t* addrs, int n) {
+  if (!r || !k || !addrs) return fail(FHERAM_ERR_INVALID, "null argument");
+  if (n < 1) return fail(FHERAM_ERR_INVALID, "n must be >= 1");
+  if (k->c != r->c) return fail(FHERAM_ERR_INVALID, "handles belong to different contexts");
+  const uint64_t max_addr = r->c->params.max_addr;
+  for (int b = 0; b < n; b++)
+    if (addrs[b] >= max_addr)
+      return fail(FHERAM_ERR_INVALID, "address %u >= max_addr %llu", addrs[b], (unsigned long long)max_addr);
+  if (!r->loaded) return fail(FHERAM_ERR_UNINIT, "unitialized memory: self.data.len()=0 (src/ram.rs:182-185)");
+  if (r->state)
+    return fail(FHERAM_ERR_STATE, "the RAM is prepared for write (read_prepare_write without its write): call fheram_ram_write first");
+  if (r->rotated)
+    return fail(FHERAM_ERR_STATE, "read_prepare_write did not complete (rpw_local_device without a successful rpw_finish_device): the RAM is rotated; finish it, then write");
+  return 0;
+}
+static bool plain_owner(const fheram_ram* r, uint32_t a) {
+  return (int)((a >> r->c->d.log_n) % (uint32_t)r->n_shards) == r->shard;
+}
+static int launch_gather_rotate(fheram_ctx* c, int* dst, const int* src, const int2* tab, int n_items) {
+  k_gather_rotate<<<c->sm_count * 8, 256, 0, c->stream>>>(dst, src, tab, n_items, c->ct_stride());
+  c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
+
+// out[b][s] = TRACE(rot(2N - j_b, data[s][h_b])) for the addresses this shard holds, into r->result ([n][word_size]
+// GLWE); the entries of the other addresses are zero, or, with a communicator, every rank's (an int32 sum over
+// zero-filled arenas: one rank contributes each entry, so it is exact).  Reads run in chunks whose work arena holds
+// the GLWEs of one chunk of a batched read (batch_chunk reads of n_local polynomials per sub-RAM).
+static int read_plain_stage(fheram_ram* r, const uint32_t* addrs, int n, const fheram_keys* k) {
+  fheram_ctx* c = r->c;
+  const Derived& d = c->d;
+  const int ws = c->params.word_size, nl = r->n_local, S = r->n_shards;
+  const long L = c->ct_stride();
+  const int chunk = batch_chunk(r) * nl;
+  // tab[0, n_own ws): (source, rotation) of the items this shard holds, in read order; sharded, tab[n_own ws + i]:
+  // where item i of the result takes its value from, relative to its chunk's first item held here, or -1
+  std::vector<int2> tab;
+  for (int b = 0; b < n; b++)
+    if (plain_owner(r, addrs[b]))
+      for (int s = 0; s < ws; s++)
+        tab.push_back(make_int2(s * nl + (int)((addrs[b] >> d.log_n) / S), (2 * kN - (int)(addrs[b] & (kN - 1))) % (2 * kN)));
+  const size_t n_own = tab.size();
+  std::vector<size_t> first_own;  // per chunk: index in tab of its first item held here
+  for (int b0 = 0, g = 0; b0 < n; b0 += chunk) {
+    first_own.push_back((size_t)g);
+    const int nb = std::min(chunk, n - b0);
+    for (int b = b0, i = 0; b < b0 + nb; b++)
+      for (int s = 0; s < ws; s++) {
+        const bool own = plain_owner(r, addrs[b]);
+        if (S > 1) tab.push_back(make_int2(own ? i : -1, 0));
+        if (own) { i++; g++; }
+      }
+  }
+  TRY(r->plain_tab.ensure(sizeof(int2) * tab.size()));
+  CU(cudaMemcpyAsync(r->plain_tab.p, tab.data(), sizeof(int2) * tab.size(), cudaMemcpyHostToDevice, c->stream));
+  const int2* d_tab = (const int2*)r->plain_tab.p;
+  const int per_chunk = std::min(chunk, n) * ws;
+  TRY(r->bufA.ensure(sizeof(int) * (size_t)per_chunk * L));
+  if (S > 1) TRY(r->bufB.ensure(sizeof(int) * (size_t)per_chunk * L));
+  TRY(r->result.ensure(sizeof(int) * (size_t)n * ws * L));
+  int* A = (int*)r->bufA.p;
+  int* Bb = (int*)r->bufB.p;
+  for (int b0 = 0, ci = 0; b0 < n; b0 += chunk, ci++) {
+    const int items = std::min(chunk, n - b0) * ws;
+    const size_t g0 = first_own[ci], g1 = (size_t)ci + 1 < first_own.size() ? first_own[ci + 1] : n_own;
+    const int m = (int)(g1 - g0);
+    int* out = (int*)r->result.p + (size_t)b0 * ws * L;
+    if (m) TRY(launch_gather_rotate(c, A, r->data, d_tab + g0, m));
+    if (m == items) {
+      TRY(run_trace_chain(c, k, m, A, nullptr, 0, 0, out, 0, d.log_n));  // src/ram.rs:457
+    } else {
+      if (m) TRY(run_trace_chain(c, k, m, A, nullptr, 0, 0, Bb, 0, d.log_n));
+      TRY(launch_gather_rotate(c, out, Bb, d_tab + n_own + (size_t)b0 * ws, items));
+    }
+  }
+  if (S > 1 && comm_matches(c, r->shard, S))
+    NC(ncclAllReduce(r->result.p, r->result.p, (size_t)n * ws * L, ncclInt32, ncclSum, c->comm, c->stream));
+  return 0;
+}
+
+extern "C" int fheram_ram_read_plain_device(fheram_ram* r, const uint32_t* addrs, int n, const fheram_keys* k,
+                                            const int32_t** d_out) {
+  TRY(check_plain_args(r, k, addrs, n));
+  if (!d_out) return fail(FHERAM_ERR_INVALID, "null argument");
+  CU(cudaSetDevice(r->c->device));
+  TRY(read_plain_stage(r, addrs, n, k));
+  *d_out = (const int32_t*)r->result.p;
+  return 0;
+}
+
+extern "C" int fheram_ram_read_plain(fheram_ram* r, const uint32_t* addrs, int n, const fheram_keys* k,
+                                     int64_t* out) {
+  if (!out) return fail(FHERAM_ERR_INVALID, "null argument");
+  const int32_t* d = nullptr;
+  TRY(fheram_ram_read_plain_device(r, addrs, n, k, &d));
+  fheram_ctx* c = r->c;
+  const size_t per = (size_t)c->params.word_size * c->ct_stride();
+  if (r->n_shards == 1 || comm_matches(c, r->shard, r->n_shards)) return download_i64(c, d, (size_t)n * per, out);
+  // a shard without a communicator fills the entries of its own addresses and leaves the others as passed
+  std::vector<int64_t> all((size_t)n * per);
+  TRY(download_i64(c, d, all.size(), all.data()));
+  for (int b = 0; b < n; b++)
+    if (plain_owner(r, addrs[b])) memcpy(out + (size_t)b * per, all.data() + (size_t)b * per, sizeof(int64_t) * per);
+  return 0;
+}
+
+// data[s][h] = normalize(data[s][h] - rot(j, T_s) + rot(j, w_s)), T_s = TRACE(rot(2N - j, data[s][h])): on the shard
+// that holds h; with a communicator every rank takes part in the broadcast of rank 0's words
+extern "C" int fheram_ram_write_plain(fheram_ram* r, uint32_t addr, const int64_t* w, const fheram_keys* k) {
+  if (!r || !k) return fail(FHERAM_ERR_INVALID, "null argument");
+  fheram_ctx* c = r->c;
+  const bool bcast = r->n_shards != 1 && comm_matches(c, r->shard, r->n_shards);
+  if (!w && !(bcast && r->shard != 0)) return fail(FHERAM_ERR_INVALID, "null argument");
+  TRY(check_plain_args(r, k, &addr, 1));
+  const bool own = plain_owner(r, addr);
+  if (!own && !bcast) return 0;
+  CU(cudaSetDevice(c->device));
+  TRY(stage_words(r, w, bcast));
+  if (!own) return 0;
+  const Derived& d = c->d;
+  const int ws = c->params.word_size, nl = r->n_local;
+  const long L = c->ct_stride();
+  const int hl = (int)((addr >> d.log_n) / r->n_shards), j = (int)(addr & (kN - 1));
+  std::vector<int2> tab(ws);
+  for (int s = 0; s < ws; s++) tab[s] = make_int2(s * nl + hl, (2 * kN - j) % (2 * kN));
+  TRY(r->plain_tab.ensure(sizeof(int2) * ws));
+  CU(cudaMemcpyAsync(r->plain_tab.p, tab.data(), sizeof(int2) * ws, cudaMemcpyHostToDevice, c->stream));
+  TRY(r->bufA.ensure(sizeof(int) * (size_t)ws * L));
+  TRY(r->bufB.ensure(sizeof(int) * (size_t)ws * L));
+  int* A = (int*)r->bufA.p;
+  int* Bb = (int*)r->bufB.p;
+  TRY(launch_gather_rotate(c, A, r->data, (const int2*)r->plain_tab.p, ws));
+  TRY(run_trace_chain(c, k, ws, A, nullptr, 0, 0, Bb, 0, d.log_n));
+  k_plain_update<<<c->sm_count * 4, 256, 0, c->stream>>>(r->data, Bb, (const int*)r->wbuf.p, j, hl, nl, ws, L);
+  c->launches++;
+  CU(cudaGetLastError());
+  // no host synchronisation, as fheram_ram_write: the words were copied out of the caller's buffer above
   return 0;
 }
 

@@ -592,5 +592,52 @@ __global__ void k_copy(int* dst, const int* src, size_t n) {
   size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
   for (; i < n; i += (size_t)gridDim.x * blockDim.x) dst[i] = src[i];
 }
+// dst[item] = src[tab[item].x] * X^tab[item].y, tab[item].y in [0, 2N), or zeros where tab[item].x < 0 (the per-item
+// glwe_rotate of the plaintext-address calls: polynomial h seen from coefficient j, and the spread of a shard's results
+// into a zero-filled arena).  Limbs move as values: the wrapped ones are negated, so -2^16 becomes +2^16.
+__global__ void k_gather_rotate(int* dst, const int* src, const int2* tab, int n_items, long ct_stride) {
+  const size_t total = (size_t)n_items * ct_stride;
+  size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+  for (; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const int item = (int)(idx / ct_stride);
+    const long off = (long)(idx % ct_stride);
+    const int2 t = tab[item];
+    if (t.x < 0) { dst[idx] = 0; continue; }
+    const int i = (int)(off & (kN - 1));
+    bool neg;
+    const int j = rot_index(i, 2 * kN - t.y, neg);  // (a X^k)[i] = +/- a[(i - k) mod 2N]
+    const int v = src[(size_t)t.x * ct_stride + off - i + j];
+    dst[idx] = neg ? -v : v;
+  }
+}
+// data[dst0 + s dst_stride] = normalize(data[...] - T[s] X^k + w[s] X^k) for s < n_items, k in [0, 2N)   (3-limb
+// ciphertexts; write_plain: write_first_step of src/ram.rs:574-576 on one polynomial seen from coefficient j).  The
+// sum is exact in integers and normalised once, as k_sub_add_normalize does.
+__global__ void k_plain_update(int* data, const int* T, const int* w, int k, int dst0, int dst_stride, int n_items,
+                               long ct_stride) {
+  const size_t total = (size_t)n_items * 2 * kN;
+  size_t idx = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+  for (; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
+    const int item = (int)(idx / (2 * kN));
+    const int r = (int)(idx % (2 * kN));  // col*N + i
+    const int i = r & (kN - 1);
+    bool neg;
+    const int e = rot_index(i, 2 * kN - k, neg);
+    int* t = data + (size_t)(dst0 + item * dst_stride) * ct_stride;
+    const int* tt = T + (size_t)item * ct_stride;
+    const int* ww = w + (size_t)item * ct_stride;
+    long long c = 0;
+#pragma unroll
+    for (int l = 2; l >= 0; l--) {
+      const int off = l * 2 * kN + r, src = off - i + e;
+      long long x = (long long)ww[src] - tt[src];
+      if (neg) x = -x;
+      const long long v = (long long)t[off] + x + c;
+      const long long d = sext17(v);
+      c = (v - d) >> kK;
+      t[off] = (int)d;
+    }
+  }
+}
 
 }  // namespace fheram

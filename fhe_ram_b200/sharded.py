@@ -201,6 +201,17 @@ class ShardedRamLib:
     def write(self, w, addr, keys) -> None:
         self.ram.write(w, addr, keys)
 
+    def read_plain(self, addrs, keys, out=None) -> np.ndarray:
+        """addrs = the same plaintext addresses on every rank; returns all n results on every rank"""
+        return self.ram.read_plain(addrs, keys, out)
+
+    def read_plain_device(self, addrs, keys) -> int:
+        return self.ram.read_plain_device(addrs, keys)
+
+    def write_plain(self, addr, w, keys) -> None:
+        """rank 0's word is written (the other ranks may pass None)"""
+        self.ram.write_plain(addr, w, keys)
+
     def store(self) -> np.ndarray:
         return self.ram.store()
 

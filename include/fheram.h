@@ -188,6 +188,39 @@ int fheram_ram_read_batch_device(fheram_ram *r, const fheram_address *addr, cons
 /* convert + copy a device result arena to host int64 limbs */
 int fheram_download_glwe(fheram_ctx *ctx, const int32_t *d_in, int n_glwe, int64_t *out);
 
+/* ---- reads and writes at plaintext addresses (DESIGN.md 3.8).  The address, and so the polynomial that is read or
+ * changed, is disclosed to the server by design: never use these calls for an address that must stay private.  The
+ * words stay encrypted and the RAM stays a valid RAM for every oblivious call.  Definitions:
+ *   rot(k, x) is glwe_rotate: x X^k, with k taken mod 2N.  It is an exact signed permutation of the limbs, with no
+ *     normalisation.
+ *   TRACE(x) is glwe_trace(0, log_n), the trace at the end of every read (src/ram.rs:457).
+ *   data[s][h] is polynomial h of sub-RAM s as fheram_ram_store lays it out.
+ *   For an address a < max_addr: h = a >> log_n and j = a & (N - 1).
+ *   read_plain: out[b][s] = TRACE(rot(2N - j_b, data[s][h_b])) for every address b and every sub-RAM s.  It decrypts
+ *     to the same value as fheram_ram_read of that address.  The limbs differ, and its noise is one trace's noise.
+ *   write_plain with w = [word_size] GLWE, as fheram_ram_write takes it (encrypting [w_s, 0, ..., 0]):
+ *     T_s = TRACE(rot(2N - j, data[s][h]))
+ *     data[s][h] <- normalize(data[s][h] - rot(j, T_s) + rot(j, w_s))
+ *     The sum is exact in integers.  It is normalised once, as k_sub_add_normalize does: balanced base-2^17 digits,
+ *     top carry dropped.  This is the reference's write_first_step (to - TRACE(to) + w, src/ram.rs:574-576) applied to
+ *     polynomial h seen from coefficient j.  Other polynomials, tree[0][0] and the state flag are untouched; a
+ *     write_plain adds one trace's key-switch noise to the N cells of polynomial h in each sub-RAM.
+ * Refusals: FHERAM_ERR_INVALID for an address >= max_addr, n < 1, null arguments or handles from another context;
+ * FHERAM_ERR_UNINIT for a RAM never loaded; FHERAM_ERR_STATE for a RAM prepared for write or left rotated by
+ * fheram_ram_rpw_local_device.  These calls neither need nor consume a read_prepare_write.
+ * Sharded RAM (polynomial h lives on shard h mod n_shards).  With a communicator every rank passes the same addresses:
+ * read_plain returns all n results on every rank (each computed by the rank that holds its polynomial, exchanged as
+ * int32 limbs), write_plain takes rank 0's words (the other ranks may pass NULL) and only the holder updates.  Without
+ * one, read_plain fills the entries of the addresses this shard holds and leaves the others as passed (zero in the
+ * _device arena); write_plain updates if this shard holds h and otherwise returns 0 having done nothing. ---- */
+/* out = [n][word_size] GLWE, as fheram_ram_read_batch; duplicate addresses are allowed */
+int fheram_ram_read_plain(fheram_ram *r, const uint32_t *addrs, int n, const fheram_keys *k, int64_t *out);
+/* the n results in the RAM's device arena, [n][word_size][limb][col][N] int32, valid until the next call on the RAM */
+int fheram_ram_read_plain_device(fheram_ram *r, const uint32_t *addrs, int n, const fheram_keys *k,
+                                 const int32_t **d_out);
+/* returns with its work queued, like fheram_ram_write; the words are copied out of w before it returns */
+int fheram_ram_write_plain(fheram_ram *r, uint32_t addr, const int64_t *w, const fheram_keys *k);
+
 /* ---- multi-GPU (SURVEY.md 8e; the reference's caller makes ONE call per read / read_prepare_write / write,
  * src/ram.rs:172-176,196-200,226-231, and so does the caller here): one context per GPU and rank, an NCCL
  * communicator over NVLink inside the library.  Rank 0 draws the id, the host program hands the 128 bytes to the

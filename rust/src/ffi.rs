@@ -84,6 +84,11 @@ extern "C" {
     pub fn fheram_ram_read_prepare_write(r: *mut fheram_ram, a: *const fheram_address, k: *const fheram_keys,
                                          out: *mut i64) -> c_int;
     pub fn fheram_ram_write(r: *mut fheram_ram, w: *const i64, a: *const fheram_address, k: *const fheram_keys) -> c_int;
+    pub fn fheram_ram_read_plain(r: *mut fheram_ram, addrs: *const u32, n: c_int, k: *const fheram_keys,
+                                 out: *mut i64) -> c_int;
+    pub fn fheram_ram_read_plain_device(r: *mut fheram_ram, addrs: *const u32, n: c_int, k: *const fheram_keys,
+                                        d_out: *mut *const i32) -> c_int;
+    pub fn fheram_ram_write_plain(r: *mut fheram_ram, addr: u32, w: *const i64, k: *const fheram_keys) -> c_int;
     pub fn fheram_source_new(seed: *const u8) -> *mut fheram_source;
     pub fn fheram_source_free(s: *mut fheram_source);
     pub fn fheram_source_position(s: *const fheram_source) -> u64;

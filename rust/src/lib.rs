@@ -237,6 +237,20 @@ impl Ram {
         let a = address.device(&mut self.params);
         check(unsafe { fheram_ram_write(self.h, flat.as_ptr(), a, keys.0) });
     }
+    /// reads at plaintext addresses (include/fheram.h): TRACE(data[s][h] X^-j) for a = h N + j, one [word_size] GLWE
+    /// per address.  The addresses are disclosed to the server; the words stay encrypted.
+    pub fn read_plain(&mut self, addrs: &[u32], keys: &EvaluationKeysPrepared) -> Vec<Vec<GLWE>> {
+        let per = self.params.word_size() * self.params.glwe_len();
+        let mut out = vec![0i64; addrs.len() * per];
+        check(unsafe { fheram_ram_read_plain(self.h, addrs.as_ptr(), addrs.len() as i32, keys.0, out.as_mut_ptr()) });
+        out.chunks(per).map(|c| self.split(c.to_vec())).collect()
+    }
+    /// write at a plaintext address: the write_first_step of Ram::write on polynomial h seen from coefficient j
+    pub fn write_plain(&mut self, addr: u32, w: &[GLWE], keys: &EvaluationKeysPrepared) {
+        assert!(w.len() == self.params.word_size());
+        let flat: Vec<i64> = w.iter().flatten().copied().collect();
+        check(unsafe { fheram_ram_write_plain(self.h, addr, flat.as_ptr(), keys.0) });
+    }
     /// every byte of the resident RAM decrypted on the device: (values, err), [max_addr][word_size] row-major (byte i of
     /// word j at j * word_size + i); the numbers of `decrypt_ram` on the stored RAM, bit for bit
     pub fn decrypt_sk(&mut self, sk: &GLWESecret) -> (Vec<i16>, Vec<i64>) {
